@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — ORB extraction throughput of the B200 front-end (BASELINE.json metric) + matching extras.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path (ORBextractor::operator(), reference ORBextractor.cc:1083-1169)
@@ -13,6 +13,8 @@ scaling; SURVEY §8e).  One JSON line is printed by rank 0:
   roofline   the dominant kernel group's algorithmic bytes / its CUDA-event time vs the measured HBM peak
   cpu_baseline  the reference's own ORBextractor.cc (oracle/_ref, compiled unmodified) on this box's host cores, bounded sample
 `--impl reference` times that CPU build alone (all host threads) and prints the same line shape.
+`--dump-outputs DIR` writes rank 0's results of the last timed step as .npy files (see dump_outputs), so that two builds
+can be compared output for output: the frames are seeded, identical from run to run.
 """
 import argparse
 import json
@@ -30,6 +32,34 @@ if ROOT not in sys.path:
 W, H, NFEAT, NLEVELS, SCALE, INI_TH, MIN_TH = 640, 480, 1000, 8, 1.2, 20, 7
 METRIC = "orb_extraction_frames_per_s_640x480_1000f"
 UNIT = "frames/s"
+
+
+DUMP_FRAMES = 64                   # frames whose keypoints and descriptors --dump-outputs writes (about 12 MB)
+
+
+def dump_outputs(out_dir, kps_d, desc_d, n_d, mono_d):
+    """What the device-resident path hands its caller for a batch, one float .npy per array:
+      n.npy, mono.npy    (B,)  keypoint count and monoIndex of every frame of the batch
+      frames.npy         (S,)  the sampled frames: a fixed seeded choice of S = min(B, DUMP_FRAMES)
+      keypoints.npy      (S, M, 7) float64  x, y, size, angle, response, octave, class_id of the sampled frames
+      descriptors.npy    (S, M, 32) float32 descriptor bytes of the sampled frames
+    M is the largest keypoint count among the sampled frames; rows past a frame's own count are zero."""
+    from visual_sgraphs_b200._lib import KEYPOINT_DTYPE
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    B = kps_d.shape[0]
+    n, mono = n_d.cpu().numpy(), mono_d.cpu().numpy()
+    frames = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_FRAMES), replace=False))
+    m = int(n[frames].max()) if len(frames) else 0
+    sel = torch.as_tensor(frames, device=kps_d.device)
+    kps = np.ascontiguousarray(kps_d[sel, :m].cpu().numpy()).view(KEYPOINT_DTYPE).reshape(len(frames), m)
+    desc = desc_d[sel, :m].cpu().numpy().astype(np.float32)
+    keys = np.stack([kps[f].astype(np.float64) for f in KEYPOINT_DTYPE.names], axis=-1)
+    valid = np.arange(m)[None, :] < n[frames][:, None]
+    keys[~valid], desc[~valid] = 0, 0
+    for name, a in (("n", n.astype(np.float64)), ("mono", mono.astype(np.float64)), ("frames", frames.astype(np.float64)),
+                    ("keypoints", keys), ("descriptors", desc)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def level_sizes(w, h):
@@ -783,7 +813,10 @@ def main():
     ap.add_argument("--batch", type=int, default=512, help="frames per step per GPU")
     ap.add_argument("--no-extras", action="store_true", help="skip the matching and cpu-baseline extras")
     ap.add_argument("--no-stage-profile", action="store_true", help="(experiments) no per-stage events in the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of --impl ours; the reference arm only times the CPU extractor")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -843,6 +876,8 @@ def main():
     stage_ms, runs = ex.stage_ms()
     ex.profile(False)
     n_kp_mean = float(n_d.float().mean().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, kps_d, desc_d, n_d, mono_d)
 
     # ---- end to end through the host-pointer C-ABI call (pinned frames in, pinned results out) ----
     # Two handles driven by two host threads, each taking half of the step's frames (every call is itself a chunked

@@ -1,10 +1,13 @@
-"""GPU parity against the REFERENCE ITSELF: the CUDA extractor behind the C ABI vs oracle/_ref/libvsg_ref.so, i.e.
-/root/reference/orb_slam3/src/ORBextractor.cc compiled unmodified (oracle/ref_build/Makefile).  The library is
-prebuilt in the build container and travels to the GPU box; /root/reference is never read here.
+"""GPU parity against the REFERENCE ITSELF: the CUDA extractor behind the C ABI vs oracle/_ref/libvsg_ref.so, i.e. the
+reference's ORBextractor.cc compiled unmodified (oracle/ref_build/Makefile).  The golden cases are also compared with
+the reference's outputs stored in tests/golden/ (tests/golden/make_golden.py), so they run where the library is not
+built; the other tests skip there.
 
 Bars (BASELINE.json north_star): keypoint sets, order, positions, sizes, responses, octaves bit-exact; angles within
 1e-3 degrees; >= 99.9 % of descriptor bits — the tests also REPORT exact equality, which holds on every frame so far.
 """
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -15,14 +18,24 @@ from visual_sgraphs_b200.synth import synth_frame
 
 pytestmark = pytest.mark.gpu
 
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
 
 @pytest.fixture(scope="module")
-def ref():
+def live_ref():
+    """The reference library where it is built, else None."""
     from oracle import ref as r
     if not r.available():
-        pytest.skip("oracle/_ref/libvsg_ref.so was not shipped")
+        return None
     r.lib()
     return r
+
+
+@pytest.fixture(scope="module")
+def ref(live_ref):
+    if live_ref is None:
+        pytest.skip("oracle/_ref/libvsg_ref.so is not built")
+    return live_ref
 
 
 def _cmp(got, want, what):
@@ -41,17 +54,24 @@ def _cmp(got, want, what):
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
-def test_golden_cases_against_the_reference(ref, case):
+def test_golden_cases_against_the_reference(live_ref, case):
     from visual_sgraphs_b200.extractor import ORBextractor
     name, src, wh, nfeat, lap = case
     frame = frame_of(src, wh)
-    r = ref.RefExtractor(nfeat)
-    want = r(frame, lap)
     ex = ORBextractor(nfeat, 1.2, 8, 20, 7)
     got = ex(frame, lap)
-    assert _cmp(got, want, name), name + ": angles / descriptors not bit-equal"
-    for level in range(8):
-        assert np.array_equal(ex.pyramid_level(level), r.level(level)), (name, level)     # mvImagePyramid[level]
+    gold = np.load(os.path.join(GOLD, name + ".npz"))                 # the reference's keypoints and descriptors
+    meta = next(c for c in json.load(open(os.path.join(GOLD, "index.json")))["cases"] if c["name"] == name)
+    assert _cmp(got, (meta["mono_index"], gold["keypoints"], gold["descriptors"]), name), \
+        name + ": angles / descriptors not bit-equal"
+    for level, lm in enumerate(meta["levels"]):                       # the reference's mvImagePyramid[level], as digests
+        assert hashlib.sha256(np.ascontiguousarray(ex.pyramid_level(level)).tobytes()).hexdigest() == lm["level_sha"], \
+            (name, level)
+    if live_ref is not None:
+        r = live_ref.RefExtractor(nfeat)
+        assert _cmp(got, r(frame, lap), name), name + ": angles / descriptors not bit-equal"
+        for level in range(8):
+            assert np.array_equal(ex.pyramid_level(level), r.level(level)), (name, level)     # mvImagePyramid[level]
 
 
 @pytest.mark.parametrize("seed", range(12))

@@ -1,6 +1,7 @@
 """CPU-only parity PIN: the reference's own ORBextractor.cc — compiled UNMODIFIED into oracle/_ref/libvsg_ref.so
 (oracle/ref_build/Makefile; OpenCV calls resolved by the cv2-pinned compat layer) — against the oracle port
-(oracle/orb_oracle.cpp) and the committed golden fixtures.
+(oracle/orb_oracle.cpp) and the committed golden fixtures.  Where that library is not built, only the comparison of
+the oracle with the golden fixtures (the reference's stored outputs) runs; the other tests skip.
 
 What this pins is everything the reference itself owns: constructor tables (ORBextractor.cc:411-470), the cell loop
 and threshold retry (:787-900), DistributeOctTree with its std::list / push_front / std::sort order (:562-785),
@@ -20,12 +21,20 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
-def ref():
+def live_ref():
+    """The reference library where it is built (or buildable from the reference's sources), else None."""
     from oracle import ref as r
     if not r.available():
-        pytest.skip("oracle/_ref not built and /root/reference absent")
+        return None
     r.build()
     return r
+
+
+@pytest.fixture(scope="module")
+def ref(live_ref):
+    if live_ref is None:
+        pytest.skip("oracle/_ref/libvsg_ref.so is not built and the reference's sources are not present")
+    return live_ref
 
 
 def _same(a, b, what):
@@ -59,17 +68,20 @@ def test_tables(ref, oracle):
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
-def test_reference_equals_oracle_and_golden(ref, oracle, case):
+def test_reference_equals_oracle_and_golden(live_ref, oracle, case):
+    """The golden fixtures hold the reference's own outputs (tests/golden/make_golden.py), so the oracle is compared
+    with them with or without the library; the level-by-level comparison needs the library."""
     name, src, wh, nfeat, lap = case
     frame = frame_of(src, wh)
-    r, o = ref.RefExtractor(nfeat), oracle.OracleExtractor(nfeat)
-    got_r, got_o = r(frame, lap), o(frame, lap)
-    _same(got_r, got_o, name)
+    o = oracle.OracleExtractor(nfeat)
+    got_o = o(frame, lap)
     gold = np.load(os.path.join(GOLD, name + ".npz"))
-    assert got_r[1].tobytes() == gold["keypoints"].tobytes()
-    assert np.array_equal(got_r[2], gold["descriptors"])
     meta = next(c for c in json.load(open(os.path.join(GOLD, "index.json")))["cases"] if c["name"] == name)
-    assert got_r[0] == meta["mono_index"] and len(got_r[1]) == meta["n_keypoints"]
+    _same(got_o, (meta["mono_index"], gold["keypoints"], gold["descriptors"]), name)
+    if live_ref is None:
+        return
+    r = live_ref.RefExtractor(nfeat)
+    _same(r(frame, lap), got_o, name)
     for level in range(8):
         assert r.level_size(level) == o.level_size(level)
         assert np.array_equal(r.level_padded(level), o.level_padded(level)), (name, level)   # incl. the 19-px frame
