@@ -321,26 +321,6 @@ def test_baseline_batch_size_properties(oracle):
         assert kd[f, :n[f]].cpu().numpy().tobytes() == kn[f, :n[f]].tobytes() and dd[f, :n[f]].cpu().numpy().tobytes() == dn[f, :n[f]].tobytes()
 
 
-def test_persistent_tma_fast_kernel_matches_the_default_grid(monkeypatch):
-    """VSG_FAST_TMA=16: FAST cells of a batch run on persistent CTAs whose cell windows are staged by the TMA unit
-    (cp.async.bulk.tensor + mbarrier, csrc/fast.cu: fast_blur_tma_kernel).  It is off by default (slower than the
-    one-CTA-per-unit grid, profiles/r02_tma_fast.md) but must stay bit-identical to it."""
-    from visual_sgraphs_b200.extractor import ORBextractor
-    frames = np.stack([synth_frame(100 + i, 640, 480) for i in range(40)])
-    want = ORBextractor(1000, 1.2, 8, 20, 7, max_batch=40).extract_batch(frames)
-    monkeypatch.setenv("VSG_FAST_TMA", "16")
-    got = ORBextractor(1000, 1.2, 8, 20, 7, max_batch=40).extract_batch(frames)
-    for a, b in zip(got, want):
-        assert a[0] == b[0] and a[1].tobytes() == b[1].tobytes() and np.array_equal(a[2], b[2])
-    # a shape with wider cells (S = 24) and two root nodes
-    frames2 = np.stack([synth_frame(300 + i, 752, 480) for i in range(20)])
-    got2 = ORBextractor(1200, 1.2, 8, 20, 7, max_batch=20).extract_batch(frames2)
-    monkeypatch.setenv("VSG_FAST_TMA", "0")
-    want2 = ORBextractor(1200, 1.2, 8, 20, 7, max_batch=20).extract_batch(frames2)
-    for a, b in zip(got2, want2):
-        assert a[0] == b[0] and a[1].tobytes() == b[1].tobytes() and np.array_equal(a[2], b[2])
-
-
 @pytest.mark.parametrize("wh", [(640, 480), (752, 480), (1241, 376), (320, 240)])
 def test_tensor_core_blur_is_bit_identical(monkeypatch, wh):
     """VSG_BLUR_TC=1: the 7x7 Gaussian blur (ORBextractor.cc:1129-1130) runs as banded u8 GEMMs on tcgen05 (csrc/blur_tc.cu).

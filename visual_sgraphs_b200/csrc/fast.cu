@@ -16,12 +16,7 @@
 // one global atomic per CTA.  The list order is not the reference's cell-row-major order; the oct-tree only
 // depends on order through the first-max-wins tie break, which octree.cu reproduces from the coordinates
 // (see order_key there).
-#include <algorithm>
-#include <climits>
-#include <cstdlib>
-
 #include "blur_device.cuh"
-#include "tma_util.cuh"
 #include "vsg_internal.cuh"
 
 namespace vsg {
@@ -107,11 +102,6 @@ __device__ __forceinline__ CellGeom cell_geom(const FrameGeom &g, int cell_block
     return c;
 }
 
-// Bytes per row of a TMA-staged raw window.  The box must START on a 16-byte boundary of the plane (measured: any other start
-// faults, tools/micro/tma_probe.cu), so it begins at x0 & ~15 and is 80 bytes wide: up to 12 bytes of lead-in + the
-// S + 4 * nq <= 60 bytes the pair re-layout reads (S <= 24).
-constexpr int kRawPitch = 80;
-
 // One FAST cell (kFastThreads threads).
 //
 // Work layout: thread t owns pair column j = t % S and walks down the cell in sweeps of RB = kFastThreads / S rows
@@ -119,13 +109,11 @@ constexpr int kRawPitch = 80;
 // column masks, the shared-memory pointers and the survivor coordinates need no per-iteration index arithmetic: one
 // pointer increment per sweep.
 //
-// The cell window comes either straight from global memory (raw == nullptr) or from a raw copy of it that the TMA unit
-// has already placed in shared memory (rows of kRawPitch bytes starting at the 16-byte aligned column x0 & ~15 of the plane).
+// The cell window is read straight from global memory: the level's pyramid plane, or the caller's level 0.
 __device__ __forceinline__ void fast_cell_body(const FrameGeom &g, const CellGeom &cell, const uint8_t *__restrict__ lvl0_base,
                                                int lvl0_pitch, int64_t lvl0_stride, const uint8_t *__restrict__ pyr,
-                                               const uint8_t *raw, uint32_t *t2, uint32_t *s2, uint32_t *list,
-                                               Cand *__restrict__ cand, int *__restrict__ cand_count, int ini_th,
-                                               int min_th, int list_cap, int frame) {
+                                               uint32_t *t2, uint32_t *s2, uint32_t *list, Cand *__restrict__ cand,
+                                               int *__restrict__ cand_count, int ini_th, int min_th, int list_cap, int frame) {
     __shared__ int s_count, s_base;
     const int level = cell.level, x0 = cell.x0, y0 = cell.y0, cw = cell.cw, ch = cell.ch;
     const LevelGeom &L = g.lv[level];
@@ -150,40 +138,32 @@ __device__ __forceinline__ void fast_cell_body(const FrameGeom &g, const CellGeo
             o.w = __byte_perm(a, b, 0x7773) & 0x00FF00FFu;
             *reinterpret_cast<uint4 *>(dst) = o;
         };
-        if (raw) {
-            for (int r = r0; qok && r < ch; r += rstep) {
-                const uint8_t *rp = raw + r * kRawPitch + (ax0 & 15) + 4 * q;
-                relayout(*reinterpret_cast<const uint32_t *>(rp), *reinterpret_cast<const uint32_t *>(rp + S),
-                         t2 + r * kT2Pitch + 4 * q);
-            }
-        } else {
-            const uint8_t *src;
-            int spitch;
-            if (level == 0) { src = lvl0_base + (int64_t)frame * lvl0_stride; spitch = lvl0_pitch; }
-            else { src = pyr + L.plane_offset + (int64_t)frame * L.plane_stride; spitch = L.pitch; }
-            const uint8_t *base = src + (int64_t)y0 * spitch + ax0;
-            const uint8_t *row = base + (int64_t)r0 * spitch + 4 * q;
-            const int64_t rinc = (int64_t)rstep * spitch;
-            uint32_t *dst = t2 + r0 * kT2Pitch + 4 * q;
-            // all global loads of the CTA are issued before the first one is consumed
-            constexpr int kLoadIters = 3;              // 3 x 20 rows of 8 quads cover the usual 44-row cell without a loop
-            uint32_t a[kLoadIters], b[kLoadIters];
+        const uint8_t *src;
+        int spitch;
+        if (level == 0) { src = lvl0_base + (int64_t)frame * lvl0_stride; spitch = lvl0_pitch; }
+        else { src = pyr + L.plane_offset + (int64_t)frame * L.plane_stride; spitch = L.pitch; }
+        const uint8_t *base = src + (int64_t)y0 * spitch + ax0;
+        const uint8_t *row = base + (int64_t)r0 * spitch + 4 * q;
+        const int64_t rinc = (int64_t)rstep * spitch;
+        uint32_t *dst = t2 + r0 * kT2Pitch + 4 * q;
+        // all global loads of the CTA are issued before the first one is consumed
+        constexpr int kLoadIters = 3;              // 3 x 20 rows of 8 quads cover the usual 44-row cell without a loop
+        uint32_t a[kLoadIters], b[kLoadIters];
 #pragma unroll
-            for (int it = 0; it < kLoadIters; ++it) {
-                if (qok && r0 + it * rstep < ch) {
-                    a[it] = __ldg(reinterpret_cast<const uint32_t *>(row + it * rinc));
-                    // the second half may reach past the window, never past the image row (x0 + cw <= W - 16)
-                    b[it] = __ldg(reinterpret_cast<const uint32_t *>(row + it * rinc + S));
-                }
+        for (int it = 0; it < kLoadIters; ++it) {
+            if (qok && r0 + it * rstep < ch) {
+                a[it] = __ldg(reinterpret_cast<const uint32_t *>(row + it * rinc));
+                // the second half may reach past the window, never past the image row (x0 + cw <= W - 16)
+                b[it] = __ldg(reinterpret_cast<const uint32_t *>(row + it * rinc + S));
             }
+        }
 #pragma unroll
-            for (int it = 0; it < kLoadIters; ++it)
-                if (qok && r0 + it * rstep < ch) relayout(a[it], b[it], dst + it * rstep * kT2Pitch);
-            for (int r = r0 + kLoadIters * rstep; qok && r < ch; r += rstep) {   // taller cells
-                const uint8_t *rp = base + (int64_t)r * spitch + 4 * q;
-                relayout(__ldg(reinterpret_cast<const uint32_t *>(rp)), __ldg(reinterpret_cast<const uint32_t *>(rp + S)),
-                         t2 + r * kT2Pitch + 4 * q);
-            }
+        for (int it = 0; it < kLoadIters; ++it)
+            if (qok && r0 + it * rstep < ch) relayout(a[it], b[it], dst + it * rstep * kT2Pitch);
+        for (int r = r0 + kLoadIters * rstep; qok && r < ch; r += rstep) {   // taller cells
+            const uint8_t *rp = base + (int64_t)r * spitch + 4 * q;
+            relayout(__ldg(reinterpret_cast<const uint32_t *>(rp)), __ldg(reinterpret_cast<const uint32_t *>(rp + S)),
+                     t2 + r * kT2Pitch + 4 * q);
         }
     }
     for (int i = tid; i < kS2Pitch; i += kFastThreads) {     // top and bottom apron rows of the strength plane
@@ -295,7 +275,7 @@ __global__ void __launch_bounds__(kFastThreads, VSG_FAST_MINB) fast_kernel(Frame
     pdl_launch_dependents();
     pdl_wait();
     const FastSmem m = fast_smem(smem, tile_rows);
-    fast_cell_body(g, cell_geom(g, blockIdx.x), lvl0_base, lvl0_pitch, lvl0_stride, pyr, nullptr, m.t2, m.s2, m.list, cand,
+    fast_cell_body(g, cell_geom(g, blockIdx.x), lvl0_base, lvl0_pitch, lvl0_stride, pyr, m.t2, m.s2, m.list, cand,
                    cand_count, ini_th, min_th, list_cap, blockIdx.y);
 }
 
@@ -340,129 +320,14 @@ __global__ void __launch_bounds__(kFastThreads, VSG_FAST_MINB) fast_blur_kernel(
         return;
     }
     const FastSmem m = fast_smem(smem, tile_rows);
-    fast_cell_body(g, cell_geom(g, role.index), lvl0_base, lvl0_pitch, lvl0_stride, pyr, nullptr, m.t2, m.s2, m.list, cand,
+    fast_cell_body(g, cell_geom(g, role.index), lvl0_base, lvl0_pitch, lvl0_stride, pyr, m.t2, m.s2, m.list, cand,
                    cand_count, ini_th, min_th, list_cap, blockIdx.y);
 }
 
-// The same grid as PERSISTENT CTAs whose cell windows are staged by the TMA unit (large batches): CTA b walks the units
-// b, b + gridDim.x, ... of the flattened (frame, unit) list.  While it scores one cell, the raw window of its next cell is
-// already on its way into the other of two shared-memory buffers — one elected thread issues a cp.async.bulk.tensor box
-// (80 bytes x the level's cell height, coordinates (x0 & ~15, y0, frame) in that level's tensor map) that completes on an
-// mbarrier — so neither the global-load latency nor the launch of a fresh CTA sits on the cell's critical path.
-struct FastTileMaps {
-    CUtensorMap m[8];       // per level: (x bytes, y rows, frame); box kRawPitch x box_rows[level] x 1
-    int box_rows[8];
-    int frame0[8];          // frame coordinate of the launch's first frame in that level's map
-};
-
-__global__ void __launch_bounds__(kFastThreads, VSG_FAST_MINB)
-fast_blur_tma_kernel(FrameGeom g, BlurLevels bl, const __grid_constant__ FastTileMaps maps, const uint8_t *__restrict__ lvl0_base,
-                     int lvl0_pitch, int64_t lvl0_stride, const uint8_t *__restrict__ pyr, uint8_t *__restrict__ blur,
-                     Cand *__restrict__ cand, int *__restrict__ cand_count, int ini_th, int min_th, int tile_rows, int list_cap,
-                     int nblur, int ratio, uint32_t group_rcp, int units_per_frame, uint32_t upf_rcp, int total_units) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t *smem = reinterpret_cast<uint8_t *>(((uintptr_t)smem_raw + 127) & ~(uintptr_t)127);
-    const int raw_bytes = (tile_rows * kRawPitch + 127) & ~127;
-    const FastSmem m = fast_smem(smem + 2 * raw_bytes, tile_rows);
-    uint64_t *bars = reinterpret_cast<uint64_t *>(m.list + ((list_cap + 1) & ~1));
-    if (threadIdx.x == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
-        mbar_init_fence();
-    }
-    __syncthreads();
-
-    auto split = [&](int u, int &frame, int &x) {        // unit -> (frame, unit of the frame)
-        frame = (int)__umulhi((uint32_t)u, upf_rcp);
-        x = u - frame * units_per_frame;
-    };
-    auto issue = [&](const CellGeom &c, int frame, int b) {   // one thread: raw window of cell c -> buffer b
-        mbar_expect_tx(&bars[b], (uint32_t)(kRawPitch * maps.box_rows[c.level]));
-        tma_load_3d(smem + b * raw_bytes, &maps.m[c.level], c.x0 & ~15, c.y0, maps.frame0[c.level] + frame, &bars[b]);
-    };
-
-    int buf = 0, have = -1;          // `have`: the unit whose window sits in (or is on its way to) rawbuf[buf]
-    uint32_t phase = 0;              // bit b: parity the next wait on buffer b uses
-    for (int u = blockIdx.x; u < total_units; u += gridDim.x) {
-        int frame, x;
-        split(u, frame, x);
-        const UnitRole role = unit_role(x, nblur, ratio, group_rcp);
-        // the unit after this one (same CTA): if it is a cell, its window is requested now
-        const int un = u + gridDim.x;
-        bool next_cell = false;
-        CellGeom cn;
-        int frame_n = 0;
-        if (un < total_units) {
-            int xn;
-            split(un, frame_n, xn);
-            const UnitRole rn = unit_role(xn, nblur, ratio, group_rcp);
-            next_cell = !rn.blur;
-            if (next_cell) cn = cell_geom(g, rn.index);
-        }
-        if (role.blur) {
-            if (next_cell && have != un) {
-                if (threadIdx.x == 0) issue(cn, frame_n, buf);
-                have = un;
-            }
-            blur_block_body(g, bl, lvl0_base, lvl0_pitch, lvl0_stride, pyr, blur, role.index, frame);
-            continue;
-        }
-        const CellGeom c = cell_geom(g, role.index);
-        if (threadIdx.x == 0) {
-            if (have != u) issue(c, frame, buf);
-            if (next_cell) issue(cn, frame_n, buf ^ 1);     // the other buffer was consumed before the last barrier
-        }
-        mbar_wait(&bars[buf], (phase >> buf) & 1u);
-        phase ^= 1u << buf;
-        fast_cell_body(g, c, lvl0_base, lvl0_pitch, lvl0_stride, pyr, smem + buf * raw_bytes, m.t2, m.s2, m.list, cand, cand_count, ini_th,
-                       min_th, list_cap, frame);
-        __syncthreads();                                    // t2 / s2 / list / rawbuf[buf] are free again
-        if (next_cell) { buf ^= 1; have = un; }
-        else have = -1;
-    }
-}
-
-// VSG_FAST_TMA = n: batches of at least n frames take the persistent TMA kernel.  OFF by default: measured on the B200 it is
-// slower than the one-CTA-per-unit grid (4.17 vs 2.26 ms per 512 frames, profiles/r02_tma_fast.md) — the hardware CTA
-// scheduler balances the unequal units (cells of eight sizes, blur strips) better than a static stride does, and the window
-// loads it hides were already covered by the other five resident CTAs.  Kept as a measured, tested alternative.
-static int fast_tma_min_frames() {
-    const char *e = getenv("VSG_FAST_TMA");
-    const int v = e ? atoi(e) : 0;
-    return v <= 0 ? INT_MAX : v;
-}
-
-// per-level 3-D tensor maps (x bytes, y rows, frame) over the pyramid planes of this launch; false if TMA cannot address them
-// (driver entry point missing, or a caller-owned level 0 whose base / pitch / stride is not 16-byte aligned)
-static bool make_fast_tile_maps(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride, const uint8_t *pyr,
-                                int nframes, FastTileMaps *maps) {
-    EncodeTiledFn fn = encode_tiled_fn();
-    if (!fn) return false;
-    for (int l = 0; l < g.nlevels; ++l) {
-        const LevelGeom &L = g.lv[l];
-        const uint8_t *base = l == 0 ? lvl0_base : pyr + L.plane_offset;
-        const int64_t pitch = l == 0 ? lvl0_pitch : L.pitch, stride = l == 0 ? lvl0_stride : L.plane_stride;
-        if (((uintptr_t)base & 15) || (pitch & 15) || (stride & 15) || pitch < kRawPitch) return false;
-        const int rows = std::min(L.h_cell + 6, 256);
-        const cuuint64_t dims[3] = {(cuuint64_t)pitch, (cuuint64_t)L.h, (cuuint64_t)nframes};
-        const cuuint64_t strides[2] = {(cuuint64_t)pitch, (cuuint64_t)stride};
-        const cuuint32_t box[3] = {(cuuint32_t)kRawPitch, (cuuint32_t)rows, 1};
-        const cuuint32_t estr[3] = {1, 1, 1};
-        if (fn(&maps->m[l], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, (void *)base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return false;
-        maps->box_rows[l] = rows;
-        maps->frame0[l] = 0;
-    }
-    for (int l = g.nlevels; l < 8; ++l) { maps->m[l] = maps->m[0]; maps->box_rows[l] = 0; maps->frame0[l] = 0; }
-    return true;
-}
-
 // blur == nullptr: FAST alone; otherwise the fused FAST + blur grid.
-vsg_status launch_fast(const FrameGeom &g, const Cell *cells, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride,
-                 const uint8_t *pyr, uint8_t *blur, Cand *cand, int *cand_count, int ini_th, int min_th, int max_cw,
-                 int max_ch, int nframes, cudaStream_t s) {
-    (void)cells;   // the kernel derives the cell geometry from the level tables
+vsg_status launch_fast(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride, const uint8_t *pyr,
+                       uint8_t *blur, Cand *cand, int *cand_count, int ini_th, int min_th, int max_cw, int max_ch, int nframes,
+                       cudaStream_t s) {
     if (g.ncells == 0) {
         if (blur) launch_blur(g, lvl0_base, lvl0_pitch, lvl0_stride, pyr, blur, nframes, s);
         return VSG_OK;
@@ -488,29 +353,9 @@ vsg_status launch_fast(const FrameGeom &g, const Cell *cells, const uint8_t *lvl
         const int nblur = bl.block_begin[g.nlevels];
         const int ratio = g.ncells / nblur;
         const uint32_t group_rcp = (uint32_t)((0x100000000ull + (uint64_t)ratio) / (uint64_t)(ratio + 1));   // ceil(2^32 / group)
-        // large batches: persistent CTAs with TMA-staged cell windows
-        const int upf = g.ncells + nblur;
-        const int64_t total = (int64_t)upf * nframes;
-        FastTileMaps maps;
-        if (nframes >= fast_tma_min_frames() && g.nlevels <= 8 && max_S <= 24 && total * upf < (1ll << 32) &&
-            make_fast_tile_maps(g, lvl0_base, lvl0_pitch, lvl0_stride, pyr, nframes, &maps)) {
-            const int raw_bytes = (tile_rows * kRawPitch + 127) & ~127;
-            const size_t smem_tma = smem + 2 * (size_t)raw_bytes + 128 + 32;
-            cudaFuncSetAttribute(fast_blur_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma);
-            int dev = 0, sms = 148, per_sm = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fast_blur_tma_kernel, kFastThreads, smem_tma);
-            const int grid = (int)std::min<int64_t>(total, (int64_t)sms * std::max(per_sm, 1));
-            const uint32_t upf_rcp = (uint32_t)((0x100000000ull + (uint64_t)upf - 1) / (uint64_t)upf);
-            launch_kernel(fast_blur_tma_kernel, dim3(grid), dim3(kFastThreads), smem_tma, s, false, g, bl, maps, lvl0_base, lvl0_pitch,
-                          lvl0_stride, pyr, blur, cand, cand_count, ini_th, min_th, tile_rows, list_cap, nblur, ratio, group_rcp, upf,
-                          upf_rcp, (int)total);
-        } else {
-            launch_kernel(fast_blur_kernel, dim3(g.ncells + nblur, nframes), dim3(kFastThreads), smem, s, true, g, bl, lvl0_base,
-                          lvl0_pitch, lvl0_stride, pyr, blur, cand, cand_count, ini_th, min_th, tile_rows, list_cap, nblur, ratio,
-                          group_rcp);
-        }
+        launch_kernel(fast_blur_kernel, dim3(g.ncells + nblur, nframes), dim3(kFastThreads), smem, s, true, g, bl, lvl0_base,
+                      lvl0_pitch, lvl0_stride, pyr, blur, cand, cand_count, ini_th, min_th, tile_rows, list_cap, nblur, ratio,
+                      group_rcp);
     }
     count_launch();
     return VSG_OK;

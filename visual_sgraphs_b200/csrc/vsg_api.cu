@@ -39,15 +39,11 @@ bool cuda_ok(cudaError_t e, const char *what) {
 void count_launch(int n) { g_launches += n; }
 // Programmatic dependent launch pays where launch latency is the cost — a handful of frames: 229 -> 213 us per
 // single-frame call — and hurts where the kernels are long: with 512 frames per launch the early-resident blocks of the
-// next kernel take 10 % off the batch rate (4.24 vs 3.85 ms per batch).  VSG_PDL: 0 = never, 1 (default) = only for
-// batches of up to kPdlMaxFrames frames, 2 = always.
+// next kernel take 10 % off the batch rate (4.24 vs 3.85 ms per batch).  So only batches of up to kPdlMaxFrames frames use it.
 static thread_local bool g_pdl_small_batch = true;
 constexpr int kPdlMaxFrames = 8;
 void pdl_scope(int nframes) { g_pdl_small_batch = nframes <= kPdlMaxFrames; }
-bool pdl_enabled() {
-    static const int mode = [] { const char *e = getenv("VSG_PDL"); return e ? atoi(e) : 1; }();
-    return mode >= 2 || (mode == 1 && g_pdl_small_batch);
-}
+bool pdl_enabled() { return g_pdl_small_batch; }
 
 static inline int cv_round(float v) { return (int)lrintf(v); }
 static inline int cv_round(double v) { return (int)lrint(v); }
@@ -66,8 +62,6 @@ struct vsg_extractor {
     static constexpr int kAuxStreams = 2;
     cudaStream_t aux[kAuxStreams] = {nullptr, nullptr};
     int chunk_frames = 128;            // launches of 64 frames reach 76 % of the 512-frame rate, 128: 89 %, 256: 96 %
-    int dev_chunk_frames = 0;          // device-resident batches: 0 = one pass on `stream`
-    bool fuse_fast_blur = true;
     uint8_t *color_d = nullptr;        // device staging of colour frames (vsg_extract_batch_color), allocated on first use
     size_t color_bytes = 0;
     // rectification maps (vsg_extractor_set_rectify_map): quantised on the host, resident on the device; independent of the
@@ -75,13 +69,7 @@ struct vsg_extractor {
     uint32_t *rect_xy[2] = {nullptr, nullptr};
     uint16_t *rect_frac[2] = {nullptr, nullptr};
     int rect_w = 0, rect_h = 0;
-    cudaEvent_t fork_ev = nullptr, join_ev[kAuxStreams] = {nullptr, nullptr};
-    // Completion of a chunked host-pointer batch can be awaited on blocking-sync events: the calling thread sleeps instead of
-    // spinning in cudaStreamSynchronize, which matters when several handles / ranks share the host's cores
-    // (off by default: on the 8-GPU box the end-to-end rate is limited by the aggregate H2D bandwidth of the host, 141 GB/s,
-    // and is the same with either wait; VSG_BLOCKING_SYNC=1 enables it; single frames always spin: lower latency).
-    cudaEvent_t done_ev[kAuxStreams + 1] = {nullptr, nullptr, nullptr};
-    bool blocking_sync = false;
+    cudaEvent_t fork_ev = nullptr;
     vsg_orb_params p{};
     std::vector<float> scale, inv_scale, sigma2, inv_sigma2;
     std::vector<int> quota;
@@ -89,11 +77,9 @@ struct vsg_extractor {
     // shape dependent state
     int cur_w = 0, cur_h = 0;
     FrameGeom g{};
-    std::vector<Cell> cells_h;
     int max_cw = 0, max_ch = 0, max_nodes = 0;
     int64_t pyr_bytes_per_frame = 0;
 
-    Cell *cells_d = nullptr;
     short4 *tabs_d = nullptr;
     PyrTile *pyr_tiles_d = nullptr;        // one-launch pyramid for small batches (pyramid.cu); nullptr = not available
     int pyr_ntiles = 0, pyr_tile_buf = 0;
@@ -144,13 +130,13 @@ struct vsg_extractor {
     bool results_on_handle = false;    // kps_d / desc_d / n_d hold the last call's results (host-pointer API)
 
     void free_shape() {
-        cudaFree(cells_d); cudaFree(tabs_d); cudaFree(pyr_tiles_d); cudaFree(pyr); cudaFree(blur); cudaFree(cand); cudaFree(node_of);
+        cudaFree(tabs_d); cudaFree(pyr_tiles_d); cudaFree(pyr); cudaFree(blur); cudaFree(cand); cudaFree(node_of);
         cudaFree(cand_count); cudaFree(level_kps); cudaFree(level_kp_count); cudaFree(slot); cudaFree(out_block_d);
         cudaFree(color_d);
         color_d = nullptr; color_bytes = 0;
         cudaFreeHost(out_block_h);
         out_block_d = out_block_h = nullptr; out_block_bytes = 0;
-        cells_d = nullptr; tabs_d = nullptr; pyr_tiles_d = nullptr; pyr_ntiles = 0; pyr = blur = nullptr; cand = nullptr; node_of = nullptr;
+        tabs_d = nullptr; pyr_tiles_d = nullptr; pyr_ntiles = 0; pyr = blur = nullptr; cand = nullptr; node_of = nullptr;
         cand_count = nullptr; level_kps = nullptr; level_kp_count = nullptr; slot = nullptr; kps_d = nullptr;
         desc_d = nullptr; n_d = mono_d = nullptr; kps_h = nullptr; desc_h = nullptr; n_h = mono_h = nullptr;
         cur_w = cur_h = 0;
@@ -222,7 +208,7 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
     FrameGeom &g = ex->g;
     memset(&g, 0, sizeof(g));
     g.nlevels = nl;
-    ex->cells_h.clear();
+    std::vector<Cell> cells;
     ex->max_cw = ex->max_ch = 7;
     ex->max_nodes = 8;
     int64_t plane_off = 0, cand_off = 0;
@@ -246,7 +232,7 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
         L.n_rows = (int)(height / 35.f);
         L.w_cell = (int)std::ceil(width / L.n_cols);
         L.h_cell = (int)std::ceil(height / L.n_rows);
-        L.cell_begin = (int)ex->cells_h.size();
+        L.cell_begin = (int)cells.size();
         int cand_cap = 0;
         for (int i = 0; i < L.n_rows; ++i) {           // :811-828
             const float ini_y = (float)(min_b + i * L.h_cell);
@@ -264,16 +250,16 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
                 c.cw = (short)((int)max_x - (int)ini_x); c.ch = (short)((int)max_y - (int)ini_y);
                 c.pad = 0;
                 if (c.cw < 7 || c.ch < 7) continue;   // cv::FAST finds nothing in such a window
-                ex->cells_h.push_back(c);
+                cells.push_back(c);
                 ex->max_cw = std::max<int>(ex->max_cw, c.cw);
                 ex->max_ch = std::max<int>(ex->max_ch, c.ch);
                 cand_cap += ((c.cw - 6 + 1) / 2) * ((c.ch - 6 + 1) / 2);
             }
         }
-        L.cell_count = (int)ex->cells_h.size() - L.cell_begin;
+        L.cell_count = (int)cells.size() - L.cell_begin;
         L.cols_eff = L.rows_eff = 0;
-        for (int k = L.cell_begin; k < (int)ex->cells_h.size(); ++k) {
-            const Cell &c = ex->cells_h[k];
+        for (int k = L.cell_begin; k < (int)cells.size(); ++k) {
+            const Cell &c = cells[k];
             L.cols_eff = std::max(L.cols_eff, (c.x0 - min_b) / L.w_cell + 1);
             L.rows_eff = std::max(L.rows_eff, (c.y0 - min_b) / L.h_cell + 1);
         }
@@ -306,7 +292,7 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
             L.resize_tma_ok = resize_tma_fits(xts[l], yts[l], L.w, L.h) ? 1 : 0;
         }
     }
-    g.ncells = (int)ex->cells_h.size();
+    g.ncells = (int)cells.size();
     for (int l = nl; l < kMaxLevels; ++l) g.lv[l].cell_begin = 0x7fffffff;   // fast.cu finds a cell's level by counting begins <= cell
     g.cand_total = cand_off;
     g.kp_total = kp_off;
@@ -331,8 +317,7 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
     // tiles of the one-launch pyramid: a 12 x 12 partition of every level; going down from the top level, a tile's region
     // is the bounding box of what it owns and of the taps of its region one level up
     if (nl >= 2) {
-        const char *ev = getenv("VSG_PYR_TILES");
-        const int ntx = ev && atoi(ev) > 0 ? atoi(ev) : 12, nty = ntx;
+        constexpr int ntx = 12, nty = 12;
         std::vector<PyrTile> tiles((size_t)ntx * nty);
         int buf = 0, ntab_max = 0, dim_max = 0;
         for (int ty = 0; ty < nty; ++ty)
@@ -367,8 +352,6 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
             ex->pyr_ntiles = (int)tiles.size();
         }
     }
-    CK(cudaMalloc(&ex->cells_d, std::max<size_t>(ex->cells_h.size(), 1) * sizeof(Cell)));
-    CK(cudaMemcpy(ex->cells_d, ex->cells_h.data(), ex->cells_h.size() * sizeof(Cell), cudaMemcpyHostToDevice));
     CK(cudaMalloc(&ex->pyr, plane_off + 256));
     CK(cudaMalloc(&ex->blur, plane_off + 256));
     CK(cudaMemset(ex->pyr, 0, plane_off + 256));
@@ -451,18 +434,16 @@ vsg_status run_pipeline(vsg_extractor *ex, cudaStream_t s, int f0, const uint8_t
         }
     }
     STAGE_MARK(1);
-    // FAST cells and the Gaussian blur share one grid (fast.cu) unless VSG_FUSE_FAST_BLUR=0
-    // large batches blur on the tensor cores instead (blur_tc.cu), as a stage of its own after the oct-tree
+    // FAST cells and the Gaussian blur share one grid (fast.cu); large batches blur on the tensor cores instead
+    // (blur_tc.cu), as a stage of its own after the oct-tree
     const BlurTcPlan *blur_tc = plan_blur_tc(g, lvl0_base, lvl0_pitch, lvl0_stride, ex->pyr, ex->blur, nframes);
-    const vsg_status fst = launch_fast(g, ex->cells_d, lvl0_base, lvl0_pitch, lvl0_stride, ex->pyr,
-                                       ex->fuse_fast_blur && !blur_tc ? ex->blur : nullptr, ex->cand, cand_count, ex->p.ini_th_fast,
-                                       ex->p.min_th_fast, ex->max_cw, ex->max_ch, nframes, s);
+    const vsg_status fst = launch_fast(g, lvl0_base, lvl0_pitch, lvl0_stride, ex->pyr, blur_tc ? nullptr : ex->blur, ex->cand,
+                                       cand_count, ex->p.ini_th_fast, ex->p.min_th_fast, ex->max_cw, ex->max_ch, nframes, s);
     if (fst != VSG_OK) return fst;
     STAGE_MARK(2);
     launch_octree(g, ex->cand, cand_count, ex->node_of, level_kps, level_kp_count, ex->max_nodes, nframes, s);
     STAGE_MARK(3);
     if (blur_tc) launch_blur_tc(blur_tc, ex->blur, s);
-    else if (!ex->fuse_fast_blur) launch_blur(g, lvl0_base, lvl0_pitch, lvl0_stride, ex->pyr, ex->blur, nframes, s);
     STAGE_MARK(4);
     launch_describe(g, lvl0_base, lvl0_pitch, lvl0_stride, ex->pyr, ex->blur, level_kps, level_kp_count, lap_x0,
                     lap_x1, kps_dev, desc_dev, out_cap, n_dev, mono_dev, slot, nframes, s);
@@ -531,12 +512,7 @@ vsg_status vsg_extractor_create(const vsg_orb_params *params, int device, int ma
         return VSG_ERR_CUDA;
     }
     if (const char *e = getenv("VSG_CHUNK_FRAMES")) ex->chunk_frames = std::max(1, atoi(e));
-    if (const char *e = getenv("VSG_DEV_CHUNK_FRAMES")) ex->dev_chunk_frames = std::max(0, atoi(e));
-    if (const char *e = getenv("VSG_FUSE_FAST_BLUR")) ex->fuse_fast_blur = atoi(e) != 0;
-    if (const char *e = getenv("VSG_BLOCKING_SYNC")) ex->blocking_sync = atoi(e) != 0;
-    for (cudaEvent_t &e : ex->done_ev) cudaEventCreateWithFlags(&e, cudaEventBlockingSync | cudaEventDisableTiming);
     cudaEventCreateWithFlags(&ex->fork_ev, cudaEventDisableTiming);
-    for (cudaEvent_t &e : ex->join_ev) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
     *out = ex;
     return VSG_OK;
 }
@@ -548,10 +524,6 @@ void vsg_extractor_destroy(vsg_extractor *ex) {
     for (cudaStream_t a : ex->aux)
         if (a) { cudaStreamSynchronize(a); cudaStreamDestroy(a); }
     if (ex->fork_ev) cudaEventDestroy(ex->fork_ev);
-    for (cudaEvent_t e : ex->done_ev)
-        if (e) cudaEventDestroy(e);
-    for (cudaEvent_t e : ex->join_ev)
-        if (e) cudaEventDestroy(e);
     if (ex->ev_created)
         for (int i = 0; i < vsg_extractor::kEvRing; ++i)
             for (int k = 0; k <= VSG_NUM_STAGES; ++k) cudaEventDestroy(ex->ev[i][k]);
@@ -700,13 +672,8 @@ static vsg_status extract_batch_host(vsg_extractor *ex, const uint8_t *images, i
                                cudaMemcpyDeviceToHost, s));
         }
     }
-    if (chunked && ex->blocking_sync) {
-        for (int k = 0; k < nstreams_used; ++k) CK(cudaEventRecord(ex->done_ev[k], k == 0 ? ex->stream : ex->aux[k - 1]));
-        for (int k = 0; k < nstreams_used; ++k) CK(cudaEventSynchronize(ex->done_ev[k]));
-    } else {
-        for (int k = 1; k < nstreams_used; ++k) CK(cudaStreamSynchronize(ex->aux[k - 1]));
-        CK(cudaStreamSynchronize(ex->stream));
-    }
+    for (int k = 1; k < nstreams_used; ++k) CK(cudaStreamSynchronize(ex->aux[k - 1]));
+    CK(cudaStreamSynchronize(ex->stream));
     vsg_status ret = VSG_OK;
     for (int f = 0; f < nframes; ++f) {
         const int n = ex->n_h[f];
@@ -812,28 +779,8 @@ vsg_status vsg_extract_batch_dev(vsg_extractor *ex, const uint8_t *images_dev, i
     }
     ex->lvl0_base = images_dev; ex->lvl0_pitch = pitch; ex->lvl0_stride = (int64_t)frame_stride; ex->last_nframes = nframes;
     ex->results_on_handle = false;
-    const int chunk = ex->dev_chunk_frames;
-    if (ex->profile || chunk <= 0 || nframes < 2 * chunk)
-        return run_pipeline(ex, ex->stream, 0, images_dev, pitch, (int64_t)frame_stride, nframes, lap_x0, lap_x1,
-                            keypoints_dev, descriptors_dev, capacity, n_dev, mono_dev);
-    // Chunks rotate over the handle's three streams so that kernels of different stages (ALU-bound FAST next to
-    // latency-bound resize / blur / describe) share the SMs; the handle's stream forks and joins the other two, so
-    // the call keeps its stream-ordered contract.
-    CK(cudaEventRecord(ex->fork_ev, ex->stream));
-    for (cudaStream_t a : ex->aux) CK(cudaStreamWaitEvent(a, ex->fork_ev, 0));
-    for (int f0 = 0, c = 0; f0 < nframes; f0 += chunk, ++c) {
-        const int nf = std::min(chunk, nframes - f0);
-        cudaStream_t s = (c % 3 == 0) ? ex->stream : ex->aux[c % 3 - 1];
-        st = run_pipeline(ex, s, f0, images_dev + (size_t)f0 * frame_stride, pitch, (int64_t)frame_stride, nf, lap_x0, lap_x1,
-                          keypoints_dev + (size_t)f0 * capacity, descriptors_dev + (size_t)f0 * capacity * 32, capacity,
-                          n_dev + f0, mono_dev + f0);
-        if (st != VSG_OK) break;       // the aux streams are joined below on the error path too
-    }
-    for (int k = 0; k < vsg_extractor::kAuxStreams; ++k) {
-        CK(cudaEventRecord(ex->join_ev[k], ex->aux[k]));
-        CK(cudaStreamWaitEvent(ex->stream, ex->join_ev[k], 0));
-    }
-    return st;
+    return run_pipeline(ex, ex->stream, 0, images_dev, pitch, (int64_t)frame_stride, nframes, lap_x0, lap_x1, keypoints_dev,
+                        descriptors_dev, capacity, n_dev, mono_dev);
 }
 
 vsg_status vsg_extractor_sync(vsg_extractor *ex) {

@@ -132,7 +132,7 @@ bool extractor_pyramid(vsg_extractor *ex, PyramidRef *out);
 // kernel of the stream is still draining; it must execute pdl_wait() before touching anything that kernel wrote.
 // Every pipeline kernel calls pdl_launch_dependents() first thing (the next kernel's blocks can be made resident as
 // soon as all of this kernel's blocks have started) and pdl_wait() ahead of its first dependent access; both are no-ops
-// for ordinary launches.  VSG_PDL=0 disables the attribute.
+// for ordinary launches.  Only batches of up to 8 frames are launched with the attribute (vsg_api.cu: pdl_enabled).
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 bool pdl_enabled();
@@ -199,9 +199,9 @@ void launch_blur_tc(const BlurTcPlan *plan, uint8_t *blur, cudaStream_t s);
 void launch_blur(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride, const uint8_t *pyr,
                  uint8_t *blur, int nframes, cudaStream_t s);
 // blur != nullptr: the Gaussian blur of the same frames runs inside the same grid (fast_blur_kernel)
-vsg_status launch_fast(const FrameGeom &g, const Cell *cells, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride,
-                 const uint8_t *pyr, uint8_t *blur, Cand *cand, int *cand_count, int ini_th, int min_th, int max_cw,
-                 int max_ch, int nframes, cudaStream_t s);
+vsg_status launch_fast(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride, const uint8_t *pyr,
+                       uint8_t *blur, Cand *cand, int *cand_count, int ini_th, int min_th, int max_cw, int max_ch, int nframes,
+                       cudaStream_t s);
 void launch_octree(const FrameGeom &g, const Cand *cand, const int *cand_count, unsigned short *node_of,
                    LevelKp *level_kps, int *level_kp_count, int max_quota_nodes, int nframes, cudaStream_t s);
 void launch_describe(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride,
