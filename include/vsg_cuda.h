@@ -70,7 +70,10 @@ int64_t vsg_launch_count(void);
  * ---------------------------------------------------------------------------------------------- */
 
 /* ORBextractor::ORBextractor (ORBextractor.cc:411-470).  `max_batch` = frames per vsg_extract_batch
- * call the handle must be able to hold (1 for the per-frame operator()). */
+ * call the handle must be able to hold (1 for the per-frame operator()).  The oct-tree keeps a level's nodes in shared
+ * memory, which bounds every level's quota (features_per_level): on a B200 a quota of more than about 3,380 features does
+ * not fit (nlevels = 1 with nfeatures = 3400, for one).  Such a handle is created, but every call that needs a frame size
+ * fails with VSG_ERR_INVALID before anything is launched; vsg_last_error names the level, its quota and the bytes needed. */
 vsg_status vsg_extractor_create(const vsg_orb_params *params, int device, int max_batch, vsg_extractor **out);
 void vsg_extractor_destroy(vsg_extractor *ex);
 

@@ -22,6 +22,7 @@
 //   * Final pick per node = highest response, FIRST in the reference's candidate order on ties
 //     (:766-782).  Candidate order is cell-row-major, then row-major inside the cell (:811-874), so
 //     the tie break is an atomicMax on (response, ~order_key(x, y)).
+#include <algorithm>
 #include <cstdio>
 
 #include "introsort.cuh"
@@ -417,25 +418,42 @@ __global__ void __launch_bounds__(kThreads) octree_kernel(FrameGeom g, const Can
 #endif
 }
 
-void launch_octree(const FrameGeom &g, const Cand *cand, const int *cand_count, unsigned short *node_of,
-                   LevelKp *level_kps, int *level_kp_count, int max_nodes, int nframes, cudaStream_t s) {
-    const int cap = (max_nodes + 3) & ~3;
+static int octree_cap(int max_nodes) { return (max_nodes + 3) & ~3; }
+
+size_t octree_smem_bytes(int max_nodes) {
     // list_a, list_b (12 B each), cc (16 B), child_pos (8 B), stay_pos, exp_list, push_off, exp_off (2 B each),
     // sort_buf (8 B), split (4 B)
-    const size_t smem = (size_t)cap * (12 + 12 + 16 + 8 + 2 + 2 + 2 + 2 + 8 + 4) + 64;
-    if (smem > 48 * 1024) cudaFuncSetAttribute(octree_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    return (size_t)octree_cap(max_nodes) * (12 + 12 + 16 + 8 + 2 + 2 + 2 + 2 + 8 + 4) + 64;
+}
+
+vsg_status octree_static_smem_bytes(size_t *bytes) {
+    cudaFuncAttributes a256, a512;
+    CK(cudaFuncGetAttributes(&a256, octree_kernel<256>));
+    CK(cudaFuncGetAttributes(&a512, octree_kernel<512>));
+    *bytes = std::max(a256.sharedSizeBytes, a512.sharedSizeBytes);
+    return VSG_OK;
+}
+
+vsg_status launch_octree(const FrameGeom &g, const Cand *cand, const int *cand_count, unsigned short *node_of,
+                         LevelKp *level_kps, int *level_kp_count, int max_nodes, int nframes, cudaStream_t s) {
+    const int cap = octree_cap(max_nodes);
+    const size_t smem = octree_smem_bytes(max_nodes);
     // A few frames: one CTA per SM at most, and a CTA of 8 warps leaves three quarters of the SM's issue slots empty while it
     // walks its keys — 16 warps: 51 -> 44 us for one 640x480 frame (24 warps: 46, 32 warps: the block-wide scans and barriers
     // cost more than the key passes gain).  Large batches fill the SMs with several 8-warp CTAs instead.
     if (nframes <= 8) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(octree_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        launch_kernel(octree_kernel<512>, dim3(g.nlevels, nframes), dim3(512), smem, s, true, g, cand, cand_count, node_of,
-                      level_kps, level_kp_count, cap);
+        if (smem > 48 * 1024)
+            CK(cudaFuncSetAttribute(octree_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CK(launch_kernel(octree_kernel<512>, dim3(g.nlevels, nframes), dim3(512), smem, s, true, g, cand, cand_count, node_of,
+                         level_kps, level_kp_count, cap));
     } else {
-        launch_kernel(octree_kernel<256>, dim3(g.nlevels, nframes), dim3(256), smem, s, true, g, cand, cand_count, node_of,
-                      level_kps, level_kp_count, cap);
+        if (smem > 48 * 1024)
+            CK(cudaFuncSetAttribute(octree_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CK(launch_kernel(octree_kernel<256>, dim3(g.nlevels, nframes), dim3(256), smem, s, true, g, cand, cand_count, node_of,
+                         level_kps, level_kp_count, cap));
     }
     count_launch();
+    return VSG_OK;
 }
 
 }  // namespace vsg

@@ -203,6 +203,12 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
         set_error("image %dx%d too large: at most %d pixels per side", w, h, kMaxImageDim);
         return VSG_ERR_INVALID;
     }
+    CK(cudaSetDevice(ex->device));
+    int smem_optin = 0;
+    size_t octree_static = 0;
+    CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ex->device));
+    const vsg_status ost = octree_static_smem_bytes(&octree_static);
+    if (ost != VSG_OK) return ost;
     ex->free_shape();
     const int nl = ex->p.nlevels;
     FrameGeom &g = ex->g;
@@ -283,6 +289,13 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
         L.kp_cap = std::max(L.quota, 4 * L.n_ini) + 4;
         L.kp_offset = kp_off;
         kp_off += L.kp_cap;
+        // the oct-tree keeps a level's nodes in shared memory; a quota whose lists do not fit cannot be launched
+        const size_t octree_need = octree_smem_bytes(L.kp_cap + 4) + octree_static;
+        if (octree_need > (size_t)smem_optin) {
+            set_error("level %d: oct-tree quota %d needs %zu bytes of shared memory per block, the device allows %d", l, L.quota,
+                      octree_need, smem_optin);
+            return VSG_ERR_INVALID;
+        }
         ex->max_nodes = std::max(ex->max_nodes, L.kp_cap + 4);
         L.scale = ex->scale[l];
         L.kp_size = (float)(int)(kPatch * ex->scale[l]);                                    // :884
@@ -300,7 +313,6 @@ vsg_status configure_shape(vsg_extractor *ex, int w, int h) {
     ex->pyr_bytes_per_frame = plane_off / ex->max_batch;
 
     const int B = ex->max_batch;
-    CK(cudaSetDevice(ex->device));
     // resize tables, one allocation
     size_t ntab = 0;
     for (int l = 1; l < nl; ++l) ntab += xts[l].size() + yts[l].size();
@@ -441,7 +453,9 @@ vsg_status run_pipeline(vsg_extractor *ex, cudaStream_t s, int f0, const uint8_t
                                        cand_count, ex->p.ini_th_fast, ex->p.min_th_fast, ex->max_cw, ex->max_ch, nframes, s);
     if (fst != VSG_OK) return fst;
     STAGE_MARK(2);
-    launch_octree(g, ex->cand, cand_count, ex->node_of, level_kps, level_kp_count, ex->max_nodes, nframes, s);
+    // nothing after this may run when the oct-tree did not: describe reads the level keypoint counts it writes
+    const vsg_status ost = launch_octree(g, ex->cand, cand_count, ex->node_of, level_kps, level_kp_count, ex->max_nodes, nframes, s);
+    if (ost != VSG_OK) return ost;
     STAGE_MARK(3);
     if (blur_tc) launch_blur_tc(blur_tc, ex->blur, s);
     STAGE_MARK(4);

@@ -202,8 +202,13 @@ void launch_blur(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, i
 vsg_status launch_fast(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride, const uint8_t *pyr,
                        uint8_t *blur, Cand *cand, int *cand_count, int ini_th, int min_th, int max_cw, int max_ch, int nframes,
                        cudaStream_t s);
-void launch_octree(const FrameGeom &g, const Cand *cand, const int *cand_count, unsigned short *node_of,
-                   LevelKp *level_kps, int *level_kp_count, int max_quota_nodes, int nframes, cudaStream_t s);
+// octree_kernel keeps its node lists in shared memory: octree_smem_bytes(max_nodes) dynamic bytes per block, plus the
+// kernel's static arrays (octree_static_smem_bytes).  Their sum must fit the device's per-block opt-in limit, so the level
+// quotas a handle accepts are bounded (configure_shape checks this before anything is allocated or launched).
+size_t octree_smem_bytes(int max_nodes);
+vsg_status octree_static_smem_bytes(size_t *bytes);
+vsg_status launch_octree(const FrameGeom &g, const Cand *cand, const int *cand_count, unsigned short *node_of,
+                         LevelKp *level_kps, int *level_kp_count, int max_nodes, int nframes, cudaStream_t s);
 void launch_describe(const FrameGeom &g, const uint8_t *lvl0_base, int lvl0_pitch, int64_t lvl0_stride,
                      const uint8_t *pyr, const uint8_t *blur, const LevelKp *level_kps, const int *level_kp_count,
                      int lap_x0, int lap_x1, vsg_keypoint *kps_out, uint8_t *desc_out, int out_cap, int *n_out,
