@@ -9,30 +9,35 @@ from visual_sgraphs_b200.synth import synth_frame
 _cache = {}
 
 
-def two_frames(oracle, seed=11, shift=(9, 5), size=(640, 480), nfeat=1000):
-    key = (seed, shift, size, nfeat)
+def two_frames(oracle, seed=11, shift=(9, 5), size=(640, 480), nfeat=1000, scale=1.2, nlevels=8):
+    key = (seed, shift, size, nfeat, scale, nlevels)
     if key not in _cache:
         a = synth_frame(seed, *size)
         rng = np.random.default_rng(seed + 1)
         b = np.roll(a, (shift[1], shift[0]), (0, 1))
         b = np.clip(b.astype(np.int16) + rng.integers(-3, 4, b.shape), 0, 255).astype(np.uint8)
-        ex = oracle.OracleExtractor(nfeat)
+        ex = oracle.OracleExtractor(nfeat, scale, nlevels)
         _, ka, da = ex(a)
         _, kb, db = ex(b)
         _cache[key] = (ka, da, kb, db)
     return _cache[key]
 
 
-def frame_data(keys, desc, size=(640, 480), stereo_seed=None):
+def scale_factors(oracle, scale=1.2, nlevels=8):
+    """mvScaleFactors of an extractor with this pyramid (the table Frame copies from its ORBextractor)."""
+    return oracle.OracleExtractor(1000, scale, nlevels).tables()["scale"]
+
+
+def frame_data(keys, desc, size=(640, 480), stereo_seed=None, bounds=None, scale_factors=None):
     u_right = None
     if stereo_seed is not None:
         rng = np.random.default_rng(stereo_seed)
         disp = rng.uniform(2, 40, len(keys)).astype(np.float32)
         u_right = np.where(rng.random(len(keys)) < 0.7, keys["x"] - disp, -1).astype(np.float32)
-    return FrameData(keys, desc, u_right=u_right, width=size[0], height=size[1])
+    return FrameData(keys, desc, u_right=u_right, bounds=bounds, scale_factors=scale_factors, width=size[0], height=size[1])
 
 
-def track_points(fd_target, kb, db, shift, seed, stereo=False):
+def track_points(fd_target, kb, db, shift, seed, stereo=False, nlevels=8):
     """Map points seen in frame B, projected into frame A (the Frame being searched)."""
     rng = np.random.default_rng(seed)
     n = len(kb)
@@ -42,7 +47,7 @@ def track_points(fd_target, kb, db, shift, seed, stereo=False):
     pts["proj_xr"] = pts["proj_x"] - rng.uniform(2, 40, n) if stereo else 0
     pts["view_cos"] = rng.uniform(0.99, 1.0, n)
     pts["depth"] = rng.uniform(1, 80, n)
-    pts["level"] = np.clip(kb["octave"] + rng.integers(-1, 2, n), 0, 7)
+    pts["level"] = np.clip(kb["octave"] + rng.integers(-1, 2, n), 0, nlevels - 1)
     pts["in_view"] = rng.random(n) < 0.9
     pts["bad"] = rng.random(n) < 0.03
     pts["blocks"] = rng.random(n) < 0.9
@@ -51,7 +56,7 @@ def track_points(fd_target, kb, db, shift, seed, stereo=False):
     return pts[order].copy(), db[order].copy(), occupied
 
 
-def proj_points(fd_cur, kb, db, shift, seed):
+def proj_points(fd_cur, kb, db, shift, seed, size=(640, 480)):
     rng = np.random.default_rng(seed)
     n = len(kb)
     pts = np.zeros(n, PROJ_POINT_DTYPE)
@@ -60,7 +65,7 @@ def proj_points(fd_cur, kb, db, shift, seed):
     pts["ur"] = pts["u"] - rng.uniform(2, 40, n)
     pts["angle"] = kb["angle"]
     pts["octave"] = kb["octave"]
-    inside = (pts["u"] >= 0) & (pts["u"] <= 640) & (pts["v"] >= 0) & (pts["v"] <= 480)
+    inside = (pts["u"] >= 0) & (pts["u"] <= size[0]) & (pts["v"] >= 0) & (pts["v"] <= size[1])
     pts["valid"] = inside & (rng.random(n) < 0.9)
     pts["blocks"] = rng.random(n) < 0.9
     occupied = (rng.random(fd_cur.n) < 0.05).astype(np.uint8)
@@ -81,7 +86,7 @@ def feature_vector(desc, nnodes=64):
     return nodes.astype(np.int32), np.array(ptr, np.int32), np.array(idx, np.int32)
 
 
-def search_points(kb, shift, seed, sigma=1.0, size=(640, 480)):
+def search_points(kb, shift, seed, sigma=1.0, size=(640, 480), nlevels=8):
     """Map points observed in frame B (keys kb), projected into frame A by the caller: vsg_search_point records."""
     from visual_sgraphs_b200._lib import SEARCH_POINT_DTYPE
     rng = np.random.default_rng(seed)
@@ -91,7 +96,7 @@ def search_points(kb, shift, seed, sigma=1.0, size=(640, 480)):
     pts["v"] = kb["y"] - shift[1] + rng.normal(0, sigma, n)
     pts["ur"] = pts["u"] - rng.uniform(2, 40, n)
     pts["angle"] = kb["angle"]
-    pts["level"] = np.clip(kb["octave"] + rng.integers(-1, 2, n), 0, 7)
+    pts["level"] = np.clip(kb["octave"] + rng.integers(-1, 2, n), 0, nlevels - 1)
     inside = (pts["u"] >= 0) & (pts["u"] < size[0]) & (pts["v"] >= 0) & (pts["v"] < size[1])
     pts["valid"] = inside & (rng.random(n) < 0.9)
     return pts
@@ -155,12 +160,14 @@ def synthetic_vocabulary(seed, k=10, levels=4, prune=0.08):
                 node_desc=np.stack(desc), word_id=word_id, weight=weight, levels=levels)
 
 
-def two_camera_scene(oracle, seed=61, size=(640, 480), nfeat=800):
+def two_camera_scene(oracle, seed=61, size=(640, 480), nfeat=800, scale=1.2, nlevels=8, bounds=None):
     """A two-camera frame (F.Nleft != -1): left / right keypoints are the two related frames of two_frames; map points are
     seen by the left camera, the right camera, or both, with their own projections and predicted levels;
     mvLeftToRightMatch / mvRightToLeftMatch pair up a third of the keypoints.  Returns a dict."""
-    ka, da, kb, db = two_frames(oracle, seed=seed, size=size, nfeat=nfeat)
-    fl, fr = frame_data(ka, da, size=size), frame_data(kb, db, size=size)
+    ka, da, kb, db = two_frames(oracle, seed=seed, size=size, nfeat=nfeat, scale=scale, nlevels=nlevels)
+    sf = None if (scale, nlevels) == (1.2, 8) else scale_factors(oracle, scale, nlevels)
+    fl = frame_data(ka, da, size=size, bounds=bounds, scale_factors=sf)
+    fr = frame_data(kb, db, size=size, bounds=bounds, scale_factors=sf)
     rng = np.random.default_rng(seed + 7)
     nl, nr = len(ka), len(kb)
     # map points: one per left keypoint and one per right keypoint, each also projected (noisily) into the other camera
@@ -172,7 +179,7 @@ def two_camera_scene(oracle, seed=61, size=(640, 480), nfeat=800):
         pts["proj_x"] = keys["x"][src] + rng.normal(0, 1.5, n)
         pts["proj_y"] = keys["y"][src] + rng.normal(0, 1.5, n)
         pts["view_cos"] = rng.uniform(0.99, 1.0, n)
-        pts["level"] = np.clip(keys["octave"][src] + rng.integers(-1, 2, n), 0, 7)
+        pts["level"] = np.clip(keys["octave"][src] + rng.integers(-1, 2, n), 0, nlevels - 1)
     pl["in_view"] = rng.random(n) < 0.7
     pr["in_view"] = rng.random(n) < 0.7
     pr["level"][rng.random(n) < 0.05] = -1                   # mnTrackScaleLevelR == -1 (:149)
@@ -192,11 +199,13 @@ def two_camera_scene(oracle, seed=61, size=(640, 480), nfeat=800):
                 occupied=occupied)
 
 
-def two_camera_last_scene(oracle, seed=61, size=(640, 480), nfeat=800):
+def two_camera_last_scene(oracle, seed=61, size=(640, 480), nfeat=800, scale=1.2, nlevels=8, bounds=None):
     """SearchByProjection(Cur, Last) with a two-camera current frame: every last-frame point comes with its projection
     into the left camera (near a left keypoint) and into the right camera (near a right keypoint or far off)."""
-    ka, da, kb, db = two_frames(oracle, seed=seed, size=size, nfeat=nfeat)
-    fl, fr = frame_data(ka, da, size=size), frame_data(kb, db, size=size)
+    ka, da, kb, db = two_frames(oracle, seed=seed, size=size, nfeat=nfeat, scale=scale, nlevels=nlevels)
+    sf = None if (scale, nlevels) == (1.2, 8) else scale_factors(oracle, scale, nlevels)
+    fl = frame_data(ka, da, size=size, bounds=bounds, scale_factors=sf)
+    fr = frame_data(kb, db, size=size, bounds=bounds, scale_factors=sf)
     rng = np.random.default_rng(seed + 11)
     nl, nr = len(ka), len(kb)
     n = nl + nr
@@ -208,7 +217,7 @@ def two_camera_last_scene(oracle, seed=61, size=(640, 480), nfeat=800):
     pr["u"] = kb["x"][src_r] + rng.normal(0, 1.0, n)
     pr["v"] = kb["y"][src_r] + rng.normal(0, 1.0, n)
     far = rng.random(n) < 0.1                                 # the right projection may land outside the image
-    pr["u"][far] += 900
+    pr["u"][far] += size[0] + 260
     lonely = rng.random(n) < 0.1                              # ... and the left window may be empty (skips the right search)
     pl["u"][lonely] = -200
     from_left = np.arange(n) < nl

@@ -211,6 +211,59 @@ def test_matcher_error_conventions():
                                    ptr(np.zeros((3, 32), np.uint8)), 2, C.byref(C.c_void_p())) == _lib.VSG_ERR_INVALID
 
 
+def test_frame_create_rejects_views_the_kernels_cannot_index():
+    """vsg_frame_create rejects a view whose level tables the searches would read out of bounds: more than kMaxLevels (16)
+    levels, no level while there are keypoints, a keypoint octave outside [0, n_levels).  A valid frame created right after
+    each rejected one still searches correctly."""
+    import ctypes as C
+    from visual_sgraphs_b200 import _lib
+    from visual_sgraphs_b200._lib import KEYPOINT_DTYPE
+    from visual_sgraphs_b200.frame import FrameData
+    from visual_sgraphs_b200.matcher import ORBmatcher
+    L = _lib.load()
+    m = ORBmatcher()
+    rng = np.random.default_rng(3)
+    keys = np.zeros(200, KEYPOINT_DTYPE)
+    keys["x"], keys["y"] = rng.uniform(0, 640, 200), rng.uniform(0, 480, 200)
+    keys["octave"] = rng.integers(0, 8, 200)
+    desc = rng.integers(0, 256, (200, 32), dtype=np.uint8)
+    scale8 = FrameData(keys, desc).scale_factors
+    scale16 = np.float32(1.1) ** np.arange(16, dtype=np.float32)
+
+    def with_octave(i, o):
+        k = keys.copy()
+        k["octave"][i] = o
+        return k
+
+    def rejected(data, what):
+        h = C.c_void_p()
+        assert L.vsg_frame_create(m._h, C.byref(data.view), C.byref(h)) == _lib.VSG_ERR_INVALID, what
+        assert not h.value, what
+        assert b"vsg_frame_create" in L.vsg_last_error(), what
+
+    valid = FrameData(keys, desc)
+    qx, qy = keys["x"][:50].copy(), keys["y"][:50].copy()
+    qr = np.full(50, 30, np.float32)
+    lo, hi = np.full(50, -1, np.int32), np.full(50, -1, np.int32)
+    want = m.area_search(m.frame(valid), qx, qy, qr, lo, hi, desc[:50])
+    assert len(want[1]) > 50
+    cases = [
+        (FrameData(keys, desc, scale_factors=np.concatenate([scale16, [np.float32(5.0)]])), "17 levels"),
+        (FrameData(keys, desc, scale_factors=np.zeros(0, np.float32)), "no level, 200 keypoints"),
+        (FrameData(with_octave(17, -1), desc), "octave -1"),
+        (FrameData(with_octave(199, 8), desc, scale_factors=scale8), "octave 8 of 8 levels"),
+        (FrameData(with_octave(0, 16), desc, scale_factors=scale16), "octave 16 of 16 levels"),
+    ]
+    for data, what in cases:
+        rejected(data, what)
+        got = m.area_search(m.frame(valid), qx, qy, qr, lo, hi, desc[:50])
+        for g, w in zip(got, want):
+            assert np.array_equal(g, w), what
+    # the limits themselves are accepted: 16 levels with a keypoint on the last one, and an empty view without levels
+    m.frame(FrameData(with_octave(0, 15), desc, scale_factors=scale16)).close()
+    m.frame(FrameData(np.zeros(0, KEYPOINT_DTYPE), np.zeros((0, 32), np.uint8), scale_factors=np.zeros(0, np.float32))).close()
+
+
 def test_knn2_full_size_properties():
     """BASELINE config 5 at its full size (100k x 1M descriptors, device-resident): size-independent properties —
     sampled queries against a numpy brute force over the whole train set, planted exact and near duplicates found at

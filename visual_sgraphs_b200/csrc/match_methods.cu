@@ -450,6 +450,17 @@ extern "C" {
 vsg_status vsg_frame_create(vsg_matcher *m, const vsg_frame_view *v, vsg_frame **out) {
     if (!m || !v || !out || v->n < 0 || v->grid_cols < 1 || v->grid_rows < 1 || (v->n > 0 && (!v->keys || !v->descriptors)))
         return VSG_ERR_INVALID;
+    // the searches index the level tables (scale factors, the Fuse gate's kMaxLevels sigma table) by keypoint octave
+    if (v->n_levels > kMaxLevels || (v->n > 0 && v->n_levels < 1)) {
+        set_error("vsg_frame_create: %d pyramid levels, %d keypoints (at most %d levels, at least 1 with keypoints)", v->n_levels,
+                  v->n, kMaxLevels);
+        return VSG_ERR_INVALID;
+    }
+    for (int i = 0; i < v->n; ++i)
+        if (v->keys[i].octave < 0 || v->keys[i].octave >= v->n_levels) {
+            set_error("vsg_frame_create: keypoint %d has octave %d outside [0, %d)", i, v->keys[i].octave, v->n_levels);
+            return VSG_ERR_INVALID;
+        }
     CK(cudaSetDevice(m->device));
     vsg_frame *f = new vsg_frame();
     f->device = m->device; f->n = v->n; f->cols = v->grid_cols; f->rows = v->grid_rows; f->n_levels = v->n_levels;
