@@ -411,6 +411,18 @@ vsg_status vsg_fuse_search(vsg_matcher *m, const vsg_frame *KF, int n, const vsg
                            const uint8_t *desc, float th, const float *inv_level_sigma2, int variant,
                            int32_t *best_idx_out, int *nfused_out);
 
+/* The searches of LocalMapping::SearchInNeighbors' loop `for (pKFi : vpTargetKFs) matcher.Fuse(pKFi, vpMapPointMatches)`
+ * (LocalMapping.cc:764-802) in one call: vsg_fuse_search(m, KFs[t], n, pts + t * n, desc, th, inv_level_sigma2[t], 0,
+ * best_idx_out + t * n, NULL) for every t < ntargets, with one upload, one kernel launch and one download whatever
+ * ntargets is.  pts and best_idx_out are [ntargets][n] (point i projected into target t with that target's pose and
+ * camera); desc (n x 32) is shared by all targets.  The two cameras of a two-camera keyframe are two targets.  Every
+ * target must live on the matcher's device.  The caller replays the bookkeeping target by target; a map point whose
+ * descriptor changes during that replay (MapPoint::Replace recomputes the survivor's) must be searched again in the
+ * later targets. */
+vsg_status vsg_fuse_search_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *KFs,
+                                 const float *const *inv_level_sigma2, int n, const vsg_search_point *pts,
+                                 const uint8_t *desc, float th, int32_t *best_idx_out);
+
 /* SearchBySim3(pKF1, pKF2, vpMatches12, S12, th) (ORBmatcher.cc:1448-1665).  pts1[i1] (KF1.n entries): map point
  * i1 of KF1 projected into KF2 (valid = present, not already matched, not bad, depth/image/distance gates);
  * pts2[i2] likewise into KF1.  matches12_out[i1] = i2 where both directions agree, else -1. */

@@ -53,6 +53,11 @@ struct Chi2Gate {            // inverse level variances for the reprojection gat
     float inv_sigma2[kMaxLevels];
 };
 
+struct FuseTarget {          // one keyframe of a multi-target Fuse search: its grid / features and its level variances
+    FrameDev f;
+    Chi2Gate gate;
+};
+
 struct AreaLists {
     const int2 *raw = nullptr;
     const int *off = nullptr, *cnt = nullptr;
@@ -68,6 +73,10 @@ vsg_status area_search(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQue
 // whole search of the methods whose queries are independent of one another.  out[k] = (index or -1, distance or INT_MAX).
 vsg_status area_best(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc, const float *inv_sigma2,
                      std::vector<int2> &out);
+// area_best with the chi-square gates over the queries of several frames at once (one copy in, one launch, one copy out):
+// query k searches frames[q_target[k]] with inv_sigma2[q_target[k]] and descriptor row qs[k].desc_idx of qdesc (n_qdesc rows).
+vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *frames, const float *const *inv_sigma2, int nq,
+                           const AreaQuery *qs, const int *q_target, int n_qdesc, const uint8_t *qdesc, std::vector<int2> &out);
 vsg_status area_search_raw(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc,
                            int n_qdesc, AreaLists *out);
 // ORBmatcher::ComputeThreeMaxima (ORBmatcher.cc:2002-2043)

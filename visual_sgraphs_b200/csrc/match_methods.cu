@@ -137,14 +137,10 @@ struct PhaseTimer {
 // distance among the keypoints that pass the window / level gates (and, for the pose-based Fuse, the chi-square reprojection
 // gates of ORBmatcher.cc:1273-1299), first candidate in the reference's scan order on ties (its updates are strict '<').
 // For the methods whose queries do not depend on one another — the Fuse searches and SearchBySim3 — this is the whole
-// search: one launch, one (index, distance) pair per query back to the host.
+// search: one launch, one (index, distance) pair per query back to the host.  Called by a whole warp for one query.
 template <bool kChi2>
-__global__ void __launch_bounds__(256) window_best_kernel(FrameDev f, int nq, const AreaQuery *__restrict__ qs,
-                                                          const uint4 *__restrict__ qdesc, Chi2Gate gate,
-                                                          int2 *__restrict__ best_out) {
-    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (q >= nq) return;
-    const AreaQuery a = qs[q];
+__device__ __forceinline__ int2 window_best(const FrameDev &f, const Chi2Gate &gate, const AreaQuery &a, const uint4 *__restrict__ qdesc,
+                                            int di, int lane) {
     const int min_cx = max(0, (int)floorf((a.x - f.min_x - a.r) * f.inv_w));
     const int max_cx = min(f.cols - 1, (int)ceilf((a.x - f.min_x + a.r) * f.inv_w));
     const int min_cy = max(0, (int)floorf((a.y - f.min_y - a.r) * f.inv_h));
@@ -153,7 +149,6 @@ __global__ void __launch_bounds__(256) window_best_kernel(FrameDev f, int nq, co
     int best = INT_MAX, best_idx = -1;
     if (ok) {
         const bool check_levels = (a.min_level > 0) || (a.max_level >= 0);
-        const int di = a.desc_idx >= 0 ? a.desc_idx : q;
         const uint4 qa = __ldg(qdesc + 2 * di), qb = __ldg(qdesc + 2 * di + 1);
         const int ncy = max_cy - min_cy + 1, ncell = (max_cx - min_cx + 1) * ncy;
         for (int base = 0; base < ncell; base += 32) {            // cells in the reference's walk order, 32 per round
@@ -201,7 +196,42 @@ __global__ void __launch_bounds__(256) window_best_kernel(FrameDev f, int nq, co
             }
         }
     }
-    if (lane == 0) best_out[q] = make_int2(best_idx, best);
+    return make_int2(best_idx, best);
+}
+
+template <bool kChi2>
+__global__ void __launch_bounds__(256) window_best_kernel(FrameDev f, int nq, const AreaQuery *__restrict__ qs,
+                                                          const uint4 *__restrict__ qdesc, Chi2Gate gate,
+                                                          int2 *__restrict__ best_out) {
+    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (q >= nq) return;
+    const AreaQuery a = qs[q];
+    const int2 r = window_best<kChi2>(f, gate, a, qdesc, a.desc_idx >= 0 ? a.desc_idx : q, lane);
+    if (lane == 0) best_out[q] = r;
+}
+
+// The same over the queries of several keyframes at once (Fuse into every neighbour of a keyframe): query q searches
+// targets[q_target[q]] with that keyframe's own grid, level and chi-square tables, and descriptor row desc_idx.
+__global__ void __launch_bounds__(256) window_best_multi_kernel(const FuseTarget *__restrict__ targets, int nq,
+                                                                const AreaQuery *__restrict__ qs, const int *__restrict__ q_target,
+                                                                const uint4 *__restrict__ qdesc, int2 *__restrict__ best_out) {
+    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (q >= nq) return;
+    const AreaQuery a = qs[q];
+    const FuseTarget &t = targets[q_target[q]];
+    const int2 r = window_best<true>(t.f, t.gate, a, qdesc, a.desc_idx, lane);
+    if (lane == 0) best_out[q] = r;
+}
+
+static FrameDev frame_dev(const vsg_frame *f) {
+    return FrameDev{f->n, f->cols, f->rows, f->min_x, f->min_y, f->inv_w, f->inv_h, f->xy, f->octave,
+                    f->has_right ? f->u_right : nullptr, (const uint4 *)f->desc, f->cell_ptr, f->cell_idx};
+}
+
+static Chi2Gate chi2_gate(const vsg_frame *f, const float *inv_sigma2) {
+    Chi2Gate gate;
+    for (int l = 0; l < kMaxLevels; ++l) gate.inv_sigma2[l] = inv_sigma2 && l < f->n_levels ? inv_sigma2[l] : 0.f;
+    return gate;
 }
 
 // Best candidate of every query (see window_best_kernel); out[k] = (keypoint index or -1, distance or INT_MAX), host memory.
@@ -217,10 +247,8 @@ vsg_status area_best(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery
         return st;
     CK(cudaMemcpyAsync(m->buf[7], qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(m->buf[8], qdesc, (size_t)nq * 32, cudaMemcpyHostToDevice, s));
-    FrameDev fd{f->n, f->cols, f->rows, f->min_x, f->min_y, f->inv_w, f->inv_h, f->xy, f->octave,
-                f->has_right ? f->u_right : nullptr, (const uint4 *)f->desc, f->cell_ptr, f->cell_idx};
-    Chi2Gate gate;
-    for (int l = 0; l < kMaxLevels; ++l) gate.inv_sigma2[l] = inv_sigma2 && l < f->n_levels ? inv_sigma2[l] : 0.f;
+    const FrameDev fd = frame_dev(f);
+    const Chi2Gate gate = chi2_gate(f, inv_sigma2);
     if (inv_sigma2)
         window_best_kernel<true><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, (const AreaQuery *)m->buf[7], (const uint4 *)m->buf[8], gate,
                                                               (int2 *)m->buf[9]);
@@ -232,6 +260,38 @@ vsg_status area_best(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery
     CK(cudaMemcpyAsync(m->hbuf[0], m->buf[9], (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     memcpy(out.data(), m->hbuf[0], (size_t)nq * sizeof(int2));
+    return VSG_OK;
+}
+
+vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *frames, const float *const *inv_sigma2, int nq,
+                           const AreaQuery *qs, const int *q_target, int n_qdesc, const uint8_t *qdesc, std::vector<int2> &out) {
+    out.assign(nq, make_int2(-1, INT_MAX));
+    if (nq == 0) return VSG_OK;
+    cudaStream_t s = m->stream;
+    vsg_status st;
+    // one staging block, one H2D copy: target table, queries, their targets, descriptor rows (16-byte aligned sections)
+    auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+    const size_t o_tgt = 0, o_q = o_tgt + up16((size_t)ntargets * sizeof(FuseTarget)),
+                 o_qt = o_q + up16((size_t)nq * sizeof(AreaQuery)), o_desc = o_qt + up16((size_t)nq * sizeof(int)),
+                 total = o_desc + (size_t)n_qdesc * 32;
+    // device slots: 17 inputs, 18 results; pinned host slots: 7 inputs, 5 results
+    if ((st = matcher_ensure(m, 17, total)) || (st = matcher_ensure(m, 18, (size_t)nq * sizeof(int2))) ||
+        (st = matcher_ensure_host(m, 7, total)) || (st = matcher_ensure_host(m, 5, (size_t)nq * sizeof(int2))))
+        return st;
+    uint8_t *h = (uint8_t *)m->hbuf[7], *d = (uint8_t *)m->buf[17];
+    FuseTarget *ht = (FuseTarget *)(h + o_tgt);
+    for (int t = 0; t < ntargets; ++t) ht[t] = FuseTarget{frame_dev(frames[t]), chi2_gate(frames[t], inv_sigma2[t])};
+    memcpy(h + o_q, qs, (size_t)nq * sizeof(AreaQuery));
+    memcpy(h + o_qt, q_target, (size_t)nq * sizeof(int));
+    memcpy(h + o_desc, qdesc, (size_t)n_qdesc * 32);
+    CK(cudaMemcpyAsync(d, h, total, cudaMemcpyHostToDevice, s));
+    window_best_multi_kernel<<<(nq + 7) / 8, 256, 0, s>>>((const FuseTarget *)(d + o_tgt), nq, (const AreaQuery *)(d + o_q),
+                                                          (const int *)(d + o_qt), (const uint4 *)(d + o_desc), (int2 *)m->buf[18]);
+    count_launch();
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(m->hbuf[5], m->buf[18], (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    memcpy(out.data(), m->hbuf[5], (size_t)nq * sizeof(int2));
     return VSG_OK;
 }
 

@@ -22,6 +22,7 @@
 #include <climits>
 #include <cmath>
 #include <cstring>
+#include <string>
 #include <vector>
 
 #include "match_internal.cuh"
@@ -30,10 +31,10 @@ using namespace vsg;
 
 namespace {
 
-// Queries for the valid points of a projected-point list: radius = th * scale[level], levels [level+lo, level+hi].
-vsg_status build_queries(const vsg_frame *F, int n, const vsg_search_point *pts, const uint8_t *desc, float th, int lo,
-                         int hi, std::vector<AreaQuery> &qs, std::vector<int> &q_src, std::vector<uint8_t> &qdesc) {
-    qs.clear(); q_src.clear();
+// Queries for the valid points of a projected-point list: radius = th * scale[level], levels [level+lo, level+hi]; appended
+// to qs, with the point's index in q_src.
+vsg_status append_queries(const vsg_frame *F, int n, const vsg_search_point *pts, float th, int lo, int hi,
+                          std::vector<AreaQuery> &qs, std::vector<int> &q_src) {
     for (int i = 0; i < n; ++i) {
         const vsg_search_point &p = pts[i];
         if (!p.valid) continue;
@@ -45,6 +46,15 @@ vsg_status build_queries(const vsg_frame *F, int n, const vsg_search_point *pts,
         qs.push_back(AreaQuery{p.u, p.v, radius, p.level + lo, p.level + hi, 0.f, -1.f});
         q_src.push_back(i);
     }
+    return VSG_OK;
+}
+
+// The same as a fresh list, with the descriptor rows of the queries gathered into qdesc.
+vsg_status build_queries(const vsg_frame *F, int n, const vsg_search_point *pts, const uint8_t *desc, float th, int lo,
+                         int hi, std::vector<AreaQuery> &qs, std::vector<int> &q_src, std::vector<uint8_t> &qdesc) {
+    qs.clear(); q_src.clear();
+    const vsg_status st = append_queries(F, n, pts, th, lo, hi, qs, q_src);
+    if (st != VSG_OK) return st;
     qdesc.resize(qs.size() * 32);
     for (size_t k = 0; k < qs.size(); ++k) memcpy(&qdesc[k * 32], desc + (size_t)q_src[k] * 32, 32);
     return VSG_OK;
@@ -225,6 +235,55 @@ vsg_status vsg_fuse_search(vsg_matcher *m, const vsg_frame *KF, int n, const vsg
         }
     }
     if (nfused_out) *nfused_out = nfused;
+    return VSG_OK;
+}
+
+// vsg_fuse_search(..., variant 0, ...) once per target keyframe, all targets in one upload, one launch and one download:
+// the searches of LocalMapping::SearchInNeighbors' loop of Fuse calls (LocalMapping.cc:764-802)
+vsg_status vsg_fuse_search_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *KFs, const float *const *inv_level_sigma2,
+                                 int n, const vsg_search_point *pts, const uint8_t *desc, float th, int32_t *best_idx_out) {
+    if (!m || ntargets < 0 || n < 0) {
+        set_error("vsg_fuse_search_multi: %d targets, %d points", ntargets, n);
+        return VSG_ERR_INVALID;
+    }
+    if (ntargets > 0 && (!KFs || !inv_level_sigma2 || (n > 0 && (!pts || !desc || !best_idx_out)))) {
+        set_error("vsg_fuse_search_multi: null target table, level table, points, descriptors or output");
+        return VSG_ERR_INVALID;
+    }
+    for (int t = 0; t < ntargets; ++t) {
+        if (!KFs[t] || !inv_level_sigma2[t]) {
+            set_error("vsg_fuse_search_multi: target %d: null keyframe or level table", t);
+            return VSG_ERR_INVALID;
+        }
+        if (KFs[t]->device != m->device) {
+            set_error("vsg_fuse_search_multi: target %d lives on device %d, the matcher on device %d", t, KFs[t]->device, m->device);
+            return VSG_ERR_INVALID;
+        }
+    }
+    CK(cudaSetDevice(m->device));
+    std::vector<AreaQuery> qs;
+    std::vector<int> q_src, q_tgt;
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_search_point *tp = pts + (size_t)t * n;
+        const size_t first = qs.size();
+        const vsg_status st = append_queries(KFs[t], n, tp, th, -1, 0, qs, q_src);      // :1246, :1270-1271
+        if (st != VSG_OK) {
+            const std::string why = vsg_last_error();
+            set_error("vsg_fuse_search_multi: target %d: %s", t, why.c_str());
+            return st;
+        }
+        for (size_t k = first; k < qs.size(); ++k) {
+            qs[k].xr = tp[q_src[k]].ur;                                                    // the chi-square gate's right coordinate
+            qs[k].desc_idx = q_src[k];                                                     // desc is shared by all targets
+        }
+        q_tgt.resize(qs.size(), t);
+    }
+    std::vector<int2> best;
+    vsg_status st = area_best_multi(m, ntargets, KFs, inv_level_sigma2, (int)qs.size(), qs.data(), q_tgt.data(), n, desc, best);
+    if (st != VSG_OK) return st;
+    for (size_t i = 0; i < (size_t)ntargets * n; ++i) best_idx_out[i] = -1;
+    for (size_t k = 0; k < qs.size(); ++k)
+        if (best[k].x >= 0 && best[k].y <= TH_LOW) best_idx_out[(size_t)q_tgt[k] * n + q_src[k]] = best[k].x;   // :1316
     return VSG_OK;
 }
 

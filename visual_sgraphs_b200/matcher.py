@@ -318,6 +318,23 @@ class ORBmatcher:
                                       int(bool(sim3_variant)), ptr(best), C.byref(nf)))
         return nf.value, best
 
+    def fuse_search_multi(self, kf_frames, inv_level_sigma2s, search_points, desc, th=3.0):
+        """FuseSearch (the pose-based variant) into every keyframe of kf_frames with one upload, one launch and one
+        download: search_points is [ntargets][n] (the points projected into each target), desc (n x 32) is shared, and
+        inv_level_sigma2s holds one table per target. Returns best_idx[ntargets][n]."""
+        T = len(kf_frames)
+        if len(inv_level_sigma2s) != T:
+            raise ValueError("fuse_search_multi: %d targets but %d level tables" % (T, len(inv_level_sigma2s)))
+        desc = np.ascontiguousarray(desc, np.uint8).reshape(-1, 32)
+        n = len(desc)
+        pts = np.ascontiguousarray(search_points, SEARCH_POINT_DTYPE).reshape(T, n)
+        sigs = [np.ascontiguousarray(s, np.float32) for s in inv_level_sigma2s]
+        frames = (C.c_void_p * max(T, 1))(*[f._h.value for f in kf_frames])
+        sig_ptrs = (C.c_void_p * max(T, 1))(*[s.ctypes.data for s in sigs])
+        best = np.zeros((T, n), np.int32)
+        check(self._L.vsg_fuse_search_multi(self._h, T, frames, sig_ptrs, n, ptr(pts), ptr(desc), float(th), ptr(best)))
+        return best
+
     def SearchBySim3(self, kf1_frame, kf2_frame, pts1, desc1, pts2, desc2, th):
         """ORBmatcher.cc:1448-1665 with both projections done by the caller. Returns (nFound, matches12[N1])."""
         pts1 = np.ascontiguousarray(pts1, SEARCH_POINT_DTYPE)

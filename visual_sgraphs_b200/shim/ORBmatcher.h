@@ -91,6 +91,10 @@ public:
     // Project MapPoints into a KeyFrame and search for duplicates (ORBmatcher.cc:1148-1335; bRight = false).
     template <class KeyFrameT, class MapPointT>
     int Fuse(KeyFrameT *pKF, const std::vector<MapPointT *> &vpMapPoints, const float th = 3.0, const bool bRight = false);
+    // LocalMapping::SearchInNeighbors' loop (LocalMapping.cc:764-802) in one call: for each target in order, Fuse(pKFi,
+    // vpMapPoints, th), then Fuse(pKFi, vpMapPoints, th, true) if pKFi->NLeft != -1.  Returns the sum of their counts.
+    template <class KeyFrameT, class MapPointT>
+    int Fuse(const std::vector<KeyFrameT *> &vpTargetKFs, const std::vector<MapPointT *> &vpMapPoints, const float th = 3.0);
 
 #ifdef SOPHUS_SIM3_HPP   // the Sim3 overloads need Sophus' own SE3/Sim3 arithmetic (include sophus/sim3.hpp first, as
                          // the reference's ORBmatcher.h does)
@@ -193,21 +197,27 @@ protected:
         v.scale_factors = out.scale.data();
         v.n_levels = (int)out.scale.size();
     }
-    struct FrameGuard {   // RAII for an uploaded frame; a frame that lives in the thread's cache is only borrowed
+    struct CacheEntry;
+    struct FrameGuard {   // RAII for an uploaded frame; a frame that lives in the thread's cache is only borrowed (and pinned)
         vsg_frame *h = nullptr;
         bool owned = true;
-        ~FrameGuard() { if (owned) vsg_frame_destroy(h); }
+        CacheEntry *pin = nullptr;
+        ~FrameGuard() {
+            if (pin) --pin->pins;
+            if (owned) vsg_frame_destroy(h);
+        }
     };
     // Uploaded frames are kept per calling thread: Tracking runs up to three projection searches on the same current frame,
     // LocalMapping / LoopClosing several on the same keyframe, and what the searches read from a Frame / KeyFrame (mvKeysUn,
     // mvKeys(Right), mDescriptors, mvuRight, the grid parameters) does not change after construction.  An entry is identified
     // by the object's address and type, its mnId (Frame.h:217, KeyFrame.h:312 — a recycled address gets a new id), which of its feature
     // lists was flattened, and the size / address of its descriptor matrix.  Types without mnId, and VSG_FRAME_CACHE=0, upload
-    // per call as before.
+    // per call as before.  An entry borrowed by a FrameGuard is pinned: a search that holds more frames than the cache has
+    // entries (the multi-target Fuse) uploads the extra ones for itself instead of evicting a frame it still reads.
     struct CacheEntry {
         const void *obj = nullptr, *desc = nullptr, *type = nullptr;
         unsigned long id = 0;
-        int kind = -1, n = 0;
+        int kind = -1, n = 0, pins = 0;
         unsigned long long stamp = 0;
         Flat flat;
         vsg_frame *h = nullptr;
@@ -239,27 +249,33 @@ protected:
             FrameCache &c = Cache();
             const void *desc = F.mDescriptors.rows > 0 ? (const void *)F.mDescriptors.ptr(0) : nullptr;
             const unsigned long id = FrameIdOf(F, 0);
-            CacheEntry *slot = &c.e[0];
+            CacheEntry *slot = nullptr;
             for (CacheEntry &x : c.e) {
                 if (x.h && x.obj == (const void *)&F && x.type == TypeKey<FrameT>() && x.id == id && x.kind == kind &&
                     x.n == F.mDescriptors.rows && x.desc == desc) {
                     x.stamp = ++c.clock;
                     ++c.hits;
+                    ++x.pins;
                     guard.h = x.h;
                     guard.owned = false;
+                    guard.pin = &x;
                     return x.flat;
                 }
-                if (x.stamp < slot->stamp) slot = &x;
+                if (!x.pins && (!slot || x.stamp < slot->stamp)) slot = &x;
             }
             ++c.misses;
-            vsg_frame_destroy(slot->h);
-            slot->h = nullptr;
-            fill(slot->flat);
-            Check(vsg_frame_create(Workspace(), &slot->flat.view, &slot->h), "vsg_frame_create");
-            slot->obj = &F; slot->type = TypeKey<FrameT>(); slot->id = id; slot->kind = kind; slot->n = F.mDescriptors.rows; slot->desc = desc; slot->stamp = ++c.clock;
-            guard.h = slot->h;
-            guard.owned = false;
-            return slot->flat;
+            if (slot) {
+                vsg_frame_destroy(slot->h);
+                slot->h = nullptr;
+                fill(slot->flat);
+                Check(vsg_frame_create(Workspace(), &slot->flat.view, &slot->h), "vsg_frame_create");
+                slot->obj = &F; slot->type = TypeKey<FrameT>(); slot->id = id; slot->kind = kind; slot->n = F.mDescriptors.rows; slot->desc = desc; slot->stamp = ++c.clock;
+                ++slot->pins;
+                guard.h = slot->h;
+                guard.owned = false;
+                guard.pin = slot;
+                return slot->flat;
+            }
         }
         fill(local);
         Check(vsg_frame_create(Workspace(), &local.view, &guard.h), "vsg_frame_create");
@@ -346,6 +362,15 @@ protected:
         if (nLeft != -1) FlattenCamera(F, false, nLeft, nullptr, out);
         else Flatten(F, out);
     }
+    // ---- Fuse(KF, vpMapPoints, th, bRight) (ORBmatcher.cc:1148-1335) in the parts the one-target and the multi-target Fuse
+    // share; defined below the class ----
+    template <class KeyFrameT>
+    static void UploadFuseTarget(KeyFrameT *pKF, bool bRight, Flat &local, FrameGuard &fr);
+    template <class KeyFrameT, class MapPointT>
+    static void ProjectForFuse(KeyFrameT *pKF, bool bRight, const std::vector<MapPointT *> &vpMapPoints, vsg_search_point *pts);
+    template <class KeyFrameT, class MapPointT, class OnReplace>
+    static int FuseReplay(KeyFrameT *pKF, bool bRight, const std::vector<MapPointT *> &vpMapPoints, const int32_t *best,
+                          OnReplace onReplace);
     template <class FrameT>
     static void RequireSingleCamera(const FrameT &F) {
         if (F.Nleft != -1)
@@ -633,36 +658,34 @@ int ORBmatcher::SearchByBoW(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<MapPoi
 }
 
 // ---- Fuse(KF, vpMapPoints, th) (ORBmatcher.cc:1148-1335) ----
-template <class KeyFrameT, class MapPointT>
-int ORBmatcher::Fuse(KeyFrameT *pKF, const std::vector<MapPointT *> &vpMapPoints, const float th, const bool bRight) {
+// The camera Fuse searches: two cameras -> mvKeys / mvKeysRight with their descriptor rows and grid
+// (KeyFrame::GetFeaturesInArea(..., bRight)); the stereo gate reads mvuRight[idx] with the camera-local index on both sides (:1266)
+template <class KeyFrameT>
+void ORBmatcher::UploadFuseTarget(KeyFrameT *pKF, bool bRight, Flat &local, FrameGuard &fr) {
     const bool bTwoCameras = pKF->NLeft != -1;
-    if (bRight && !bTwoCameras) throw std::runtime_error("vsg ORBmatcher::Fuse: bRight needs a two-camera keyframe");
-    Flat flatLocal;
-    FrameGuard fr;
-    // two cameras: the camera searched — mvKeys / mvKeysRight with their descriptor rows and grid (KeyFrame::GetFeaturesInArea(...,
-    // bRight)); the stereo gate reads mvuRight[idx] with the camera-local index on both sides (:1266)
-    const Flat &flat = Upload(*pKF, bTwoCameras ? 3 + (bRight ? 1 : 0) : 0, [&](Flat &o) {
+    Upload(*pKF, bTwoCameras ? 3 + (bRight ? 1 : 0) : 0, [&](Flat &o) {
         if (bTwoCameras) {
             const int n = (int)(bRight ? pKF->mvKeysRight : pKF->mvKeys).size();
             FlattenCamera(*pKF, bRight, pKF->NLeft, (int)pKF->mvuRight.size() >= n && n > 0 ? pKF->mvuRight.data() : nullptr, o);
         } else {
             Flatten(*pKF, o);
         }
-    }, flatLocal, fr);
+    }, local, fr);
+}
+
+// The projection of every map point into the camera (:1154-1244); pts[i].valid = the point reaches GetFeaturesInArea.
+template <class KeyFrameT, class MapPointT>
+void ORBmatcher::ProjectForFuse(KeyFrameT *pKF, bool bRight, const std::vector<MapPointT *> &vpMapPoints, vsg_search_point *pts) {
     const auto Tcw = bRight ? pKF->GetRightPose() : pKF->GetPose();                          // :1154-1165
     const auto Ow = bRight ? pKF->GetRightCameraCenter() : pKF->GetCameraCenter();
     auto *pCamera = bRight ? pKF->mpCamera2 : pKF->mpCamera;
-    const int idxOffset = bRight ? pKF->NLeft : 0;                                            // :1295-1296
     const float &bf = pKF->mbf;
-    const int nMPs = (int)vpMapPoints.size();
-    std::vector<vsg_search_point> pts(nMPs);
-    std::vector<uint8_t> desc((size_t)nMPs * 32, 0);
-    for (int i = 0; i < nMPs; ++i) {
+    for (size_t i = 0; i < vpMapPoints.size(); ++i) {
         vsg_search_point &p = pts[i];
         std::memset(&p, 0, sizeof(p));
         MapPointT *pMP = vpMapPoints[i];
         if (!pMP) continue;
-        // isBad() / IsInKeyFrame() change while the reference's loop runs: they are evaluated in the replay below,
+        // isBad() / IsInKeyFrame() change while the reference's loop runs: they are evaluated in the replay,
         // at the same point of the iteration order; the search itself does not depend on them.
         const auto p3Dw = pMP->GetWorldPos();
         const auto p3Dc = Tcw * p3Dw;
@@ -674,28 +697,123 @@ int ORBmatcher::Fuse(KeyFrameT *pKF, const std::vector<MapPointT *> &vpMapPoints
         if (!DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, true, p)) continue;
         p.u = uv(0); p.v = uv(1);
         p.valid = 1;
-        CopyDescriptor(pMP, desc, (size_t)i);
     }
-    std::vector<int32_t> best(nMPs, -1);
-    Check(vsg_fuse_search(Workspace(), fr.h, nMPs, pts.data(), desc.data(), th, pKF->mvInvLevelSigma2.data(), 0, best.data(),
-                          nullptr), "vsg_fuse_search");
+}
+
+// The bookkeeping of :1173-1332 in point order, from the searched camera's best keypoints (-1: none).  onReplace(survivor)
+// follows every Replace.
+template <class KeyFrameT, class MapPointT, class OnReplace>
+int ORBmatcher::FuseReplay(KeyFrameT *pKF, bool bRight, const std::vector<MapPointT *> &vpMapPoints, const int32_t *best,
+                           OnReplace onReplace) {
+    const int idxOffset = bRight ? pKF->NLeft : 0;                                            // :1295-1296
     int nFused = 0;
-    for (int i = 0; i < nMPs; ++i) {                                                        // :1173-1332 in order
+    for (size_t i = 0; i < vpMapPoints.size(); ++i) {
         MapPointT *pMP = vpMapPoints[i];
         if (!pMP || pMP->isBad() || pMP->IsInKeyFrame(pKF)) continue;
         if (best[i] < 0) continue;
-        best[i] += idxOffset;
-        MapPointT *pMPinKF = pKF->GetMapPoint(best[i]);
+        const int idx = best[i] + idxOffset;
+        MapPointT *pMPinKF = pKF->GetMapPoint(idx);
         if (pMPinKF) {
             if (!pMPinKF->isBad()) {
-                if (pMPinKF->Observations() > pMP->Observations()) pMP->Replace(pMPinKF);
-                else pMPinKF->Replace(pMP);
+                if (pMPinKF->Observations() > pMP->Observations()) { pMP->Replace(pMPinKF); onReplace(pMPinKF); }
+                else { pMPinKF->Replace(pMP); onReplace(pMP); }
             }
         } else {
-            pMP->AddObservation(pKF, best[i]);
-            pKF->AddMapPoint(pMP, best[i]);
+            pMP->AddObservation(pKF, idx);
+            pKF->AddMapPoint(pMP, idx);
         }
         nFused++;
+    }
+    return nFused;
+}
+
+template <class KeyFrameT, class MapPointT>
+int ORBmatcher::Fuse(KeyFrameT *pKF, const std::vector<MapPointT *> &vpMapPoints, const float th, const bool bRight) {
+    if (bRight && pKF->NLeft == -1) throw std::runtime_error("vsg ORBmatcher::Fuse: bRight needs a two-camera keyframe");
+    Flat flatLocal;
+    FrameGuard fr;
+    UploadFuseTarget(pKF, bRight, flatLocal, fr);
+    const int nMPs = (int)vpMapPoints.size();
+    std::vector<vsg_search_point> pts(nMPs);
+    ProjectForFuse(pKF, bRight, vpMapPoints, pts.data());
+    std::vector<uint8_t> desc((size_t)nMPs * 32, 0);
+    for (int i = 0; i < nMPs; ++i)
+        if (pts[i].valid) CopyDescriptor(vpMapPoints[i], desc, (size_t)i);
+    std::vector<int32_t> best(nMPs, -1);
+    Check(vsg_fuse_search(Workspace(), fr.h, nMPs, pts.data(), desc.data(), th, pKF->mvInvLevelSigma2.data(), 0, best.data(),
+                          nullptr), "vsg_fuse_search");
+    return FuseReplay(pKF, bRight, vpMapPoints, best.data(), [](MapPointT *) {});
+}
+
+template <class KeyFrameT, class MapPointT>
+int ORBmatcher::Fuse(const std::vector<KeyFrameT *> &vpTargetKFs, const std::vector<MapPointT *> &vpMapPoints, const float th) {
+    std::vector<std::pair<KeyFrameT *, bool>> targets;                                        // (keyframe, bRight) in loop order
+    for (KeyFrameT *pKF : vpTargetKFs) {
+        targets.emplace_back(pKF, false);
+        if (pKF->NLeft != -1) targets.emplace_back(pKF, true);
+    }
+    const int T = (int)targets.size(), n = (int)vpMapPoints.size();
+    if (T == 0) return 0;
+    std::vector<Flat> local(T);
+    std::vector<FrameGuard> fr(T);
+    std::vector<const vsg_frame *> frames(T);
+    std::vector<const float *> sigma(T);
+    std::vector<vsg_search_point> pts((size_t)T * n);
+    std::vector<uint8_t> searched(n, 0), desc((size_t)n * 32, 0);
+    for (int t = 0; t < T; ++t) {
+        KeyFrameT *pKF = targets[t].first;
+        UploadFuseTarget(pKF, targets[t].second, local[t], fr[t]);
+        frames[t] = fr[t].h;
+        sigma[t] = pKF->mvInvLevelSigma2.data();
+        ProjectForFuse(pKF, targets[t].second, vpMapPoints, &pts[(size_t)t * n]);
+        for (int i = 0; i < n; ++i) searched[i] |= pts[(size_t)t * n + i].valid;
+    }
+    for (int i = 0; i < n; ++i)
+        if (searched[i]) CopyDescriptor(vpMapPoints[i], desc, (size_t)i);
+    std::vector<int32_t> best((size_t)T * n, -1);
+    Check(vsg_fuse_search_multi(Workspace(), T, frames.data(), sigma.data(), n, pts.data(), desc.data(), th, best.data()),
+          "vsg_fuse_search_multi");
+    // Stale descriptors.  The loop searches target t with the descriptors the map points have when Fuse(target t) starts, and
+    // MapPoint::Replace ends with the survivor's ComputeDistinctiveDescriptors(): a survivor that is one of vpMapPoints may
+    // enter the later targets with a new descriptor and pick another keypoint there.  So after each target's replay, every
+    // query that survived a Replace is compared with its uploaded row; the ones that changed are searched again, with the
+    // new rows, in all later targets (one more call), before the next target is replayed.
+    std::vector<std::pair<MapPointT *, int>> queryOf;                                         // map point -> its query indices
+    for (int i = 0; i < n; ++i)
+        if (searched[i]) queryOf.emplace_back(vpMapPoints[i], i);
+    std::sort(queryOf.begin(), queryOf.end());
+    std::vector<int> survivors, stale;
+    auto onReplace = [&](MapPointT *pSurvivor) {
+        auto it = std::lower_bound(queryOf.begin(), queryOf.end(), std::make_pair(pSurvivor, 0));
+        for (; it != queryOf.end() && it->first == pSurvivor; ++it) survivors.push_back(it->second);
+    };
+    int nFused = 0;
+    for (int t = 0; t < T; ++t) {
+        nFused += FuseReplay(targets[t].first, targets[t].second, vpMapPoints, &best[(size_t)t * n], onReplace);
+        if (t + 1 == T || survivors.empty()) continue;
+        std::sort(survivors.begin(), survivors.end());
+        survivors.erase(std::unique(survivors.begin(), survivors.end()), survivors.end());
+        stale.clear();
+        for (int i : survivors) {
+            const cv::Mat d = vpMapPoints[i]->GetDescriptor();
+            if (std::memcmp(d.ptr(0), &desc[(size_t)i * 32], 32) == 0) continue;
+            std::memcpy(&desc[(size_t)i * 32], d.ptr(0), 32);
+            stale.push_back(i);
+        }
+        survivors.clear();
+        if (stale.empty()) continue;
+        const int R = T - t - 1, ns = (int)stale.size();
+        std::vector<vsg_search_point> rpts((size_t)R * ns);
+        std::vector<uint8_t> rdesc((size_t)ns * 32);
+        for (int j = 0; j < ns; ++j) {
+            std::memcpy(&rdesc[(size_t)j * 32], &desc[(size_t)stale[j] * 32], 32);
+            for (int r = 0; r < R; ++r) rpts[(size_t)r * ns + j] = pts[(size_t)(t + 1 + r) * n + stale[j]];
+        }
+        std::vector<int32_t> rbest((size_t)R * ns);
+        Check(vsg_fuse_search_multi(Workspace(), R, frames.data() + t + 1, sigma.data() + t + 1, ns, rpts.data(), rdesc.data(), th,
+                                    rbest.data()), "vsg_fuse_search_multi");
+        for (int r = 0; r < R; ++r)
+            for (int j = 0; j < ns; ++j) best[(size_t)(t + 1 + r) * n + stale[j]] = rbest[(size_t)r * ns + j];
     }
     return nFused;
 }
