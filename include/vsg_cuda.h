@@ -373,6 +373,26 @@ vsg_status vsg_search_by_bow_2cam(vsg_matcher *m, const vsg_frame_view *KF, cons
                                   const int32_t *f_ptr, const int32_t *f_idx, float nnratio, int check_ori,
                                   int32_t *matches_f_out, int *nmatches_out);
 
+/* One side of a BoW search: a frame or keyframe view, its map-point flags (mp_valid[i] = map point i present and not bad;
+ * not read for the frame of vsg_search_by_bow_multi) and its DBoW2::FeatureVector as the node ids / CSR lists the
+ * single-target calls take. */
+typedef struct vsg_bow_side {
+    vsg_frame_view view;
+    const uint8_t *mp_valid;
+    int32_t nnodes;
+    const int32_t *nodes, *ptr, *idx;
+} vsg_bow_side;
+
+/* Tracking::Relocalization's loop `for (i : candidates) matcher.SearchByBoW(pKF_i, mCurrentFrame, vvpMapPointMatches[i])`
+ * (Tracking.cc:3687-3854) in one call: for every t < ntargets, vsg_search_by_bow_2cam(m, &KFs[t]->view, KFs[t]->mp_valid,
+ * &F->view, f_nleft, <KFs[t]'s feature vector>, <F's feature vector>, nnratio, check_ori, matches_f_out + t * F->view.n,
+ * &nmatches_out[t]), with one upload, one kernel launch (none if no target shares a node with F) and one download.  F is
+ * shared by all targets; the same keyframe may appear more than once.  ntargets == 0 does nothing.  A null or malformed
+ * target, or a feature index out of range, returns VSG_ERR_INVALID before anything is launched, and vsg_last_error names
+ * the target. */
+vsg_status vsg_search_by_bow_multi(vsg_matcher *m, int ntargets, const vsg_bow_side *const *KFs, const vsg_bow_side *F,
+                                   int f_nleft, float nnratio, int check_ori, int32_t *matches_f_out, int *nmatches_out);
+
 /* A map point already projected into the searched Frame / KeyFrame by the caller: the pose, Sim3 and
  * camera-model arithmetic ahead of GetFeaturesInArea (e.g. ORBmatcher.cc:444-486, 1182-1238, 1904-1929) stays
  * with the reference's Sophus / GeometricCamera classes; everything from the window query on runs here. */
@@ -438,6 +458,14 @@ vsg_status vsg_search_by_bow_kf(vsg_matcher *m, const vsg_frame_view *KF1, const
                                 const int32_t *nodes1, const int32_t *ptr1, const int32_t *idx1, int nnodes2,
                                 const int32_t *nodes2, const int32_t *ptr2, const int32_t *idx2, float nnratio,
                                 int check_ori, int32_t *matches12_out, int *nmatches_out);
+
+/* LoopClosing::DetectCommonRegionsFromBoW's loop `for (j : vpCovKFi) matcherBoW.SearchByBoW(mpCurrentKF, vpCovKFi[j],
+ * vvpMatchedMPs[j])` (LoopClosing.cc:573-642) in one call: for every t < ntargets, vsg_search_by_bow_kf(m, &KF1->view,
+ * KF1->mp_valid, &KF2s[t]->view, KF2s[t]->mp_valid, <KF1's feature vector>, <KF2s[t]'s feature vector>, nnratio, check_ori,
+ * matches12_out + t * KF1->view.n, &nmatches_out[t]), with one upload, one kernel launch (none if no target shares a node with
+ * KF1) and one download.  KF1 is shared by all targets.  Argument rules as vsg_search_by_bow_multi. */
+vsg_status vsg_search_by_bow_kf_multi(vsg_matcher *m, const vsg_bow_side *KF1, int ntargets, const vsg_bow_side *const *KF2s,
+                                      float nnratio, int check_ori, int32_t *matches12_out, int *nmatches_out);
 
 /* The Hamming-distance half of the BoW-guided pairings, for callers that own the per-pair geometry test — two-camera
  * SearchForTriangulation (ORBmatcher.cc:902-1146 with mpCamera2 != NULL), where the epipolar test is the caller's

@@ -36,6 +36,12 @@ class FrameView(C.Structure):
                 ("grid_rows", C.c_int32), ("scale_factors", C.c_void_p), ("n_levels", C.c_int32)]
 
 
+class BowSide(C.Structure):
+    """vsg_bow_side (include/vsg_cuda.h): a view, its map-point flags and its flattened FeatureVector."""
+    _fields_ = [("view", FrameView), ("mp_valid", C.c_void_p), ("nnodes", C.c_int32), ("nodes", C.c_void_p),
+                ("ptr", C.c_void_p), ("idx", C.c_void_p)]
+
+
 TRACK_POINT_DTYPE = np.dtype([("proj_x", "<f4"), ("proj_y", "<f4"), ("proj_xr", "<f4"), ("view_cos", "<f4"),
                               ("depth", "<f4"), ("level", "<i4"), ("in_view", "u1"), ("bad", "u1"), ("blocks", "u1"),
                               ("pad", "u1")])
@@ -127,6 +133,8 @@ _SIGNATURES = {
     "vsg_search_by_bow_2cam": (C.c_int, [C.c_void_p, C.POINTER(FrameView), C.c_void_p, C.POINTER(FrameView), C.c_int, C.c_int,
                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_float, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
+    "vsg_search_by_bow_multi": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(BowSide), C.c_int, C.c_float, C.c_int,
+                                          C.c_void_p, C.c_void_p]),
     "vsg_search_by_projection_reloc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                                  C.c_float, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
     "vsg_search_by_projection_sim3": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
@@ -140,6 +148,8 @@ _SIGNATURES = {
     "vsg_search_by_bow_kf": (C.c_int, [C.c_void_p, C.POINTER(FrameView), C.c_void_p, C.POINTER(FrameView), C.c_void_p,
                                        C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_float, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
+    "vsg_search_by_bow_kf_multi": (C.c_int, [C.c_void_p, C.POINTER(BowSide), C.c_int, C.c_void_p, C.c_float, C.c_int,
+                                             C.c_void_p, C.c_void_p]),
     "vsg_bow_pair_distances": (C.c_int, [C.c_void_p, C.POINTER(FrameView), C.c_void_p, C.POINTER(FrameView), C.c_int, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int),

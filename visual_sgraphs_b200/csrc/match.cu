@@ -179,7 +179,7 @@ __global__ void window_match_kernel(const uint4 *__restrict__ query, int nq, con
                                     const uint8_t *__restrict__ skip, const int *__restrict__ train_level,
                                     int init_dist, int *__restrict__ best_idx, int *__restrict__ best_dist,
                                     int *__restrict__ second_dist, int *__restrict__ best_level,
-                                    int *__restrict__ second_level, int *__restrict__ all_dist) {
+                                    int *__restrict__ second_level) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= nq) return;
     const uint4 qa = __ldg(query + 2 * q), qb = __ldg(query + 2 * q + 1);
@@ -188,7 +188,6 @@ __global__ void window_match_kernel(const uint4 *__restrict__ query, int nq, con
     for (int c = cand_ptr[q]; c < e; ++c) {
         const int j = cand[c];
         const int d = hamming256(qa, qb, __ldg(train + 2 * j), __ldg(train + 2 * j + 1));
-        if (all_dist) all_dist[c] = d;
         if (skip && skip[j]) continue;
         const int lvl = train_level ? train_level[j] : -1;
         if (d < bd) { bd2 = bd; bd = d; bl2 = bl; bl = lvl; bi = j; }
@@ -201,12 +200,33 @@ __global__ void window_match_kernel(const uint4 *__restrict__ query, int nq, con
     if (second_level) second_level[q] = bl2;
 }
 
-void launch_window_dists(vsg_matcher *m, const uint8_t *query_dev, int nq, const uint8_t *train_dev,
-                         const int *cand_ptr_dev, const int *cand_dev, int *all_dist_dev) {
-    if (nq <= 0) return;
-    window_match_kernel<<<(nq + 127) / 128, 128, 0, m->stream>>>((const uint4 *)query_dev, nq, (const uint4 *)train_dev,
-                                                                cand_ptr_dev, cand_dev, nullptr, nullptr, 256, nullptr,
-                                                                nullptr, nullptr, nullptr, nullptr, all_dist_dev);
+// ------------------------------------------------------------------------------------------------
+// BoW in-node distances: one thread per (segment, candidate) pair of every merge walk of a call.  Segment s = (query
+// descriptor row, first candidate in the uploaded FeatureVector idx arrays, the candidate side's first descriptor row,
+// first output slot); the segments are sorted by output slot and end with a sentinel whose slot is npairs.  A thread
+// finds its segment by binary search over the slots and writes its distance in walk order (0..256 fits 16 bits).
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) bow_dists_multi_kernel(const int4 *__restrict__ segs, int nseg, const int *__restrict__ idx,
+                                                              const uint4 *__restrict__ desc, int npairs,
+                                                              unsigned short *__restrict__ out) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npairs) return;
+    int lo = 0, hi = nseg - 1;                           // last segment whose first slot is <= p
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(&segs[mid].w) <= p) lo = mid;
+        else hi = mid - 1;
+    }
+    const int4 s = __ldg(segs + lo);
+    const int j = s.z + __ldg(idx + s.y + (p - s.w));
+    out[p] = (unsigned short)hamming256(__ldg(desc + 2 * s.x), __ldg(desc + 2 * s.x + 1), __ldg(desc + 2 * j), __ldg(desc + 2 * j + 1));
+}
+
+void launch_bow_dists(vsg_matcher *m, const int4 *segs_dev, int nseg, const int *idx_dev, const uint8_t *desc_dev, int npairs,
+                      uint16_t *out_dev) {
+    if (npairs <= 0) return;
+    bow_dists_multi_kernel<<<(npairs + 255) / 256, 256, 0, m->stream>>>(segs_dev, nseg, idx_dev, (const uint4 *)desc_dev, npairs,
+                                                                        out_dev);
     count_launch();
 }
 
@@ -412,7 +432,7 @@ vsg_status vsg_match_window(vsg_matcher *m, const uint8_t *query, int nq, const 
     window_match_kernel<<<(nq + 127) / 128, 128, 0, s>>>((const uint4 *)m->buf[1], nq, (const uint4 *)m->buf[2],
                                                         (const int *)m->buf[3], (const int *)m->buf[4],
                                                         skip ? skip_dev : nullptr, train_level ? lvl_dev : nullptr,
-                                                        init_dist, o, o + nq, o + 2 * nq, o + 3 * nq, o + 4 * nq, nullptr);
+                                                        init_dist, o, o + nq, o + 2 * nq, o + 3 * nq, o + 4 * nq);
     count_launch();
     CK(cudaGetLastError());
     int32_t *outs[5] = {best_idx, best_dist, second_dist, best_level, second_level};

@@ -79,6 +79,35 @@ vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const 
                            const AreaQuery *qs, const int *q_target, int n_qdesc, const uint8_t *qdesc, std::vector<int2> &out);
 vsg_status area_search_raw(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc,
                            int n_qdesc, AreaLists *out);
+// ---- BoW-guided pairings (SearchByBoW x 2, SearchForTriangulation; match_methods_kf.cu) ----
+struct FeatVec {             // a flattened DBoW2::FeatureVector: node ids ascending, node k's features idx[ptr[k] .. ptr[k+1])
+    int nnodes;
+    const int32_t *nodes, *ptr, *idx;
+};
+// One merge walk over two FeatureVectors (e.g. ORBmatcher.cc:785-872): every feature i1 of side 1 with use1[i1] != 0 inside
+// a node both vectors share is a query whose candidates are ALL features of that node on side 2.
+struct BowWalk {
+    const vsg_frame_view *v1;
+    const uint8_t *use1;
+    FeatVec a;
+    const vsg_frame_view *v2;
+    FeatVec b;
+};
+// A query of a walk: feature i1 of side 1, its candidates b.idx[jb .. je) in the reference's scan order, their distances
+// dist[off .. off + je - jb).
+struct BowSeg {
+    int i1, jb, je, off;
+};
+bool featvec_ok(int nn, const int32_t *nodes, const int32_t *ptr, const int32_t *idx);
+// Appends the queries of one walk to segs, output slots continuing from *npairs; rejects feature indices out of range.
+vsg_status bow_walk(const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs);
+// The distances of every in-node pair of the walks: one copy in (segments, every distinct descriptor table once, every
+// distinct side-2 idx array once), one launch of bow_dists_multi_kernel (none if npairs == 0), one copy out.  segs[seg_ptr[k]
+// .. seg_ptr[k+1]) are walk k's.  *dist points into the matcher's pinned staging and stays valid until its next BoW call.
+vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std::vector<BowSeg> &segs, const int *seg_ptr,
+                     int64_t npairs, const uint16_t **dist);
+// What is wrong with one side of a multi-target BoW call (nullptr: nothing); the map-point flags only if it needs them.
+const char *bow_side_problem(const vsg_bow_side *s, bool needs_valid);
 // ORBmatcher::ComputeThreeMaxima (ORBmatcher.cc:2002-2043)
 void three_maxima(const std::vector<int> *hist, int L, int &ind1, int &ind2, int &ind3);
 // rotation-histogram bin (ORBmatcher.cc:351-358)

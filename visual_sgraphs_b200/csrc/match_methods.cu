@@ -21,6 +21,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cmath>
+#include <string>
 #include <vector>
 
 #include "match_internal.cuh"
@@ -499,6 +500,55 @@ int rot_bin(float a1, float a2) {   // :351-358 — factor is 1/HISTO_LENGTH, C 
     int bin = (int)std::round(rot * factor);
     if (bin == HISTO_LENGTH) bin = 0;
     return bin;
+}
+
+// The KF-F replay of SearchByBoW (ORBmatcher.cc:256-392) over one walk's distances: frame features matched by an earlier
+// keyframe feature skipped (:282-283, :303-304), best / second best per camera (:298-322), TH_LOW and ratio gates (the right
+// camera's inside the left one's TH_LOW block with its ratio test disabled, :362-366), rotation histogram.  Returns nmatches.
+static int bow_replay_kf_f(const vsg_frame_view *KF, const vsg_frame_view *F, int f_nleft, const FeatVec &fb, const BowSeg *segs,
+                           int nseg, const uint16_t *dist, float nnratio, int check_ori, int32_t *matches_f_out) {
+    for (int i = 0; i < F->n; ++i) matches_f_out[i] = -1;
+    std::vector<int> rot_hist[HISTO_LENGTH];
+    int nmatches = 0;
+    const int nleft = f_nleft < 0 ? F->n : f_nleft;                  // single camera: every feature is a "left" one
+    for (int k = 0; k < nseg; ++k) {
+        const BowSeg &sg = segs[k];
+        int best1 = 256, best_idx_f = -1, best2 = 256;
+        int best1r = 256, best_idx_fr = -1, best2r = 256;
+        for (int j = sg.jb; j < sg.je; ++j) {
+            const int real_f = fb.idx[j];
+            if (matches_f_out[real_f] >= 0) continue;                // :282-283, :303-304
+            const int d = dist[sg.off + j - sg.jb];
+            if (real_f < nleft) {
+                if (d < best1) { best2 = best1; best1 = d; best_idx_f = real_f; }
+                else if (d < best2) best2 = d;
+            } else {
+                if (d < best1r) { best2r = best1r; best1r = d; best_idx_fr = real_f; }
+                else if (d < best2r) best2r = d;
+            }
+        }
+        if (best1 <= TH_LOW) {
+            if (static_cast<float>(best1) < nnratio * static_cast<float>(best2)) {
+                matches_f_out[best_idx_f] = sg.i1;
+                if (check_ori) rot_hist[rot_bin(KF->keys[sg.i1].angle, F->keys[best_idx_f].angle)].push_back(best_idx_f);
+                ++nmatches;
+            }
+            if (best1r <= TH_LOW) {                                  // ratio test `|| true` (:366)
+                matches_f_out[best_idx_fr] = sg.i1;
+                if (check_ori) rot_hist[rot_bin(KF->keys[sg.i1].angle, F->keys[best_idx_fr].angle)].push_back(best_idx_fr);
+                ++nmatches;
+            }
+        }
+    }
+    if (check_ori) {
+        int ind1 = -1, ind2 = -1, ind3 = -1;
+        three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
+        for (int i = 0; i < HISTO_LENGTH; ++i) {
+            if (i == ind1 || i == ind2 || i == ind3) continue;
+            for (int idx : rot_hist[i]) { matches_f_out[idx] = -1; --nmatches; }
+        }
+    }
+    return nmatches;
 }
 
 }  // namespace vsg
@@ -1240,90 +1290,67 @@ vsg_status vsg_search_by_bow_2cam(vsg_matcher *m, const vsg_frame_view *KF, cons
     CK(cudaSetDevice(m->device));
     // the merge walk over the two FeatureVectors (:248-376): one query per keyframe feature with a usable map
     // point inside a common node; its candidates are the frame features of that node, in vIndicesF order
-    std::vector<int> q_kf, cptr(1, 0), cand;
-    int a = 0, b = 0;
-    while (a < kf_nnodes && b < f_nnodes) {
-        if (kf_nodes[a] == f_nodes[b]) {
-            for (int ik = kf_ptr[a]; ik < kf_ptr[a + 1]; ++ik) {
-                const int real_kf = kf_idx[ik];
-                if (real_kf < 0 || real_kf >= KF->n) { set_error("bow: keyframe index out of range"); return VSG_ERR_INVALID; }
-                if (!kf_mp_valid[real_kf]) continue;
-                q_kf.push_back(real_kf);
-                for (int jf = f_ptr[b]; jf < f_ptr[b + 1]; ++jf) {
-                    if (f_idx[jf] < 0 || f_idx[jf] >= F->n) { set_error("bow: frame index out of range"); return VSG_ERR_INVALID; }
-                    cand.push_back(f_idx[jf]);
-                }
-                cptr.push_back((int)cand.size());
-            }
-            ++a; ++b;
-        } else if (kf_nodes[a] < f_nodes[b]) {
-            while (a < kf_nnodes && kf_nodes[a] < f_nodes[b]) ++a;
-        } else {
-            while (b < f_nnodes && f_nodes[b] < kf_nodes[a]) ++b;
-        }
-    }
-    const int nq = (int)q_kf.size(), ncand = (int)cand.size();
-    std::vector<int> dist(ncand);
-    if (nq > 0 && ncand > 0) {
-        std::vector<uint8_t> qdesc((size_t)nq * 32);
-        for (int k = 0; k < nq; ++k) memcpy(&qdesc[(size_t)k * 32], KF->descriptors + (size_t)q_kf[k] * 32, 32);
-        vsg_status st;
-        if ((st = matcher_ensure(m, 1, (size_t)nq * 32)) || (st = matcher_ensure(m, 2, (size_t)std::max(F->n, 1) * 32)) ||
-            (st = matcher_ensure(m, 3, (size_t)(nq + 1) * 4)) || (st = matcher_ensure(m, 4, (size_t)ncand * 4)) ||
-            (st = matcher_ensure(m, 6, (size_t)ncand * 4)))
-            return st;
-        cudaStream_t s = m->stream;
-        CK(cudaMemcpyAsync(m->buf[1], qdesc.data(), (size_t)nq * 32, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(m->buf[2], F->descriptors, (size_t)F->n * 32, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(m->buf[3], cptr.data(), (size_t)(nq + 1) * 4, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(m->buf[4], cand.data(), (size_t)ncand * 4, cudaMemcpyHostToDevice, s));
-        launch_window_dists(m, (const uint8_t *)m->buf[1], nq, (const uint8_t *)m->buf[2], (const int *)m->buf[3],
-                            (const int *)m->buf[4], (int *)m->buf[6]);
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(dist.data(), m->buf[6], (size_t)ncand * 4, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    for (int i = 0; i < F->n; ++i) matches_f_out[i] = -1;
-    std::vector<int> rot_hist[HISTO_LENGTH];
-    int nmatches = 0;
-    const int nleft = f_nleft < 0 ? F->n : f_nleft;                  // single camera: every feature is a "left" one
-    for (int k = 0; k < nq; ++k) {                                   // :256-392 with the distances looked up
-        int best1 = 256, best_idx_f = -1, best2 = 256;
-        int best1r = 256, best_idx_fr = -1, best2r = 256;
-        for (int c = cptr[k]; c < cptr[k + 1]; ++c) {
-            const int real_f = cand[c];
-            if (matches_f_out[real_f] >= 0) continue;                // :282-283, :303-304
-            const int d = dist[c];
-            if (real_f < nleft) {
-                if (d < best1) { best2 = best1; best1 = d; best_idx_f = real_f; }
-                else if (d < best2) best2 = d;
-            } else {
-                if (d < best1r) { best2r = best1r; best1r = d; best_idx_fr = real_f; }
-                else if (d < best2r) best2r = d;
-            }
-        }
-        if (best1 <= TH_LOW) {
-            if (static_cast<float>(best1) < nnratio * static_cast<float>(best2)) {
-                matches_f_out[best_idx_f] = q_kf[k];
-                if (check_ori) rot_hist[rot_bin(KF->keys[q_kf[k]].angle, F->keys[best_idx_f].angle)].push_back(best_idx_f);
-                ++nmatches;
-            }
-            if (best1r <= TH_LOW) {                                  // ratio test `|| true` (:366)
-                matches_f_out[best_idx_fr] = q_kf[k];
-                if (check_ori) rot_hist[rot_bin(KF->keys[q_kf[k]].angle, F->keys[best_idx_fr].angle)].push_back(best_idx_fr);
-                ++nmatches;
-            }
-        }
-    }
-    if (check_ori) {
-        int ind1 = -1, ind2 = -1, ind3 = -1;
-        three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
-        for (int i = 0; i < HISTO_LENGTH; ++i) {
-            if (i == ind1 || i == ind2 || i == ind3) continue;
-            for (int idx : rot_hist[i]) { matches_f_out[idx] = -1; --nmatches; }
-        }
-    }
+    const BowWalk w{KF, kf_mp_valid, FeatVec{kf_nnodes, kf_nodes, kf_ptr, kf_idx}, F, FeatVec{f_nnodes, f_nodes, f_ptr, f_idx}};
+    std::vector<BowSeg> segs;
+    int64_t npairs = 0;
+    const uint16_t *dist;
+    vsg_status st = bow_walk(w, segs, &npairs);
+    const int seg_ptr[2] = {0, (int)segs.size()};
+    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
+    const int nmatches = bow_replay_kf_f(KF, F, f_nleft, w.b, segs.data(), (int)segs.size(), dist, nnratio, check_ori, matches_f_out);
     if (nmatches_out) *nmatches_out = nmatches;
+    return VSG_OK;
+}
+
+// vsg_search_by_bow_2cam(KFs[t] against F) for every target in one upload, one launch and one download
+vsg_status vsg_search_by_bow_multi(vsg_matcher *m, int ntargets, const vsg_bow_side *const *KFs, const vsg_bow_side *F,
+                                   int f_nleft, float nnratio, int check_ori, int32_t *matches_f_out, int *nmatches_out) {
+    if (!m || ntargets < 0) {
+        set_error("vsg_search_by_bow_multi: %d targets", ntargets);
+        return VSG_ERR_INVALID;
+    }
+    if (ntargets == 0) return VSG_OK;
+    const char *why;
+    if (!KFs || !nmatches_out || (F && F->view.n > 0 && !matches_f_out)) {
+        set_error("vsg_search_by_bow_multi: null target table or output");
+        return VSG_ERR_INVALID;
+    }
+    if ((why = bow_side_problem(F, false))) {
+        set_error("vsg_search_by_bow_multi: F: %s", why);
+        return VSG_ERR_INVALID;
+    }
+    if (f_nleft < -1 || f_nleft > F->view.n) {
+        set_error("vsg_search_by_bow_multi: f_nleft %d outside [-1, %d]", f_nleft, F->view.n);
+        return VSG_ERR_INVALID;
+    }
+    for (int t = 0; t < ntargets; ++t)
+        if ((why = bow_side_problem(KFs[t], true))) {
+            set_error("vsg_search_by_bow_multi: target %d: %s", t, why);
+            return VSG_ERR_INVALID;
+        }
+    CK(cudaSetDevice(m->device));
+    std::vector<BowWalk> walks;
+    std::vector<BowSeg> segs;
+    std::vector<int> seg_ptr(1, 0);
+    int64_t npairs = 0;
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_bow_side &a = *KFs[t];
+        walks.push_back(BowWalk{&a.view, a.mp_valid, FeatVec{a.nnodes, a.nodes, a.ptr, a.idx}, &F->view,
+                                FeatVec{F->nnodes, F->nodes, F->ptr, F->idx}});
+        if (bow_walk(walks.back(), segs, &npairs) != VSG_OK) {
+            const std::string err = vsg_last_error();
+            set_error("vsg_search_by_bow_multi: target %d: %s", t, err.c_str());
+            return VSG_ERR_INVALID;
+        }
+        seg_ptr.push_back((int)segs.size());
+    }
+    const uint16_t *dist;
+    vsg_status st = bow_dists(m, ntargets, walks.data(), segs, seg_ptr.data(), npairs, &dist);
+    if (st != VSG_OK) return st;
+    for (int t = 0; t < ntargets; ++t)                                               // in target order, as the loop runs
+        nmatches_out[t] = bow_replay_kf_f(&KFs[t]->view, &F->view, f_nleft, walks[t].b, segs.data() + seg_ptr[t],
+                                          seg_ptr[t + 1] - seg_ptr[t], dist, nnratio, check_ori,
+                                          matches_f_out + (size_t)t * F->view.n);
     return VSG_OK;
 }
 

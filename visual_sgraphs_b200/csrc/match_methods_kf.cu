@@ -13,8 +13,8 @@
 //   Pinhole::epipolarConstrain                                                    orb_slam3/src/CameraModels/Pinhole.cpp:118-141
 //
 // Same split of work as match_methods.cu: the GPU answers every window query of a call at once (grid walk +
-// 256-bit Hamming distance of each candidate: area_search_kernel), or every in-node descriptor pair of a BoW
-// walk (window_match_kernel); the order-dependent bookkeeping is replayed on the host over those lists.
+// 256-bit Hamming distance of each candidate: area_search_kernel), or every in-node descriptor pair of the BoW
+// walks of a call (bow_dists_multi_kernel); the order-dependent bookkeeping is replayed on the host over those lists.
 // KeyFrame::GetFeaturesInArea is Frame::GetFeaturesInArea without the level filter; the callers' per-candidate
 // level gate (kpLevel < nPredictedLevel-1 || kpLevel > nPredictedLevel) is the same filter applied later, so it
 // is folded into the query (min_level = level-1, max_level = level >= 0, which always enables the check).
@@ -60,67 +60,6 @@ vsg_status build_queries(const vsg_frame *F, int n, const vsg_search_point *pts,
     return VSG_OK;
 }
 
-struct FeatVec {
-    int nnodes;
-    const int32_t *nodes, *ptr, *idx;
-};
-
-// The merge walk over two DBoW2::FeatureVectors (e.g. :785-872): for every feature of vector 1 that passes
-// `use1`, inside a node both vectors share, one query whose candidates are ALL features of that node in vector 2
-// (in vIndices order; per-candidate gates are applied in the replay).  Distances come from the GPU.
-template <class Use1>
-vsg_status bow_pair_dists(vsg_matcher *m, const vsg_frame_view *V1, const vsg_frame_view *V2, const FeatVec &a,
-                          const FeatVec &b, Use1 use1, std::vector<int> &q1, std::vector<int> &cptr,
-                          std::vector<int> &cand, std::vector<int> &dist) {
-    q1.clear(); cand.clear(); cptr.assign(1, 0);
-    int ia = 0, ib = 0;
-    while (ia < a.nnodes && ib < b.nnodes) {
-        if (a.nodes[ia] == b.nodes[ib]) {
-            for (int k = a.ptr[ia]; k < a.ptr[ia + 1]; ++k) {
-                const int i1 = a.idx[k];
-                if (i1 < 0 || i1 >= V1->n) { set_error("bow: feature index out of range"); return VSG_ERR_INVALID; }
-                if (!use1(i1)) continue;
-                q1.push_back(i1);
-                for (int j = b.ptr[ib]; j < b.ptr[ib + 1]; ++j) {
-                    if (b.idx[j] < 0 || b.idx[j] >= V2->n) { set_error("bow: feature index out of range"); return VSG_ERR_INVALID; }
-                    cand.push_back(b.idx[j]);
-                }
-                cptr.push_back((int)cand.size());
-            }
-            ++ia; ++ib;
-        } else if (a.nodes[ia] < b.nodes[ib]) {
-            while (ia < a.nnodes && a.nodes[ia] < b.nodes[ib]) ++ia;      // lower_bound
-        } else {
-            while (ib < b.nnodes && b.nodes[ib] < a.nodes[ia]) ++ib;
-        }
-    }
-    const int nq = (int)q1.size(), ncand = (int)cand.size();
-    dist.assign(ncand, 0);
-    if (nq == 0 || ncand == 0) return VSG_OK;
-    std::vector<uint8_t> qdesc((size_t)nq * 32);
-    for (int k = 0; k < nq; ++k) memcpy(&qdesc[(size_t)k * 32], V1->descriptors + (size_t)q1[k] * 32, 32);
-    vsg_status st;
-    if ((st = matcher_ensure(m, 1, (size_t)nq * 32)) || (st = matcher_ensure(m, 2, (size_t)std::max(V2->n, 1) * 32)) ||
-        (st = matcher_ensure(m, 3, (size_t)(nq + 1) * 4)) || (st = matcher_ensure(m, 4, (size_t)ncand * 4)) ||
-        (st = matcher_ensure(m, 6, (size_t)ncand * 4)))
-        return st;
-    cudaStream_t s = m->stream;
-    CK(cudaMemcpyAsync(m->buf[1], qdesc.data(), (size_t)nq * 32, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[2], V2->descriptors, (size_t)V2->n * 32, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[3], cptr.data(), (size_t)(nq + 1) * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[4], cand.data(), (size_t)ncand * 4, cudaMemcpyHostToDevice, s));
-    launch_window_dists(m, (const uint8_t *)m->buf[1], nq, (const uint8_t *)m->buf[2], (const int *)m->buf[3],
-                        (const int *)m->buf[4], (int *)m->buf[6]);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(dist.data(), m->buf[6], (size_t)ncand * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return VSG_OK;
-}
-
-bool featvec_ok(int nn, const int32_t *nodes, const int32_t *ptr, const int32_t *idx) {
-    return nn >= 0 && (nn == 0 || (nodes && ptr && idx));
-}
-
 // the rotation-consistency filter shared by the methods: everything outside the three dominant bins is dropped
 template <class Drop>
 void apply_rot_filter(const std::vector<int> *rot_hist, Drop drop) {
@@ -133,6 +72,162 @@ void apply_rot_filter(const std::vector<int> *rot_hist, Drop drop) {
 }
 
 }  // namespace
+
+namespace vsg {
+
+bool featvec_ok(int nn, const int32_t *nodes, const int32_t *ptr, const int32_t *idx) {
+    return nn >= 0 && (nn == 0 || (nodes && ptr && (idx || ptr[nn] == 0)));
+}
+
+// The CSR lists of a FeatureVector must be well formed: the device reads side 2's idx[ptr[k] .. ptr[k+1]) from a copy of
+// idx[0 .. ptr[nnodes]), so the offsets start at 0 and never decrease.  nullptr: nothing wrong.
+static const char *featvec_problem(const FeatVec &v) {
+    if (v.nnodes < 0) return "negative node count";
+    if (v.nnodes == 0) return nullptr;
+    if (!v.nodes || !v.ptr) return "null node or offset array";
+    if (v.ptr[0] != 0) return "first list offset is not 0";
+    for (int k = 0; k < v.nnodes; ++k)
+        if (v.ptr[k + 1] < v.ptr[k]) return "list offsets decrease";
+    if (v.ptr[v.nnodes] > 0 && !v.idx) return "null feature index array";
+    return nullptr;
+}
+
+vsg_status bow_walk(const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs) {
+    const FeatVec &a = w.a, &b = w.b;
+    for (const FeatVec *v : {&a, &b})
+        if (const char *why = featvec_problem(*v)) {
+            set_error("bow: malformed feature vector: %s", why);
+            return VSG_ERR_INVALID;
+        }
+    int ia = 0, ib = 0;
+    while (ia < a.nnodes && ib < b.nnodes) {
+        if (a.nodes[ia] == b.nodes[ib]) {
+            const int jb = b.ptr[ib], je = b.ptr[ib + 1];
+            bool checked = false;                                         // side 2's node, once a query uses it
+            for (int k = a.ptr[ia]; k < a.ptr[ia + 1]; ++k) {
+                const int i1 = a.idx[k];
+                if (i1 < 0 || i1 >= w.v1->n) {
+                    set_error("bow: feature index %d out of range (%d features)", i1, w.v1->n);
+                    return VSG_ERR_INVALID;
+                }
+                if (!w.use1[i1]) continue;
+                for (int j = jb; j < je && !checked; ++j)
+                    if (b.idx[j] < 0 || b.idx[j] >= w.v2->n) {
+                        set_error("bow: feature index %d out of range (%d features)", b.idx[j], w.v2->n);
+                        return VSG_ERR_INVALID;
+                    }
+                checked = true;
+                segs.push_back(BowSeg{i1, jb, je, (int)std::min<int64_t>(*npairs, INT_MAX)});
+                *npairs += je - jb;
+            }
+            ++ia; ++ib;
+        } else if (a.nodes[ia] < b.nodes[ib]) {
+            while (ia < a.nnodes && a.nodes[ia] < b.nodes[ib]) ++ia;      // lower_bound
+        } else {
+            while (ib < b.nnodes && b.nodes[ib] < a.nodes[ia]) ++ib;
+        }
+    }
+    return VSG_OK;
+}
+
+vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std::vector<BowSeg> &segs, const int *seg_ptr,
+                     int64_t npairs, const uint16_t **dist) {
+    *dist = nullptr;
+    if (npairs == 0) return VSG_OK;
+    if (npairs > INT_MAX) {
+        set_error("bow: %lld descriptor pairs in one call (at most %d)", (long long)npairs, INT_MAX);
+        return VSG_ERR_INVALID;
+    }
+    // every distinct descriptor table and side-2 idx array once: a frame shared by all walks, a keyframe passed twice
+    struct Table { const void *p; int n, first; };
+    std::vector<Table> tabs, idxs;
+    int rows = 0, nidx = 0;
+    auto place = [](std::vector<Table> &v, const void *p, int n, int &total) {
+        for (const Table &t : v)
+            if (t.p == p && t.n == n) return t.first;
+        v.push_back(Table{p, n, total});
+        total += n;
+        return v.back().first;
+    };
+    std::vector<int4> dsegs;
+    for (int k = 0; k < nwalks; ++k) {
+        const BowWalk &w = walks[k];
+        int row1 = -1, row2 = -1, idx0 = -1;
+        for (int q = seg_ptr[k]; q < seg_ptr[k + 1]; ++q) {
+            const BowSeg &sg = segs[q];
+            if (sg.je == sg.jb) continue;
+            if (row1 < 0) {
+                row1 = place(tabs, w.v1->descriptors, w.v1->n, rows);
+                row2 = place(tabs, w.v2->descriptors, w.v2->n, rows);
+                idx0 = place(idxs, w.b.idx, w.b.ptr[w.b.nnodes], nidx);
+            }
+            dsegs.push_back(make_int4(row1 + sg.i1, idx0 + sg.jb, row2, sg.off));
+        }
+    }
+    dsegs.push_back(make_int4(0, 0, 0, (int)npairs));                     // sentinel
+    auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+    const size_t o_seg = 0, o_desc = up16(dsegs.size() * sizeof(int4)), o_idx = o_desc + (size_t)rows * 32,
+                 o_out = up16(o_idx + (size_t)nidx * sizeof(int)), total = o_out + (size_t)npairs * sizeof(uint16_t);
+    vsg_status st;
+    // device slot 19 and pinned host slot 8: inputs, then the distances
+    if ((st = matcher_ensure(m, 19, total)) || (st = matcher_ensure_host(m, 8, total))) return st;
+    uint8_t *h = (uint8_t *)m->hbuf[8], *d = (uint8_t *)m->buf[19];
+    memcpy(h + o_seg, dsegs.data(), dsegs.size() * sizeof(int4));
+    for (const Table &t : tabs) memcpy(h + o_desc + (size_t)t.first * 32, t.p, (size_t)t.n * 32);
+    for (const Table &t : idxs) memcpy(h + o_idx + (size_t)t.first * sizeof(int), t.p, (size_t)t.n * sizeof(int));
+    cudaStream_t s = m->stream;
+    CK(cudaMemcpyAsync(d, h, o_out, cudaMemcpyHostToDevice, s));
+    launch_bow_dists(m, (const int4 *)(d + o_seg), (int)dsegs.size(), (const int *)(d + o_idx), d + o_desc, (int)npairs,
+                     (uint16_t *)(d + o_out));
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h + o_out, d + o_out, (size_t)npairs * sizeof(uint16_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    *dist = (const uint16_t *)(h + o_out);
+    return VSG_OK;
+}
+
+const char *bow_side_problem(const vsg_bow_side *s, bool needs_valid) {
+    if (!s) return "null side";
+    if (s->view.n < 0) return "negative feature count";
+    if (s->view.n > 0 && (!s->view.descriptors || !s->view.keys)) return "null keypoints or descriptors";
+    if (needs_valid && s->view.n > 0 && !s->mp_valid) return "null map-point flags";
+    if (!featvec_ok(s->nnodes, s->nodes, s->ptr, s->idx)) return "malformed feature vector";
+    return nullptr;
+}
+
+// The KF-KF replay of SearchByBoW (ORBmatcher.cc:785-900) over one walk's distances: already-matched and map-point-less
+// candidates skipped (:821-825), best / second best, TH_LOW (strict) and ratio gates, rotation histogram.  Returns nmatches.
+static int bow_replay_kf(const vsg_frame_view *KF1, const vsg_frame_view *KF2, const uint8_t *mp_valid2, const FeatVec &b2,
+                         const BowSeg *segs, int nseg, const uint16_t *dist, float nnratio, int check_ori, int32_t *matches12_out) {
+    for (int i = 0; i < KF1->n; ++i) matches12_out[i] = -1;
+    std::vector<uint8_t> matched2(KF2->n, 0);
+    std::vector<int> rot_hist[HISTO_LENGTH];
+    int nmatches = 0;
+    for (int k = 0; k < nseg; ++k) {
+        const BowSeg &sg = segs[k];
+        const int i1 = sg.i1;
+        int best1 = 256, best_idx2 = -1, best2 = 256;
+        for (int j = sg.jb; j < sg.je; ++j) {
+            const int i2 = b2.idx[j];
+            if (matched2[i2] || !mp_valid2[i2]) continue;                            // :821-825
+            const int d = dist[sg.off + j - sg.jb];
+            if (d < best1) { best2 = best1; best1 = d; best_idx2 = i2; }
+            else if (d < best2) best2 = d;
+        }
+        if (best1 < TH_LOW) {                                                        // :843 (strict)
+            if (static_cast<float>(best1) < nnratio * static_cast<float>(best2)) {
+                matches12_out[i1] = best_idx2;
+                matched2[best_idx2] = 1;
+                if (check_ori) rot_hist[rot_bin(KF1->keys[i1].angle, KF2->keys[best_idx2].angle)].push_back(i1);
+                ++nmatches;
+            }
+        }
+    }
+    if (check_ori) apply_rot_filter(rot_hist, [&](int i1) { matches12_out[i1] = -1; --nmatches; });
+    return nmatches;
+}
+
+}  // namespace vsg
 
 extern "C" {
 
@@ -335,35 +430,63 @@ vsg_status vsg_search_by_bow_kf(vsg_matcher *m, const vsg_frame_view *KF1, const
         (KF1->n > 0 && (!mp_valid1 || !matches12_out)) || (KF2->n > 0 && !mp_valid2))
         return VSG_ERR_INVALID;
     CK(cudaSetDevice(m->device));
-    std::vector<int> q1, cptr, cand, dist;
-    vsg_status st = bow_pair_dists(m, KF1, KF2, FeatVec{nnodes1, nodes1, ptr1, idx1}, FeatVec{nnodes2, nodes2, ptr2, idx2},
-                                   [&](int i1) { return mp_valid1[i1] != 0; }, q1, cptr, cand, dist);
-    if (st != VSG_OK) return st;
-    for (int i = 0; i < KF1->n; ++i) matches12_out[i] = -1;
-    std::vector<uint8_t> matched2(KF2->n, 0);
-    std::vector<int> rot_hist[HISTO_LENGTH];
-    int nmatches = 0;
-    for (size_t k = 0; k < q1.size(); ++k) {
-        const int i1 = q1[k];
-        int best1 = 256, best_idx2 = -1, best2 = 256;
-        for (int c = cptr[k]; c < cptr[k + 1]; ++c) {
-            const int i2 = cand[c];
-            if (matched2[i2] || !mp_valid2[i2]) continue;                            // :821-825
-            const int d = dist[c];
-            if (d < best1) { best2 = best1; best1 = d; best_idx2 = i2; }
-            else if (d < best2) best2 = d;
-        }
-        if (best1 < TH_LOW) {                                                        // :843 (strict)
-            if (static_cast<float>(best1) < nnratio * static_cast<float>(best2)) {
-                matches12_out[i1] = best_idx2;
-                matched2[best_idx2] = 1;
-                if (check_ori) rot_hist[rot_bin(KF1->keys[i1].angle, KF2->keys[best_idx2].angle)].push_back(i1);
-                ++nmatches;
-            }
-        }
-    }
-    if (check_ori) apply_rot_filter(rot_hist, [&](int i1) { matches12_out[i1] = -1; --nmatches; });
+    const BowWalk w{KF1, mp_valid1, FeatVec{nnodes1, nodes1, ptr1, idx1}, KF2, FeatVec{nnodes2, nodes2, ptr2, idx2}};
+    std::vector<BowSeg> segs;
+    int64_t npairs = 0;
+    const uint16_t *dist;
+    vsg_status st = bow_walk(w, segs, &npairs);
+    const int seg_ptr[2] = {0, (int)segs.size()};
+    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
+    const int nmatches = bow_replay_kf(KF1, KF2, mp_valid2, w.b, segs.data(), (int)segs.size(), dist, nnratio, check_ori, matches12_out);
     if (nmatches_out) *nmatches_out = nmatches;
+    return VSG_OK;
+}
+
+// vsg_search_by_bow_kf(KF1 against KF2s[t]) for every target in one upload, one launch and one download
+vsg_status vsg_search_by_bow_kf_multi(vsg_matcher *m, const vsg_bow_side *KF1, int ntargets, const vsg_bow_side *const *KF2s,
+                                      float nnratio, int check_ori, int32_t *matches12_out, int *nmatches_out) {
+    if (!m || ntargets < 0) {
+        set_error("vsg_search_by_bow_kf_multi: %d targets", ntargets);
+        return VSG_ERR_INVALID;
+    }
+    if (ntargets == 0) return VSG_OK;
+    const char *why;
+    if (!KF2s || !nmatches_out || (KF1 && KF1->view.n > 0 && !matches12_out)) {
+        set_error("vsg_search_by_bow_kf_multi: null target table or output");
+        return VSG_ERR_INVALID;
+    }
+    if ((why = bow_side_problem(KF1, true))) {
+        set_error("vsg_search_by_bow_kf_multi: KF1: %s", why);
+        return VSG_ERR_INVALID;
+    }
+    for (int t = 0; t < ntargets; ++t)
+        if ((why = bow_side_problem(KF2s[t], true))) {
+            set_error("vsg_search_by_bow_kf_multi: target %d: %s", t, why);
+            return VSG_ERR_INVALID;
+        }
+    CK(cudaSetDevice(m->device));
+    std::vector<BowWalk> walks;
+    std::vector<BowSeg> segs;
+    std::vector<int> seg_ptr(1, 0);
+    int64_t npairs = 0;
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_bow_side &b = *KF2s[t];
+        walks.push_back(BowWalk{&KF1->view, KF1->mp_valid, FeatVec{KF1->nnodes, KF1->nodes, KF1->ptr, KF1->idx}, &b.view,
+                                FeatVec{b.nnodes, b.nodes, b.ptr, b.idx}});
+        if (bow_walk(walks.back(), segs, &npairs) != VSG_OK) {
+            const std::string err = vsg_last_error();
+            set_error("vsg_search_by_bow_kf_multi: target %d: %s", t, err.c_str());
+            return VSG_ERR_INVALID;
+        }
+        seg_ptr.push_back((int)segs.size());
+    }
+    const uint16_t *dist;
+    vsg_status st = bow_dists(m, ntargets, walks.data(), segs, seg_ptr.data(), npairs, &dist);
+    if (st != VSG_OK) return st;
+    for (int t = 0; t < ntargets; ++t)                                               // in target order, as the loop runs
+        nmatches_out[t] = bow_replay_kf(&KF1->view, &KF2s[t]->view, KF2s[t]->mp_valid, walks[t].b, segs.data() + seg_ptr[t],
+                                        seg_ptr[t + 1] - seg_ptr[t], dist, nnratio, check_ori,
+                                        matches12_out + (size_t)t * KF1->view.n);
     return VSG_OK;
 }
 
@@ -379,17 +502,27 @@ vsg_status vsg_bow_pair_distances(vsg_matcher *m, const vsg_frame_view *KF1, con
         (KF1->n > 0 && !use1) || !nq_out || !total_out)
         return VSG_ERR_INVALID;
     CK(cudaSetDevice(m->device));
-    std::vector<int> q1, cptr, cand, dist;
-    vsg_status st = bow_pair_dists(m, KF1, KF2, FeatVec{nnodes1, nodes1, ptr1, idx1}, FeatVec{nnodes2, nodes2, ptr2, idx2},
-                                   [&](int i1) { return use1[i1] != 0; }, q1, cptr, cand, dist);
-    if (st != VSG_OK) return st;
-    *nq_out = (int)q1.size();
-    *total_out = (int)cand.size();
-    if ((int)q1.size() > q_capacity || (int)cand.size() > capacity) return VSG_ERR_CAPACITY;
-    if ((!q1.empty() && (!q1_out || !cand_ptr_out)) || (!cand.empty() && (!cand_idx2_out || !cand_dist_out))) return VSG_ERR_INVALID;
-    for (size_t k = 0; k < q1.size(); ++k) { q1_out[k] = q1[k]; cand_ptr_out[k] = cptr[k]; }
-    if (cand_ptr_out) cand_ptr_out[q1.size()] = (int)cand.size();
-    for (size_t c = 0; c < cand.size(); ++c) { cand_idx2_out[c] = cand[c]; cand_dist_out[c] = dist[c]; }
+    const BowWalk w{KF1, use1, FeatVec{nnodes1, nodes1, ptr1, idx1}, KF2, FeatVec{nnodes2, nodes2, ptr2, idx2}};
+    std::vector<BowSeg> segs;
+    int64_t npairs = 0;
+    const uint16_t *dist;
+    vsg_status st = bow_walk(w, segs, &npairs);
+    const int seg_ptr[2] = {0, (int)segs.size()};
+    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
+    *nq_out = (int)segs.size();
+    *total_out = (int)npairs;
+    if ((int)segs.size() > q_capacity || npairs > capacity) return VSG_ERR_CAPACITY;
+    if ((!segs.empty() && (!q1_out || !cand_ptr_out)) || (npairs && (!cand_idx2_out || !cand_dist_out))) return VSG_ERR_INVALID;
+    for (size_t k = 0; k < segs.size(); ++k) {
+        const BowSeg &sg = segs[k];
+        q1_out[k] = sg.i1;
+        cand_ptr_out[k] = sg.off;
+        for (int j = sg.jb; j < sg.je; ++j) {
+            cand_idx2_out[sg.off + j - sg.jb] = idx2[j];
+            cand_dist_out[sg.off + j - sg.jb] = dist[sg.off + j - sg.jb];
+        }
+    }
+    if (cand_ptr_out) cand_ptr_out[segs.size()] = (int)npairs;
     return VSG_OK;
 }
 
@@ -408,25 +541,29 @@ vsg_status vsg_search_for_triangulation(vsg_matcher *m, const vsg_frame_view *KF
     CK(cudaSetDevice(m->device));
     auto stereo1 = [&](int i) { return KF1->u_right && KF1->u_right[i] >= 0; };       // :977
     auto stereo2 = [&](int i) { return KF2->u_right && KF2->u_right[i] >= 0; };       // :1005
-    std::vector<int> q1, cptr, cand, dist;
-    vsg_status st = bow_pair_dists(m, KF1, KF2, FeatVec{nnodes1, nodes1, ptr1, idx1}, FeatVec{nnodes2, nodes2, ptr2, idx2},
-                                   [&](int i1) { return !has_mp1[i1] && (!only_stereo || stereo1(i1)); },   // :971-981
-                                   q1, cptr, cand, dist);
-    if (st != VSG_OK) return st;
+    std::vector<uint8_t> use1(KF1->n);
+    for (int i = 0; i < KF1->n; ++i) use1[i] = !has_mp1[i] && (!only_stereo || stereo1(i));   // :971-981
+    const BowWalk w{KF1, use1.data(), FeatVec{nnodes1, nodes1, ptr1, idx1}, KF2, FeatVec{nnodes2, nodes2, ptr2, idx2}};
+    std::vector<BowSeg> segs;
+    int64_t npairs = 0;
+    const uint16_t *dist;
+    vsg_status st = bow_walk(w, segs, &npairs);
+    const int seg_ptr[2] = {0, (int)segs.size()};
+    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
     for (int i = 0; i < KF1->n; ++i) matches12_out[i] = -1;
     std::vector<int> rot_hist[HISTO_LENGTH];
     int nmatches = 0;
-    for (size_t k = 0; k < q1.size(); ++k) {
-        const int i1 = q1[k];
+    for (const BowSeg &sg : segs) {
+        const int i1 = sg.i1;
         const vsg_keypoint &kp1 = KF1->keys[i1];
         const bool b_stereo1 = stereo1(i1);
         int best = TH_LOW, best_idx2 = -1;
-        for (int c = cptr[k]; c < cptr[k + 1]; ++c) {
-            const int i2 = cand[c];
+        for (int j = sg.jb; j < sg.je; ++j) {
+            const int i2 = idx2[j];
             if (has_mp2[i2]) continue;                                               // :1001 (vbMatched2 is never set, SURVEY C#3)
             const bool b_stereo2 = stereo2(i2);
             if (only_stereo && !b_stereo2) continue;
-            const int d = dist[c];
+            const int d = dist[sg.off + j - sg.jb];
             if (d > TH_LOW || d > best) continue;                                    // :1014
             const vsg_keypoint &kp2 = KF2->keys[i2];
             if (!b_stereo1 && !b_stereo2) {                                          // :1023-1031

@@ -88,8 +88,8 @@ struct vsg_matcher {
     cudaStream_t stream = nullptr;
     void *buf[20] = {};      // device scratch slots; each entry point documents the slots it owns
     size_t cap[20] = {};
-    void *hbuf[8] = {};      // pinned host staging (grows on demand): results come back without page faults
-    size_t hcap[8] = {};
+    void *hbuf[9] = {};      // pinned host staging (grows on demand): results come back without page faults
+    size_t hcap[9] = {};
     std::vector<char> scratch[2];   // reusable host scratch of the search methods (query lists), kept across calls
     int sm_count = 148;
 };
@@ -105,9 +105,10 @@ vsg_status launch_knn2_merge_parts(vsg_matcher *m, const int32_t *idx_parts, con
 bool knn2_tc_supported(int nq, int nt);
 vsg_status knn2_tc_device(vsg_matcher *m, const uint8_t *q_dev, int nq, const uint8_t *t_dev, int nt, int offset, int *idx_dev,
                           int *dist_dev);
-// distances of every CSR candidate: all_dist[c] = |query[q] xor train[cand[c]]| for c in [cand_ptr[q], cand_ptr[q+1])
-void launch_window_dists(vsg_matcher *m, const uint8_t *query_dev, int nq, const uint8_t *train_dev,
-                         const int *cand_ptr_dev, const int *cand_dev, int *all_dist_dev);
+// bow_dists_multi_kernel (match.cu): out[segs[s].w + k] = |desc[segs[s].x] xor desc[segs[s].z + idx[segs[s].y + k]]| for the
+// k-th candidate of segment s; segs holds nseg segments sorted by .w, the last one a sentinel with .w = npairs
+void launch_bow_dists(vsg_matcher *m, const int4 *segs_dev, int nseg, const int *idx_dev, const uint8_t *desc_dev, int npairs,
+                      uint16_t *out_dev);
 
 // Read-only view of an extractor's device pyramid of its last call (for the stereo matcher).
 struct PyramidRef {

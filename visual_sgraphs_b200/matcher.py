@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import PROJ_POINT_DTYPE, SEARCH_POINT_DTYPE, TRACK_POINT_DTYPE, check, ptr
+from ._lib import PROJ_POINT_DTYPE, SEARCH_POINT_DTYPE, TRACK_POINT_DTYPE, BowSide, check, ptr
 from .frame import DeviceFrame, FrameData
 
 TH_HIGH = 100     # ORBmatcher.cc:34
@@ -40,6 +40,19 @@ def projection_map_resolve_shard(frame_data, blocked, assign, shard_begin, track
                                              ptr(cand_ptr), ptr(cand_idx), ptr(cand_dist), float(np.float32(nnratio)),
                                              ptr(assign), C.byref(nm)))
     return nm.value
+
+
+def _bow_side(data, mp_valid, featvec, keep):
+    """A vsg_bow_side for (FrameData, map-point flags or None, (nodes, ptr, idx)); the arrays it points to go into `keep`."""
+    nodes, ptr_, idx = (np.ascontiguousarray(a, np.int32) for a in featvec)
+    valid = None if mp_valid is None else np.ascontiguousarray(mp_valid, np.uint8)
+    keep.extend([data, nodes, ptr_, idx, valid])
+    return BowSide(data.view, ptr(valid), len(nodes), ptr(nodes), ptr(ptr_), ptr(idx))
+
+
+def _side_table(sides):
+    """const vsg_bow_side *const[] over `sides` (the structs stay referenced by the returned table's owner)."""
+    return (C.c_void_p * max(len(sides), 1))(*[C.addressof(s) for s in sides])
 
 
 class ORBmatcher:
@@ -281,6 +294,20 @@ class ORBmatcher:
                                              float(self.mfNNratio), int(self.mbCheckOrientation), ptr(out), C.byref(nm)))
         return nm.value, out
 
+    def SearchByBoWMulti(self, targets, f_data, f_featvec, f_nleft=-1):
+        """SearchByBoW with one frame against many keyframes (Tracking::Relocalization's loop over its candidates) in one
+        upload, one launch and one download: targets is a list of (kf_data, kf_mp_valid, kf_featvec).  Returns
+        (nmatches[T], matches_f[T, F.N]), target for target what SearchByBoW returns."""
+        keep = []
+        sides = [_bow_side(d, v, fv, keep) for d, v, fv in targets]
+        F = _bow_side(f_data, None, f_featvec, keep)
+        T = len(sides)
+        out = np.zeros((T, f_data.n), np.int32)
+        nm = np.zeros(T, np.int32)
+        check(self._L.vsg_search_by_bow_multi(self._h, T, _side_table(sides), C.byref(F), int(f_nleft), float(self.mfNNratio),
+                                              int(self.mbCheckOrientation), ptr(out), ptr(nm)))
+        return nm, out
+
     def SearchByProjectionReloc(self, cur_frame, occupied, search_points, desc, th, ORBdist):
         """SearchByProjection(Frame&, KeyFrame*, sAlreadyFound, th, ORBdist) (ORBmatcher.cc:1880-2000) with the
         projection done by the caller. Returns (nmatches, assign[N])."""
@@ -358,6 +385,20 @@ class ORBmatcher:
                                            len(n1), ptr(n1), ptr(p1), ptr(i1), len(n2), ptr(n2), ptr(p2), ptr(i2),
                                            float(self.mfNNratio), int(self.mbCheckOrientation), ptr(out), C.byref(nm)))
         return nm.value, out
+
+    def SearchByBoWKFMulti(self, kf1_data, mp_valid1, featvec1, targets):
+        """SearchByBoWKF of one keyframe against many (LoopClosing::DetectCommonRegionsFromBoW's loop over the candidates
+        and their covisibles) in one upload, one launch and one download: targets is a list of (kf2_data, mp_valid2,
+        featvec2).  Returns (nmatches[T], matches12[T, N1]), target for target what SearchByBoWKF returns."""
+        keep = []
+        K1 = _bow_side(kf1_data, mp_valid1, featvec1, keep)
+        sides = [_bow_side(d, v, fv, keep) for d, v, fv in targets]
+        T = len(sides)
+        out = np.zeros((T, kf1_data.n), np.int32)
+        nm = np.zeros(T, np.int32)
+        check(self._L.vsg_search_by_bow_kf_multi(self._h, C.byref(K1), T, _side_table(sides), float(self.mfNNratio),
+                                                 int(self.mbCheckOrientation), ptr(out), ptr(nm)))
+        return nm, out
 
     def SearchForTriangulation(self, kf1_data, has_mp1, kf2_data, has_mp2, featvec1, featvec2, F12, ep, level_sigma2_2,
                                bOnlyStereo=False, bCoarse=False):

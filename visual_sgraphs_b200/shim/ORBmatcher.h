@@ -88,6 +88,18 @@ public:
     template <class KeyFrameT, class MapPointT>
     int SearchByBoW(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<MapPointT *> &vpMatches12);
 
+    // Tracking::Relocalization's loop over its candidates (Tracking.cc:3687-3854) in one call: vvpMapPointMatches[i] and
+    // element i of the result are what SearchByBoW(vpKFs[i], F, vvpMapPointMatches[i]) gives.  The caller skips bad
+    // keyframes itself, as the loop does.
+    template <class KeyFrameT, class FrameT, class MapPointT>
+    std::vector<int> SearchByBoW(const std::vector<KeyFrameT *> &vpKFs, FrameT &F,
+                                 std::vector<std::vector<MapPointT *>> &vvpMapPointMatches);
+    // LoopClosing::DetectCommonRegionsFromBoW's loop over the candidates and their covisibles (LoopClosing.cc:573-642) in one
+    // call: vvpMatches12[i] and element i of the result are what SearchByBoW(pKF1, vpKF2s[i], vvpMatches12[i]) gives.
+    template <class KeyFrameT, class MapPointT>
+    std::vector<int> SearchByBoW(KeyFrameT *pKF1, const std::vector<KeyFrameT *> &vpKF2s,
+                                 std::vector<std::vector<MapPointT *>> &vvpMatches12);
+
     // Project MapPoints into a KeyFrame and search for duplicates (ORBmatcher.cc:1148-1335; bRight = false).
     template <class KeyFrameT, class MapPointT>
     int Fuse(KeyFrameT *pKF, const std::vector<MapPointT *> &vpMapPoints, const float th = 3.0, const bool bRight = false);
@@ -292,6 +304,33 @@ protected:
             ptr.push_back((int32_t)idx.size());
         }
     }
+    // One side of a BoW search, flattened as the SearchByBoW overloads read it: both cameras of a two-camera frame /
+    // keyframe or mvKeysUn, FeatureVector entries >= limit dropped, map-point flags from GetMapPointMatches() / isBad()
+    // (all zero without vpMPs).  Not copyable: side points into the other members.
+    struct BowSide {
+        Flat flat;
+        std::vector<uint8_t> valid;
+        std::vector<int32_t> nodes, ptr, idx;
+        vsg_bow_side side;
+        BowSide() = default;
+        BowSide(const BowSide &) = delete;
+        BowSide &operator=(const BowSide &) = delete;
+    };
+    template <class FrameT, class MapPointT>
+    static void FlattenBowSide(const FrameT &F, bool bothCameras, size_t limit, const std::vector<MapPointT *> *vpMPs, BowSide &o) {
+        if (bothCameras) FlattenBothCameras(F, o.flat); else Flatten(F, o.flat);
+        o.valid.assign(o.flat.view.n, 0);
+        if (vpMPs)
+            for (int i = 0; i < o.flat.view.n; ++i) o.valid[i] = (*vpMPs)[i] && !(*vpMPs)[i]->isBad();   // :262-266, :800-804
+        FlattenFeatVec(F.mFeatVec, o.nodes, o.ptr, o.idx, limit);
+        o.side.view = o.flat.view;
+        o.side.mp_valid = o.valid.data();
+        o.side.nnodes = (int32_t)o.nodes.size();
+        o.side.nodes = o.nodes.data(); o.side.ptr = o.ptr.data(); o.side.idx = o.idx.data();
+    }
+    // SearchByBoW(KF, KF): two-camera keyframes take part with the features that have an entry in mvKeysUn (:793-796)
+    template <class KeyFrameT>
+    static size_t BowKFLimit(const KeyFrameT *pKF) { return pKF->NLeft != -1 ? pKF->mvKeysUn.size() : (size_t)-1; }
     template <class MapPointT>
     static void CopyDescriptor(MapPointT *pMP, std::vector<uint8_t> &desc, size_t i) {
         const cv::Mat d = pMP->GetDescriptor();
@@ -535,33 +574,45 @@ template <class KeyFrameT, class FrameT, class MapPointT>
 int ORBmatcher::SearchByBoW(KeyFrameT *pKF, FrameT &F, std::vector<MapPointT *> &vpMapPointMatches) {
     const std::vector<MapPointT *> vpMapPointsKF = pKF->GetMapPointMatches();
     vpMapPointMatches = std::vector<MapPointT *>(F.N, static_cast<MapPointT *>(nullptr));
-    Flat kf, fr;
+    BowSide kf, fr;
     // two-camera frames / keyframes: the left camera's keypoints followed by the right camera's, the order of
     // mDescriptors and of the indices in mFeatVec (:298-322, :341-343, :348-350)
-    if (pKF->mpCamera2) FlattenBothCameras(*pKF, kf); else Flatten(*pKF, kf);
-    if (F.Nleft != -1) FlattenBothCameras(F, fr); else Flatten(F, fr);
-    std::vector<uint8_t> valid(kf.view.n, 0);
-    for (int i = 0; i < kf.view.n; ++i)
-        if (vpMapPointsKF[i] && !vpMapPointsKF[i]->isBad()) valid[i] = 1;                    // :262-266
-    auto flatten_fv = [](const auto &fv, std::vector<int32_t> &nodes, std::vector<int32_t> &ptr, std::vector<int32_t> &idx) {
-        ptr.push_back(0);
-        for (const auto &kv : fv) {           // DBoW2::FeatureVector = std::map<NodeId, std::vector<unsigned>>
-            nodes.push_back((int32_t)kv.first);
-            for (unsigned v : kv.second) idx.push_back((int32_t)v);
-            ptr.push_back((int32_t)idx.size());
-        }
-    };
-    std::vector<int32_t> kn, kp, ki, fn, fp, fi;
-    flatten_fv(pKF->mFeatVec, kn, kp, ki);
-    flatten_fv(F.mFeatVec, fn, fp, fi);
-    std::vector<int32_t> matches(fr.view.n, -1);
+    FlattenBowSide(*pKF, pKF->mpCamera2 != nullptr, (size_t)-1, &vpMapPointsKF, kf);
+    FlattenBowSide(F, F.Nleft != -1, (size_t)-1, static_cast<const std::vector<MapPointT *> *>(nullptr), fr);
+    std::vector<int32_t> matches(fr.flat.view.n, -1);
     int nmatches = 0;
-    Check(vsg_search_by_bow_2cam(Workspace(), &kf.view, valid.data(), &fr.view, F.Nleft, (int)kn.size(), kn.data(), kp.data(),
-                                 ki.data(), (int)fn.size(), fn.data(), fp.data(), fi.data(), mfNNratio,
+    Check(vsg_search_by_bow_2cam(Workspace(), &kf.flat.view, kf.valid.data(), &fr.flat.view, F.Nleft, kf.side.nnodes, kf.side.nodes,
+                                 kf.side.ptr, kf.side.idx, fr.side.nnodes, fr.side.nodes, fr.side.ptr, fr.side.idx, mfNNratio,
                                  mbCheckOrientation ? 1 : 0, matches.data(), &nmatches), "vsg_search_by_bow");
-    for (int j = 0; j < fr.view.n; ++j)
+    for (int j = 0; j < fr.flat.view.n; ++j)
         if (matches[j] >= 0) vpMapPointMatches[j] = vpMapPointsKF[matches[j]];               // :339
     return nmatches;
+}
+
+template <class KeyFrameT, class FrameT, class MapPointT>
+std::vector<int> ORBmatcher::SearchByBoW(const std::vector<KeyFrameT *> &vpKFs, FrameT &F,
+                                         std::vector<std::vector<MapPointT *>> &vvpMapPointMatches) {
+    const size_t T = vpKFs.size();
+    std::vector<std::vector<MapPointT *>> vpMapPointsKF(T);
+    std::vector<BowSide> kfs(T);
+    std::vector<const vsg_bow_side *> table(T);
+    for (size_t t = 0; t < T; ++t) {                                                  // each target as the one-target call has it
+        vpMapPointsKF[t] = vpKFs[t]->GetMapPointMatches();
+        FlattenBowSide(*vpKFs[t], vpKFs[t]->mpCamera2 != nullptr, (size_t)-1, &vpMapPointsKF[t], kfs[t]);
+        table[t] = &kfs[t].side;
+    }
+    BowSide fr;
+    FlattenBowSide(F, F.Nleft != -1, (size_t)-1, static_cast<const std::vector<MapPointT *> *>(nullptr), fr);
+    const size_t n = (size_t)fr.flat.view.n;
+    std::vector<int32_t> matches(T * n, -1);
+    std::vector<int> counts(T, 0);
+    Check(vsg_search_by_bow_multi(Workspace(), (int)T, table.data(), &fr.side, F.Nleft, mfNNratio, mbCheckOrientation ? 1 : 0,
+                                  matches.data(), counts.data()), "vsg_search_by_bow_multi");
+    vvpMapPointMatches.assign(T, std::vector<MapPointT *>(F.N, static_cast<MapPointT *>(nullptr)));
+    for (size_t t = 0; t < T; ++t)
+        for (size_t j = 0; j < n; ++j)
+            if (matches[t * n + j] >= 0) vvpMapPointMatches[t][j] = vpMapPointsKF[t][matches[t * n + j]];   // :339
+    return counts;
 }
 
 template <class FrameT>
@@ -633,28 +684,47 @@ template <class KeyFrameT, class MapPointT>
 int ORBmatcher::SearchByBoW(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<MapPointT *> &vpMatches12) {
     // two-camera keyframes: only the features with an entry in mvKeysUn take part (`idx >= mvKeysUn.size()` -> continue,
     // :793-796, :814-817); they are dropped from the flattened FeatureVectors
-    const size_t lim1 = pKF1->NLeft != -1 ? pKF1->mvKeysUn.size() : (size_t)-1;
-    const size_t lim2 = pKF2->NLeft != -1 ? pKF2->mvKeysUn.size() : (size_t)-1;
     const std::vector<MapPointT *> vpMapPoints1 = pKF1->GetMapPointMatches();
     const std::vector<MapPointT *> vpMapPoints2 = pKF2->GetMapPointMatches();
     vpMatches12 = std::vector<MapPointT *>(vpMapPoints1.size(), static_cast<MapPointT *>(nullptr));
-    Flat k1, k2;
-    Flatten(*pKF1, k1);
-    Flatten(*pKF2, k2);
-    std::vector<uint8_t> v1(k1.view.n, 0), v2(k2.view.n, 0);
-    for (int i = 0; i < k1.view.n; ++i) v1[i] = vpMapPoints1[i] && !vpMapPoints1[i]->isBad();   // :800-804
-    for (int i = 0; i < k2.view.n; ++i) v2[i] = vpMapPoints2[i] && !vpMapPoints2[i]->isBad();   // :820-826
-    std::vector<int32_t> n1, p1, i1, n2, p2, i2;
-    FlattenFeatVec(pKF1->mFeatVec, n1, p1, i1, lim1);
-    FlattenFeatVec(pKF2->mFeatVec, n2, p2, i2, lim2);
-    std::vector<int32_t> m12(k1.view.n, -1);
+    BowSide k1, k2;
+    FlattenBowSide(*pKF1, false, BowKFLimit(pKF1), &vpMapPoints1, k1);                 // :800-804
+    FlattenBowSide(*pKF2, false, BowKFLimit(pKF2), &vpMapPoints2, k2);                 // :820-826
+    std::vector<int32_t> m12(k1.flat.view.n, -1);
     int nmatches = 0;
-    Check(vsg_search_by_bow_kf(Workspace(), &k1.view, v1.data(), &k2.view, v2.data(), (int)n1.size(), n1.data(), p1.data(),
-                               i1.data(), (int)n2.size(), n2.data(), p2.data(), i2.data(), mfNNratio,
-                               mbCheckOrientation ? 1 : 0, m12.data(), &nmatches), "vsg_search_by_bow_kf");
-    for (int i = 0; i < k1.view.n; ++i)
+    Check(vsg_search_by_bow_kf(Workspace(), &k1.flat.view, k1.valid.data(), &k2.flat.view, k2.valid.data(), k1.side.nnodes,
+                               k1.side.nodes, k1.side.ptr, k1.side.idx, k2.side.nnodes, k2.side.nodes, k2.side.ptr, k2.side.idx,
+                               mfNNratio, mbCheckOrientation ? 1 : 0, m12.data(), &nmatches), "vsg_search_by_bow_kf");
+    for (int i = 0; i < k1.flat.view.n; ++i)
         if (m12[i] >= 0) vpMatches12[i] = vpMapPoints2[m12[i]];                           // :847
     return nmatches;
+}
+
+template <class KeyFrameT, class MapPointT>
+std::vector<int> ORBmatcher::SearchByBoW(KeyFrameT *pKF1, const std::vector<KeyFrameT *> &vpKF2s,
+                                         std::vector<std::vector<MapPointT *>> &vvpMatches12) {
+    const size_t T = vpKF2s.size();
+    const std::vector<MapPointT *> vpMapPoints1 = pKF1->GetMapPointMatches();
+    BowSide k1;
+    FlattenBowSide(*pKF1, false, BowKFLimit(pKF1), &vpMapPoints1, k1);
+    std::vector<std::vector<MapPointT *>> vpMapPoints2(T);
+    std::vector<BowSide> k2s(T);
+    std::vector<const vsg_bow_side *> table(T);
+    for (size_t t = 0; t < T; ++t) {                                                  // each target as the one-target call has it
+        vpMapPoints2[t] = vpKF2s[t]->GetMapPointMatches();
+        FlattenBowSide(*vpKF2s[t], false, BowKFLimit(vpKF2s[t]), &vpMapPoints2[t], k2s[t]);
+        table[t] = &k2s[t].side;
+    }
+    const size_t n = (size_t)k1.flat.view.n;
+    std::vector<int32_t> m12(T * n, -1);
+    std::vector<int> counts(T, 0);
+    Check(vsg_search_by_bow_kf_multi(Workspace(), &k1.side, (int)T, table.data(), mfNNratio, mbCheckOrientation ? 1 : 0, m12.data(),
+                                     counts.data()), "vsg_search_by_bow_kf_multi");
+    vvpMatches12.assign(T, std::vector<MapPointT *>(vpMapPoints1.size(), static_cast<MapPointT *>(nullptr)));
+    for (size_t t = 0; t < T; ++t)
+        for (size_t i = 0; i < n; ++i)
+            if (m12[t * n + i] >= 0) vvpMatches12[t][i] = vpMapPoints2[t][m12[t * n + i]];   // :847
+    return counts;
 }
 
 // ---- Fuse(KF, vpMapPoints, th) (ORBmatcher.cc:1148-1335) ----
