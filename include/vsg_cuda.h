@@ -484,7 +484,8 @@ vsg_status vsg_bow_pair_distances(vsg_matcher *m, const vsg_frame_view *KF1, con
  * pinhole camera per keyframe (mpCamera2 == NULL).  has_mp1/2[i] = GetMapPoint(i) != NULL.  f12 = the
  * fundamental matrix of Pinhole::epipolarConstrain (Pinhole.cpp:118-141), row-major; ep = epipole of KF1 in KF2
  * (:914).  level_sigma2_2 = pKF2->mvLevelSigma2.  matches12_out[i1] = i2 or -1 (vMatchedPairs = the pairs with
- * i2 >= 0 in increasing i1). */
+ * i2 >= 0 in increasing i1).  vsg_triangulation_candidates_multi with one target, then vsg_triangulation_resolve: the
+ * same argument rules (a keypoint octave of KF2 outside [0, n_levels) is rejected). */
 vsg_status vsg_search_for_triangulation(vsg_matcher *m, const vsg_frame_view *KF1, const uint8_t *has_mp1,
                                         const vsg_frame_view *KF2, const uint8_t *has_mp2, int nnodes1,
                                         const int32_t *nodes1, const int32_t *ptr1, const int32_t *idx1, int nnodes2,
@@ -492,6 +493,34 @@ vsg_status vsg_search_for_triangulation(vsg_matcher *m, const vsg_frame_view *KF
                                         int only_stereo, int coarse, const float *f12, const float *ep,
                                         const float *level_sigma2_2, int check_ori, int32_t *matches12_out,
                                         int *nmatches_out);
+
+/* One neighbour of LocalMapping::CreateNewMapPoints' loop (LocalMapping.cc:406,460): keyframe 2 of
+ * SearchForTriangulation, single pinhole camera.  kf2.mp_valid[i] = pKF2->GetMapPoint(i) != NULL (bad points included,
+ * ORBmatcher.cc:998-1001).  f12 / ep as in vsg_search_for_triangulation; level_sigma2 = pKF2->mvLevelSigma2
+ * (kf2.view.n_levels entries; may be NULL when the call is coarse). */
+typedef struct vsg_triangulation_target {
+    vsg_bow_side kf2;
+    float f12[9];
+    float ep[2];
+    const float *level_sigma2;
+} vsg_triangulation_target;
+
+/* The searches of every target at once: best12_out is [ntargets][KF1->view.n].  KF1->mp_valid[i] = pKF1->GetMapPoint(i)
+ * != NULL at this call.  best12_out[t][i1] = the keyframe-2 feature the reference's inner loop picks for i1 in target t,
+ * -1 if none, -2 if i1 was not searched because it had a map point.  One upload, at most one launch, one download.
+ * ntargets == 0 does nothing.  A null target, a malformed feature vector, a feature index out of range, a KF1 feature
+ * listed twice in its feature vector, a null level_sigma2 when !coarse or a target keypoint octave outside [0, n_levels)
+ * returns VSG_ERR_INVALID before anything is launched, and vsg_last_error names the target. */
+vsg_status vsg_triangulation_candidates_multi(vsg_matcher *m, const vsg_bow_side *KF1, int ntargets,
+                                              const vsg_triangulation_target *const *targets, int only_stereo, int coarse,
+                                              int32_t *best12_out);
+
+/* Host only, no device: SearchForTriangulation's result for one target from its row of best12, with KF1's map points as
+ * they are NOW (has_mp1).  Equal to vsg_search_for_triangulation(KF1, has_mp1, KF2, …) as long as KF1 has gained, never
+ * lost, map points since the candidates call.  A feature that is -2 and has no map point now returns
+ * VSG_ERR_INVALID, naming the feature. */
+vsg_status vsg_triangulation_resolve(const vsg_frame_view *KF1, const vsg_frame_view *KF2, const uint8_t *has_mp1,
+                                     const int32_t *best12, int check_ori, int32_t *matches12_out, int *nmatches_out);
 
 /* ------------------------------------------------------------------------------------------------
  * BoW transform — the per-feature tree walk of DBoW2::TemplatedVocabulary::transform as called by Frame::ComputeBoW /

@@ -42,6 +42,12 @@ class BowSide(C.Structure):
                 ("ptr", C.c_void_p), ("idx", C.c_void_p)]
 
 
+class TriangulationTarget(C.Structure):
+    """vsg_triangulation_target (include/vsg_cuda.h): keyframe 2 of SearchForTriangulation with its F12, epipole and
+    level variances."""
+    _fields_ = [("kf2", BowSide), ("f12", C.c_float * 9), ("ep", C.c_float * 2), ("level_sigma2", C.c_void_p)]
+
+
 TRACK_POINT_DTYPE = np.dtype([("proj_x", "<f4"), ("proj_y", "<f4"), ("proj_xr", "<f4"), ("view_cos", "<f4"),
                               ("depth", "<f4"), ("level", "<i4"), ("in_view", "u1"), ("bad", "u1"), ("blocks", "u1"),
                               ("pad", "u1")])
@@ -158,6 +164,10 @@ _SIGNATURES = {
                                                C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
+    "vsg_triangulation_candidates_multi": (C.c_int, [C.c_void_p, C.POINTER(BowSide), C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                                     C.c_void_p]),
+    "vsg_triangulation_resolve": (C.c_int, [C.POINTER(FrameView), C.POINTER(FrameView), C.c_void_p, C.c_void_p, C.c_int,
+                                            C.c_void_p, C.POINTER(C.c_int)]),
     "vsg_vocabulary_create": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                         C.POINTER(C.c_void_p)]),
     "vsg_vocabulary_destroy": (None, [C.c_void_p]),

@@ -230,6 +230,74 @@ void launch_bow_dists(vsg_matcher *m, const int4 *segs_dev, int nseg, const int 
     count_launch();
 }
 
+// ------------------------------------------------------------------------------------------------
+// SearchForTriangulation's per-pair test (ORBmatcher.cc:998-1077 with Pinhole::epipolarConstrain, Pinhole.cpp:126-140): one
+// warp per segment, lanes stride over the candidates.  The reference keeps bestDist starting at TH_LOW and accepts on
+// `d <= bestDist`, and no gate reads bestDist, so it ends with the minimum distance among the passing candidates, the last
+// one in scan order on ties: a warp minimum over (d << 32 | ~position).  The float arithmetic is spelled out with _rn
+// intrinsics (no contraction whatever --fmad says, IEEE division) and the chi-square gate compares in double, as the
+// reference's `dsqr < 3.84 * sigma2` does.
+// ------------------------------------------------------------------------------------------------
+constexpr int kTriWarps = 8;
+
+__global__ void __launch_bounds__(kTriWarps * 32) triangulation_best_kernel(const TriSeg *__restrict__ segs, int nseg,
+                                                                            const TriTarget *__restrict__ targets,
+                                                                            const int *__restrict__ idx, const uint4 *__restrict__ desc,
+                                                                            const TriKey *__restrict__ keys,
+                                                                            const float2 *__restrict__ lvl, int only_stereo,
+                                                                            int coarse, int *__restrict__ out) {
+    const int s = blockIdx.x * kTriWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (s >= nseg) return;                                                    // whole warps only
+    const TriSeg sg = segs[s];
+    const TriTarget &tg = targets[sg.target];
+    const uint4 qa = __ldg(desc + 2 * sg.q_row), qb = __ldg(desc + 2 * sg.q_row + 1);
+    const float ep0 = __ldg(&tg.ep[0]), ep1 = __ldg(&tg.ep[1]);
+    const int desc0 = __ldg(&tg.desc0), key0 = __ldg(&tg.key0), lvl0 = __ldg(&tg.lvl0);
+    float a = 0.f, b = 0.f, c = 0.f;                                          // Pinhole.cpp:126-128
+    if (!coarse) {
+        const float *f = tg.f12;
+        a = __fadd_rn(__fadd_rn(__fmul_rn(sg.x1, __ldg(f + 0)), __fmul_rn(sg.y1, __ldg(f + 3))), __ldg(f + 6));
+        b = __fadd_rn(__fadd_rn(__fmul_rn(sg.x1, __ldg(f + 1)), __fmul_rn(sg.y1, __ldg(f + 4))), __ldg(f + 7));
+        c = __fadd_rn(__fadd_rn(__fmul_rn(sg.x1, __ldg(f + 2)), __fmul_rn(sg.y1, __ldg(f + 5))), __ldg(f + 8));
+    }
+    unsigned long long best = ~0ull;
+    for (int p = lane; p < sg.ncand; p += 32) {
+        const int i2 = __ldg(idx + sg.cand + p);
+        const int4 kr = __ldg((const int4 *)(keys + key0 + i2));
+        const float x2 = __int_as_float(kr.x), y2 = __int_as_float(kr.y);
+        if (kr.w & kTriHasMp) continue;                                       // :1001 (vbMatched2 is never set)
+        const bool stereo2 = kr.w & kTriStereo;
+        if (only_stereo && !stereo2) continue;                                // :1008
+        const int d = hamming256(qa, qb, __ldg(desc + 2 * (desc0 + i2)), __ldg(desc + 2 * (desc0 + i2) + 1));
+        if (d > 50) continue;                                                 // :1014, TH_LOW
+        const float2 lv = __ldg(lvl + lvl0 + kr.z);
+        if (!sg.stereo1 && !stereo2) {                                        // :1023-1031
+            const float ex = __fsub_rn(ep0, x2), ey = __fsub_rn(ep1, y2);
+            if (__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)) < __fmul_rn(100.f, lv.x)) continue;
+        }
+        if (!coarse) {                                                        // Pinhole.cpp:130-140
+            const float num = __fadd_rn(__fadd_rn(__fmul_rn(a, x2), __fmul_rn(b, y2)), c);
+            const float den = __fadd_rn(__fmul_rn(a, a), __fmul_rn(b, b));
+            if (den == 0.f) continue;
+            const float dsqr = __fdiv_rn(__fmul_rn(num, num), den);
+            if (!((double)dsqr < __dmul_rn(3.84, (double)lv.y))) continue;
+        }
+        best = min(best, ((unsigned long long)d << 32) | (unsigned)~p);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
+    if (lane == 0) out[s] = best == ~0ull ? -1 : __ldg(idx + sg.cand + (int)~(unsigned)best);
+}
+
+void launch_triangulation_best(vsg_matcher *m, const TriSeg *segs_dev, int nseg, const TriTarget *targets_dev, const int *idx_dev,
+                               const uint8_t *desc_dev, const TriKey *keys_dev, const float2 *lvl_dev, int only_stereo, int coarse,
+                               int *out_dev) {
+    if (nseg <= 0) return;
+    triangulation_best_kernel<<<(nseg + kTriWarps - 1) / kTriWarps, kTriWarps * 32, 0, m->stream>>>(
+        segs_dev, nseg, targets_dev, idx_dev, (const uint4 *)desc_dev, keys_dev, lvl_dev, only_stereo, coarse, out_dev);
+    count_launch();
+}
+
 static void knn2_plan(const vsg_matcher *m, int nq, int nt, int *qtiles, int *nchunks, int *chunk_rows) {
     *qtiles = (nq + kKnnThreads * kKnnQ - 1) / (kKnnThreads * kKnnQ);
     // enough CTAs for ~4 waves over the SMs, chunks a multiple of the tile size and below the key's index range

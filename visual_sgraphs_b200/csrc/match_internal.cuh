@@ -98,6 +98,20 @@ struct BowWalk {
 struct BowSeg {
     int i1, jb, je, off;
 };
+// Host tables laid out back to back in one upload, each distinct one once (a frame shared by all walks, a keyframe passed
+// twice): place() returns the first element of (p, n), appending it if it is not there yet.
+struct TablePlacer {
+    struct Table { const void *p; int n, first; };
+    std::vector<Table> tabs;
+    int total = 0;
+    int place(const void *p, int n) {
+        for (const Table &t : tabs)
+            if (t.p == p && t.n == n) return t.first;
+        tabs.push_back(Table{p, n, total});
+        total += n;
+        return tabs.back().first;
+    }
+};
 bool featvec_ok(int nn, const int32_t *nodes, const int32_t *ptr, const int32_t *idx);
 // Appends the queries of one walk to segs, output slots continuing from *npairs; rejects feature indices out of range.
 vsg_status bow_walk(const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs);

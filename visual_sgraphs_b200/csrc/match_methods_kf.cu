@@ -71,6 +71,14 @@ void apply_rot_filter(const std::vector<int> *rot_hist, Drop drop) {
     }
 }
 
+size_t up16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// The placed descriptor tables (32-byte rows) and FeatureVector index arrays of a BoW upload into the staging buffer h.
+void copy_tables(uint8_t *h, size_t o_desc, size_t o_idx, const TablePlacer &descs, const TablePlacer &idxs) {
+    for (const TablePlacer::Table &t : descs.tabs) memcpy(h + o_desc + (size_t)t.first * 32, t.p, (size_t)t.n * 32);
+    for (const TablePlacer::Table &t : idxs.tabs) memcpy(h + o_idx + (size_t)t.first * sizeof(int), t.p, (size_t)t.n * sizeof(int));
+}
+
 }  // namespace
 
 namespace vsg {
@@ -138,17 +146,7 @@ vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std
         set_error("bow: %lld descriptor pairs in one call (at most %d)", (long long)npairs, INT_MAX);
         return VSG_ERR_INVALID;
     }
-    // every distinct descriptor table and side-2 idx array once: a frame shared by all walks, a keyframe passed twice
-    struct Table { const void *p; int n, first; };
-    std::vector<Table> tabs, idxs;
-    int rows = 0, nidx = 0;
-    auto place = [](std::vector<Table> &v, const void *p, int n, int &total) {
-        for (const Table &t : v)
-            if (t.p == p && t.n == n) return t.first;
-        v.push_back(Table{p, n, total});
-        total += n;
-        return v.back().first;
-    };
+    TablePlacer descs, idxs;
     std::vector<int4> dsegs;
     for (int k = 0; k < nwalks; ++k) {
         const BowWalk &w = walks[k];
@@ -157,24 +155,22 @@ vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std
             const BowSeg &sg = segs[q];
             if (sg.je == sg.jb) continue;
             if (row1 < 0) {
-                row1 = place(tabs, w.v1->descriptors, w.v1->n, rows);
-                row2 = place(tabs, w.v2->descriptors, w.v2->n, rows);
-                idx0 = place(idxs, w.b.idx, w.b.ptr[w.b.nnodes], nidx);
+                row1 = descs.place(w.v1->descriptors, w.v1->n);
+                row2 = descs.place(w.v2->descriptors, w.v2->n);
+                idx0 = idxs.place(w.b.idx, w.b.ptr[w.b.nnodes]);
             }
             dsegs.push_back(make_int4(row1 + sg.i1, idx0 + sg.jb, row2, sg.off));
         }
     }
     dsegs.push_back(make_int4(0, 0, 0, (int)npairs));                     // sentinel
-    auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
-    const size_t o_seg = 0, o_desc = up16(dsegs.size() * sizeof(int4)), o_idx = o_desc + (size_t)rows * 32,
-                 o_out = up16(o_idx + (size_t)nidx * sizeof(int)), total = o_out + (size_t)npairs * sizeof(uint16_t);
+    const size_t o_seg = 0, o_desc = up16(dsegs.size() * sizeof(int4)), o_idx = o_desc + (size_t)descs.total * 32,
+                 o_out = up16(o_idx + (size_t)idxs.total * sizeof(int)), total = o_out + (size_t)npairs * sizeof(uint16_t);
     vsg_status st;
     // device slot 19 and pinned host slot 8: inputs, then the distances
     if ((st = matcher_ensure(m, 19, total)) || (st = matcher_ensure_host(m, 8, total))) return st;
     uint8_t *h = (uint8_t *)m->hbuf[8], *d = (uint8_t *)m->buf[19];
     memcpy(h + o_seg, dsegs.data(), dsegs.size() * sizeof(int4));
-    for (const Table &t : tabs) memcpy(h + o_desc + (size_t)t.first * 32, t.p, (size_t)t.n * 32);
-    for (const Table &t : idxs) memcpy(h + o_idx + (size_t)t.first * sizeof(int), t.p, (size_t)t.n * sizeof(int));
+    copy_tables(h, o_desc, o_idx, descs, idxs);
     cudaStream_t s = m->stream;
     CK(cudaMemcpyAsync(d, h, o_out, cudaMemcpyHostToDevice, s));
     launch_bow_dists(m, (const int4 *)(d + o_seg), (int)dsegs.size(), (const int *)(d + o_idx), d + o_desc, (int)npairs,
@@ -225,6 +221,139 @@ static int bow_replay_kf(const vsg_frame_view *KF1, const vsg_frame_view *KF2, c
     }
     if (check_ori) apply_rot_filter(rot_hist, [&](int i1) { matches12_out[i1] = -1; --nmatches; });
     return nmatches;
+}
+
+// vsg_triangulation_candidates_multi under the name `who` (vsg_search_for_triangulation runs it with one target).  The host
+// does the merge walks; every segment with candidates goes to the device with its target's tables, and
+// triangulation_best_kernel picks each segment's bestIdx2.
+static vsg_status triangulation_candidates(vsg_matcher *m, const char *who, const vsg_bow_side *KF1, int ntargets,
+                                           const vsg_triangulation_target *const *targets, int only_stereo, int coarse,
+                                           int32_t *best12_out) {
+    if (!m || ntargets < 0) {
+        set_error("%s: %d targets", who, ntargets);
+        return VSG_ERR_INVALID;
+    }
+    if (ntargets == 0) return VSG_OK;
+    const char *why;
+    if (!targets || (KF1 && KF1->view.n > 0 && !best12_out)) {
+        set_error("%s: null target table or output", who);
+        return VSG_ERR_INVALID;
+    }
+    if ((why = bow_side_problem(KF1, true))) {
+        set_error("%s: KF1: %s", who, why);
+        return VSG_ERR_INVALID;
+    }
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_triangulation_target *tg = targets[t];
+        why = tg ? bow_side_problem(&tg->kf2, true) : "null target";
+        if (!why && !coarse && !tg->level_sigma2) why = "null level_sigma2 (the call is not coarse)";
+        if (!why && tg->kf2.view.n > 0 && !tg->kf2.view.scale_factors) why = "null scale factors";
+        if (why) {
+            set_error("%s: target %d: %s", who, t, why);
+            return VSG_ERR_INVALID;
+        }
+        const vsg_frame_view &v = tg->kf2.view;                           // the device indexes the level tables by octave
+        for (int i = 0; i < v.n; ++i)
+            if (v.keys[i].octave < 0 || v.keys[i].octave >= v.n_levels) {
+                set_error("%s: target %d: keypoint %d: octave %d outside [0, %d)", who, t, i, v.keys[i].octave, v.n_levels);
+                return VSG_ERR_INVALID;
+            }
+    }
+    CK(cudaSetDevice(m->device));
+    const vsg_frame_view &v1 = KF1->view;
+    auto stereo = [](const vsg_frame_view &v, int i) { return v.u_right && v.u_right[i] >= 0; };   // :977, :1005
+    std::vector<uint8_t> use1(v1.n);
+    for (int i = 0; i < v1.n; ++i) use1[i] = !KF1->mp_valid[i] && (!only_stereo || stereo(v1, i));   // :968-981
+    // the walks; a KF1 feature listed twice would be searched twice in one target, which one row of best12 cannot say
+    std::vector<BowSeg> segs;
+    std::vector<int> seg_ptr(1, 0), seen(v1.n, -1);
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_bow_side &b = targets[t]->kf2;
+        int64_t npairs = 0;
+        if (bow_walk(BowWalk{&v1, use1.data(), FeatVec{KF1->nnodes, KF1->nodes, KF1->ptr, KF1->idx}, &b.view,
+                             FeatVec{b.nnodes, b.nodes, b.ptr, b.idx}}, segs, &npairs) != VSG_OK) {
+            const std::string err = vsg_last_error();
+            set_error("%s: target %d: %s", who, t, err.c_str());
+            return VSG_ERR_INVALID;
+        }
+        for (size_t k = seg_ptr.back(); k < segs.size(); ++k) {
+            if (seen[segs[k].i1] == t) {
+                set_error("%s: target %d: KF1 feature %d is listed twice in its feature vector", who, t, segs[k].i1);
+                return VSG_ERR_INVALID;
+            }
+            seen[segs[k].i1] = t;
+        }
+        seg_ptr.push_back((int)segs.size());
+    }
+    for (int t = 0; t < ntargets; ++t)
+        for (int i = 0; i < v1.n; ++i) best12_out[(size_t)t * v1.n + i] = KF1->mp_valid[i] ? -2 : -1;
+    // the segments with candidates and the tables they read
+    TablePlacer descs, idxs;
+    std::vector<TriSeg> dsegs;
+    std::vector<size_t> dseg_out;                                         // best12_out slot of each uploaded segment
+    std::vector<TriTarget> dtargets(ntargets, TriTarget{});
+    std::vector<int> used;                                                // targets with segments, in order
+    int nkeys = 0, nlvl = 0;
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_triangulation_target &tg = *targets[t];
+        const vsg_bow_side &b = tg.kf2;
+        int row1 = -1, idx0 = -1;
+        for (int k = seg_ptr[t]; k < seg_ptr[t + 1]; ++k) {
+            const BowSeg &sg = segs[k];
+            if (sg.je == sg.jb) continue;
+            if (row1 < 0) {
+                row1 = descs.place(v1.descriptors, v1.n);
+                TriTarget &d = dtargets[t];
+                memcpy(d.f12, tg.f12, sizeof d.f12);
+                memcpy(d.ep, tg.ep, sizeof d.ep);
+                d.desc0 = descs.place(b.view.descriptors, b.view.n);
+                d.key0 = nkeys;
+                d.lvl0 = nlvl;
+                nkeys += b.view.n;
+                nlvl += b.view.n_levels;
+                idx0 = idxs.place(b.idx, b.ptr[b.nnodes]);
+                used.push_back(t);
+            }
+            const vsg_keypoint &kp1 = v1.keys[sg.i1];
+            dsegs.push_back(TriSeg{kp1.x, kp1.y, row1 + sg.i1, idx0 + sg.jb, sg.je - sg.jb, t, stereo(v1, sg.i1) ? 1 : 0, 0});
+            dseg_out.push_back((size_t)t * v1.n + sg.i1);
+        }
+    }
+    if (dsegs.empty()) return VSG_OK;
+    const int nseg = (int)dsegs.size();
+    const size_t o_seg = 0, o_tg = up16((size_t)nseg * sizeof(TriSeg)), o_desc = up16(o_tg + (size_t)ntargets * sizeof(TriTarget)),
+                 o_idx = o_desc + (size_t)descs.total * 32, o_key = up16(o_idx + (size_t)idxs.total * sizeof(int)),
+                 o_lvl = o_key + (size_t)nkeys * sizeof(TriKey), o_out = up16(o_lvl + (size_t)nlvl * sizeof(float2)),
+                 total = o_out + (size_t)nseg * sizeof(int);
+    vsg_status st;
+    // device slot 19 and pinned host slot 8, as bow_dists: inputs, then one index per segment
+    if ((st = matcher_ensure(m, 19, total)) || (st = matcher_ensure_host(m, 8, total))) return st;
+    uint8_t *h = (uint8_t *)m->hbuf[8], *d = (uint8_t *)m->buf[19];
+    memcpy(h + o_seg, dsegs.data(), (size_t)nseg * sizeof(TriSeg));
+    memcpy(h + o_tg, dtargets.data(), (size_t)ntargets * sizeof(TriTarget));
+    copy_tables(h, o_desc, o_idx, descs, idxs);
+    TriKey *keys = (TriKey *)(h + o_key);
+    float2 *lvl = (float2 *)(h + o_lvl);
+    for (int t : used) {
+        const vsg_triangulation_target &tg = *targets[t];
+        const vsg_frame_view &v = tg.kf2.view;
+        for (int i = 0; i < v.n; ++i)
+            keys[dtargets[t].key0 + i] = TriKey{v.keys[i].x, v.keys[i].y, v.keys[i].octave,
+                                                (stereo(v, i) ? kTriStereo : 0) | (tg.kf2.mp_valid[i] ? kTriHasMp : 0)};
+        for (int l = 0; l < v.n_levels; ++l)
+            lvl[dtargets[t].lvl0 + l] = make_float2(v.scale_factors[l], tg.level_sigma2 ? tg.level_sigma2[l] : 0.f);
+    }
+    cudaStream_t s = m->stream;
+    CK(cudaMemcpyAsync(d, h, o_out, cudaMemcpyHostToDevice, s));
+    launch_triangulation_best(m, (const TriSeg *)(d + o_seg), nseg, (const TriTarget *)(d + o_tg), (const int *)(d + o_idx),
+                              d + o_desc, (const TriKey *)(d + o_key), (const float2 *)(d + o_lvl), only_stereo, coarse,
+                              (int *)(d + o_out));
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h + o_out, d + o_out, (size_t)nseg * sizeof(int), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    const int *best = (const int *)(h + o_out);
+    for (int k = 0; k < nseg; ++k) best12_out[dseg_out[k]] = best[k];
+    return VSG_OK;
 }
 
 }  // namespace vsg
@@ -526,7 +655,7 @@ vsg_status vsg_bow_pair_distances(vsg_matcher *m, const vsg_frame_view *KF1, con
     return VSG_OK;
 }
 
-// ORBmatcher.cc:902-1146 (mpCamera2 == NULL, Pinhole::epipolarConstrain)
+// ORBmatcher.cc:902-1146 (mpCamera2 == NULL, Pinhole::epipolarConstrain): the candidates of one target, then the resolve
 vsg_status vsg_search_for_triangulation(vsg_matcher *m, const vsg_frame_view *KF1, const uint8_t *has_mp1,
                                         const vsg_frame_view *KF2, const uint8_t *has_mp2, int nnodes1,
                                         const int32_t *nodes1, const int32_t *ptr1, const int32_t *idx1, int nnodes2,
@@ -538,57 +667,51 @@ vsg_status vsg_search_for_triangulation(vsg_matcher *m, const vsg_frame_view *KF
         (KF1->n > 0 && (!has_mp1 || !matches12_out)) || (KF2->n > 0 && !has_mp2) || !ep || (!coarse && (!f12 || !level_sigma2_2)) ||
         (KF2->n > 0 && !KF2->scale_factors))
         return VSG_ERR_INVALID;
-    CK(cudaSetDevice(m->device));
-    auto stereo1 = [&](int i) { return KF1->u_right && KF1->u_right[i] >= 0; };       // :977
-    auto stereo2 = [&](int i) { return KF2->u_right && KF2->u_right[i] >= 0; };       // :1005
-    std::vector<uint8_t> use1(KF1->n);
-    for (int i = 0; i < KF1->n; ++i) use1[i] = !has_mp1[i] && (!only_stereo || stereo1(i));   // :971-981
-    const BowWalk w{KF1, use1.data(), FeatVec{nnodes1, nodes1, ptr1, idx1}, KF2, FeatVec{nnodes2, nodes2, ptr2, idx2}};
-    std::vector<BowSeg> segs;
-    int64_t npairs = 0;
-    const uint16_t *dist;
-    vsg_status st = bow_walk(w, segs, &npairs);
-    const int seg_ptr[2] = {0, (int)segs.size()};
-    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
-    for (int i = 0; i < KF1->n; ++i) matches12_out[i] = -1;
+    const vsg_bow_side side1{*KF1, has_mp1, nnodes1, nodes1, ptr1, idx1};
+    vsg_triangulation_target tg{vsg_bow_side{*KF2, has_mp2, nnodes2, nodes2, ptr2, idx2}, {}, {ep[0], ep[1]}, level_sigma2_2};
+    if (f12) memcpy(tg.f12, f12, sizeof tg.f12);
+    const vsg_triangulation_target *tp = &tg;
+    std::vector<int32_t> best12(KF1->n);
+    vsg_status st = triangulation_candidates(m, "vsg_search_for_triangulation", &side1, 1, &tp, only_stereo, coarse, best12.data());
+    if (st != VSG_OK) return st;
+    return vsg_triangulation_resolve(KF1, KF2, has_mp1, best12.data(), check_ori, matches12_out, nmatches_out);
+}
+
+// LocalMapping::CreateNewMapPoints' searches (LocalMapping.cc:406,460), every neighbour in one upload, one launch and one download
+vsg_status vsg_triangulation_candidates_multi(vsg_matcher *m, const vsg_bow_side *KF1, int ntargets,
+                                              const vsg_triangulation_target *const *targets, int only_stereo, int coarse,
+                                              int32_t *best12_out) {
+    return triangulation_candidates(m, "vsg_triangulation_candidates_multi", KF1, ntargets, targets, only_stereo, coarse, best12_out);
+}
+
+// The rest of ORBmatcher.cc:998-1137 for one target: the features without a map point now keep their candidate, then the
+// rotation check.  Each feature has one row entry, so the histogram holds the same members in every order of the walk, and
+// ComputeThreeMaxima reads only the bin sizes.
+vsg_status vsg_triangulation_resolve(const vsg_frame_view *KF1, const vsg_frame_view *KF2, const uint8_t *has_mp1,
+                                     const int32_t *best12, int check_ori, int32_t *matches12_out, int *nmatches_out) {
+    if (!KF1 || !KF2 || KF1->n < 0 || KF2->n < 0 || (KF1->n > 0 && (!has_mp1 || !best12 || !matches12_out || !KF1->keys))) {
+        set_error("vsg_triangulation_resolve: null or negative-sized keyframe, map-point flags, candidates or output");
+        return VSG_ERR_INVALID;
+    }
+    for (int i = 0; i < KF1->n; ++i) {
+        const int b = best12[i];
+        if (b == -2 && !has_mp1[i]) {
+            set_error("vsg_triangulation_resolve: feature %d was not searched (it had a map point) and has no map point now", i);
+            return VSG_ERR_INVALID;
+        }
+        if (b < -2 || b >= KF2->n || (b >= 0 && !KF2->keys)) {
+            set_error("vsg_triangulation_resolve: feature %d: candidate %d out of range (%d features)", i, b, KF2->n);
+            return VSG_ERR_INVALID;
+        }
+    }
     std::vector<int> rot_hist[HISTO_LENGTH];
     int nmatches = 0;
-    for (const BowSeg &sg : segs) {
-        const int i1 = sg.i1;
-        const vsg_keypoint &kp1 = KF1->keys[i1];
-        const bool b_stereo1 = stereo1(i1);
-        int best = TH_LOW, best_idx2 = -1;
-        for (int j = sg.jb; j < sg.je; ++j) {
-            const int i2 = idx2[j];
-            if (has_mp2[i2]) continue;                                               // :1001 (vbMatched2 is never set, SURVEY C#3)
-            const bool b_stereo2 = stereo2(i2);
-            if (only_stereo && !b_stereo2) continue;
-            const int d = dist[sg.off + j - sg.jb];
-            if (d > TH_LOW || d > best) continue;                                    // :1014
-            const vsg_keypoint &kp2 = KF2->keys[i2];
-            if (!b_stereo1 && !b_stereo2) {                                          // :1023-1031
-                const float distex = ep[0] - kp2.x, distey = ep[1] - kp2.y;
-                if (distex * distex + distey * distey < 100 * KF2->scale_factors[kp2.octave]) continue;
-            }
-            bool ok = coarse != 0;
-            if (!ok) {                                                               // Pinhole.cpp:126-140
-                const float a = kp1.x * f12[0] + kp1.y * f12[3] + f12[6];
-                const float b = kp1.x * f12[1] + kp1.y * f12[4] + f12[7];
-                const float cc = kp1.x * f12[2] + kp1.y * f12[5] + f12[8];
-                const float num = a * kp2.x + b * kp2.y + cc;
-                const float den = a * a + b * b;
-                if (den != 0) {
-                    const float dsqr = num * num / den;
-                    ok = dsqr < 3.84 * level_sigma2_2[kp2.octave];
-                }
-            }
-            if (ok) { best_idx2 = i2; best = d; }
-        }
-        if (best_idx2 >= 0) {
-            matches12_out[i1] = best_idx2;
-            ++nmatches;
-            if (check_ori) rot_hist[rot_bin(kp1.angle, KF2->keys[best_idx2].angle)].push_back(i1);
-        }
+    for (int i = 0; i < KF1->n; ++i) {
+        matches12_out[i] = -1;
+        if (has_mp1[i] || best12[i] < 0) continue;                               // :968-970
+        matches12_out[i] = best12[i];                                            // :1080-1100
+        ++nmatches;
+        if (check_ori) rot_hist[rot_bin(KF1->keys[i].angle, KF2->keys[best12[i]].angle)].push_back(i);
     }
     if (check_ori) apply_rot_filter(rot_hist, [&](int i1) { matches12_out[i1] = -1; --nmatches; });
     if (nmatches_out) *nmatches_out = nmatches;

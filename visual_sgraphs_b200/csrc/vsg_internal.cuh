@@ -109,6 +109,35 @@ vsg_status knn2_tc_device(vsg_matcher *m, const uint8_t *q_dev, int nq, const ui
 // k-th candidate of segment s; segs holds nseg segments sorted by .w, the last one a sentinel with .w = npairs
 void launch_bow_dists(vsg_matcher *m, const int4 *segs_dev, int nseg, const int *idx_dev, const uint8_t *desc_dev, int npairs,
                       uint16_t *out_dev);
+// triangulation_best_kernel (match.cu): SearchForTriangulation's inner loop (ORBmatcher.cc:998-1077, pinhole) for every
+// segment of every target of a call.  A segment is one (target, KF1 feature) query of a BoW merge walk; its candidates are
+// idx[cand .. cand + ncand) (target-local feature indices, the reference's scan order).
+struct TriSeg {
+    float x1, y1;            // KF1 keypoint
+    int q_row;               // KF1 descriptor row in the uploaded descriptor tables
+    int cand, ncand;
+    int target;
+    int stereo1;             // KF1->u_right && KF1->u_right[i1] >= 0
+    int pad;
+};
+struct TriTarget {
+    float f12[9], ep[2];
+    int desc0;               // first descriptor row of the target
+    int key0;                // first TriKey of the target
+    int lvl0;                // first level entry of the target
+    int pad[2];
+};
+struct TriKey {
+    float x, y;
+    int octave;              // validated on the host: inside [0, n_levels)
+    int flags;               // kTriStereo | kTriHasMp
+};
+constexpr int kTriStereo = 1, kTriHasMp = 2;
+// out[s] = the target feature the reference ends with as bestIdx2 for segment s, or -1.  lvl[lvl0 + octave] = (scale factor,
+// level sigma^2).  Nothing is launched when nseg == 0.
+void launch_triangulation_best(vsg_matcher *m, const TriSeg *segs_dev, int nseg, const TriTarget *targets_dev, const int *idx_dev,
+                               const uint8_t *desc_dev, const TriKey *keys_dev, const float2 *lvl_dev, int only_stereo, int coarse,
+                               int *out_dev);
 
 // Read-only view of an extractor's device pyramid of its last call (for the stereo matcher).
 struct PyramidRef {

@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import PROJ_POINT_DTYPE, SEARCH_POINT_DTYPE, TRACK_POINT_DTYPE, BowSide, check, ptr
+from ._lib import PROJ_POINT_DTYPE, SEARCH_POINT_DTYPE, TRACK_POINT_DTYPE, BowSide, TriangulationTarget, check, ptr
 from .frame import DeviceFrame, FrameData
 
 TH_HIGH = 100     # ORBmatcher.cc:34
@@ -415,6 +415,37 @@ class ORBmatcher:
                                                    len(n1), ptr(n1), ptr(p1), ptr(i1), len(n2), ptr(n2), ptr(p2), ptr(i2),
                                                    int(bOnlyStereo), int(bCoarse), ptr(F12), ptr(ep), ptr(sig),
                                                    int(self.mbCheckOrientation), ptr(out), C.byref(nm)))
+        return nm.value, out
+
+    def SearchForTriangulationMulti(self, kf1_data, has_mp1, featvec1, targets, bOnlyStereo=False, bCoarse=False):
+        """The searches of LocalMapping::CreateNewMapPoints' loop over the neighbours in one upload, at most one launch and
+        one download: targets is a list of (kf2_data, has_mp2, featvec2, F12, ep, level_sigma2_2) (level_sigma2_2 may be
+        None when bCoarse).  Returns best12[T, N1]: the keyframe-2 feature each KF1 feature ends with, -1 none, -2 not
+        searched (it has a map point).  ResolveTriangulation turns a row into SearchForTriangulation's result."""
+        keep = []
+        K1 = _bow_side(kf1_data, has_mp1, featvec1, keep)
+        tgs = []
+        for kf2, h2, fv2, f12, ep, sig in targets:
+            sig = None if sig is None else np.ascontiguousarray(sig, np.float32)
+            keep.append(sig)
+            tg = TriangulationTarget(_bow_side(kf2, h2, fv2, keep), (C.c_float * 9)(*np.asarray(f12, np.float32).reshape(9)),
+                                     (C.c_float * 2)(*np.asarray(ep, np.float32).reshape(2)), ptr(sig))
+            tgs.append(tg)
+        T = len(tgs)
+        out = np.zeros((T, kf1_data.n), np.int32)
+        table = (C.c_void_p * max(T, 1))(*[C.addressof(t) for t in tgs])
+        check(self._L.vsg_triangulation_candidates_multi(self._h, C.byref(K1), T, table, int(bOnlyStereo), int(bCoarse), ptr(out)))
+        return out
+
+    def ResolveTriangulation(self, kf1_data, kf2_data, has_mp1, best12):
+        """vsg_triangulation_resolve (host code): SearchForTriangulation's result for one target from its row of best12
+        with KF1's map points as they are now. Returns (nmatches, matches12[N1])."""
+        h1 = np.ascontiguousarray(has_mp1, np.uint8)
+        best12 = np.ascontiguousarray(best12, np.int32)
+        out = np.zeros(kf1_data.n, np.int32)
+        nm = C.c_int(0)
+        check(self._L.vsg_triangulation_resolve(C.byref(kf1_data.view), C.byref(kf2_data.view), ptr(h1), ptr(best12),
+                                                int(self.mbCheckOrientation), ptr(out), C.byref(nm)))
         return nm.value, out
 
     def ComputeStereoMatches(self, ex_left, ex_right, keys_l, desc_l, keys_r, desc_r, mb, mbf, frame_l=0, frame_r=0):

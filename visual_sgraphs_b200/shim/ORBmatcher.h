@@ -27,6 +27,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <set>
 #include <tuple>
 #include <type_traits>
@@ -133,6 +134,21 @@ public:
     template <class KeyFrameT>
     int SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<std::pair<size_t, size_t>> &vMatchedPairs,
                                const bool bOnlyStereo, const bool bCoarse = false);
+
+    // LocalMapping::CreateNewMapPoints' loop `for (i) SearchForTriangulation(pKF1, vpKF2s[i], vMatchedPairs, bOnlyStereo,
+    // bCoarse)` (LocalMapping.cc:406,460) in two halves: one device call for every neighbour up front, then, inside the loop,
+    // SearchForTriangulation(search, i, vMatchedPairs), which returns exactly what the single-target call returns at that
+    // moment.  The batch searches each feature of KF1 that has no map point; a resolve keeps the ones that still have none
+    // and applies the rotation check.  A target is searched again by the single-target call when it is a two-camera
+    // keyframe (or KF1 is one), when one of its map-point slots or either pose changed since the batch, or when a KF1
+    // feature that had a map point at the batch has lost it.
+    template <class KeyFrameT>
+    struct TriangulationSearch;
+    template <class KeyFrameT>
+    TriangulationSearch<KeyFrameT> SearchForTriangulation(KeyFrameT *pKF1, const std::vector<KeyFrameT *> &vpKF2s,
+                                                          const bool bOnlyStereo, const bool bCoarse);
+    template <class KeyFrameT>
+    int SearchForTriangulation(TriangulationSearch<KeyFrameT> &search, size_t i, std::vector<std::pair<size_t, size_t>> &vMatchedPairs);
 
 public:
     static const int TH_LOW = 50;
@@ -410,6 +426,20 @@ protected:
     template <class KeyFrameT, class MapPointT, class OnReplace>
     static int FuseReplay(KeyFrameT *pKF, bool bRight, const std::vector<MapPointT *> &vpMapPoints, const int32_t *best,
                           OnReplace onReplace);
+    // ---- SearchForTriangulation (ORBmatcher.cc:902-1146) in the parts the one-target and the multi-target forms share ----
+    // epipole of KF1 in KF2 and the fundamental matrix of Pinhole::epipolarConstrain (Pinhole.cpp:120-124), built with the
+    // reference's own Eigen expressions (f12 is left zero when bCoarse: nothing reads it)
+    template <class KeyFrameT>
+    static void TriangulationGeometry(KeyFrameT *pKF1, KeyFrameT *pKF2, bool bCoarse, float f12[9], float ep[2]);
+    // KF1 or a target as the C ABI reads it: mvKeysUn, mDescriptors, mFeatVec and GetMapPoint(i) != NULL (:968, :998)
+    template <class KeyFrameT>
+    static void FlattenTriangulationSide(KeyFrameT &KF, BowSide &o) {
+        using MapPointT = typename std::remove_pointer<decltype(KF.GetMapPoint(0))>::type;
+        FlattenBowSide(KF, false, (size_t)-1, static_cast<const std::vector<MapPointT *> *>(nullptr), o);
+        for (int i = 0; i < o.flat.view.n; ++i) o.valid[i] = KF.GetMapPoint(i) ? 1 : 0;
+    }
+    template <class KeyFrameT>
+    static bool TwoCameraKF(const KeyFrameT *pKF) { return pKF->NLeft != -1 || pKF->mpCamera2; }
     template <class FrameT>
     static void RequireSingleCamera(const FrameT &F) {
         if (F.Nleft != -1)
@@ -1064,12 +1094,7 @@ int ORBmatcher::Fuse(KeyFrameT *pKF, Sophus::Sim3f &Scw, const std::vector<MapPo
 
 // ---- SearchForTriangulation (ORBmatcher.cc:902-1146) ----
 template <class KeyFrameT>
-int ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<std::pair<size_t, size_t>> &vMatchedPairs,
-                                       const bool bOnlyStereo, const bool bCoarse) {
-    if (pKF1->NLeft != -1 || pKF2->NLeft != -1 || pKF1->mpCamera2 || pKF2->mpCamera2)
-        return SearchForTriangulationTwoCameras(pKF1, pKF2, vMatchedPairs, bOnlyStereo, bCoarse);
-    // epipole in the second image and the fundamental matrix of Pinhole::epipolarConstrain (Pinhole.cpp:120-124),
-    // built once with the reference's own Eigen expressions (it does not depend on the keypoints)
+void ORBmatcher::TriangulationGeometry(KeyFrameT *pKF1, KeyFrameT *pKF2, bool bCoarse, float f12[9], float epf[2]) {
     const auto T1w = pKF1->GetPose();
     const auto T2w = pKF2->GetPose();
     const auto Tw2 = pKF2->GetPoseInverse();
@@ -1079,7 +1104,7 @@ int ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::ve
     const auto T12 = T1w * Tw2;
     const auto R12 = T12.rotationMatrix();
     const auto t12 = T12.translation();
-    float f12[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+    for (int k = 0; k < 9; ++k) f12[k] = 0;
     if (!bCoarse) {
         typename std::decay<decltype(R12)>::type t12x;
         t12x << 0, -t12(2), t12(1), t12(2), 0, -t12(0), -t12(1), t12(0), 0;                 // Sophus::SO3f::hat(t12)
@@ -1089,7 +1114,16 @@ int ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::ve
         for (int r = 0; r < 3; ++r)
             for (int c = 0; c < 3; ++c) f12[3 * r + c] = F12(r, c);
     }
-    const float epf[2] = {ep(0), ep(1)};
+    epf[0] = ep(0);
+    epf[1] = ep(1);
+}
+
+template <class KeyFrameT>
+int ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<std::pair<size_t, size_t>> &vMatchedPairs,
+                                       const bool bOnlyStereo, const bool bCoarse) {
+    if (TwoCameraKF(pKF1) || TwoCameraKF(pKF2)) return SearchForTriangulationTwoCameras(pKF1, pKF2, vMatchedPairs, bOnlyStereo, bCoarse);
+    float f12[9], epf[2];
+    TriangulationGeometry(pKF1, pKF2, bCoarse, f12, epf);
     Flat k1, k2;
     Flatten(*pKF1, k1);
     Flatten(*pKF2, k2);
@@ -1111,6 +1145,92 @@ int ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::ve
         if (m12[i] < 0) continue;
         vMatchedPairs.push_back(std::make_pair(i, (size_t)m12[i]));
     }
+    return nmatches;
+}
+
+template <class KeyFrameT>
+struct ORBmatcher::TriangulationSearch {
+    KeyFrameT *pKF1 = nullptr;
+    std::vector<KeyFrameT *> vpKF2s;
+    bool bOnlyStereo = false, bCoarse = false;
+    // what the batch call searched with: KF1, every target (row[t] = its row of best12, -1 if it was not batched), and
+    // each target's f12 and epipole (11 floats)
+    std::unique_ptr<BowSide> k1;
+    std::vector<BowSide> k2;
+    std::vector<int> row;
+    std::vector<float> geom;
+    std::vector<int32_t> best12;
+};
+
+template <class KeyFrameT>
+ORBmatcher::TriangulationSearch<KeyFrameT> ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, const std::vector<KeyFrameT *> &vpKF2s,
+                                                                              const bool bOnlyStereo, const bool bCoarse) {
+    TriangulationSearch<KeyFrameT> s;
+    const size_t T = vpKF2s.size();
+    s.pKF1 = pKF1;
+    s.vpKF2s = vpKF2s;
+    s.bOnlyStereo = bOnlyStereo;
+    s.bCoarse = bCoarse;
+    s.k2 = std::vector<BowSide>(T);
+    s.row.assign(T, -1);
+    s.geom.assign(T * 11, 0.f);
+    if (TwoCameraKF(pKF1)) return s;                                                       // all targets take the single call
+    s.k1.reset(new BowSide());
+    FlattenTriangulationSide(*pKF1, *s.k1);
+    std::vector<vsg_triangulation_target> tgs;
+    tgs.reserve(T);
+    for (size_t t = 0; t < T; ++t) {
+        KeyFrameT *pKF2 = vpKF2s[t];
+        if (TwoCameraKF(pKF2)) continue;
+        FlattenTriangulationSide(*pKF2, s.k2[t]);
+        float *g = &s.geom[t * 11];
+        TriangulationGeometry(pKF1, pKF2, bCoarse, g, g + 9);
+        vsg_triangulation_target tg;
+        tg.kf2 = s.k2[t].side;
+        std::memcpy(tg.f12, g, sizeof tg.f12);
+        std::memcpy(tg.ep, g + 9, sizeof tg.ep);
+        tg.level_sigma2 = pKF2->mvLevelSigma2.data();
+        s.row[t] = (int)tgs.size();
+        tgs.push_back(tg);
+    }
+    std::vector<const vsg_triangulation_target *> table(tgs.size());
+    for (size_t r = 0; r < tgs.size(); ++r) table[r] = &tgs[r];
+    s.best12.assign(tgs.size() * (size_t)s.k1->flat.view.n, -1);
+    Check(vsg_triangulation_candidates_multi(Workspace(), &s.k1->side, (int)tgs.size(), table.data(), bOnlyStereo ? 1 : 0,
+                                             bCoarse ? 1 : 0, s.best12.data()), "vsg_triangulation_candidates_multi");
+    return s;
+}
+
+template <class KeyFrameT>
+int ORBmatcher::SearchForTriangulation(TriangulationSearch<KeyFrameT> &search, size_t i,
+                                       std::vector<std::pair<size_t, size_t>> &vMatchedPairs) {
+    KeyFrameT *pKF1 = search.pKF1, *pKF2 = search.vpKF2s.at(i);
+    const int r = search.row[i];
+    bool current = r >= 0;
+    const BowSide &k2 = search.k2[i];
+    for (int j = 0; current && j < k2.flat.view.n; ++j)                                    // the target's map-point slots
+        current = (pKF2->GetMapPoint(j) != nullptr) == (k2.valid[j] != 0);
+    if (current) {                                                                          // both poses
+        float g[11];
+        TriangulationGeometry(pKF1, pKF2, search.bCoarse, g, g + 9);
+        current = std::memcmp(g, &search.geom[i * 11], sizeof g) == 0;
+    }
+    const int n1 = current ? search.k1->flat.view.n : 0;
+    const int32_t *best = current ? &search.best12[(size_t)r * n1] : nullptr;
+    std::vector<uint8_t> h1(n1);
+    for (int j = 0; current && j < n1; ++j) {                                               // KF1's map points: gained, never lost
+        h1[j] = pKF1->GetMapPoint(j) ? 1 : 0;
+        current = best[j] != -2 || h1[j];
+    }
+    if (!current) return SearchForTriangulation(pKF1, pKF2, vMatchedPairs, search.bOnlyStereo, search.bCoarse);
+    std::vector<int32_t> m12(n1, -1);
+    int nmatches = 0;
+    Check(vsg_triangulation_resolve(&search.k1->flat.view, &k2.flat.view, h1.data(), best, mbCheckOrientation ? 1 : 0, m12.data(),
+                                    &nmatches), "vsg_triangulation_resolve");
+    vMatchedPairs.clear();
+    vMatchedPairs.reserve(nmatches);
+    for (int j = 0; j < n1; j++)                                                            // :1136-1143
+        if (m12[j] >= 0) vMatchedPairs.push_back(std::make_pair((size_t)j, (size_t)m12[j]));
     return nmatches;
 }
 
