@@ -160,6 +160,24 @@ def test_shard_by_shard_replay_equals_the_one_call_resolve(oracle):
         assert total == wnm and np.array_equal(assign, wassign), world
 
 
+def test_shard_replay_rejects_a_bad_index_before_writing(oracle):
+    """A candidate index out of range in the last map point's list: vsg_projection_map_resolve_shard fails and leaves the
+    claim state and the assignments untouched, although earlier map points of the shard would have matched."""
+    from visual_sgraphs_b200 import _lib
+    from visual_sgraphs_b200.matcher import projection_map_resolve_shard
+    fd, pts, desc, occ = _proj_scenario(oracle)
+    cp, ci, cd = _cpu_candidates(oracle, fd, pts, desc, 3.0)
+    assert projection_map_resolve_shard(fd, np.ascontiguousarray(occ, np.uint8).copy(), np.full(fd.n, -1, np.int32), 0,
+                                        pts[:-1], cp[:-1], ci, cd, 0.8) > 0
+    ci, cd, cp = np.append(ci, fd.n).astype(np.int32), np.append(cd, 0).astype(np.int32), cp.copy()
+    cp[-1] += 1
+    blocked = np.ascontiguousarray(occ, np.uint8).copy()
+    assign = np.full(fd.n, -1, np.int32)
+    with pytest.raises(_lib.VsgError, match="candidate index out of range"):
+        projection_map_resolve_shard(fd, blocked, assign, 0, pts, cp, ci, cd, 0.8)
+    assert np.array_equal(blocked, np.ascontiguousarray(occ, np.uint8)) and (assign == -1).all()
+
+
 def _ring_worker(rank, world, port, out_dir):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)

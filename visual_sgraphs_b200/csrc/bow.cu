@@ -101,12 +101,12 @@ vsg_status vsg_bow_transform(vsg_matcher *m, const vsg_vocabulary *voc, const ui
     if (n == 0) return VSG_OK;
     CK(cudaSetDevice(m->device));
     vsg_status st;
-    if ((st = matcher_ensure(m, 1, (size_t)n * 32)) || (st = matcher_ensure(m, 6, (size_t)n * 8))) return st;
+    if ((st = matcher_ensure(m, kSlotArg1, (size_t)n * 32)) || (st = matcher_ensure(m, kSlotOut, (size_t)n * 8))) return st;
     cudaStream_t s = m->stream;
-    CK(cudaMemcpyAsync(m->buf[1], descriptors, (size_t)n * 32, cudaMemcpyHostToDevice, s));
-    int *leaf = (int *)m->buf[6], *nid = leaf + n;
+    CK(cudaMemcpyAsync(m->buf[kSlotArg1], descriptors, (size_t)n * 32, cudaMemcpyHostToDevice, s));
+    int *leaf = (int *)m->buf[kSlotOut], *nid = leaf + n;
     bow_transform_kernel<<<(n + 127) / 128, 128, 0, s>>>(voc->child_ptr, voc->child_idx, voc->node_desc,
-                                                        (const uint4 *)m->buf[1], n, voc->levels - levelsup, leaf, nid);
+                                                        (const uint4 *)m->buf[kSlotArg1], n, voc->levels - levelsup, leaf, nid);
     count_launch();
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(leaf_node_out, leaf, (size_t)n * 4, cudaMemcpyDeviceToHost, s));

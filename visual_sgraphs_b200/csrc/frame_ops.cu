@@ -93,13 +93,13 @@ vsg_status vsg_undistort_keypoints(vsg_matcher *m, int n, const float *xy_in, do
     }
     CK(cudaSetDevice(m->device));
     vsg_status st;
-    if ((st = matcher_ensure(m, 6, (size_t)n * 8)) || (st = matcher_ensure(m, 7, (size_t)n * 8))) return st;
+    if ((st = matcher_ensure(m, kSlotOut, (size_t)n * 8)) || (st = matcher_ensure(m, kSlotAreaQueries, (size_t)n * 8))) return st;
     cudaStream_t s = m->stream;
-    CK(cudaMemcpyAsync(m->buf[6], xy_in, (size_t)n * 8, cudaMemcpyHostToDevice, s));
-    undistort_kernel<<<(n + 127) / 128, 128, 0, s>>>(c, (const float2 *)m->buf[6], n, (float2 *)m->buf[7]);
+    CK(cudaMemcpyAsync(m->buf[kSlotOut], xy_in, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+    undistort_kernel<<<(n + 127) / 128, 128, 0, s>>>(c, (const float2 *)m->buf[kSlotOut], n, (float2 *)m->buf[kSlotAreaQueries]);
     count_launch();
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(xy_out, m->buf[7], (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(xy_out, m->buf[kSlotAreaQueries], (size_t)n * 8, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VSG_OK;
 }
@@ -127,13 +127,13 @@ vsg_status vsg_undistort_keypoints_batch(vsg_matcher *m, vsg_extractor *ex, int 
     CK(cudaStreamSynchronize(pr.stream));
     const int cap = pr.out_cap;
     vsg_status st;
-    if ((st = matcher_ensure(m, 7, (size_t)nframes * cap * 8))) return st;
+    if ((st = matcher_ensure(m, kSlotAreaQueries, (size_t)nframes * cap * 8))) return st;
     cudaStream_t s = m->stream;
     undistort_batch_kernel<<<dim3((cap + 127) / 128, nframes), 128, 0, s>>>(c, pr.kps_dev, pr.n_dev, cap, identity,
-                                                                            (float2 *)m->buf[7]);
+                                                                            (float2 *)m->buf[kSlotAreaQueries]);
     count_launch();
     CK(cudaGetLastError());
-    CK(cudaMemcpy2DAsync(xy_out, (size_t)capacity * 8, m->buf[7], (size_t)cap * 8, (size_t)cap * 8, nframes,
+    CK(cudaMemcpy2DAsync(xy_out, (size_t)capacity * 8, m->buf[kSlotAreaQueries], (size_t)cap * 8, (size_t)cap * 8, nframes,
                          cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VSG_OK;

@@ -257,11 +257,11 @@ vsg_status knn2_tc_device(vsg_matcher *m, const uint8_t *q_dev, int nq, const ui
     nseg = (ntiles + tiles_per_seg - 1) / tiles_per_seg;
     const int nitems = n_mb * nseg;
     vsg_status st;
-    if ((st = matcher_ensure(m, 14, (size_t)nq * 256)) || (st = matcher_ensure(m, 15, (size_t)nt * 256)) ||
-        (st = matcher_ensure(m, 16, (size_t)nseg * nq * 2 * sizeof(int32_t) * 2)))
+    if ((st = matcher_ensure(m, kSlotTcQuery, (size_t)nq * 256)) || (st = matcher_ensure(m, kSlotTcTrain, (size_t)nt * 256)) ||
+        (st = matcher_ensure(m, kSlotTcParts, (size_t)nseg * nq * 2 * sizeof(int32_t) * 2)))
         return st;
-    int8_t *q8 = (int8_t *)m->buf[14], *t8 = (int8_t *)m->buf[15];
-    int32_t *part_idx = (int32_t *)m->buf[16], *part_dist = part_idx + (size_t)nseg * nq * 2;
+    int8_t *q8 = (int8_t *)m->buf[kSlotTcQuery], *t8 = (int8_t *)m->buf[kSlotTcTrain];
+    int32_t *part_idx = (int32_t *)m->buf[kSlotTcParts], *part_dist = part_idx + (size_t)nseg * nq * 2;
     cudaStream_t s = m->stream;
     expand_pm1_kernel<<<(unsigned)(((int64_t)nq * 8 + 255) / 256), 256, 0, s>>>((const uint32_t *)q_dev, nq, q8);
     expand_pm1_kernel<<<(unsigned)(((int64_t)nt * 8 + 255) / 256), 256, 0, s>>>((const uint32_t *)t_dev, nt, t8);

@@ -86,19 +86,19 @@ vsg_status vsg_distinctive_descriptors(vsg_matcher *m, const uint8_t *descriptor
     if (total > 0 && !descriptors) return VSG_ERR_INVALID;
     CK(cudaSetDevice(m->device));
     vsg_status st;
-    if ((st = matcher_ensure(m, 1, (size_t)std::max(total, 1) * 32)) || (st = matcher_ensure(m, 3, (size_t)(npoints + 1) * 4)) ||
-        (st = matcher_ensure(m, 6, (size_t)npoints * 4)))
+    if ((st = matcher_ensure(m, kSlotArg1, (size_t)std::max(total, 1) * 32)) || (st = matcher_ensure(m, kSlotArg3, (size_t)(npoints + 1) * 4)) ||
+        (st = matcher_ensure(m, kSlotOut, (size_t)npoints * 4)))
         return st;
     cudaStream_t s = m->stream;
-    if (total > 0) CK(cudaMemcpyAsync(m->buf[1], descriptors, (size_t)total * 32, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[3], ptr, (size_t)(npoints + 1) * 4, cudaMemcpyHostToDevice, s));
+    if (total > 0) CK(cudaMemcpyAsync(m->buf[kSlotArg1], descriptors, (size_t)total * 32, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(m->buf[kSlotArg3], ptr, (size_t)(npoints + 1) * 4, cudaMemcpyHostToDevice, s));
     const size_t smem = (size_t)std::min(longest, kDistinctSmemRows) * 32;
     if (smem > 48 * 1024) CK(cudaFuncSetAttribute(distinctive_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    distinctive_kernel<<<npoints, kDistinctThreads, smem, s>>>((const uint4 *)m->buf[1], (const int *)m->buf[3], npoints,
-                                                             (int *)m->buf[6]);
+    distinctive_kernel<<<npoints, kDistinctThreads, smem, s>>>((const uint4 *)m->buf[kSlotArg1], (const int *)m->buf[kSlotArg3], npoints,
+                                                             (int *)m->buf[kSlotOut]);
     count_launch();
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(best_out, m->buf[6], (size_t)npoints * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(best_out, m->buf[kSlotOut], (size_t)npoints * 4, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VSG_OK;
 }

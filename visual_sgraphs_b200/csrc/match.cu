@@ -17,7 +17,7 @@
 
 namespace vsg {
 
-vsg_status matcher_ensure(vsg_matcher *m, int slot, size_t bytes) {
+vsg_status matcher_ensure(vsg_matcher *m, DevSlot slot, size_t bytes) {
     if (m->cap[slot] >= bytes) return VSG_OK;
     if (m->buf[slot]) cudaFree(m->buf[slot]);
     m->buf[slot] = nullptr;
@@ -27,7 +27,7 @@ vsg_status matcher_ensure(vsg_matcher *m, int slot, size_t bytes) {
     m->cap[slot] = want;
     return VSG_OK;
 }
-vsg_status matcher_ensure_host(vsg_matcher *m, int slot, size_t bytes) {
+vsg_status matcher_ensure_host(vsg_matcher *m, HostSlot slot, size_t bytes) {
     if (m->hcap[slot] >= bytes) return VSG_OK;
     if (m->hbuf[slot]) cudaFreeHost(m->hbuf[slot]);
     m->hbuf[slot] = nullptr;
@@ -37,7 +37,6 @@ vsg_status matcher_ensure_host(vsg_matcher *m, int slot, size_t bytes) {
     m->hcap[slot] = want;
     return VSG_OK;
 }
-static vsg_status ensure(vsg_matcher *m, int slot, size_t bytes) { return matcher_ensure(m, slot, bytes); }
 
 __device__ __forceinline__ int hamming256(const uint4 &a0, const uint4 &a1, const uint4 &b0, const uint4 &b1) {
     return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) +
@@ -323,9 +322,9 @@ static vsg_status knn2_device(vsg_matcher *m, const uint8_t *q_dev, int nq, cons
     if (knn2_tc_supported(nq, nt)) return knn2_tc_device(m, q_dev, nq, t_dev, nt, offset, idx_dev, dist_dev);
     int qtiles, nchunks, chunk_rows;
     knn2_plan(m, nq, nt, &qtiles, &nchunks, &chunk_rows);
-    vsg_status st = ensure(m, 0, (size_t)nchunks * nq * 2 * sizeof(unsigned));
+    vsg_status st = matcher_ensure(m, kSlotKnnParts, (size_t)nchunks * nq * 2 * sizeof(unsigned));
     if (st != VSG_OK) return st;
-    unsigned *part = (unsigned *)m->buf[0];
+    unsigned *part = (unsigned *)m->buf[kSlotKnnParts];
     if (nt > 0) {
         knn2_kernel<<<dim3(qtiles, nchunks), kKnnThreads, 0, m->stream>>>((const uint4 *)q_dev, nq, (const uint4 *)t_dev, nt,
                                                                           chunk_rows, part);
@@ -394,13 +393,13 @@ vsg_status vsg_descriptor_distance(vsg_matcher *m, const uint8_t *a, const uint8
     if (n == 0) return VSG_OK;
     CK(cudaSetDevice(m->device));
     vsg_status st;
-    if ((st = ensure(m, 1, (size_t)n * 32)) || (st = ensure(m, 2, (size_t)n * 32)) || (st = ensure(m, 3, (size_t)n * 4))) return st;
-    CK(cudaMemcpyAsync(m->buf[1], a, (size_t)n * 32, cudaMemcpyHostToDevice, m->stream));
-    CK(cudaMemcpyAsync(m->buf[2], b, (size_t)n * 32, cudaMemcpyHostToDevice, m->stream));
-    pair_distance_kernel<<<(n + 255) / 256, 256, 0, m->stream>>>((const uint4 *)m->buf[1], (const uint4 *)m->buf[2], n,
-                                                                (int *)m->buf[3]);
+    if ((st = matcher_ensure(m, kSlotArg1, (size_t)n * 32)) || (st = matcher_ensure(m, kSlotArg2, (size_t)n * 32)) || (st = matcher_ensure(m, kSlotArg3, (size_t)n * 4))) return st;
+    CK(cudaMemcpyAsync(m->buf[kSlotArg1], a, (size_t)n * 32, cudaMemcpyHostToDevice, m->stream));
+    CK(cudaMemcpyAsync(m->buf[kSlotArg2], b, (size_t)n * 32, cudaMemcpyHostToDevice, m->stream));
+    pair_distance_kernel<<<(n + 255) / 256, 256, 0, m->stream>>>((const uint4 *)m->buf[kSlotArg1], (const uint4 *)m->buf[kSlotArg2], n,
+                                                                (int *)m->buf[kSlotArg3]);
     count_launch();
-    CK(cudaMemcpyAsync(out, m->buf[3], (size_t)n * 4, cudaMemcpyDeviceToHost, m->stream));
+    CK(cudaMemcpyAsync(out, m->buf[kSlotArg3], (size_t)n * 4, cudaMemcpyDeviceToHost, m->stream));
     CK(cudaStreamSynchronize(m->stream));
     return VSG_OK;
 }
@@ -420,16 +419,16 @@ vsg_status vsg_knn2(vsg_matcher *m, const uint8_t *query, int nq, const uint8_t 
     if (nq == 0) return VSG_OK;
     CK(cudaSetDevice(m->device));
     vsg_status st;
-    if ((st = ensure(m, 1, (size_t)nq * 32)) || (st = ensure(m, 2, (size_t)std::max(nt, 1) * 32)) ||
-        (st = ensure(m, 3, (size_t)nq * 8)) || (st = ensure(m, 4, (size_t)nq * 8)))
+    if ((st = matcher_ensure(m, kSlotArg1, (size_t)nq * 32)) || (st = matcher_ensure(m, kSlotArg2, (size_t)std::max(nt, 1) * 32)) ||
+        (st = matcher_ensure(m, kSlotArg3, (size_t)nq * 8)) || (st = matcher_ensure(m, kSlotArg4, (size_t)nq * 8)))
         return st;
-    CK(cudaMemcpyAsync(m->buf[1], query, (size_t)nq * 32, cudaMemcpyHostToDevice, m->stream));
-    if (nt) CK(cudaMemcpyAsync(m->buf[2], train, (size_t)nt * 32, cudaMemcpyHostToDevice, m->stream));
-    st = knn2_device(m, (const uint8_t *)m->buf[1], nq, (const uint8_t *)m->buf[2], nt, train_index_offset, (int *)m->buf[3],
-                     (int *)m->buf[4]);
+    CK(cudaMemcpyAsync(m->buf[kSlotArg1], query, (size_t)nq * 32, cudaMemcpyHostToDevice, m->stream));
+    if (nt) CK(cudaMemcpyAsync(m->buf[kSlotArg2], train, (size_t)nt * 32, cudaMemcpyHostToDevice, m->stream));
+    st = knn2_device(m, (const uint8_t *)m->buf[kSlotArg1], nq, (const uint8_t *)m->buf[kSlotArg2], nt, train_index_offset, (int *)m->buf[kSlotArg3],
+                     (int *)m->buf[kSlotArg4]);
     if (st != VSG_OK) return st;
-    CK(cudaMemcpyAsync(out_idx, m->buf[3], (size_t)nq * 8, cudaMemcpyDeviceToHost, m->stream));
-    CK(cudaMemcpyAsync(out_dist, m->buf[4], (size_t)nq * 8, cudaMemcpyDeviceToHost, m->stream));
+    CK(cudaMemcpyAsync(out_idx, m->buf[kSlotArg3], (size_t)nq * 8, cudaMemcpyDeviceToHost, m->stream));
+    CK(cudaMemcpyAsync(out_dist, m->buf[kSlotArg4], (size_t)nq * 8, cudaMemcpyDeviceToHost, m->stream));
     CK(cudaStreamSynchronize(m->stream));
     return VSG_OK;
 }
@@ -460,8 +459,8 @@ vsg_status vsg_knn2_sharded(vsg_comm *comm, vsg_matcher *m, const uint8_t *query
     const int nranks = comm_size(comm);
     const size_t part = (size_t)nq * 2 * sizeof(int32_t);
     vsg_status st;
-    if ((st = ensure(m, 13, 2 * part * (size_t)(nranks + 1)))) return st;
-    int32_t *my_idx = (int32_t *)m->buf[13], *my_dist = my_idx + (size_t)nq * 2;
+    if ((st = matcher_ensure(m, kSlotKnnSharded, 2 * part * (size_t)(nranks + 1)))) return st;
+    int32_t *my_idx = (int32_t *)m->buf[kSlotKnnSharded], *my_dist = my_idx + (size_t)nq * 2;
     int32_t *all_idx = my_dist + (size_t)nq * 2, *all_dist = all_idx + (size_t)nq * 2 * nranks;
     if ((st = knn2_device(m, query_dev, nq, train_shard_dev, nt_shard, train_index_offset, my_idx, my_dist)) != VSG_OK) return st;
     if ((st = comm_all_gather(comm, my_idx, all_idx, part, m->stream)) != VSG_OK) return st;
@@ -482,23 +481,22 @@ vsg_status vsg_match_window(vsg_matcher *m, const uint8_t *query, int nq, const 
     if (ncand < 0 || (ncand > 0 && (!cand || !train))) return VSG_ERR_INVALID;
     CK(cudaSetDevice(m->device));
     vsg_status st;
-    // slots: 1 query, 2 train, 3 cand_ptr, 4 cand, 5 skip + level, 6 outputs (5 x nq ints)
-    if ((st = ensure(m, 1, (size_t)nq * 32)) || (st = ensure(m, 2, (size_t)std::max(nt, 1) * 32)) ||
-        (st = ensure(m, 3, (size_t)(nq + 1) * 4)) || (st = ensure(m, 4, (size_t)std::max(ncand, 1) * 4)) ||
-        (st = ensure(m, 5, (size_t)std::max(nt, 1) * 5 + 16)) || (st = ensure(m, 6, (size_t)nq * 20)))
+    if ((st = matcher_ensure(m, kSlotArg1, (size_t)nq * 32)) || (st = matcher_ensure(m, kSlotArg2, (size_t)std::max(nt, 1) * 32)) ||
+        (st = matcher_ensure(m, kSlotArg3, (size_t)(nq + 1) * 4)) || (st = matcher_ensure(m, kSlotArg4, (size_t)std::max(ncand, 1) * 4)) ||
+        (st = matcher_ensure(m, kSlotArg5, (size_t)std::max(nt, 1) * 5 + 16)) || (st = matcher_ensure(m, kSlotOut, (size_t)nq * 20)))
         return st;
     cudaStream_t s = m->stream;
-    CK(cudaMemcpyAsync(m->buf[1], query, (size_t)nq * 32, cudaMemcpyHostToDevice, s));
-    if (nt) CK(cudaMemcpyAsync(m->buf[2], train, (size_t)nt * 32, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[3], cand_ptr, (size_t)(nq + 1) * 4, cudaMemcpyHostToDevice, s));
-    if (ncand) CK(cudaMemcpyAsync(m->buf[4], cand, (size_t)ncand * 4, cudaMemcpyHostToDevice, s));
-    int *lvl_dev = (int *)m->buf[5];
-    uint8_t *skip_dev = (uint8_t *)m->buf[5] + (size_t)std::max(nt, 1) * 4;
+    CK(cudaMemcpyAsync(m->buf[kSlotArg1], query, (size_t)nq * 32, cudaMemcpyHostToDevice, s));
+    if (nt) CK(cudaMemcpyAsync(m->buf[kSlotArg2], train, (size_t)nt * 32, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(m->buf[kSlotArg3], cand_ptr, (size_t)(nq + 1) * 4, cudaMemcpyHostToDevice, s));
+    if (ncand) CK(cudaMemcpyAsync(m->buf[kSlotArg4], cand, (size_t)ncand * 4, cudaMemcpyHostToDevice, s));
+    int *lvl_dev = (int *)m->buf[kSlotArg5];
+    uint8_t *skip_dev = (uint8_t *)m->buf[kSlotArg5] + (size_t)std::max(nt, 1) * 4;
     if (train_level && nt) CK(cudaMemcpyAsync(lvl_dev, train_level, (size_t)nt * 4, cudaMemcpyHostToDevice, s));
     if (skip && nt) CK(cudaMemcpyAsync(skip_dev, skip, (size_t)nt, cudaMemcpyHostToDevice, s));
-    int *o = (int *)m->buf[6];
-    window_match_kernel<<<(nq + 127) / 128, 128, 0, s>>>((const uint4 *)m->buf[1], nq, (const uint4 *)m->buf[2],
-                                                        (const int *)m->buf[3], (const int *)m->buf[4],
+    int *o = (int *)m->buf[kSlotOut];
+    window_match_kernel<<<(nq + 127) / 128, 128, 0, s>>>((const uint4 *)m->buf[kSlotArg1], nq, (const uint4 *)m->buf[kSlotArg2],
+                                                        (const int *)m->buf[kSlotArg3], (const int *)m->buf[kSlotArg4],
                                                         skip ? skip_dev : nullptr, train_level ? lvl_dev : nullptr,
                                                         init_dist, o, o + nq, o + 2 * nq, o + 3 * nq, o + 4 * nq);
     count_launch();

@@ -242,25 +242,26 @@ vsg_status area_best(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery
     if (nq == 0) return VSG_OK;
     cudaStream_t s = m->stream;
     vsg_status st;
-    // device slots: 7 queries, 8 qdesc, 9 results; pinned host slot 0
-    if ((st = matcher_ensure(m, 7, (size_t)nq * sizeof(AreaQuery))) || (st = matcher_ensure(m, 8, (size_t)nq * 32)) ||
-        (st = matcher_ensure(m, 9, (size_t)nq * sizeof(int2))) || (st = matcher_ensure_host(m, 0, (size_t)nq * sizeof(int2))))
+    if ((st = matcher_ensure(m, kSlotAreaQueries, (size_t)nq * sizeof(AreaQuery))) ||
+        (st = matcher_ensure(m, kSlotAreaQdesc, (size_t)nq * 32)) || (st = matcher_ensure(m, kSlotAreaCounts, (size_t)nq * sizeof(int2))) ||
+        (st = matcher_ensure_host(m, kHostAreaCounts, (size_t)nq * sizeof(int2))))
         return st;
-    CK(cudaMemcpyAsync(m->buf[7], qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[8], qdesc, (size_t)nq * 32, cudaMemcpyHostToDevice, s));
+    AreaQuery *qs_d = (AreaQuery *)m->buf[kSlotAreaQueries];
+    uint4 *qdesc_d = (uint4 *)m->buf[kSlotAreaQdesc];
+    int2 *best_d = (int2 *)m->buf[kSlotAreaCounts];
+    CK(cudaMemcpyAsync(qs_d, qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(qdesc_d, qdesc, (size_t)nq * 32, cudaMemcpyHostToDevice, s));
     const FrameDev fd = frame_dev(f);
     const Chi2Gate gate = chi2_gate(f, inv_sigma2);
     if (inv_sigma2)
-        window_best_kernel<true><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, (const AreaQuery *)m->buf[7], (const uint4 *)m->buf[8], gate,
-                                                              (int2 *)m->buf[9]);
+        window_best_kernel<true><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, qs_d, qdesc_d, gate, best_d);
     else
-        window_best_kernel<false><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, (const AreaQuery *)m->buf[7], (const uint4 *)m->buf[8], gate,
-                                                               (int2 *)m->buf[9]);
+        window_best_kernel<false><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, qs_d, qdesc_d, gate, best_d);
     count_launch();
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(m->hbuf[0], m->buf[9], (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(m->hbuf[kHostAreaCounts], best_d, (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    memcpy(out.data(), m->hbuf[0], (size_t)nq * sizeof(int2));
+    memcpy(out.data(), m->hbuf[kHostAreaCounts], (size_t)nq * sizeof(int2));
     return VSG_OK;
 }
 
@@ -271,15 +272,13 @@ vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const 
     cudaStream_t s = m->stream;
     vsg_status st;
     // one staging block, one H2D copy: target table, queries, their targets, descriptor rows (16-byte aligned sections)
-    auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
     const size_t o_tgt = 0, o_q = o_tgt + up16((size_t)ntargets * sizeof(FuseTarget)),
                  o_qt = o_q + up16((size_t)nq * sizeof(AreaQuery)), o_desc = o_qt + up16((size_t)nq * sizeof(int)),
                  total = o_desc + (size_t)n_qdesc * 32;
-    // device slots: 17 inputs, 18 results; pinned host slots: 7 inputs, 5 results
-    if ((st = matcher_ensure(m, 17, total)) || (st = matcher_ensure(m, 18, (size_t)nq * sizeof(int2))) ||
-        (st = matcher_ensure_host(m, 7, total)) || (st = matcher_ensure_host(m, 5, (size_t)nq * sizeof(int2))))
+    if ((st = matcher_ensure(m, kSlotBestMultiIn, total)) || (st = matcher_ensure(m, kSlotBestMultiOut, (size_t)nq * sizeof(int2))) ||
+        (st = matcher_ensure_host(m, kHostBestMultiIn, total)) || (st = matcher_ensure_host(m, kHostBestMultiOut, (size_t)nq * sizeof(int2))))
         return st;
-    uint8_t *h = (uint8_t *)m->hbuf[7], *d = (uint8_t *)m->buf[17];
+    uint8_t *h = (uint8_t *)m->hbuf[kHostBestMultiIn], *d = (uint8_t *)m->buf[kSlotBestMultiIn];
     FuseTarget *ht = (FuseTarget *)(h + o_tgt);
     for (int t = 0; t < ntargets; ++t) ht[t] = FuseTarget{frame_dev(frames[t]), chi2_gate(frames[t], inv_sigma2[t])};
     memcpy(h + o_q, qs, (size_t)nq * sizeof(AreaQuery));
@@ -287,13 +286,54 @@ vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const 
     memcpy(h + o_desc, qdesc, (size_t)n_qdesc * 32);
     CK(cudaMemcpyAsync(d, h, total, cudaMemcpyHostToDevice, s));
     window_best_multi_kernel<<<(nq + 7) / 8, 256, 0, s>>>((const FuseTarget *)(d + o_tgt), nq, (const AreaQuery *)(d + o_q),
-                                                          (const int *)(d + o_qt), (const uint4 *)(d + o_desc), (int2 *)m->buf[18]);
+                                                          (const int *)(d + o_qt), (const uint4 *)(d + o_desc),
+                                                          (int2 *)m->buf[kSlotBestMultiOut]);
     count_launch();
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(m->hbuf[5], m->buf[18], (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(m->hbuf[kHostBestMultiOut], m->buf[kSlotBestMultiOut], (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    memcpy(out.data(), m->hbuf[5], (size_t)nq * sizeof(int2));
+    memcpy(out.data(), m->hbuf[kHostBestMultiOut], (size_t)nq * sizeof(int2));
     return VSG_OK;
+}
+
+// The window search both list forms share: uploads the queries and n_qdesc descriptor rows, launches area_search_kernel with
+// room for init_cap entries (or more if the slot already has it) and, if the lists overflow that, once more with room for all
+// of them.  The lists stay on the device (kSlotAreaCounts: off[nq], cnt[nq], total; kSlotAreaRaw: the entries); host slot
+// kHostAreaCounts (host_ints ints) receives off, cnt and total if with_offsets, else the total alone.
+static vsg_status area_search_launch(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc,
+                                     int n_qdesc, size_t init_cap, bool with_offsets, size_t host_ints, PhaseTimer &pt, int *total) {
+    cudaStream_t s = m->stream;
+    vsg_status st;
+    if ((st = matcher_ensure(m, kSlotAreaQueries, (size_t)nq * sizeof(AreaQuery))) ||
+        (st = matcher_ensure(m, kSlotAreaQdesc, (size_t)n_qdesc * 32)) ||
+        (st = matcher_ensure(m, kSlotAreaCounts, (size_t)(2 * nq + 1) * sizeof(int))) ||
+        (st = matcher_ensure_host(m, kHostAreaCounts, host_ints * sizeof(int))))
+        return st;
+    CK(cudaMemcpyAsync(m->buf[kSlotAreaQueries], qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(m->buf[kSlotAreaQdesc], qdesc, (size_t)n_qdesc * 32, cudaMemcpyHostToDevice, s));
+    int *off_d = (int *)m->buf[kSlotAreaCounts], *total_d = off_d + 2 * nq;
+    int *host = (int *)m->hbuf[kHostAreaCounts];
+    const FrameDev fd = frame_dev(f);
+    size_t cap = std::max<size_t>(m->cap[kSlotAreaRaw] / sizeof(int2), init_cap);
+    for (int attempt = 0; attempt < 2; ++attempt) {
+        if ((st = matcher_ensure(m, kSlotAreaRaw, cap * sizeof(int2)))) return st;
+        CK(cudaMemsetAsync(total_d, 0, sizeof(int), s));
+        area_search_kernel<<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, (const AreaQuery *)m->buf[kSlotAreaQueries],
+                                                       (const uint4 *)m->buf[kSlotAreaQdesc], off_d, off_d + nq,
+                                                       (int2 *)m->buf[kSlotAreaRaw], (int)cap, total_d);
+        count_launch();
+        if (with_offsets)
+            CK(cudaMemcpyAsync(host, off_d, (size_t)(2 * nq + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
+        else
+            CK(cudaMemcpyAsync(host, total_d, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        pt.mark(with_offsets ? "H2D + kernel + D2H of offsets" : "H2D + kernel + D2H of the total");
+        *total = host[with_offsets ? 2 * nq : 0];
+        if ((size_t)*total <= cap) return VSG_OK;
+        cap = (size_t)*total + 1024;             // retry once with the exact size
+    }
+    set_error("area_search: candidate buffer overflow");
+    return VSG_ERR_CAPACITY;
 }
 
 vsg_status area_search_raw(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc,
@@ -301,46 +341,20 @@ vsg_status area_search_raw(vsg_matcher *m, const vsg_frame *f, int nq, const Are
     PhaseTimer pt("area_search");
     *out = AreaLists();
     if (nq == 0) return VSG_OK;
-    cudaStream_t s = m->stream;
-    vsg_status st;
-    // device slots: 7 queries, 8 qdesc, 9 off/cnt/total, 10 out entries; pinned host slots: 0 off/cnt/total, 1 entries
-    if ((st = matcher_ensure(m, 7, (size_t)nq * sizeof(AreaQuery))) || (st = matcher_ensure(m, 8, (size_t)n_qdesc * 32)) ||
-        (st = matcher_ensure(m, 9, (size_t)(2 * nq + 1) * sizeof(int))) ||
-        (st = matcher_ensure_host(m, 0, (size_t)(2 * nq + 1) * sizeof(int))))
-        return st;
-    CK(cudaMemcpyAsync(m->buf[7], qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[8], qdesc, (size_t)n_qdesc * 32, cudaMemcpyHostToDevice, s));
-    int *off_d = (int *)m->buf[9], *cnt_d = off_d + nq, *total_d = off_d + 2 * nq;
-    int *host = (int *)m->hbuf[0];
-    FrameDev fd{f->n, f->cols, f->rows, f->min_x, f->min_y, f->inv_w, f->inv_h, f->xy, f->octave,
-                f->has_right ? f->u_right : nullptr, (const uint4 *)f->desc, f->cell_ptr, f->cell_idx};
-    size_t cap = std::max<size_t>(m->cap[10] / sizeof(int2), (size_t)nq * 32);
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        if ((st = matcher_ensure(m, 10, cap * sizeof(int2)))) return st;
-        CK(cudaMemsetAsync(total_d, 0, sizeof(int), s));
-        area_search_kernel<<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, (const AreaQuery *)m->buf[7], (const uint4 *)m->buf[8],
-                                                       off_d, cnt_d, (int2 *)m->buf[10], (int)cap, total_d);
-        count_launch();
-        CK(cudaMemcpyAsync(host, off_d, (size_t)(2 * nq + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        pt.mark("H2D + kernel + D2H of offsets");
-        const int total = host[2 * nq];
-        if ((size_t)total <= cap) {
-            if ((st = matcher_ensure_host(m, 1, (size_t)std::max(total, 1) * sizeof(int2)))) return st;
-            if (total) {
-                CK(cudaMemcpyAsync(m->hbuf[1], m->buf[10], (size_t)total * sizeof(int2), cudaMemcpyDeviceToHost, s));
-                CK(cudaStreamSynchronize(s));
-            }
-            pt.mark("D2H of entries");
-            out->raw = (const int2 *)m->hbuf[1];
-            out->off = host;
-            out->cnt = host + nq;
-            return VSG_OK;
-        }
-        cap = (size_t)total + 1024;             // retry once with the exact size
+    int total;
+    vsg_status st = area_search_launch(m, f, nq, qs, qdesc, n_qdesc, (size_t)nq * 32, true, (size_t)(2 * nq + 1), pt, &total);
+    if (st != VSG_OK || (st = matcher_ensure_host(m, kHostAreaEnt, (size_t)std::max(total, 1) * sizeof(int2)))) return st;
+    if (total) {
+        CK(cudaMemcpyAsync(m->hbuf[kHostAreaEnt], m->buf[kSlotAreaRaw], (size_t)total * sizeof(int2), cudaMemcpyDeviceToHost,
+                           m->stream));
+        CK(cudaStreamSynchronize(m->stream));
     }
-    set_error("area_search: candidate buffer overflow");
-    return VSG_ERR_CAPACITY;
+    pt.mark("D2H of entries");
+    const int *host = (const int *)m->hbuf[kHostAreaCounts];
+    out->raw = (const int2 *)m->hbuf[kHostAreaEnt];
+    out->off = host;
+    out->cnt = host + nq;
+    return VSG_OK;
 }
 
 // Exclusive prefix sum of the per-query counts by one CTA (tiles of 1024 with a running carry): ptr[q] = position of query
@@ -406,67 +420,44 @@ vsg_status area_search_ordered(vsg_matcher *m, const vsg_frame *f, int nq, const
     PhaseTimer pt("area_search");
     *out = OrderedLists();
     if (nq == 0) return VSG_OK;
-    cudaStream_t s = m->stream;
-    vsg_status st;
-    // device slots: 7 queries, 8 qdesc, 9 off/cnt/total, 10 raw entries, 11 ptr + qid, 6 ordered entries;
-    // pinned host slots: 0 ptr, 1 entries, 4 qid
-    if ((st = matcher_ensure(m, 7, (size_t)nq * sizeof(AreaQuery))) || (st = matcher_ensure(m, 8, (size_t)n_qdesc * 32)) ||
-        (st = matcher_ensure(m, 9, (size_t)(2 * nq + 1) * sizeof(int))) ||
-        (st = matcher_ensure_host(m, 0, (size_t)(nq + 2) * sizeof(int))))
+    int total;
+    vsg_status st = area_search_launch(m, f, nq, qs, qdesc, n_qdesc, (size_t)nq * 4, false, (size_t)nq + 2, pt, &total);
+    if (st != VSG_OK) return st;
+    if ((st = matcher_ensure(m, kSlotAreaOrder, ((size_t)nq + 1 + std::max(total, 1)) * sizeof(int))) ||
+        (st = matcher_ensure(m, kSlotOut, (size_t)std::max(total, 1) * sizeof(int2))) ||
+        (st = matcher_ensure_host(m, kHostAreaEnt, (size_t)std::max(total, 1) * sizeof(int2))) ||
+        (st = matcher_ensure_host(m, kHostAreaQid, (size_t)std::max(total, 1) * sizeof(int))))
         return st;
-    CK(cudaMemcpyAsync(m->buf[7], qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[8], qdesc, (size_t)n_qdesc * 32, cudaMemcpyHostToDevice, s));
-    int *off_d = (int *)m->buf[9], *cnt_d = off_d + nq, *total_d = off_d + 2 * nq;
-    int *host = (int *)m->hbuf[0];
-    FrameDev fd{f->n, f->cols, f->rows, f->min_x, f->min_y, f->inv_w, f->inv_h, f->xy, f->octave,
-                f->has_right ? f->u_right : nullptr, (const uint4 *)f->desc, f->cell_ptr, f->cell_idx};
-    size_t cap = std::max<size_t>(m->cap[10] / sizeof(int2), (size_t)nq * 4);
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        if ((st = matcher_ensure(m, 10, cap * sizeof(int2)))) return st;
-        CK(cudaMemsetAsync(total_d, 0, sizeof(int), s));
-        area_search_kernel<<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, (const AreaQuery *)m->buf[7], (const uint4 *)m->buf[8],
-                                                       off_d, cnt_d, (int2 *)m->buf[10], (int)cap, total_d);
-        count_launch();
-        CK(cudaMemcpyAsync(host, total_d, sizeof(int), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        pt.mark("H2D + kernel + D2H of the total");
-        const int total = host[0];
-        if ((size_t)total > cap) { cap = (size_t)total + 1024; continue; }   // retry once with the exact size
-        if ((st = matcher_ensure(m, 11, ((size_t)nq + 1 + std::max(total, 1)) * sizeof(int))) ||
-            (st = matcher_ensure(m, 6, (size_t)std::max(total, 1) * sizeof(int2))) ||
-            (st = matcher_ensure_host(m, 1, (size_t)std::max(total, 1) * sizeof(int2))) ||
-            (st = matcher_ensure_host(m, 4, (size_t)std::max(total, 1) * sizeof(int))))
-            return st;
-        int *ptr_d = (int *)m->buf[11], *qid_d = ptr_d + nq + 1;
-        scan_counts_kernel<<<1, 1024, 0, s>>>(cnt_d, nq, ptr_d);
-        order_segments_kernel<<<(nq + 255) / 256, 256, 0, s>>>((const int2 *)m->buf[10], off_d, cnt_d, ptr_d, nq, (int2 *)m->buf[6],
-                                                               qid_d);
-        count_launch(2);
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(host, ptr_d, (size_t)(nq + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
-        if (total) {
-            CK(cudaMemcpyAsync(m->hbuf[1], m->buf[6], (size_t)total * sizeof(int2), cudaMemcpyDeviceToHost, s));
-            CK(cudaMemcpyAsync(m->hbuf[4], qid_d, (size_t)total * sizeof(int), cudaMemcpyDeviceToHost, s));
-        }
-        CK(cudaStreamSynchronize(s));
-        pt.mark("ordering + D2H of the lists");
-        out->ent = (const int2 *)m->hbuf[1];
-        out->qid = (const int *)m->hbuf[4];
-        out->ptr = host;
-        out->total = total;
-        return VSG_OK;
+    cudaStream_t s = m->stream;
+    const int *off_d = (const int *)m->buf[kSlotAreaCounts], *cnt_d = off_d + nq;
+    int *ptr_d = (int *)m->buf[kSlotAreaOrder], *qid_d = ptr_d + nq + 1;
+    int *host = (int *)m->hbuf[kHostAreaCounts];
+    scan_counts_kernel<<<1, 1024, 0, s>>>(cnt_d, nq, ptr_d);
+    order_segments_kernel<<<(nq + 255) / 256, 256, 0, s>>>((const int2 *)m->buf[kSlotAreaRaw], off_d, cnt_d, ptr_d, nq,
+                                                           (int2 *)m->buf[kSlotOut], qid_d);
+    count_launch(2);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(host, ptr_d, (size_t)(nq + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (total) {
+        CK(cudaMemcpyAsync(m->hbuf[kHostAreaEnt], m->buf[kSlotOut], (size_t)total * sizeof(int2), cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(m->hbuf[kHostAreaQid], qid_d, (size_t)total * sizeof(int), cudaMemcpyDeviceToHost, s));
     }
-    set_error("area_search: candidate buffer overflow");
-    return VSG_ERR_CAPACITY;
+    CK(cudaStreamSynchronize(s));
+    pt.mark("ordering + D2H of the lists");
+    out->ent = (const int2 *)m->hbuf[kHostAreaEnt];
+    out->qid = (const int *)m->hbuf[kHostAreaQid];
+    out->ptr = host;
+    out->total = total;
+    return VSG_OK;
 }
 
 // Runs the area search for nq queries and brings the lists back: ptr[nq+1] and (idx, dist) pairs in query order.
-vsg_status area_search(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc,
+vsg_status area_search(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc, int n_qdesc,
                        std::vector<int> &ptr, std::vector<int2> &ent) {
     ptr.assign(nq + 1, 0);
     ent.clear();
     AreaLists L;
-    vsg_status st = area_search_raw(m, f, nq, qs, qdesc, nq, &L);
+    vsg_status st = area_search_raw(m, f, nq, qs, qdesc, n_qdesc, &L);
     if (st != VSG_OK || nq == 0) return st;
     int total = 0;
     for (int q = 0; q < nq; ++q) total += L.cnt[q];
@@ -540,15 +531,114 @@ static int bow_replay_kf_f(const vsg_frame_view *KF, const vsg_frame_view *F, in
             }
         }
     }
-    if (check_ori) {
-        int ind1 = -1, ind2 = -1, ind3 = -1;
-        three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
-        for (int i = 0; i < HISTO_LENGTH; ++i) {
-            if (i == ind1 || i == ind2 || i == ind3) continue;
-            for (int idx : rot_hist[i]) { matches_f_out[idx] = -1; --nmatches; }
+    if (check_ori) apply_rot_filter(rot_hist, [&](int idx) { matches_f_out[idx] = -1; --nmatches; });
+    return nmatches;
+}
+
+// The window query of map point i (:60-74; the right camera's :146-151): RadiusByViewingCos (:218-224), times th unless th == 1, times the scale
+// of the predicted level; levels [level - 1, level]; descriptor row i.  `side` names the camera in the error message.
+static vsg_status map_point_query(const vsg_frame *F, const vsg_track_point &mp, int i, float th, float xr, int max_dist,
+                                  const char *side, AreaQuery *q) {
+    if (mp.level < 0 || mp.level >= (int)F->scale.size()) {
+        set_error("map point %d: %slevel %d out of range", i, side, mp.level);
+        return VSG_ERR_INVALID;
+    }
+    float r = (mp.view_cos > 0.998) ? 2.5f : 4.0f;
+    if (th != 1.0) r *= th;
+    const float win = r * F->scale[mp.level];
+    *q = AreaQuery{mp.proj_x, mp.proj_y, win, mp.level - 1, mp.level, xr, win, max_dist, i};
+    return VSG_OK;
+}
+
+// :48-74 for a single-camera frame: the queries of the map points that reach GetFeaturesInArea into qs and their map point
+// indices into q_mp (room for n_mp each), their number into *nq
+static vsg_status map_queries(const vsg_frame *F, int n_mp, const vsg_track_point *pts, float th, int far_points, float th_far,
+                              int max_dist, AreaQuery *qs, int *q_mp, int *nq) {
+    int k = 0;
+    for (int i = 0; i < n_mp; ++i) {
+        const vsg_track_point &mp = pts[i];
+        if (!mp.in_view) continue;
+        if (far_points && mp.depth > th_far) continue;
+        if (mp.bad) continue;
+        const vsg_status st = map_point_query(F, mp, i, th, mp.proj_xr, max_dist, "", qs + k);
+        if (st != VSG_OK) return st;
+        q_mp[k++] = i;
+    }
+    *nq = k;
+    return VSG_OK;
+}
+
+// The best / second-best-by-level scan of :76-141 over one map point's n candidates, cand(c) = (keypoint, distance), skipping
+// the blocked keypoints: whether the map point matches, and the keypoint it would take in *best_idx.
+enum class MapScan { NoCandidate, RatioRejected, Match };   // none <= TH_HIGH (:123); the `continue` of :124-125; a match
+template <class Cand>
+static MapScan map_scan(int n, Cand cand, const uint8_t *blocked, const vsg_keypoint *keys, float nnratio, int *best_idx) {
+    int best = 256, best_level = -1, best2 = 256, best_level2 = -1, idx = -1;
+    for (int c = 0; c < n; ++c) {
+        const int2 e = cand(c);
+        if (blocked[e.x]) continue;
+        if (e.y < best) { best2 = best; best = e.y; best_level2 = best_level; best_level = keys[e.x].octave; idx = e.x; }
+        else if (e.y < best2) { best_level2 = keys[e.x].octave; best2 = e.y; }
+    }
+    *best_idx = idx;
+    if (best > TH_HIGH) return MapScan::NoCandidate;
+    if (best_level == best_level2 && best > nnratio * best2) return MapScan::RatioRejected;
+    return MapScan::Match;
+}
+
+// ORBmatcher.cc:1667-1878 over the ncam cameras of the current frame Cur[0 .. ncam): the points of the last frame searched in
+// camera c around pts[c] (pts[0] carries the point's octave, angle and flags), their descriptors in desc.  With two cameras a
+// point's right-camera search (:1785-1852) is skipped when its left window was empty, whose `continue` (:1727-1728) skips it.
+static vsg_status projection_last(vsg_matcher *m, int ncam, const vsg_frame *const *Cur, const uint8_t *occupied, int n_last,
+                                  const vsg_proj_point *const *pts, const uint8_t *desc, float th, int mode, int check_ori,
+                                  int32_t *assign_out, int *nmatches_out) {
+    CK(cudaSetDevice(m->device));
+    std::vector<AreaQuery> qs[2];
+    std::vector<int> q_src;
+    for (int i = 0; i < n_last; ++i) {
+        const vsg_proj_point &p = pts[0][i];
+        if (!p.valid) continue;
+        if (p.octave < 0 || p.octave >= (int)Cur[0]->scale.size()) { set_error("point %d: octave %d out of range", i, p.octave); return VSG_ERR_INVALID; }
+        const float radius = th * Cur[0]->scale[p.octave];
+        int lo, hi;
+        if (mode == 1) { lo = p.octave; hi = -1; }                 // forward  (:1719-1720)
+        else if (mode == 2) { lo = 0; hi = p.octave; }             // backward (:1721-1722)
+        else { lo = p.octave - 1; hi = p.octave + 1; }             // :1723-1724
+        for (int cam = 0; cam < ncam; ++cam)
+            qs[cam].push_back(AreaQuery{pts[cam][i].u, pts[cam][i].v, radius, lo, hi, ncam == 1 ? p.ur : 0.f, radius});
+        q_src.push_back(i);
+    }
+    const int nq = (int)q_src.size();
+    std::vector<uint8_t> qdesc((size_t)nq * 32);
+    for (int k = 0; k < nq; ++k) memcpy(&qdesc[(size_t)k * 32], desc + (size_t)q_src[k] * 32, 32);
+    std::vector<int> ptr[2];
+    std::vector<int2> ent[2];
+    int N = 0;
+    for (int cam = 0; cam < ncam; ++cam) {
+        const vsg_status st = area_search(m, Cur[cam], nq, qs[cam].data(), qdesc.data(), nq, ptr[cam], ent[cam]);
+        if (st != VSG_OK) return st;
+        N += Cur[cam]->n;
+    }
+    std::vector<uint8_t> blocked(occupied, occupied + N);
+    for (int i = 0; i < N; ++i) assign_out[i] = -1;
+    std::vector<int> rot_hist[HISTO_LENGTH];
+    int nmatches = 0;
+    for (int k = 0; k < nq; ++k) {
+        const vsg_proj_point &p = pts[0][q_src[k]];
+        if (ncam == 2 && ptr[0][k] == ptr[0][k + 1]) continue;     // vIndices2.empty() -> continue: no right-camera search either
+        for (int cam = 0, offset = 0; cam < ncam; offset += Cur[cam]->n, ++cam) {
+            const int2 b = nearest_unclaimed(ent[cam].data() + ptr[cam][k], ent[cam].data() + ptr[cam][k + 1], blocked.data() + offset);
+            if (b.x <= TH_HIGH) {
+                assign_out[b.y + offset] = q_src[k];
+                blocked[b.y + offset] = p.blocks;
+                ++nmatches;
+                if (check_ori) rot_hist[rot_bin(p.angle, Cur[cam]->keys[b.y].angle)].push_back(b.y + offset);
+            }
         }
     }
-    return nmatches;
+    if (check_ori) apply_rot_filter(rot_hist, [&](int idx) { assign_out[idx] = -2; --nmatches; });
+    if (nmatches_out) *nmatches_out = nmatches;
+    return VSG_OK;
 }
 
 }  // namespace vsg
@@ -597,14 +687,13 @@ vsg_status vsg_frame_create(vsg_matcher *m, const vsg_frame_view *v, vsg_frame *
     // One pinned staging block, one stream-ordered device allocation, one H2D copy (a Search* call of the drop-in
     // classes uploads a frame every time: six cudaMalloc / cudaFree pairs per call cost more than the search itself).
     const size_t n1 = std::max(v->n, 1);
-    auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
     const size_t o_xy = 0, o_oct = o_xy + up16(n1 * sizeof(float2)), o_ur = o_oct + up16(n1 * sizeof(int)),
                  o_desc = o_ur + up16(n1 * sizeof(float)), o_cptr = o_desc + up16(n1 * 32),
                  o_cidx = o_cptr + up16((size_t)(ncell + 1) * sizeof(int)),
                  total = o_cidx + up16(std::max<size_t>(cidx.size(), 1) * sizeof(int));
-    vsg_status st = matcher_ensure_host(m, 2, total);
+    vsg_status st = matcher_ensure_host(m, kHostFrameStaging, total);
     if (st != VSG_OK) { delete f; return st; }
-    uint8_t *h = (uint8_t *)m->hbuf[2];
+    uint8_t *h = (uint8_t *)m->hbuf[kHostFrameStaging];
     float2 *hxy = (float2 *)(h + o_xy);
     int *hoct = (int *)(h + o_oct);
     for (int i = 0; i < v->n; ++i) { hxy[i] = make_float2(v->keys[i].x, v->keys[i].y); hoct[i] = v->keys[i].octave; }
@@ -644,7 +733,7 @@ vsg_status vsg_area_search(vsg_matcher *m, const vsg_frame *f, int nq, const flo
         qs[i] = AreaQuery{qx[i], qy[i], qr[i], min_level ? min_level[i] : -1, max_level ? max_level[i] : -1, 0.f, -1.f};
     std::vector<int> ptr;
     std::vector<int2> ent;
-    vsg_status st = area_search(m, f, nq, qs.data(), qdesc, ptr, ent);
+    vsg_status st = area_search(m, f, nq, qs.data(), qdesc, nq, ptr, ent);
     if (st != VSG_OK) return st;
     for (int i = 0; i <= nq; ++i) cand_ptr[i] = ptr[i];
     if (total_out) *total_out = (int)ent.size();
@@ -656,64 +745,13 @@ vsg_status vsg_area_search(vsg_matcher *m, const vsg_frame *f, int nq, const flo
     return VSG_OK;
 }
 
-// ORBmatcher.cc:48-74: the map points that reach GetFeaturesInArea, as window queries
-// Candidates at distance d > TH_HIGH with nnratio * d >= TH_HIGH can neither become the best match (:123) nor, as the
+// The largest candidate distance the replay of ORBmatcher.cc:76-141 can use.  Candidates at distance d > TH_HIGH with nnratio * d >= TH_HIGH can neither become the best match (:123) nor, as the
 // second best, trigger the ratio rejection (:125: best <= TH_HIGH <= nnratio * d), and every candidate that stays is
 // closer than every one dropped — so the replay over the pruned lists gives the identical result.
 static int projection_map_max_dist(float nnratio) {
     int d = TH_HIGH + 1;
     while (d < 256 && !(nnratio * (float)d >= (float)TH_HIGH)) ++d;
     return d - 1;
-}
-
-static vsg_status projection_map_queries(const std::vector<float> &scale, int n_mp, const vsg_track_point *pts, float th,
-                                         int far_points, float th_far, int max_dist, std::vector<AreaQuery> &qs,
-                                         std::vector<int> &q_mp) {
-    const bool b_factor = th != 1.0;
-    qs.clear(); q_mp.clear();
-    qs.reserve(n_mp); q_mp.reserve(n_mp);
-    for (int i = 0; i < n_mp; ++i) {
-        const vsg_track_point &mp = pts[i];
-        if (!mp.in_view) continue;
-        if (far_points && mp.depth > th_far) continue;
-        if (mp.bad) continue;
-        if (mp.level < 0 || mp.level >= (int)scale.size()) { set_error("map point %d: level %d out of range", i, mp.level); return VSG_ERR_INVALID; }
-        float r = (mp.view_cos > 0.998) ? 2.5f : 4.0f;    // RadiusByViewingCos (:218-224)
-        if (b_factor) r *= th;
-        const float win = r * scale[mp.level];
-        qs.push_back(AreaQuery{mp.proj_x, mp.proj_y, win, mp.level - 1, mp.level, mp.proj_xr, win, max_dist});
-        q_mp.push_back(i);
-    }
-    return VSG_OK;
-}
-
-// ORBmatcher.cc:76-141: the sequential replay over per-map-point candidate lists (ptr has n_mp + 1 entries; map points
-// that never reached GetFeaturesInArea have empty lists)
-static int projection_map_resolve(int n_kp, const vsg_keypoint *keys, const uint8_t *occupied, int n_mp,
-                                  const vsg_track_point *pts, const int32_t *ptr, const int32_t *cand_idx,
-                                  const int32_t *cand_dist, float nnratio, int32_t *assign_out) {
-    std::vector<uint8_t> blocked(occupied, occupied + n_kp);
-    for (int i = 0; i < n_kp; ++i) assign_out[i] = -1;
-    int nmatches = 0;
-    for (int k = 0; k < n_mp; ++k) {
-        if (ptr[k] == ptr[k + 1]) continue;
-        int best = 256, best_level = -1, best2 = 256, best_level2 = -1, best_idx = -1;
-        for (int c = ptr[k]; c < ptr[k + 1]; ++c) {
-            const int idx = cand_idx[c], dist = cand_dist[c];
-            if (blocked[idx]) continue;
-            if (dist < best) { best2 = best; best = dist; best_level2 = best_level; best_level = keys[idx].octave; best_idx = idx; }
-            else if (dist < best2) { best_level2 = keys[idx].octave; best2 = dist; }
-        }
-        if (best <= TH_HIGH) {
-            if (best_level == best_level2 && best > nnratio * best2) continue;
-            if (best_level != best_level2 || best <= nnratio * best2) {
-                assign_out[best_idx] = k;
-                blocked[best_idx] = pts[k].blocks;
-                ++nmatches;
-            }
-        }
-    }
-    return nmatches;
 }
 
 // GPU half of SearchByProjection(Frame&, vector<MapPoint*>&): candidate lists of every map point
@@ -723,21 +761,20 @@ vsg_status vsg_projection_map_candidates(vsg_matcher *m, const vsg_frame *F, int
                                          int *total_out) {
     if (!m || !F || n_mp < 0 || !cand_ptr || (n_mp > 0 && (!pts || !mp_desc))) return VSG_ERR_INVALID;
     CK(cudaSetDevice(m->device));
-    std::vector<AreaQuery> qs;
-    std::vector<int> q_mp;
-    vsg_status st = projection_map_queries(F->scale, n_mp, pts, th, far_points, th_far, 256, qs, q_mp);   // full lists: the
-    if (st != VSG_OK) return st;                                                           // resolve's nnratio is not known here
-    std::vector<uint8_t> qdesc(qs.size() * 32);
-    for (size_t k = 0; k < qs.size(); ++k) memcpy(&qdesc[k * 32], mp_desc + (size_t)q_mp[k] * 32, 32);
+    std::vector<AreaQuery> qs(std::max(n_mp, 1));
+    std::vector<int> q_mp(std::max(n_mp, 1));
+    int nq;
+    vsg_status st = map_queries(F, n_mp, pts, th, far_points, th_far, 256, qs.data(), q_mp.data(), &nq);   // full lists: the
+    if (st != VSG_OK) return st;                                                                     // resolve's nnratio is not known here
     std::vector<int> ptr;
     std::vector<int2> ent;
-    if ((st = area_search(m, F, (int)qs.size(), qs.data(), qdesc.data(), ptr, ent)) != VSG_OK) return st;
+    if ((st = area_search(m, F, nq, qs.data(), mp_desc, n_mp, ptr, ent)) != VSG_OK) return st;
     if (total_out) *total_out = (int)ent.size();
     // expand to one list per map point
-    size_t q = 0;
+    int q = 0;
     for (int i = 0; i < n_mp; ++i) {
-        cand_ptr[i] = q < qs.size() ? ptr[q] : (int)ent.size();
-        if (q < qs.size() && q_mp[q] == i) ++q;
+        cand_ptr[i] = q < nq ? ptr[q] : (int)ent.size();
+        if (q < nq && q_mp[q] == i) ++q;
     }
     cand_ptr[n_mp] = (int)ent.size();
     if ((int)ent.size() > capacity) return VSG_ERR_CAPACITY;
@@ -753,19 +790,18 @@ vsg_status vsg_projection_map_candidates(vsg_matcher *m, const vsg_frame *F, int
 vsg_status vsg_projection_map_resolve(const vsg_frame_view *F, const uint8_t *occupied, int n_mp,
                                       const vsg_track_point *pts, const int32_t *cand_ptr, const int32_t *cand_idx,
                                       const int32_t *cand_dist, float nnratio, int32_t *assign_out, int *nmatches_out) {
-    if (!F || n_mp < 0 || !cand_ptr || (F->n > 0 && (!occupied || !assign_out || !F->keys)) ||
-        (n_mp > 0 && !pts) || (cand_ptr[n_mp] > 0 && (!cand_idx || !cand_dist)))
-        return VSG_ERR_INVALID;
-    for (int c = 0; c < cand_ptr[n_mp]; ++c)
-        if (cand_idx[c] < 0 || cand_idx[c] >= F->n) { set_error("resolve: candidate index out of range"); return VSG_ERR_INVALID; }
-    const int nm = projection_map_resolve(F->n, F->keys, occupied, n_mp, pts, cand_ptr, cand_idx, cand_dist, nnratio, assign_out);
-    if (nmatches_out) *nmatches_out = nm;
-    return VSG_OK;
+    if (!F || F->n < 0 || (F->n > 0 && (!occupied || !assign_out))) return VSG_ERR_INVALID;
+    std::vector<uint8_t> blocked(occupied, occupied + F->n);
+    std::vector<int32_t> assign(F->n, -1);                 // assign_out stays as it was if the call is rejected
+    const vsg_status st = vsg_projection_map_resolve_shard(F, blocked.data(), 0, n_mp, pts, cand_ptr, cand_idx, cand_dist, nnratio,
+                                                           assign.data(), nmatches_out);
+    if (st == VSG_OK) std::copy(assign.begin(), assign.end(), assign_out);
+    return st;
 }
 
 // ---- SearchByProjection(Frame&, vector<MapPoint*>&) in two halves that the one-call and the sharded entry points share ----
 // GPU half: window queries of the map points that reach GetFeaturesInArea (:48-74), candidate lists with distances back
-// on the host (pinned staging of the matcher; valid until its next search).
+// on the host (pinned staging of the matcher; valid until its next area search).
 struct MapSearch {
     int nq = 0;
     const int *q_mp = nullptr;   // query -> map point index (local to the pts array given)
@@ -780,40 +816,29 @@ static vsg_status projection_map_search(vsg_matcher *m, const vsg_frame *F, int 
     PhaseTimer pt("search_by_projection_map");
     // query list in the matcher's pinned staging (a 200k-point map is 7 MB of queries: no fresh pages per call, and the
     // upload runs at the PCIe rate instead of the pageable-memory rate)
-    {
-        vsg_status qst = matcher_ensure_host(m, 3, (size_t)std::max(n_mp, 1) * sizeof(AreaQuery));
-        if (qst != VSG_OK) return qst;
-    }
-    m->scratch[1].resize((size_t)std::max(n_mp, 1) * sizeof(int));
-    AreaQuery *qs = reinterpret_cast<AreaQuery *>(m->hbuf[3]);
-    int *q_mp = reinterpret_cast<int *>(m->scratch[1].data());
-    int nq = 0;
-    {
-        const bool b_factor = th != 1.0;
-        const int max_dist = projection_map_max_dist(nnratio);
-        for (int i = 0; i < n_mp; ++i) {                      // :48-74
-            const vsg_track_point &mp = pts[i];
-            if (!mp.in_view) continue;
-            if (far_points && mp.depth > th_far) continue;
-            if (mp.bad) continue;
-            if (mp.level < 0 || mp.level >= (int)F->scale.size()) { set_error("map point %d: level %d out of range", i, mp.level); return VSG_ERR_INVALID; }
-            float r = (mp.view_cos > 0.998) ? 2.5f : 4.0f;    // RadiusByViewingCos (:218-224)
-            if (b_factor) r *= th;
-            const float win = r * F->scale[mp.level];
-            qs[nq] = AreaQuery{mp.proj_x, mp.proj_y, win, mp.level - 1, mp.level, mp.proj_xr, win, max_dist, i};   // desc row i
-            q_mp[nq++] = i;
-        }
-    }
+    vsg_status st = matcher_ensure_host(m, kHostMapQueries, (size_t)std::max(n_mp, 1) * sizeof(AreaQuery));
+    if (st != VSG_OK) return st;
+    m->scratch.resize(std::max(n_mp, 1));
+    AreaQuery *qs = reinterpret_cast<AreaQuery *>(m->hbuf[kHostMapQueries]);
+    int nq;
+    st = map_queries(F, n_mp, pts, th, far_points, th_far, projection_map_max_dist(nnratio), qs, m->scratch.data(), &nq);
+    if (st != VSG_OK) return st;
     pt.mark("queries");
     out->nq = nq;
-    out->q_mp = q_mp;
+    out->q_mp = m->scratch.data();
     out->ordered = nq >= kOrderedReplayMinQueries;
     // tracking-sized calls (a local map of a few thousand points): the lists come back as the kernel left them and the
     // replay visits them query by query — two kernels and a copy less than the ordered form
-    const vsg_status st = out->ordered ? area_search_ordered(m, F, nq, qs, mp_desc, n_mp, &out->L)
-                                       : area_search_raw(m, F, nq, qs, mp_desc, n_mp, &out->R);
+    st = out->ordered ? area_search_ordered(m, F, nq, qs, mp_desc, n_mp, &out->L) : area_search_raw(m, F, nq, qs, mp_desc, n_mp, &out->R);
     pt.mark("area_search total");
     return st;
+}
+
+// The first entry from e on whose keypoint is not claimed (total if none).  Out of line on purpose: inlined next to map_scan,
+// the loop index is spilled to the stack and every skipped entry of the ordered replay pays a store and a reload.
+__attribute__((noinline)) static int first_unclaimed(const int2 *ent, int e, int total, const uint8_t *blocked) {
+    while (e < total && blocked[ent[e].x]) ++e;
+    return e;
 }
 
 // Host half: the sequential replay of :76-141 in map order.  `blocked` (keypoints holding a map point with observations,
@@ -825,21 +850,11 @@ static int projection_map_replay(const vsg_frame *F, uint8_t *blocked, const Map
     const int *q_mp = S.q_mp;
     int nmatches = 0;
     auto scan = [&](const int2 *c, const int2 *ce, int k) {
-        int best = 256, best_level = -1, best2 = 256, best_level2 = -1, best_idx = -1;
-        for (; c < ce; ++c) {
-            const int idx = c->x, dist = c->y;
-            if (blocked[idx]) continue;
-            if (dist < best) { best2 = best; best = dist; best_level2 = best_level; best_level = keys[idx].octave; best_idx = idx; }
-            else if (dist < best2) { best_level2 = keys[idx].octave; best2 = dist; }
-        }
-        if (best <= TH_HIGH) {
-            if (best_level == best_level2 && best > nnratio * best2) return;
-            if (best_level != best_level2 || best <= nnratio * best2) {
-                assign_out[best_idx] = index_offset + q_mp[k];
-                blocked[best_idx] = pts[q_mp[k]].blocks;
-                ++nmatches;
-            }
-        }
+        int idx;
+        if (map_scan((int)(ce - c), [c](int j) { return c[j]; }, blocked, keys, nnratio, &idx) != MapScan::Match) return;
+        assign_out[idx] = index_offset + q_mp[k];
+        blocked[idx] = pts[q_mp[k]].blocks;
+        ++nmatches;
     };
     if (!S.ordered) {
         for (int k = 0; k < S.nq; ++k) scan(S.R.raw + S.R.off[k], S.R.raw + S.R.off[k] + S.R.cnt[k], k);
@@ -849,8 +864,7 @@ static int projection_map_replay(const vsg_frame *F, uint8_t *blocked, const Map
     // with a map much larger than the frame that is nearly every entry — and only the first unclaimed entry of a query
     // triggers the scan of that query's list.  (Claims only ever appear, so an entry found claimed stays irrelevant.)
     const OrderedLists &L = S.L;
-    for (int e = 0; e < L.total;) {
-        if (blocked[L.ent[e].x]) { ++e; continue; }
+    for (int e = first_unclaimed(L.ent, 0, L.total, blocked); e < L.total; e = first_unclaimed(L.ent, e, L.total, blocked)) {
         const int k = L.qid[e];
         const int2 *c = L.ent + e, *ce = L.ent + L.ptr[k + 1];
         e = L.ptr[k + 1];
@@ -896,10 +910,10 @@ vsg_status vsg_search_by_projection_map_sharded(vsg_comm *comm, vsg_matcher *m, 
     if (st != VSG_OK) return st;
     // device: token (N bytes, padded), my record (N + 1 ints), everyone's records; pinned host mirrors
     const size_t tok_bytes = ((size_t)N + 15) & ~(size_t)15, rec_ints = (size_t)N + 1;
-    if ((st = matcher_ensure(m, 12, tok_bytes + rec_ints * 4 * (1 + (size_t)nranks) + 64)) ||
-        (st = matcher_ensure_host(m, 6, tok_bytes + rec_ints * 4 * (1 + (size_t)nranks) + 64)))
+    if ((st = matcher_ensure(m, kSlotMapShardToken, tok_bytes + rec_ints * 4 * (1 + (size_t)nranks) + 64)) ||
+        (st = matcher_ensure_host(m, kHostMapShardToken, tok_bytes + rec_ints * 4 * (1 + (size_t)nranks) + 64)))
         return st;
-    uint8_t *tok_d = (uint8_t *)m->buf[12], *tok_h = (uint8_t *)m->hbuf[6];
+    uint8_t *tok_d = (uint8_t *)m->buf[kSlotMapShardToken], *tok_h = (uint8_t *)m->hbuf[kHostMapShardToken];
     int32_t *rec_d = (int32_t *)(tok_d + tok_bytes), *all_d = rec_d + rec_ints;
     int32_t *rec_h = (int32_t *)(tok_h + tok_bytes), *all_h = rec_h + rec_ints;
     cudaStream_t s = m->stream;
@@ -941,24 +955,22 @@ vsg_status vsg_projection_map_resolve_shard(const vsg_frame_view *F, uint8_t *bl
     if (!F || n_local < 0 || !cand_ptr || (F->n > 0 && (!blocked || !assign_out || !F->keys)) || (n_local > 0 && !pts_local) ||
         (cand_ptr[n_local] > 0 && (!cand_idx || !cand_dist)))
         return VSG_ERR_INVALID;
+    // every index a list can reach is checked before anything is written (one flat pass: lists are short)
+    int lo = cand_ptr[0], hi = cand_ptr[0];
+    for (int k = 1; k <= n_local; ++k) { lo = std::min(lo, cand_ptr[k]); hi = std::max(hi, cand_ptr[k]); }
+    if (lo < 0) { set_error("resolve: negative candidate list offset"); return VSG_ERR_INVALID; }
+    for (int c = lo; c < hi; ++c)
+        if (cand_idx[c] < 0 || cand_idx[c] >= F->n) { set_error("resolve: candidate index out of range"); return VSG_ERR_INVALID; }
     int nmatches = 0;
     for (int k = 0; k < n_local; ++k) {
-        int best = 256, best_level = -1, best2 = 256, best_level2 = -1, best_idx = -1;
-        for (int c = cand_ptr[k]; c < cand_ptr[k + 1]; ++c) {
-            const int idx = cand_idx[c], dist = cand_dist[c];
-            if (idx < 0 || idx >= F->n) { set_error("resolve: candidate index out of range"); return VSG_ERR_INVALID; }
-            if (blocked[idx]) continue;
-            if (dist < best) { best2 = best; best = dist; best_level2 = best_level; best_level = F->keys[idx].octave; best_idx = idx; }
-            else if (dist < best2) { best_level2 = F->keys[idx].octave; best2 = dist; }
-        }
-        if (best <= TH_HIGH) {
-            if (best_level == best_level2 && best > nnratio * best2) continue;
-            if (best_level != best_level2 || best <= nnratio * best2) {
-                assign_out[best_idx] = shard_begin + k;
-                blocked[best_idx] = pts_local[k].blocks;
-                ++nmatches;
-            }
-        }
+        const int32_t *ci = cand_idx + cand_ptr[k], *cd = cand_dist + cand_ptr[k];
+        int idx;
+        if (map_scan(cand_ptr[k + 1] - cand_ptr[k], [ci, cd](int c) { return make_int2(ci[c], cd[c]); }, blocked, F->keys, nnratio,
+                     &idx) != MapScan::Match)
+            continue;
+        assign_out[idx] = shard_begin + k;
+        blocked[idx] = pts_local[k].blocks;
+        ++nmatches;
     }
     if (nmatches_out) *nmatches_out = nmatches;
     return VSG_OK;
@@ -979,10 +991,8 @@ vsg_status vsg_search_by_projection_map_2cam(vsg_matcher *m, const vsg_frame *FL
         return VSG_ERR_INVALID;
     }
     CK(cudaSetDevice(m->device));
-    const int nL = FL->n, nR = FR->n, N = nL + nR;
-    const bool b_factor = th != 1.0;
+    const int nL = FL->n, N = nL + FR->n;
     const int max_dist = projection_map_max_dist(nnratio);
-    const int nlev = (int)FL->scale.size();
     // queries of both cameras; q_of[cam][i] = query number of map point i or -1
     std::vector<AreaQuery> qs[2];
     std::vector<int> q_of[2];
@@ -992,20 +1002,17 @@ vsg_status vsg_search_by_projection_map_2cam(vsg_matcher *m, const vsg_frame *FL
         if (!l.in_view && !r.in_view) continue;                                 // :52-53
         if (far_points && l.depth > th_far) continue;                           // :55-56
         if (l.bad) continue;                                                    // :58-59
+        AreaQuery q;
+        vsg_status st;
         if (l.in_view) {
-            if (l.level < 0 || l.level >= nlev) { set_error("map point %d: level %d out of range", i, l.level); return VSG_ERR_INVALID; }
-            float rad = (l.view_cos > 0.998) ? 2.5f : 4.0f;
-            if (b_factor) rad *= th;
-            const float win = rad * FL->scale[l.level];
+            if ((st = map_point_query(FL, l, i, th, 0.f, max_dist, "", &q)) != VSG_OK) return st;
             q_of[0][i] = (int)qs[0].size();
-            qs[0].push_back(AreaQuery{l.proj_x, l.proj_y, win, l.level - 1, l.level, 0.f, win, max_dist, i});
+            qs[0].push_back(q);
         }
-        if (r.in_view && r.level != -1) {                                       // :146-150
-            if (r.level < 0 || r.level >= nlev) { set_error("map point %d: right level %d out of range", i, r.level); return VSG_ERR_INVALID; }
-            const float rad = (r.view_cos > 0.998) ? 2.5f : 4.0f;              // no th factor on this side (:151)
-            const float win = rad * FR->scale[r.level];
+        if (r.in_view && r.level != -1) {                                       // :146-150; no th factor on this side (:151)
+            if ((st = map_point_query(FR, r, i, 1.f, 0.f, max_dist, "right ", &q)) != VSG_OK) return st;
             q_of[1][i] = (int)qs[1].size();
-            qs[1].push_back(AreaQuery{r.proj_x, r.proj_y, win, r.level - 1, r.level, 0.f, win, max_dist, i});
+            qs[1].push_back(q);
         }
     }
     // the two searches share the matcher's staging: the left lists are copied out before the right search runs
@@ -1030,43 +1037,25 @@ vsg_status vsg_search_by_projection_map_2cam(vsg_matcher *m, const vsg_frame *FL
     int nmatches = 0;
     auto claim = [&](int slot, int mp) { assign_out[slot] = mp; blocked[slot] = pts_left[mp].blocks; };
     for (int i = 0; i < n_mp; ++i) {
-        if (q_of[0][i] < 0 && q_of[1][i] < 0) continue;
-        bool skip_right = false;
+        int idx;
         if (q_of[0][i] >= 0) {
-            const int k = q_of[0][i];
-            int best = 256, best_level = -1, best2 = 256, best_level2 = -1, best_idx = -1;
-            const int2 *c = raw_l.data() + off_l[k], *ce = c + cnt_l[k];
-            for (; c < ce; ++c) {
-                const int idx = c->x, dist = c->y;
-                if (blocked[idx]) continue;
-                if (dist < best) { best2 = best; best = dist; best_level2 = best_level; best_level = FL->keys[idx].octave; best_idx = idx; }
-                else if (dist < best2) { best_level2 = FL->keys[idx].octave; best2 = dist; }
-            }
-            if (best <= TH_HIGH) {
-                if (best_level == best_level2 && best > nnratio * best2) skip_right = true;   // `continue` at :124-125
-                else {
-                    claim(best_idx, i);
-                    if (left_to_right[best_idx] != -1) { claim(left_to_right[best_idx] + nL, i); ++nmatches; }   // :131-136
-                    ++nmatches;
-                }
+            const int2 *c = raw_l.data() + off_l[q_of[0][i]];
+            const MapScan r = map_scan(cnt_l[q_of[0][i]], [c](int j) { return c[j]; }, blocked.data(), FL->keys.data(), nnratio, &idx);
+            if (r == MapScan::RatioRejected) continue;                          // `continue` at :124-125: no right-camera search
+            if (r == MapScan::Match) {
+                claim(idx, i);
+                if (left_to_right[idx] != -1) { claim(left_to_right[idx] + nL, i); ++nmatches; }   // :131-136
+                ++nmatches;
             }
         }
-        if (skip_right || q_of[1][i] < 0) continue;
-        const int k = q_of[1][i];
-        int best = 256, best_level = -1, best2 = 256, best_level2 = -1, best_idx = -1;
-        const int2 *c = R.raw + R.off[k], *ce = c + R.cnt[k];
-        for (; c < ce; ++c) {
-            const int idx = c->x, dist = c->y;
-            if (blocked[idx + nL]) continue;                                    // :176-178
-            if (dist < best) { best2 = best; best = dist; best_level2 = best_level; best_level = FR->keys[idx].octave; best_idx = idx; }
-            else if (dist < best2) { best_level2 = FR->keys[idx].octave; best2 = dist; }
-        }
-        if (best <= TH_HIGH) {
-            if (best_level == best_level2 && best > nnratio * best2) continue;
-            if (right_to_left[best_idx] != -1) { claim(right_to_left[best_idx], i); ++nmatches; }   // :203-208
-            claim(best_idx + nL, i);
-            ++nmatches;
-        }
+        if (q_of[1][i] < 0) continue;
+        const int2 *c = R.raw + R.off[q_of[1][i]];
+        if (map_scan(R.cnt[q_of[1][i]], [c](int j) { return c[j]; }, blocked.data() + nL, FR->keys.data(), nnratio, &idx) !=
+            MapScan::Match)                                                     // :176-178: the right camera's claims
+            continue;
+        if (right_to_left[idx] != -1) { claim(right_to_left[idx], i); ++nmatches; }   // :203-208
+        claim(idx + nL, i);
+        ++nmatches;
     }
     if (nmatches_out) *nmatches_out = nmatches;
     return VSG_OK;
@@ -1077,61 +1066,12 @@ vsg_status vsg_search_by_projection_last(vsg_matcher *m, const vsg_frame *Cur, c
                                          const vsg_proj_point *pts, const uint8_t *desc, float th, int mode,
                                          int check_ori, int32_t *assign_out, int *nmatches_out) {
     if (!m || !Cur || n_last < 0 || !assign_out || (n_last > 0 && (!pts || !desc)) || (Cur->n > 0 && !occupied)) return VSG_ERR_INVALID;
-    CK(cudaSetDevice(m->device));
-    std::vector<AreaQuery> qs;
-    std::vector<int> q_src;
-    for (int i = 0; i < n_last; ++i) {
-        const vsg_proj_point &p = pts[i];
-        if (!p.valid) continue;
-        if (p.octave < 0 || p.octave >= (int)Cur->scale.size()) { set_error("point %d: octave %d out of range", i, p.octave); return VSG_ERR_INVALID; }
-        const float radius = th * Cur->scale[p.octave];
-        int lo, hi;
-        if (mode == 1) { lo = p.octave; hi = -1; }                 // forward  (:1719-1720)
-        else if (mode == 2) { lo = 0; hi = p.octave; }             // backward (:1721-1722)
-        else { lo = p.octave - 1; hi = p.octave + 1; }             // :1723-1724
-        qs.push_back(AreaQuery{p.u, p.v, radius, lo, hi, p.ur, radius});
-        q_src.push_back(i);
-    }
-    std::vector<uint8_t> qdesc(qs.size() * 32);
-    for (size_t k = 0; k < qs.size(); ++k) memcpy(&qdesc[k * 32], desc + (size_t)q_src[k] * 32, 32);
-    std::vector<int> ptr;
-    std::vector<int2> ent;
-    vsg_status st = area_search(m, Cur, (int)qs.size(), qs.data(), qdesc.data(), ptr, ent);
-    if (st != VSG_OK) return st;
-    std::vector<uint8_t> blocked(occupied, occupied + Cur->n);
-    for (int i = 0; i < Cur->n; ++i) assign_out[i] = -1;
-    std::vector<int> rot_hist[HISTO_LENGTH];
-    int nmatches = 0;
-    for (size_t k = 0; k < qs.size(); ++k) {
-        int best = 256, best_idx = -1;
-        for (int c = ptr[k]; c < ptr[k + 1]; ++c) {
-            const int i2 = ent[c].x, dist = ent[c].y;
-            if (blocked[i2]) continue;
-            if (dist < best) { best = dist; best_idx = i2; }
-        }
-        if (best <= TH_HIGH) {
-            const vsg_proj_point &p = pts[q_src[k]];
-            assign_out[best_idx] = q_src[k];
-            blocked[best_idx] = p.blocks;
-            ++nmatches;
-            if (check_ori) rot_hist[rot_bin(p.angle, Cur->keys[best_idx].angle)].push_back(best_idx);
-        }
-    }
-    if (check_ori) {
-        int ind1 = -1, ind2 = -1, ind3 = -1;
-        three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
-        for (int i = 0; i < HISTO_LENGTH; ++i) {
-            if (i == ind1 || i == ind2 || i == ind3) continue;
-            for (int idx : rot_hist[i]) { assign_out[idx] = -2; --nmatches; }
-        }
-    }
-    if (nmatches_out) *nmatches_out = nmatches;
-    return VSG_OK;
+    return projection_last(m, 1, &Cur, occupied, n_last, &pts, desc, th, mode, check_ori, assign_out, nmatches_out);
 }
 
 // ORBmatcher.cc:1667-1878 with a two-camera current frame (CurrentFrame.Nleft != -1): per last-frame point the left-camera
-// search (:1709-1784) and — unless the left window was empty, whose `continue` (:1727-1728) skips it — the right-camera
-// search around its projection through mTrl (:1785-1852).
+// search (:1709-1784) and — unless the left window was empty — the right-camera search around its projection through mTrl
+// (:1785-1852).
 vsg_status vsg_search_by_projection_last_2cam(vsg_matcher *m, const vsg_frame *CurL, const vsg_frame *CurR,
                                               const uint8_t *occupied, int n_last, const vsg_proj_point *pts_left,
                                               const vsg_proj_point *pts_right, const uint8_t *desc, float th, int mode,
@@ -1143,65 +1083,9 @@ vsg_status vsg_search_by_projection_last_2cam(vsg_matcher *m, const vsg_frame *C
         set_error("vsg_search_by_projection_last_2cam: the per-camera frames of a two-camera rig carry no uRight");
         return VSG_ERR_INVALID;
     }
-    CK(cudaSetDevice(m->device));
-    const int nL = CurL->n, N = CurL->n + CurR->n, nlev = (int)CurL->scale.size();
-    std::vector<AreaQuery> qs[2];
-    std::vector<int> q_src;
-    for (int i = 0; i < n_last; ++i) {
-        const vsg_proj_point &p = pts_left[i];
-        if (!p.valid) continue;
-        if (p.octave < 0 || p.octave >= nlev) { set_error("point %d: octave %d out of range", i, p.octave); return VSG_ERR_INVALID; }
-        const float radius = th * CurL->scale[p.octave];
-        int lo, hi;
-        if (mode == 1) { lo = p.octave; hi = -1; }
-        else if (mode == 2) { lo = 0; hi = p.octave; }
-        else { lo = p.octave - 1; hi = p.octave + 1; }
-        qs[0].push_back(AreaQuery{p.u, p.v, radius, lo, hi, 0.f, radius, 256, (int)q_src.size()});
-        qs[1].push_back(AreaQuery{pts_right[i].u, pts_right[i].v, radius, lo, hi, 0.f, radius, 256, (int)q_src.size()});
-        q_src.push_back(i);
-    }
-    const int nq = (int)q_src.size();
-    std::vector<uint8_t> qdesc((size_t)std::max(nq, 1) * 32);
-    for (int k = 0; k < nq; ++k) memcpy(&qdesc[(size_t)k * 32], desc + (size_t)q_src[k] * 32, 32);
-    std::vector<int> ptr[2];
-    std::vector<int2> ent[2];
-    vsg_status st;
-    if ((st = area_search(m, CurL, nq, qs[0].data(), qdesc.data(), ptr[0], ent[0])) != VSG_OK) return st;
-    if ((st = area_search(m, CurR, nq, qs[1].data(), qdesc.data(), ptr[1], ent[1])) != VSG_OK) return st;
-    std::vector<uint8_t> blocked(occupied, occupied + N);
-    for (int i = 0; i < N; ++i) assign_out[i] = -1;
-    std::vector<int> rot_hist[HISTO_LENGTH];
-    int nmatches = 0;
-    for (int k = 0; k < nq; ++k) {
-        const vsg_proj_point &p = pts_left[q_src[k]];
-        if (ptr[0][k] == ptr[0][k + 1]) continue;                  // vIndices2.empty() -> continue: no right-camera search either
-        for (int cam = 0; cam < 2; ++cam) {
-            const vsg_frame *F = cam == 0 ? CurL : CurR;
-            const int offset = cam == 0 ? 0 : nL;
-            int best = 256, best_idx = -1;
-            for (int c = ptr[cam][k]; c < ptr[cam][k + 1]; ++c) {
-                const int i2 = ent[cam][c].x, dist = ent[cam][c].y;
-                if (blocked[i2 + offset]) continue;
-                if (dist < best) { best = dist; best_idx = i2; }
-            }
-            if (best <= TH_HIGH) {
-                assign_out[best_idx + offset] = q_src[k];
-                blocked[best_idx + offset] = p.blocks;
-                ++nmatches;
-                if (check_ori) rot_hist[rot_bin(p.angle, F->keys[best_idx].angle)].push_back(best_idx + offset);
-            }
-        }
-    }
-    if (check_ori) {
-        int ind1 = -1, ind2 = -1, ind3 = -1;
-        three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
-        for (int i = 0; i < HISTO_LENGTH; ++i) {
-            if (i == ind1 || i == ind2 || i == ind3) continue;
-            for (int idx : rot_hist[i]) { assign_out[idx] = -2; --nmatches; }
-        }
-    }
-    if (nmatches_out) *nmatches_out = nmatches;
-    return VSG_OK;
+    const vsg_frame *cur[2] = {CurL, CurR};
+    const vsg_proj_point *pts[2] = {pts_left, pts_right};
+    return projection_last(m, 2, cur, occupied, n_last, pts, desc, th, mode, check_ori, assign_out, nmatches_out);
 }
 
 // ORBmatcher.cc:643-756
@@ -1222,7 +1106,7 @@ vsg_status vsg_search_for_initialization(vsg_matcher *m, const vsg_frame_view *F
     for (size_t k = 0; k < qs.size(); ++k) memcpy(&qdesc[k * 32], F1->descriptors + (size_t)q_src[k] * 32, 32);
     std::vector<int> ptr;
     std::vector<int2> ent;
-    vsg_status st = area_search(m, F2, (int)qs.size(), qs.data(), qdesc.data(), ptr, ent);
+    vsg_status st = area_search(m, F2, (int)qs.size(), qs.data(), qdesc.data(), (int)qs.size(), ptr, ent);
     if (st != VSG_OK) return st;
     int nmatches = 0;
     for (int i = 0; i < F1->n; ++i) matches12_out[i] = -1;
@@ -1248,15 +1132,8 @@ vsg_status vsg_search_for_initialization(vsg_matcher *m, const vsg_frame_view *F
             }
         }
     }
-    if (check_ori) {
-        int ind1 = -1, ind2 = -1, ind3 = -1;
-        three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
-        for (int i = 0; i < HISTO_LENGTH; ++i) {
-            if (i == ind1 || i == ind2 || i == ind3) continue;
-            for (int idx1 : rot_hist[i])
-                if (matches12_out[idx1] >= 0) { matches12_out[idx1] = -1; --nmatches; }
-        }
-    }
+    if (check_ori)                                                  // a match stolen later is still in its bin
+        apply_rot_filter(rot_hist, [&](int i1) { if (matches12_out[i1] >= 0) { matches12_out[i1] = -1; --nmatches; } });
     for (int i1 = 0; i1 < F1->n; ++i1)                              // :748-751
         if (matches12_out[i1] >= 0) {
             prev_matched[2 * i1] = F2->keys[matches12_out[i1]].x;
@@ -1294,9 +1171,8 @@ vsg_status vsg_search_by_bow_2cam(vsg_matcher *m, const vsg_frame_view *KF, cons
     std::vector<BowSeg> segs;
     int64_t npairs = 0;
     const uint16_t *dist;
-    vsg_status st = bow_walk(w, segs, &npairs);
-    const int seg_ptr[2] = {0, (int)segs.size()};
-    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
+    const vsg_status st = bow_walk_dists(m, w, segs, &npairs, &dist);
+    if (st != VSG_OK) return st;
     const int nmatches = bow_replay_kf_f(KF, F, f_nleft, w.b, segs.data(), (int)segs.size(), dist, nnratio, check_ori, matches_f_out);
     if (nmatches_out) *nmatches_out = nmatches;
     return VSG_OK;
@@ -1323,30 +1199,22 @@ vsg_status vsg_search_by_bow_multi(vsg_matcher *m, int ntargets, const vsg_bow_s
         set_error("vsg_search_by_bow_multi: f_nleft %d outside [-1, %d]", f_nleft, F->view.n);
         return VSG_ERR_INVALID;
     }
-    for (int t = 0; t < ntargets; ++t)
-        if ((why = bow_side_problem(KFs[t], true))) {
-            set_error("vsg_search_by_bow_multi: target %d: %s", t, why);
-            return VSG_ERR_INVALID;
-        }
-    CK(cudaSetDevice(m->device));
     std::vector<BowWalk> walks;
     std::vector<BowSeg> segs;
-    std::vector<int> seg_ptr(1, 0);
+    std::vector<int> seg_ptr;
     int64_t npairs = 0;
-    for (int t = 0; t < ntargets; ++t) {
-        const vsg_bow_side &a = *KFs[t];
-        walks.push_back(BowWalk{&a.view, a.mp_valid, FeatVec{a.nnodes, a.nodes, a.ptr, a.idx}, &F->view,
-                                FeatVec{F->nnodes, F->nodes, F->ptr, F->idx}});
-        if (bow_walk(walks.back(), segs, &npairs) != VSG_OK) {
-            const std::string err = vsg_last_error();
-            set_error("vsg_search_by_bow_multi: target %d: %s", t, err.c_str());
-            return VSG_ERR_INVALID;
-        }
-        seg_ptr.push_back((int)segs.size());
-    }
-    const uint16_t *dist;
-    vsg_status st = bow_dists(m, ntargets, walks.data(), segs, seg_ptr.data(), npairs, &dist);
+    vsg_status st = bow_walk_targets(
+        "vsg_search_by_bow_multi", ntargets, [&](int t) { return bow_side_problem(KFs[t], true); },
+        [&](int t) {
+            const vsg_bow_side &a = *KFs[t];
+            return BowWalk{&a.view, a.mp_valid, FeatVec{a.nnodes, a.nodes, a.ptr, a.idx}, &F->view,
+                           FeatVec{F->nnodes, F->nodes, F->ptr, F->idx}};
+        },
+        walks, segs, seg_ptr, &npairs);
     if (st != VSG_OK) return st;
+    CK(cudaSetDevice(m->device));
+    const uint16_t *dist;
+    if ((st = bow_dists(m, ntargets, walks.data(), segs, seg_ptr.data(), npairs, &dist)) != VSG_OK) return st;
     for (int t = 0; t < ntargets; ++t)                                               // in target order, as the loop runs
         nmatches_out[t] = bow_replay_kf_f(&KFs[t]->view, &F->view, f_nleft, walks[t].b, segs.data() + seg_ptr[t],
                                           seg_ptr[t + 1] - seg_ptr[t], dist, nnratio, check_ori,

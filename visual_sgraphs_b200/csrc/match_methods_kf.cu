@@ -21,6 +21,7 @@
 #include <algorithm>
 #include <climits>
 #include <cmath>
+#include <cstdio>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -59,19 +60,6 @@ vsg_status build_queries(const vsg_frame *F, int n, const vsg_search_point *pts,
     for (size_t k = 0; k < qs.size(); ++k) memcpy(&qdesc[k * 32], desc + (size_t)q_src[k] * 32, 32);
     return VSG_OK;
 }
-
-// the rotation-consistency filter shared by the methods: everything outside the three dominant bins is dropped
-template <class Drop>
-void apply_rot_filter(const std::vector<int> *rot_hist, Drop drop) {
-    int ind1 = -1, ind2 = -1, ind3 = -1;
-    three_maxima(rot_hist, HISTO_LENGTH, ind1, ind2, ind3);
-    for (int i = 0; i < HISTO_LENGTH; ++i) {
-        if (i == ind1 || i == ind2 || i == ind3) continue;
-        for (int idx : rot_hist[i]) drop(idx);
-    }
-}
-
-size_t up16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 // The placed descriptor tables (32-byte rows) and FeatureVector index arrays of a BoW upload into the staging buffer h.
 void copy_tables(uint8_t *h, size_t o_desc, size_t o_idx, const TablePlacer &descs, const TablePlacer &idxs) {
@@ -166,9 +154,8 @@ vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std
     const size_t o_seg = 0, o_desc = up16(dsegs.size() * sizeof(int4)), o_idx = o_desc + (size_t)descs.total * 32,
                  o_out = up16(o_idx + (size_t)idxs.total * sizeof(int)), total = o_out + (size_t)npairs * sizeof(uint16_t);
     vsg_status st;
-    // device slot 19 and pinned host slot 8: inputs, then the distances
-    if ((st = matcher_ensure(m, 19, total)) || (st = matcher_ensure_host(m, 8, total))) return st;
-    uint8_t *h = (uint8_t *)m->hbuf[8], *d = (uint8_t *)m->buf[19];
+    if ((st = matcher_ensure(m, kSlotBow, total)) || (st = matcher_ensure_host(m, kHostBow, total))) return st;
+    uint8_t *h = (uint8_t *)m->hbuf[kHostBow], *d = (uint8_t *)m->buf[kSlotBow];
     memcpy(h + o_seg, dsegs.data(), dsegs.size() * sizeof(int4));
     copy_tables(h, o_desc, o_idx, descs, idxs);
     cudaStream_t s = m->stream;
@@ -180,6 +167,12 @@ vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std
     CK(cudaStreamSynchronize(s));
     *dist = (const uint16_t *)(h + o_out);
     return VSG_OK;
+}
+
+vsg_status bow_walk_dists(vsg_matcher *m, const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs, const uint16_t **dist) {
+    const vsg_status st = bow_walk(w, segs, npairs);
+    const int seg_ptr[2] = {0, (int)segs.size()};
+    return st != VSG_OK ? st : bow_dists(m, 1, &w, segs, seg_ptr, *npairs, dist);
 }
 
 const char *bow_side_problem(const vsg_bow_side *s, bool needs_valid) {
@@ -243,48 +236,48 @@ static vsg_status triangulation_candidates(vsg_matcher *m, const char *who, cons
         set_error("%s: KF1: %s", who, why);
         return VSG_ERR_INVALID;
     }
-    for (int t = 0; t < ntargets; ++t) {
-        const vsg_triangulation_target *tg = targets[t];
-        why = tg ? bow_side_problem(&tg->kf2, true) : "null target";
-        if (!why && !coarse && !tg->level_sigma2) why = "null level_sigma2 (the call is not coarse)";
-        if (!why && tg->kf2.view.n > 0 && !tg->kf2.view.scale_factors) why = "null scale factors";
-        if (why) {
-            set_error("%s: target %d: %s", who, t, why);
-            return VSG_ERR_INVALID;
-        }
-        const vsg_frame_view &v = tg->kf2.view;                           // the device indexes the level tables by octave
-        for (int i = 0; i < v.n; ++i)
-            if (v.keys[i].octave < 0 || v.keys[i].octave >= v.n_levels) {
-                set_error("%s: target %d: keypoint %d: octave %d outside [0, %d)", who, t, i, v.keys[i].octave, v.n_levels);
-                return VSG_ERR_INVALID;
-            }
-    }
-    CK(cudaSetDevice(m->device));
     const vsg_frame_view &v1 = KF1->view;
     auto stereo = [](const vsg_frame_view &v, int i) { return v.u_right && v.u_right[i] >= 0; };   // :977, :1005
     std::vector<uint8_t> use1(v1.n);
     for (int i = 0; i < v1.n; ++i) use1[i] = !KF1->mp_valid[i] && (!only_stereo || stereo(v1, i));   // :968-981
-    // the walks; a KF1 feature listed twice would be searched twice in one target, which one row of best12 cannot say
-    std::vector<BowSeg> segs;
-    std::vector<int> seg_ptr(1, 0), seen(v1.n, -1);
-    for (int t = 0; t < ntargets; ++t) {
+    char octave_problem[96];
+    auto problem = [&](int t) -> const char * {
+        const vsg_triangulation_target *tg = targets[t];
+        if (!tg) return "null target";
+        if (const char *w = bow_side_problem(&tg->kf2, true)) return w;
+        if (!coarse && !tg->level_sigma2) return "null level_sigma2 (the call is not coarse)";
+        if (tg->kf2.view.n > 0 && !tg->kf2.view.scale_factors) return "null scale factors";
+        const vsg_frame_view &v = tg->kf2.view;                           // the device indexes the level tables by octave
+        for (int i = 0; i < v.n; ++i)
+            if (v.keys[i].octave < 0 || v.keys[i].octave >= v.n_levels) {
+                snprintf(octave_problem, sizeof octave_problem, "keypoint %d: octave %d outside [0, %d)", i, v.keys[i].octave,
+                         v.n_levels);
+                return octave_problem;
+            }
+        return nullptr;
+    };
+    auto walk = [&](int t) {
         const vsg_bow_side &b = targets[t]->kf2;
-        int64_t npairs = 0;
-        if (bow_walk(BowWalk{&v1, use1.data(), FeatVec{KF1->nnodes, KF1->nodes, KF1->ptr, KF1->idx}, &b.view,
-                             FeatVec{b.nnodes, b.nodes, b.ptr, b.idx}}, segs, &npairs) != VSG_OK) {
-            const std::string err = vsg_last_error();
-            set_error("%s: target %d: %s", who, t, err.c_str());
-            return VSG_ERR_INVALID;
-        }
-        for (size_t k = seg_ptr.back(); k < segs.size(); ++k) {
+        return BowWalk{&v1, use1.data(), FeatVec{KF1->nnodes, KF1->nodes, KF1->ptr, KF1->idx}, &b.view,
+                       FeatVec{b.nnodes, b.nodes, b.ptr, b.idx}};
+    };
+    std::vector<BowWalk> walks;
+    std::vector<BowSeg> segs;
+    std::vector<int> seg_ptr;
+    int64_t npairs = 0;
+    vsg_status st = bow_walk_targets(who, ntargets, problem, walk, walks, segs, seg_ptr, &npairs);
+    if (st != VSG_OK) return st;
+    // a KF1 feature listed twice would be searched twice in one target, which one row of best12 cannot say
+    std::vector<int> seen(v1.n, -1);
+    for (int t = 0; t < ntargets; ++t)
+        for (int k = seg_ptr[t]; k < seg_ptr[t + 1]; ++k) {
             if (seen[segs[k].i1] == t) {
                 set_error("%s: target %d: KF1 feature %d is listed twice in its feature vector", who, t, segs[k].i1);
                 return VSG_ERR_INVALID;
             }
             seen[segs[k].i1] = t;
         }
-        seg_ptr.push_back((int)segs.size());
-    }
+    CK(cudaSetDevice(m->device));
     for (int t = 0; t < ntargets; ++t)
         for (int i = 0; i < v1.n; ++i) best12_out[(size_t)t * v1.n + i] = KF1->mp_valid[i] ? -2 : -1;
     // the segments with candidates and the tables they read
@@ -325,10 +318,9 @@ static vsg_status triangulation_candidates(vsg_matcher *m, const char *who, cons
                  o_idx = o_desc + (size_t)descs.total * 32, o_key = up16(o_idx + (size_t)idxs.total * sizeof(int)),
                  o_lvl = o_key + (size_t)nkeys * sizeof(TriKey), o_out = up16(o_lvl + (size_t)nlvl * sizeof(float2)),
                  total = o_out + (size_t)nseg * sizeof(int);
-    vsg_status st;
-    // device slot 19 and pinned host slot 8, as bow_dists: inputs, then one index per segment
-    if ((st = matcher_ensure(m, 19, total)) || (st = matcher_ensure_host(m, 8, total))) return st;
-    uint8_t *h = (uint8_t *)m->hbuf[8], *d = (uint8_t *)m->buf[19];
+    // inputs, then one index per segment
+    if ((st = matcher_ensure(m, kSlotBow, total)) || (st = matcher_ensure_host(m, kHostBow, total))) return st;
+    uint8_t *h = (uint8_t *)m->hbuf[kHostBow], *d = (uint8_t *)m->buf[kSlotBow];
     memcpy(h + o_seg, dsegs.data(), (size_t)nseg * sizeof(TriSeg));
     memcpy(h + o_tg, dtargets.data(), (size_t)ntargets * sizeof(TriTarget));
     copy_tables(h, o_desc, o_idx, descs, idxs);
@@ -372,23 +364,18 @@ vsg_status vsg_search_by_projection_reloc(vsg_matcher *m, const vsg_frame *Cur, 
     std::vector<int2> ent;
     vsg_status st = build_queries(Cur, n, pts, desc, th, -1, +1, qs, q_src, qdesc);   // :1927
     if (st != VSG_OK) return st;
-    if ((st = area_search(m, Cur, (int)qs.size(), qs.data(), qdesc.data(), ptr, ent)) != VSG_OK) return st;
+    if ((st = area_search(m, Cur, (int)qs.size(), qs.data(), qdesc.data(), (int)qs.size(), ptr, ent)) != VSG_OK) return st;
     std::vector<uint8_t> taken(occupied, occupied + Cur->n);                          // CurrentFrame.mvpMapPoints[i2]
     for (int i = 0; i < Cur->n; ++i) assign_out[i] = -1;
     std::vector<int> rot_hist[HISTO_LENGTH];
     int nmatches = 0;
     for (size_t k = 0; k < qs.size(); ++k) {
-        int best = 256, best_idx = -1;
-        for (int c = ptr[k]; c < ptr[k + 1]; ++c) {
-            const int i2 = ent[c].x, dist = ent[c].y;
-            if (taken[i2]) continue;                                                 // :1939-1940
-            if (dist < best) { best = dist; best_idx = i2; }
-        }
-        if (best <= orb_dist && best_idx >= 0) {                                     // :1952
-            assign_out[best_idx] = q_src[k];
-            taken[best_idx] = 1;
+        const int2 b = nearest_unclaimed(ent.data() + ptr[k], ent.data() + ptr[k + 1], taken.data());   // :1939-1940
+        if (b.x <= orb_dist && b.y >= 0) {                                                               // :1952
+            assign_out[b.y] = q_src[k];
+            taken[b.y] = 1;
             ++nmatches;
-            if (check_ori) rot_hist[rot_bin(pts[q_src[k]].angle, Cur->keys[best_idx].angle)].push_back(best_idx);
+            if (check_ori) rot_hist[rot_bin(pts[q_src[k]].angle, Cur->keys[b.y].angle)].push_back(b.y);
         }
     }
     if (check_ori) apply_rot_filter(rot_hist, [&](int idx) { assign_out[idx] = -2; --nmatches; });
@@ -408,21 +395,16 @@ vsg_status vsg_search_by_projection_sim3(vsg_matcher *m, const vsg_frame *KF, co
     std::vector<int2> ent;
     vsg_status st = build_queries(KF, n, pts, desc, (float)th, -1, 0, qs, q_src, qdesc);   // :486, :502-503
     if (st != VSG_OK) return st;
-    if ((st = area_search(m, KF, (int)qs.size(), qs.data(), qdesc.data(), ptr, ent)) != VSG_OK) return st;
+    if ((st = area_search(m, KF, (int)qs.size(), qs.data(), qdesc.data(), (int)qs.size(), ptr, ent)) != VSG_OK) return st;
     std::vector<uint8_t> taken(matched, matched + KF->n);                            // vpMatched[idx]
     for (int i = 0; i < KF->n; ++i) assign_out[i] = -1;
     int nmatches = 0;
     const float gate = TH_LOW * ratio_hamming;                                       // :520
     for (size_t k = 0; k < qs.size(); ++k) {
-        int best = 256, best_idx = -1;
-        for (int c = ptr[k]; c < ptr[k + 1]; ++c) {
-            const int idx = ent[c].x, dist = ent[c].y;
-            if (taken[idx]) continue;                                                // :497-498
-            if (dist < best) { best = dist; best_idx = idx; }
-        }
-        if ((float)best <= gate && best_idx >= 0) {
-            assign_out[best_idx] = q_src[k];
-            taken[best_idx] = 1;
+        const int2 b = nearest_unclaimed(ent.data() + ptr[k], ent.data() + ptr[k + 1], taken.data());   // :497-498
+        if ((float)b.x <= gate && b.y >= 0) {
+            assign_out[b.y] = q_src[k];
+            taken[b.y] = 1;
             ++nmatches;
         }
     }
@@ -563,9 +545,8 @@ vsg_status vsg_search_by_bow_kf(vsg_matcher *m, const vsg_frame_view *KF1, const
     std::vector<BowSeg> segs;
     int64_t npairs = 0;
     const uint16_t *dist;
-    vsg_status st = bow_walk(w, segs, &npairs);
-    const int seg_ptr[2] = {0, (int)segs.size()};
-    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
+    const vsg_status st = bow_walk_dists(m, w, segs, &npairs, &dist);
+    if (st != VSG_OK) return st;
     const int nmatches = bow_replay_kf(KF1, KF2, mp_valid2, w.b, segs.data(), (int)segs.size(), dist, nnratio, check_ori, matches12_out);
     if (nmatches_out) *nmatches_out = nmatches;
     return VSG_OK;
@@ -588,30 +569,22 @@ vsg_status vsg_search_by_bow_kf_multi(vsg_matcher *m, const vsg_bow_side *KF1, i
         set_error("vsg_search_by_bow_kf_multi: KF1: %s", why);
         return VSG_ERR_INVALID;
     }
-    for (int t = 0; t < ntargets; ++t)
-        if ((why = bow_side_problem(KF2s[t], true))) {
-            set_error("vsg_search_by_bow_kf_multi: target %d: %s", t, why);
-            return VSG_ERR_INVALID;
-        }
-    CK(cudaSetDevice(m->device));
     std::vector<BowWalk> walks;
     std::vector<BowSeg> segs;
-    std::vector<int> seg_ptr(1, 0);
+    std::vector<int> seg_ptr;
     int64_t npairs = 0;
-    for (int t = 0; t < ntargets; ++t) {
-        const vsg_bow_side &b = *KF2s[t];
-        walks.push_back(BowWalk{&KF1->view, KF1->mp_valid, FeatVec{KF1->nnodes, KF1->nodes, KF1->ptr, KF1->idx}, &b.view,
-                                FeatVec{b.nnodes, b.nodes, b.ptr, b.idx}});
-        if (bow_walk(walks.back(), segs, &npairs) != VSG_OK) {
-            const std::string err = vsg_last_error();
-            set_error("vsg_search_by_bow_kf_multi: target %d: %s", t, err.c_str());
-            return VSG_ERR_INVALID;
-        }
-        seg_ptr.push_back((int)segs.size());
-    }
-    const uint16_t *dist;
-    vsg_status st = bow_dists(m, ntargets, walks.data(), segs, seg_ptr.data(), npairs, &dist);
+    vsg_status st = bow_walk_targets(
+        "vsg_search_by_bow_kf_multi", ntargets, [&](int t) { return bow_side_problem(KF2s[t], true); },
+        [&](int t) {
+            const vsg_bow_side &b = *KF2s[t];
+            return BowWalk{&KF1->view, KF1->mp_valid, FeatVec{KF1->nnodes, KF1->nodes, KF1->ptr, KF1->idx}, &b.view,
+                           FeatVec{b.nnodes, b.nodes, b.ptr, b.idx}};
+        },
+        walks, segs, seg_ptr, &npairs);
     if (st != VSG_OK) return st;
+    CK(cudaSetDevice(m->device));
+    const uint16_t *dist;
+    if ((st = bow_dists(m, ntargets, walks.data(), segs, seg_ptr.data(), npairs, &dist)) != VSG_OK) return st;
     for (int t = 0; t < ntargets; ++t)                                               // in target order, as the loop runs
         nmatches_out[t] = bow_replay_kf(&KF1->view, &KF2s[t]->view, KF2s[t]->mp_valid, walks[t].b, segs.data() + seg_ptr[t],
                                         seg_ptr[t + 1] - seg_ptr[t], dist, nnratio, check_ori,
@@ -635,9 +608,8 @@ vsg_status vsg_bow_pair_distances(vsg_matcher *m, const vsg_frame_view *KF1, con
     std::vector<BowSeg> segs;
     int64_t npairs = 0;
     const uint16_t *dist;
-    vsg_status st = bow_walk(w, segs, &npairs);
-    const int seg_ptr[2] = {0, (int)segs.size()};
-    if (st != VSG_OK || (st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
+    const vsg_status st = bow_walk_dists(m, w, segs, &npairs, &dist);
+    if (st != VSG_OK) return st;
     *nq_out = (int)segs.size();
     *total_out = (int)npairs;
     if ((int)segs.size() > q_capacity || npairs > capacity) return VSG_ERR_CAPACITY;

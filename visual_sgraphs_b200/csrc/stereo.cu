@@ -337,26 +337,26 @@ extern "C" vsg_status vsg_stereo_match(vsg_matcher *m, vsg_extractor *left, vsg_
     for (int i = 0; i < n_l; ++i)
         if (keys_l[i].octave < 0 || keys_l[i].octave >= nl) { set_error("vsg_stereo_match: left keypoint %d has octave %d", i, keys_l[i].octave); return VSG_ERR_INVALID; }
     vsg_status st;
-    // slots: 1 keys_l, 2 desc_l, 3 right kps, 4 desc_r, 6 best dist/idx/sad (3 x n_l ints), 7 u_right/depth (2 x n_l floats)
-    if ((st = matcher_ensure(m, 1, (size_t)n_l * sizeof(vsg_keypoint))) || (st = matcher_ensure(m, 2, (size_t)n_l * 32)) ||
-        (st = matcher_ensure(m, 3, (size_t)n_r * sizeof(RightKp))) || (st = matcher_ensure(m, 4, (size_t)n_r * 32)) ||
-        (st = matcher_ensure(m, 6, (size_t)n_l * 12)) || (st = matcher_ensure(m, 7, (size_t)n_l * 8)))
+    // best dist/idx/sad: 3 x n_l ints; u_right/depth: 2 x n_l floats
+    if ((st = matcher_ensure(m, kSlotArg1, (size_t)n_l * sizeof(vsg_keypoint))) || (st = matcher_ensure(m, kSlotArg2, (size_t)n_l * 32)) ||
+        (st = matcher_ensure(m, kSlotArg3, (size_t)n_r * sizeof(RightKp))) || (st = matcher_ensure(m, kSlotArg4, (size_t)n_r * 32)) ||
+        (st = matcher_ensure(m, kSlotOut, (size_t)n_l * 12)) || (st = matcher_ensure(m, kSlotAreaQueries, (size_t)n_l * 8)))
         return st;
     cudaStream_t s = m->stream;
-    CK(cudaMemcpyAsync(m->buf[1], keys_l, (size_t)n_l * sizeof(vsg_keypoint), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[2], desc_l, (size_t)n_l * 32, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[3], rk.data(), (size_t)n_r * sizeof(RightKp), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(m->buf[4], desc_r, (size_t)n_r * 32, cudaMemcpyHostToDevice, s));
-    int *bd = (int *)m->buf[6], *bi = bd + n_l, *sad = bi + n_l;
-    float *ur = (float *)m->buf[7], *dp = ur + n_l;
+    CK(cudaMemcpyAsync(m->buf[kSlotArg1], keys_l, (size_t)n_l * sizeof(vsg_keypoint), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(m->buf[kSlotArg2], desc_l, (size_t)n_l * 32, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(m->buf[kSlotArg3], rk.data(), (size_t)n_r * sizeof(RightKp), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(m->buf[kSlotArg4], desc_r, (size_t)n_r * 32, cudaMemcpyHostToDevice, s));
+    int *bd = (int *)m->buf[kSlotOut], *bi = bd + n_l, *sad = bi + n_l;
+    float *ur = (float *)m->buf[kSlotAreaQueries], *dp = ur + n_l;
     const float max_d = mbf / mb;                             // :987-989
     const size_t smem = (size_t)n_r * sizeof(RightKp);
     if (smem > 200 * 1024) { set_error("vsg_stereo_match: too many right keypoints (%d)", n_r); return VSG_ERR_INVALID; }
     if (smem > 48 * 1024) CK(cudaFuncSetAttribute(stereo_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    stereo_search_kernel<<<(n_l + 127) / 128, 128, smem, s>>>((const vsg_keypoint *)m->buf[1], (const uint4 *)m->buf[2], n_l,
-                                                             (const RightKp *)m->buf[3], (const uint4 *)m->buf[4], n_r,
+    stereo_search_kernel<<<(n_l + 127) / 128, 128, smem, s>>>((const vsg_keypoint *)m->buf[kSlotArg1], (const uint4 *)m->buf[kSlotArg2], n_l,
+                                                             (const RightKp *)m->buf[kSlotArg3], (const uint4 *)m->buf[kSlotArg4], n_r,
                                                              n_rows, max_d, bd, bi);
-    stereo_sad_kernel<<<(n_l + 7) / 8, 256, 0, s>>>(P, (const vsg_keypoint *)m->buf[1], n_l, (const RightKp *)m->buf[3], bd, bi,
+    stereo_sad_kernel<<<(n_l + 7) / 8, 256, 0, s>>>(P, (const vsg_keypoint *)m->buf[kSlotArg1], n_l, (const RightKp *)m->buf[kSlotArg3], bd, bi,
                                                    max_d, mbf, sad, ur, dp);
     count_launch(2);
     CK(cudaGetLastError());
@@ -411,9 +411,9 @@ extern "C" vsg_status vsg_stereo_match_batch(vsg_matcher *m, vsg_extractor *ex, 
     P.n_rows = pr.geom->lv[0].h;
     vsg_status st;
     const size_t n = (size_t)npairs * cap;
-    if ((st = matcher_ensure(m, 6, n * 12)) || (st = matcher_ensure(m, 7, n * 8))) return st;
-    int *bd = (int *)m->buf[6], *bi = bd + n, *sad = bi + n;
-    float *ur = (float *)m->buf[7], *dp = ur + n;
+    if ((st = matcher_ensure(m, kSlotOut, n * 12)) || (st = matcher_ensure(m, kSlotAreaQueries, n * 8))) return st;
+    int *bd = (int *)m->buf[kSlotOut], *bi = bd + n, *sad = bi + n;
+    float *ur = (float *)m->buf[kSlotAreaQueries], *dp = ur + n;
     cudaStream_t s = m->stream;
     const float max_d = mbf / mb;
     const size_t smem = (size_t)cap * sizeof(RightKp);

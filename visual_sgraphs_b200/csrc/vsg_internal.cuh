@@ -81,23 +81,72 @@ struct __align__(8) LevelKp {
 
 }  // namespace vsg
 
+namespace vsg {
+
+// Device scratch slots of a matcher (vsg_matcher::buf).  A slot's contents are only valid inside the call that wrote them
+// unless its line says otherwise; a function must not call another user of a slot while it still needs that slot's contents.
+enum DevSlot : int {
+    kSlotKnnParts = 0,     // knn2_device (match.cu): per-chunk top-2 partials
+    kSlotArg1,             // one-shot inputs: query descriptors (vsg_descriptor_distance, vsg_knn2, vsg_match_window), left
+                           // keypoints (stereo.cu), descriptors (mappoint.cu, bow.cu)
+    kSlotArg2,             // train descriptors (match.cu), left descriptors (stereo.cu)
+    kSlotArg3,             // distances / indices (match.cu), right keypoints (stereo.cu), list offsets (mappoint.cu)
+    kSlotArg4,             // distances / candidates (match.cu), right descriptors (stereo.cu)
+    kSlotArg5,             // vsg_match_window: train levels and skip flags
+    kSlotOut,              // one-shot results (vsg_match_window, stereo.cu, mappoint.cu, bow.cu), undistort input (frame_ops.cu);
+                           // area_search_ordered: the entries in query order
+    kSlotAreaQueries,      // area_search_raw / _ordered, area_best: the queries; second one-shot result (frame_ops.cu, stereo.cu)
+    kSlotAreaQdesc,        // area_search_raw / _ordered, area_best: the query descriptors
+    kSlotAreaCounts,       // area_search_raw / _ordered: per-query offset and count, the total; area_best: the results
+    kSlotAreaRaw,          // area_search_raw / _ordered: the entries as the kernel writes them (its size carries over as the
+                           // next search's first capacity)
+    kSlotAreaOrder,        // area_search_ordered: list pointers and the query of every entry
+    kSlotMapShardToken,    // vsg_search_by_projection_map_sharded: claim token and per-rank records
+    kSlotKnnSharded,       // vsg_knn2_sharded: own and gathered top-2 lists
+    kSlotTcQuery,          // knn2_tc_device (knn_tc.cu): expanded query descriptors
+    kSlotTcTrain,          // knn2_tc_device: expanded train descriptors
+    kSlotTcParts,          // knn2_tc_device: per-segment top-2 partials
+    kSlotBestMultiIn,      // area_best_multi: targets, queries and descriptors
+    kSlotBestMultiOut,     // area_best_multi: the results
+    kSlotBow,              // bow_dists, triangulation_candidates (match_methods_kf.cu): inputs, then results
+    kNumDevSlots
+};
+
+// Pinned host staging slots of a matcher (vsg_matcher::hbuf): results come back without page faults.  Same rule as DevSlot.
+enum HostSlot : int {
+    kHostAreaCounts = 0,   // area_search_raw: offsets, counts and total (AreaLists::off / cnt); area_search_ordered: list
+                           // pointers (OrderedLists::ptr) — both valid until the next area search; area_best: its results
+    kHostAreaEnt,          // area_search_raw / _ordered: the entries (AreaLists::raw, OrderedLists::ent), valid until the next
+                           // area search
+    kHostFrameStaging,     // vsg_frame_create: the frame's arrays on their way to the device
+    kHostMapQueries,       // projection_map_search: the map points' window queries
+    kHostAreaQid,          // area_search_ordered: the query of every entry (OrderedLists::qid), valid until the next area search
+    kHostBestMultiOut,     // area_best_multi: the results
+    kHostMapShardToken,    // vsg_search_by_projection_map_sharded: claim token and per-rank records
+    kHostBestMultiIn,      // area_best_multi: targets, queries and descriptors
+    kHostBow,              // bow_dists: inputs, then the distances (valid until the next BoW call); triangulation_candidates
+    kNumHostSlots
+};
+
+}  // namespace vsg
+
 // Matcher workspace: a stream plus scratch buffers that grow on demand (defined here so that match.cu and
 // match_methods.cu share it).
 struct vsg_matcher {
     int device = 0;
     cudaStream_t stream = nullptr;
-    void *buf[20] = {};      // device scratch slots; each entry point documents the slots it owns
-    size_t cap[20] = {};
-    void *hbuf[9] = {};      // pinned host staging (grows on demand): results come back without page faults
-    size_t hcap[9] = {};
-    std::vector<char> scratch[2];   // reusable host scratch of the search methods (query lists), kept across calls
+    void *buf[vsg::kNumDevSlots] = {};
+    size_t cap[vsg::kNumDevSlots] = {};
+    void *hbuf[vsg::kNumHostSlots] = {};
+    size_t hcap[vsg::kNumHostSlots] = {};
+    std::vector<int> scratch;   // projection_map_search: query -> map point (MapSearch::q_mp), valid until the next map search
     int sm_count = 148;
 };
 
 namespace vsg {
 
-vsg_status matcher_ensure(vsg_matcher *m, int slot, size_t bytes);
-vsg_status matcher_ensure_host(vsg_matcher *m, int slot, size_t bytes);
+vsg_status matcher_ensure(vsg_matcher *m, DevSlot slot, size_t bytes);
+vsg_status matcher_ensure_host(vsg_matcher *m, HostSlot slot, size_t bytes);
 // merge of `nparts` per-shard / per-segment top-2 lists ([nparts][nq][2]) by (distance, index) on the matcher's stream
 vsg_status launch_knn2_merge_parts(vsg_matcher *m, const int32_t *idx_parts, const int32_t *dist_parts, int nparts, int nq,
                                    int32_t *out_idx, int32_t *out_dist);
