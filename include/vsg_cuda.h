@@ -366,7 +366,9 @@ vsg_status vsg_search_by_bow(vsg_matcher *m, const vsg_frame_view *KF, const uin
 
 /* The same with a two-camera frame (F.Nleft = f_nleft != -1; ORBmatcher.cc:298-322, :362-390): F (and KF, if it has a
  * second camera) list the left camera's keypoints / descriptor rows first, then the right camera's, as mDescriptors does;
- * best and second-best are kept per camera.  f_nleft == -1 is vsg_search_by_bow. */
+ * best and second-best are kept per camera.  f_nleft == -1 is vsg_search_by_bow.  Both run vsg_search_by_bow_multi with one
+ * target and share its argument rules; vsg_last_error names a rejected argument.  A view with n > 0 needs both its keys
+ * and its descriptors, also when check_ori == 0. */
 vsg_status vsg_search_by_bow_2cam(vsg_matcher *m, const vsg_frame_view *KF, const uint8_t *kf_mp_valid,
                                   const vsg_frame_view *F, int f_nleft, int kf_nnodes, const int32_t *kf_nodes,
                                   const int32_t *kf_ptr, const int32_t *kf_idx, int f_nnodes, const int32_t *f_nodes,
@@ -426,7 +428,9 @@ vsg_status vsg_search_by_projection_sim3(vsg_matcher *m, const vsg_frame *KF, co
  * best_idx_out[i] = the keyframe feature the reference picks for point i (bestDist <= TH_LOW), else -1.  The
  * search of a point does not depend on the map-point bookkeeping of earlier points, so the caller applies
  * Replace / AddObservation / AddMapPoint in order afterwards, re-checking isBad() / IsInKeyFrame() as the
- * reference does at the top of each iteration.  *nfused_out counts the entries >= 0. */
+ * reference does at the top of each iteration.  *nfused_out counts the entries >= 0.  Variant 0 is
+ * vsg_fuse_search_multi with one target, variant 1 the same search without the gates; both share its argument rules,
+ * so KF must live on the matcher's device. */
 vsg_status vsg_fuse_search(vsg_matcher *m, const vsg_frame *KF, int n, const vsg_search_point *pts,
                            const uint8_t *desc, float th, const float *inv_level_sigma2, int variant,
                            int32_t *best_idx_out, int *nfused_out);
@@ -452,7 +456,8 @@ vsg_status vsg_search_by_sim3(vsg_matcher *m, const vsg_frame *KF1, const vsg_fr
                               int *nfound_out);
 
 /* SearchByBoW(KeyFrame* pKF1, KeyFrame* pKF2, vpMatches12) (ORBmatcher.cc:758-900).  mp_valid1/2[i] = map point
- * present and not bad.  matches12_out[i1] = i2 (the reference stores vpMapPoints2[i2]) or -1. */
+ * present and not bad.  matches12_out[i1] = i2 (the reference stores vpMapPoints2[i2]) or -1.  vsg_search_by_bow_kf_multi
+ * with one target: the same argument rules (a view with n > 0 needs both its keys and its descriptors). */
 vsg_status vsg_search_by_bow_kf(vsg_matcher *m, const vsg_frame_view *KF1, const uint8_t *mp_valid1,
                                 const vsg_frame_view *KF2, const uint8_t *mp_valid2, int nnodes1,
                                 const int32_t *nodes1, const int32_t *ptr1, const int32_t *idx1, int nnodes2,

@@ -103,12 +103,13 @@ vsg_status vsg_search_for_initialization(vsg_matcher *, const vsg_frame_view *F1
     *nmatches_out = orc_search_for_initialization(V(F1), V(F2), prev_matched, window_size, nnratio, check_ori, matches12_out);
     return VSG_OK;
 }
-vsg_status vsg_search_by_bow_2cam(vsg_matcher *, const vsg_frame_view *KF, const uint8_t *kf_mp_valid, const vsg_frame_view *F, int f_nleft,
-                                  int kf_nnodes, const int32_t *kf_nodes, const int32_t *kf_ptr, const int32_t *kf_idx, int f_nnodes,
-                                  const int32_t *f_nodes, const int32_t *f_ptr, const int32_t *f_idx, float nnratio, int check_ori,
-                                  int32_t *matches_f_out, int *nmatches_out) {
-    *nmatches_out = orc_search_by_bow_2cam(V(KF), kf_mp_valid, V(F), f_nleft, kf_nnodes, kf_nodes, kf_ptr, kf_idx, f_nnodes, f_nodes, f_ptr,
-                                           f_idx, nnratio, check_ori, matches_f_out);
+vsg_status vsg_search_by_bow_multi(vsg_matcher *, int ntargets, const vsg_bow_side *const *KFs, const vsg_bow_side *F, int f_nleft,
+                                   float nnratio, int check_ori, int32_t *matches_f_out, int *nmatches_out) {
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_bow_side &a = *KFs[t];
+        nmatches_out[t] = orc_search_by_bow_2cam(V(&a.view), a.mp_valid, V(&F->view), f_nleft, a.nnodes, a.nodes, a.ptr, a.idx, F->nnodes,
+                                                 F->nodes, F->ptr, F->idx, nnratio, check_ori, matches_f_out + (size_t)t * F->view.n);
+    }
     return VSG_OK;
 }
 vsg_status vsg_search_by_projection_reloc(vsg_matcher *, const vsg_frame *Cur, const uint8_t *occupied, int n, const vsg_search_point *pts,
@@ -130,18 +131,27 @@ vsg_status vsg_fuse_search(vsg_matcher *, const vsg_frame *KF, int n, const vsg_
     if (nfused_out) *nfused_out = nf;
     return VSG_OK;
 }
+vsg_status vsg_fuse_search_multi(vsg_matcher *, int ntargets, const vsg_frame *const *KFs, const float *const *inv_level_sigma2, int n,
+                                 const vsg_search_point *pts, const uint8_t *desc, float th, int32_t *best_idx_out) {
+    for (int t = 0; t < ntargets; ++t)
+        orc_fuse_search(V(KFs[t]), n, reinterpret_cast<const orc_search_point *>(pts) + (size_t)t * n, desc, th, inv_level_sigma2[t], 0,
+                        best_idx_out + (size_t)t * n);
+    return VSG_OK;
+}
 vsg_status vsg_search_by_sim3(vsg_matcher *, const vsg_frame *KF1, const vsg_frame *KF2, int n1, const vsg_search_point *pts1, const uint8_t *desc1,
                               int n2, const vsg_search_point *pts2, const uint8_t *desc2, float th, int32_t *matches12_out, int *nfound_out) {
     *nfound_out = orc_search_by_sim3_n(V(KF1), V(KF2), n1, reinterpret_cast<const orc_search_point *>(pts1), desc1, n2,
                                        reinterpret_cast<const orc_search_point *>(pts2), desc2, th, matches12_out);
     return VSG_OK;
 }
-vsg_status vsg_search_by_bow_kf(vsg_matcher *, const vsg_frame_view *KF1, const uint8_t *mp_valid1, const vsg_frame_view *KF2,
-                                const uint8_t *mp_valid2, int nn1, const int32_t *nodes1, const int32_t *ptr1, const int32_t *idx1, int nn2,
-                                const int32_t *nodes2, const int32_t *ptr2, const int32_t *idx2, float nnratio, int check_ori,
-                                int32_t *matches12_out, int *nmatches_out) {
-    *nmatches_out = orc_search_by_bow_kf(V(KF1), mp_valid1, V(KF2), mp_valid2, nn1, nodes1, ptr1, idx1, nn2, nodes2, ptr2, idx2, nnratio,
-                                         check_ori, matches12_out);
+vsg_status vsg_search_by_bow_kf_multi(vsg_matcher *, const vsg_bow_side *KF1, int ntargets, const vsg_bow_side *const *KF2s, float nnratio,
+                                      int check_ori, int32_t *matches12_out, int *nmatches_out) {
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_bow_side &b = *KF2s[t];
+        nmatches_out[t] = orc_search_by_bow_kf(V(&KF1->view), KF1->mp_valid, V(&b.view), b.mp_valid, KF1->nnodes, KF1->nodes, KF1->ptr,
+                                               KF1->idx, b.nnodes, b.nodes, b.ptr, b.idx, nnratio, check_ori,
+                                               matches12_out + (size_t)t * KF1->view.n);
+    }
     return VSG_OK;
 }
 vsg_status vsg_bow_pair_distances(vsg_matcher *, const vsg_frame_view *KF1, const uint8_t *use1, const vsg_frame_view *KF2, int nn1,

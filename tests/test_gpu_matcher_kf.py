@@ -69,6 +69,47 @@ def test_search_by_sim3(oracle):
     assert nf > 100
 
 
+def _tie_scene():
+    """A query at (320, 240) with radius 30 walks 7 x 7 grid cells (64 x 48 cells on 640 x 480), 32 per warp round.  The
+    keyframe has two keypoints with the query's own descriptor: keypoint 0 in cell (29, 21), the first of round 0, and
+    keypoint 1 in cell (35, 27), the 49th, in round 1; keypoint 2 is farther.  The reference's strict '<' keeps keypoint 0."""
+    from visual_sgraphs_b200._lib import KEYPOINT_DTYPE, SEARCH_POINT_DTYPE
+
+    def keys(xy):
+        k = np.zeros(len(xy), KEYPOINT_DTYPE)
+        k["x"], k["y"] = np.array(xy, np.float32).T
+        k["size"] = 31
+        return k
+
+    d = np.random.default_rng(3).integers(0, 256, 32, dtype=np.uint8)
+    kf = sc.frame_data(keys([(292, 212), (348, 268), (330, 250)]), np.stack([d, d, d ^ 0xFF]))
+    q = np.zeros(1, SEARCH_POINT_DTYPE)
+    q["u"], q["v"], q["valid"] = 320, 240, 1
+    return kf, q, d[None].copy(), keys
+
+
+@pytest.mark.parametrize("variant", [0, 1])
+def test_fuse_search_tie_across_rounds(oracle, variant):
+    kf, q, d, _ = _tie_scene()
+    inv_sigma2 = np.full(8, 1e-4, np.float32)              # chi-square gates wide enough for the 28-px offsets
+    m = _matcher()
+    nf, best = m.FuseSearch(m.frame(kf), q, d, 30.0, inv_sigma2, sim3_variant=bool(variant))
+    wnf, wbest = oracle.fuse_search(kf.view, q, d, 30.0, inv_sigma2, variant)
+    assert nf == wnf == 1 and np.array_equal(best, wbest) and best[0] == 0
+
+
+def test_search_by_sim3_tie_across_rounds(oracle):
+    kf2, q, d, keys = _tie_scene()
+    kf1 = sc.frame_data(keys([(100, 100)]), d)                # its one point projects onto the window; KF2's keypoint 0
+    p2 = np.zeros(kf2.n, q.dtype)                             # projects back onto it
+    p2[0]["u"], p2[0]["v"], p2[0]["valid"] = 100, 100, 1
+    d2 = np.ascontiguousarray(kf2.descriptors)
+    m = _matcher()
+    nf, m12 = m.SearchBySim3(m.frame(kf1), m.frame(kf2), q, d, p2, d2, 30.0)
+    wnf, wm12 = oracle.search_by_sim3(kf1.view, kf2.view, q, d, p2, d2, 30.0)
+    assert nf == wnf == 1 and np.array_equal(m12, wm12) and m12[0] == 0
+
+
 @pytest.mark.parametrize("check_ori", [True, False])
 def test_search_by_bow_kf(oracle, check_ori):
     ka, da, kb, db = sc.two_frames(oracle, shift=(3, 2))

@@ -3,7 +3,7 @@ size-dependent paths of the device code (run on the B200 with -m gpu).
 
 test_gpu_matcher_methods.py / test_gpu_matcher_kf.py check every method on one 640x480 scene with integer bounds and
 an 8 x 1.2 pyramid.  The device code depends on exactly what that scene holds fixed:
-  - the grid geometry: area_search_kernel / window_best_kernel find cells with floorf / ceilf((x - min_x +- r) * inv_w),
+  - the grid geometry: area_search_kernel / window_best_multi_kernel find cells with floorf / ceilf((x - min_x +- r) * inv_w),
     vsg_frame_create bins keypoints with std::round and drops the ones outside the grid;
   - the level tables: windows scale with scale[level], levels [level - 1, level] (min_level = -1 at level 0), the Fuse
     chi-square gate reads inv_sigma2[octave];

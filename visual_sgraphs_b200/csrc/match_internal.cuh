@@ -70,12 +70,10 @@ struct AreaLists {
 // n_qdesc rows of qdesc are uploaded (queries pick theirs by desc_idx).
 vsg_status area_search(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc, int n_qdesc,
                        std::vector<int> &ptr, std::vector<int2> &ent);
-// Best candidate per query on the device (window / level gates, optional chi-square gates when inv_sigma2 != nullptr): the
-// whole search of the methods whose queries are independent of one another.  out[k] = (index or -1, distance or INT_MAX).
-vsg_status area_best(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc, const float *inv_sigma2,
-                     std::vector<int2> &out);
-// area_best with the chi-square gates over the queries of several frames at once (one copy in, one launch, one copy out):
-// query k searches frames[q_target[k]] with inv_sigma2[q_target[k]] and descriptor row qs[k].desc_idx of qdesc (n_qdesc rows).
+// Best candidate per query on the device, over the queries of one or several frames at once (one copy in, one launch, one
+// copy out): the whole search of the methods whose queries are independent of one another.  Query k searches
+// frames[q_target[k]] with descriptor row qs[k].desc_idx of qdesc (n_qdesc rows), through the window / level gates and, unless
+// inv_sigma2 is nullptr, the chi-square gates with inv_sigma2[q_target[k]].  out[k] = (index or -1, distance or INT_MAX).
 vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *frames, const float *const *inv_sigma2, int nq,
                            const AreaQuery *qs, const int *q_target, int n_qdesc, const uint8_t *qdesc, std::vector<int2> &out);
 // area_search without the re-pack into query order
@@ -132,8 +130,6 @@ vsg_status bow_walk(const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs
 // .. seg_ptr[k+1]) are walk k's.  *dist points into the matcher's pinned staging and stays valid until its next BoW call.
 vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std::vector<BowSeg> &segs, const int *seg_ptr,
                      int64_t npairs, const uint16_t **dist);
-// bow_walk and bow_dists for the one walk of a single-target call.
-vsg_status bow_walk_dists(vsg_matcher *m, const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs, const uint16_t **dist);
 // What is wrong with one side of a multi-target BoW call (nullptr: nothing); the map-point flags only if it needs them.
 const char *bow_side_problem(const vsg_bow_side *s, bool needs_valid);
 // The target loop of the multi-target BoW calls: problem(t) says what is wrong with target t (nullptr: nothing), and

@@ -200,19 +200,9 @@ __device__ __forceinline__ int2 window_best(const FrameDev &f, const Chi2Gate &g
     return make_int2(best_idx, best);
 }
 
+// window_best over the queries of one or several keyframes (Fuse into every neighbour of a keyframe): query q searches
+// targets[q_target[q]] with that keyframe's own grid, level and (kChi2) chi-square tables, and descriptor row desc_idx.
 template <bool kChi2>
-__global__ void __launch_bounds__(256) window_best_kernel(FrameDev f, int nq, const AreaQuery *__restrict__ qs,
-                                                          const uint4 *__restrict__ qdesc, Chi2Gate gate,
-                                                          int2 *__restrict__ best_out) {
-    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (q >= nq) return;
-    const AreaQuery a = qs[q];
-    const int2 r = window_best<kChi2>(f, gate, a, qdesc, a.desc_idx >= 0 ? a.desc_idx : q, lane);
-    if (lane == 0) best_out[q] = r;
-}
-
-// The same over the queries of several keyframes at once (Fuse into every neighbour of a keyframe): query q searches
-// targets[q_target[q]] with that keyframe's own grid, level and chi-square tables, and descriptor row desc_idx.
 __global__ void __launch_bounds__(256) window_best_multi_kernel(const FuseTarget *__restrict__ targets, int nq,
                                                                 const AreaQuery *__restrict__ qs, const int *__restrict__ q_target,
                                                                 const uint4 *__restrict__ qdesc, int2 *__restrict__ best_out) {
@@ -220,7 +210,7 @@ __global__ void __launch_bounds__(256) window_best_multi_kernel(const FuseTarget
     if (q >= nq) return;
     const AreaQuery a = qs[q];
     const FuseTarget &t = targets[q_target[q]];
-    const int2 r = window_best<true>(t.f, t.gate, a, qdesc, a.desc_idx, lane);
+    const int2 r = window_best<kChi2>(t.f, t.gate, a, qdesc, a.desc_idx, lane);
     if (lane == 0) best_out[q] = r;
 }
 
@@ -233,36 +223,6 @@ static Chi2Gate chi2_gate(const vsg_frame *f, const float *inv_sigma2) {
     Chi2Gate gate;
     for (int l = 0; l < kMaxLevels; ++l) gate.inv_sigma2[l] = inv_sigma2 && l < f->n_levels ? inv_sigma2[l] : 0.f;
     return gate;
-}
-
-// Best candidate of every query (see window_best_kernel); out[k] = (keypoint index or -1, distance or INT_MAX), host memory.
-vsg_status area_best(vsg_matcher *m, const vsg_frame *f, int nq, const AreaQuery *qs, const uint8_t *qdesc, const float *inv_sigma2,
-                     std::vector<int2> &out) {
-    out.assign(nq, make_int2(-1, INT_MAX));
-    if (nq == 0) return VSG_OK;
-    cudaStream_t s = m->stream;
-    vsg_status st;
-    if ((st = matcher_ensure(m, kSlotAreaQueries, (size_t)nq * sizeof(AreaQuery))) ||
-        (st = matcher_ensure(m, kSlotAreaQdesc, (size_t)nq * 32)) || (st = matcher_ensure(m, kSlotAreaCounts, (size_t)nq * sizeof(int2))) ||
-        (st = matcher_ensure_host(m, kHostAreaCounts, (size_t)nq * sizeof(int2))))
-        return st;
-    AreaQuery *qs_d = (AreaQuery *)m->buf[kSlotAreaQueries];
-    uint4 *qdesc_d = (uint4 *)m->buf[kSlotAreaQdesc];
-    int2 *best_d = (int2 *)m->buf[kSlotAreaCounts];
-    CK(cudaMemcpyAsync(qs_d, qs, (size_t)nq * sizeof(AreaQuery), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(qdesc_d, qdesc, (size_t)nq * 32, cudaMemcpyHostToDevice, s));
-    const FrameDev fd = frame_dev(f);
-    const Chi2Gate gate = chi2_gate(f, inv_sigma2);
-    if (inv_sigma2)
-        window_best_kernel<true><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, qs_d, qdesc_d, gate, best_d);
-    else
-        window_best_kernel<false><<<(nq + 7) / 8, 256, 0, s>>>(fd, nq, qs_d, qdesc_d, gate, best_d);
-    count_launch();
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(m->hbuf[kHostAreaCounts], best_d, (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    memcpy(out.data(), m->hbuf[kHostAreaCounts], (size_t)nq * sizeof(int2));
-    return VSG_OK;
 }
 
 vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *frames, const float *const *inv_sigma2, int nq,
@@ -280,14 +240,15 @@ vsg_status area_best_multi(vsg_matcher *m, int ntargets, const vsg_frame *const 
         return st;
     uint8_t *h = (uint8_t *)m->hbuf[kHostBestMultiIn], *d = (uint8_t *)m->buf[kSlotBestMultiIn];
     FuseTarget *ht = (FuseTarget *)(h + o_tgt);
-    for (int t = 0; t < ntargets; ++t) ht[t] = FuseTarget{frame_dev(frames[t]), chi2_gate(frames[t], inv_sigma2[t])};
+    for (int t = 0; t < ntargets; ++t)
+        ht[t] = FuseTarget{frame_dev(frames[t]), chi2_gate(frames[t], inv_sigma2 ? inv_sigma2[t] : nullptr)};
     memcpy(h + o_q, qs, (size_t)nq * sizeof(AreaQuery));
     memcpy(h + o_qt, q_target, (size_t)nq * sizeof(int));
     memcpy(h + o_desc, qdesc, (size_t)n_qdesc * 32);
     CK(cudaMemcpyAsync(d, h, total, cudaMemcpyHostToDevice, s));
-    window_best_multi_kernel<<<(nq + 7) / 8, 256, 0, s>>>((const FuseTarget *)(d + o_tgt), nq, (const AreaQuery *)(d + o_q),
-                                                          (const int *)(d + o_qt), (const uint4 *)(d + o_desc),
-                                                          (int2 *)m->buf[kSlotBestMultiOut]);
+    const auto kernel = inv_sigma2 ? window_best_multi_kernel<true> : window_best_multi_kernel<false>;
+    kernel<<<(nq + 7) / 8, 256, 0, s>>>((const FuseTarget *)(d + o_tgt), nq, (const AreaQuery *)(d + o_q), (const int *)(d + o_qt),
+                                        (const uint4 *)(d + o_desc), (int2 *)m->buf[kSlotBestMultiOut]);
     count_launch();
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(m->hbuf[kHostBestMultiOut], m->buf[kSlotBestMultiOut], (size_t)nq * sizeof(int2), cudaMemcpyDeviceToHost, s));
@@ -1156,26 +1117,20 @@ vsg_status vsg_search_by_bow(vsg_matcher *m, const vsg_frame_view *KF, const uin
 // The same with a two-camera frame (F.Nleft = f_nleft != -1): F's features [0, f_nleft) are the left camera's, the rest
 // the right camera's; best / second-best are kept per camera (:298-322) and the right-camera match is taken inside the
 // left one's `bestDist1 <= TH_LOW` block with its ratio test disabled (`|| true`, :364-366).  f_nleft == -1: single camera.
+// vsg_search_by_bow_multi with one target.
 vsg_status vsg_search_by_bow_2cam(vsg_matcher *m, const vsg_frame_view *KF, const uint8_t *kf_mp_valid,
                                   const vsg_frame_view *F, int f_nleft, int kf_nnodes, const int32_t *kf_nodes,
                                   const int32_t *kf_ptr, const int32_t *kf_idx, int f_nnodes, const int32_t *f_nodes,
                                   const int32_t *f_ptr, const int32_t *f_idx, float nnratio, int check_ori,
                                   int32_t *matches_f_out, int *nmatches_out) {
-    if (!m || !KF || !F || !matches_f_out || kf_nnodes < 0 || f_nnodes < 0 || (KF->n > 0 && !kf_mp_valid) || f_nleft < -1 ||
-        f_nleft > F->n)
+    if (!KF || !F || !matches_f_out) {
+        set_error("vsg_search_by_bow_2cam: null keyframe, frame or output");
         return VSG_ERR_INVALID;
-    CK(cudaSetDevice(m->device));
-    // the merge walk over the two FeatureVectors (:248-376): one query per keyframe feature with a usable map
-    // point inside a common node; its candidates are the frame features of that node, in vIndicesF order
-    const BowWalk w{KF, kf_mp_valid, FeatVec{kf_nnodes, kf_nodes, kf_ptr, kf_idx}, F, FeatVec{f_nnodes, f_nodes, f_ptr, f_idx}};
-    std::vector<BowSeg> segs;
-    int64_t npairs = 0;
-    const uint16_t *dist;
-    const vsg_status st = bow_walk_dists(m, w, segs, &npairs, &dist);
-    if (st != VSG_OK) return st;
-    const int nmatches = bow_replay_kf_f(KF, F, f_nleft, w.b, segs.data(), (int)segs.size(), dist, nnratio, check_ori, matches_f_out);
-    if (nmatches_out) *nmatches_out = nmatches;
-    return VSG_OK;
+    }
+    const vsg_bow_side kf{*KF, kf_mp_valid, kf_nnodes, kf_nodes, kf_ptr, kf_idx}, f{*F, nullptr, f_nnodes, f_nodes, f_ptr, f_idx};
+    const vsg_bow_side *kfs = &kf;
+    int nmatches;
+    return vsg_search_by_bow_multi(m, 1, &kfs, &f, f_nleft, nnratio, check_ori, matches_f_out, nmatches_out ? nmatches_out : &nmatches);
 }
 
 // vsg_search_by_bow_2cam(KFs[t] against F) for every target in one upload, one launch and one download
@@ -1203,6 +1158,8 @@ vsg_status vsg_search_by_bow_multi(vsg_matcher *m, int ntargets, const vsg_bow_s
     std::vector<BowSeg> segs;
     std::vector<int> seg_ptr;
     int64_t npairs = 0;
+    // the merge walk over the two FeatureVectors (:248-376): one query per keyframe feature with a usable map
+    // point inside a common node; its candidates are the frame features of that node, in vIndicesF order
     vsg_status st = bow_walk_targets(
         "vsg_search_by_bow_multi", ntargets, [&](int t) { return bow_side_problem(KFs[t], true); },
         [&](int t) {

@@ -33,7 +33,7 @@ using namespace vsg;
 namespace {
 
 // Queries for the valid points of a projected-point list: radius = th * scale[level], levels [level+lo, level+hi]; appended
-// to qs, with the point's index in q_src.
+// to qs, with the point's index in q_src.  The point's index is also its descriptor row: the callers upload the whole table.
 vsg_status append_queries(const vsg_frame *F, int n, const vsg_search_point *pts, float th, int lo, int hi,
                           std::vector<AreaQuery> &qs, std::vector<int> &q_src) {
     for (int i = 0; i < n; ++i) {
@@ -44,20 +44,9 @@ vsg_status append_queries(const vsg_frame *F, int n, const vsg_search_point *pts
             return VSG_ERR_INVALID;
         }
         const float radius = th * F->scale[p.level];
-        qs.push_back(AreaQuery{p.u, p.v, radius, p.level + lo, p.level + hi, 0.f, -1.f});
+        qs.push_back(AreaQuery{p.u, p.v, radius, p.level + lo, p.level + hi, 0.f, -1.f, 256, i});
         q_src.push_back(i);
     }
-    return VSG_OK;
-}
-
-// The same as a fresh list, with the descriptor rows of the queries gathered into qdesc.
-vsg_status build_queries(const vsg_frame *F, int n, const vsg_search_point *pts, const uint8_t *desc, float th, int lo,
-                         int hi, std::vector<AreaQuery> &qs, std::vector<int> &q_src, std::vector<uint8_t> &qdesc) {
-    qs.clear(); q_src.clear();
-    const vsg_status st = append_queries(F, n, pts, th, lo, hi, qs, q_src);
-    if (st != VSG_OK) return st;
-    qdesc.resize(qs.size() * 32);
-    for (size_t k = 0; k < qs.size(); ++k) memcpy(&qdesc[k * 32], desc + (size_t)q_src[k] * 32, 32);
     return VSG_OK;
 }
 
@@ -167,12 +156,6 @@ vsg_status bow_dists(vsg_matcher *m, int nwalks, const BowWalk *walks, const std
     CK(cudaStreamSynchronize(s));
     *dist = (const uint16_t *)(h + o_out);
     return VSG_OK;
-}
-
-vsg_status bow_walk_dists(vsg_matcher *m, const BowWalk &w, std::vector<BowSeg> &segs, int64_t *npairs, const uint16_t **dist) {
-    const vsg_status st = bow_walk(w, segs, npairs);
-    const int seg_ptr[2] = {0, (int)segs.size()};
-    return st != VSG_OK ? st : bow_dists(m, 1, &w, segs, seg_ptr, *npairs, dist);
 }
 
 const char *bow_side_problem(const vsg_bow_side *s, bool needs_valid) {
@@ -348,6 +331,54 @@ static vsg_status triangulation_candidates(vsg_matcher *m, const char *who, cons
     return VSG_OK;
 }
 
+// vsg_fuse_search_multi under the name `who` (vsg_fuse_search runs it with one target); inv_level_sigma2 == nullptr searches
+// without the chi-square gates (Fuse(KF, Scw, ...)).  Every map point's search is independent of the others: the best
+// candidate is picked on the device, one (index, distance) pair per query comes back.
+static vsg_status fuse_search(vsg_matcher *m, const char *who, int ntargets, const vsg_frame *const *KFs,
+                              const float *const *inv_level_sigma2, int n, const vsg_search_point *pts, const uint8_t *desc, float th,
+                              int32_t *best_idx_out) {
+    if (!m || ntargets < 0 || n < 0) {
+        set_error("%s: %d targets, %d points", who, ntargets, n);
+        return VSG_ERR_INVALID;
+    }
+    if (ntargets > 0 && (!KFs || (n > 0 && (!pts || !desc || !best_idx_out)))) {
+        set_error("%s: null target table, points, descriptors or output", who);
+        return VSG_ERR_INVALID;
+    }
+    for (int t = 0; t < ntargets; ++t) {
+        if (!KFs[t] || (inv_level_sigma2 && !inv_level_sigma2[t])) {
+            set_error("%s: target %d: null keyframe or level table", who, t);
+            return VSG_ERR_INVALID;
+        }
+        if (KFs[t]->device != m->device) {
+            set_error("%s: target %d lives on device %d, the matcher on device %d", who, t, KFs[t]->device, m->device);
+            return VSG_ERR_INVALID;
+        }
+    }
+    CK(cudaSetDevice(m->device));
+    std::vector<AreaQuery> qs;
+    std::vector<int> q_src, q_tgt;
+    for (int t = 0; t < ntargets; ++t) {
+        const vsg_search_point *tp = pts + (size_t)t * n;
+        const size_t first = qs.size();
+        const vsg_status st = append_queries(KFs[t], n, tp, th, -1, 0, qs, q_src);      // :1246, :1270-1271
+        if (st != VSG_OK) {
+            const std::string why = vsg_last_error();
+            set_error("%s: target %d: %s", who, t, why.c_str());
+            return st;
+        }
+        for (size_t k = first; k < qs.size(); ++k) qs[k].xr = tp[q_src[k]].ur;          // the chi-square gate's right coordinate
+        q_tgt.resize(qs.size(), t);
+    }
+    std::vector<int2> best;
+    vsg_status st = area_best_multi(m, ntargets, KFs, inv_level_sigma2, (int)qs.size(), qs.data(), q_tgt.data(), n, desc, best);
+    if (st != VSG_OK) return st;
+    for (size_t i = 0; i < (size_t)ntargets * n; ++i) best_idx_out[i] = -1;
+    for (size_t k = 0; k < qs.size(); ++k)
+        if (best[k].x >= 0 && best[k].y <= TH_LOW) best_idx_out[(size_t)q_tgt[k] * n + q_src[k]] = best[k].x;   // :1316, :1428
+    return VSG_OK;
+}
+
 }  // namespace vsg
 
 extern "C" {
@@ -360,11 +391,10 @@ vsg_status vsg_search_by_projection_reloc(vsg_matcher *m, const vsg_frame *Cur, 
     CK(cudaSetDevice(m->device));
     std::vector<AreaQuery> qs;
     std::vector<int> q_src, ptr;
-    std::vector<uint8_t> qdesc;
     std::vector<int2> ent;
-    vsg_status st = build_queries(Cur, n, pts, desc, th, -1, +1, qs, q_src, qdesc);   // :1927
+    vsg_status st = append_queries(Cur, n, pts, th, -1, +1, qs, q_src);              // :1927
     if (st != VSG_OK) return st;
-    if ((st = area_search(m, Cur, (int)qs.size(), qs.data(), qdesc.data(), (int)qs.size(), ptr, ent)) != VSG_OK) return st;
+    if ((st = area_search(m, Cur, (int)qs.size(), qs.data(), desc, n, ptr, ent)) != VSG_OK) return st;
     std::vector<uint8_t> taken(occupied, occupied + Cur->n);                          // CurrentFrame.mvpMapPoints[i2]
     for (int i = 0; i < Cur->n; ++i) assign_out[i] = -1;
     std::vector<int> rot_hist[HISTO_LENGTH];
@@ -391,11 +421,10 @@ vsg_status vsg_search_by_projection_sim3(vsg_matcher *m, const vsg_frame *KF, co
     CK(cudaSetDevice(m->device));
     std::vector<AreaQuery> qs;
     std::vector<int> q_src, ptr;
-    std::vector<uint8_t> qdesc;
     std::vector<int2> ent;
-    vsg_status st = build_queries(KF, n, pts, desc, (float)th, -1, 0, qs, q_src, qdesc);   // :486, :502-503
+    vsg_status st = append_queries(KF, n, pts, (float)th, -1, 0, qs, q_src);          // :486, :502-503
     if (st != VSG_OK) return st;
-    if ((st = area_search(m, KF, (int)qs.size(), qs.data(), qdesc.data(), (int)qs.size(), ptr, ent)) != VSG_OK) return st;
+    if ((st = area_search(m, KF, (int)qs.size(), qs.data(), desc, n, ptr, ent)) != VSG_OK) return st;
     std::vector<uint8_t> taken(matched, matched + KF->n);                            // vpMatched[idx]
     for (int i = 0; i < KF->n; ++i) assign_out[i] = -1;
     int nmatches = 0;
@@ -412,85 +441,30 @@ vsg_status vsg_search_by_projection_sim3(vsg_matcher *m, const vsg_frame *KF, co
     return VSG_OK;
 }
 
-// the search part of ORBmatcher.cc:1148-1335 (variant 0) and :1337-1446 (variant 1)
+// the search part of ORBmatcher.cc:1148-1335 (variant 0) and :1337-1446 (variant 1): vsg_fuse_search_multi with one target,
+// and for variant 1 without the chi-square gates
 vsg_status vsg_fuse_search(vsg_matcher *m, const vsg_frame *KF, int n, const vsg_search_point *pts,
                            const uint8_t *desc, float th, const float *inv_level_sigma2, int variant,
                            int32_t *best_idx_out, int *nfused_out) {
-    if (!m || !KF || n < 0 || (n > 0 && (!pts || !desc || !best_idx_out)) || (variant == 0 && !inv_level_sigma2) ||
-        (variant != 0 && variant != 1))
+    if ((variant != 0 && variant != 1) || (variant == 0 && !inv_level_sigma2)) {
+        set_error("vsg_fuse_search: variant %d%s", variant, variant == 0 ? " without a level table" : " is not 0 or 1");
         return VSG_ERR_INVALID;
-    CK(cudaSetDevice(m->device));
-    std::vector<AreaQuery> qs;
-    std::vector<int> q_src;
-    std::vector<uint8_t> qdesc;
-    vsg_status st = build_queries(KF, n, pts, desc, th, -1, 0, qs, q_src, qdesc);     // :1246, :1270-1271
-    if (st != VSG_OK) return st;
-    if (variant == 0)
-        for (size_t k = 0; k < qs.size(); ++k) qs[k].xr = pts[q_src[k]].ur;         // the right coordinate of the chi-square gate
-    // every map point's search is independent of the others: the best candidate (with the chi-square gates of :1273-1299 for
-    // the pose-based variant) is picked on the device, one (index, distance) pair per point comes back
-    std::vector<int2> best;
-    if ((st = area_best(m, KF, (int)qs.size(), qs.data(), qdesc.data(), variant == 0 ? inv_level_sigma2 : nullptr, best)) != VSG_OK)
-        return st;
-    for (int i = 0; i < n; ++i) best_idx_out[i] = -1;
-    int nfused = 0;
-    for (size_t k = 0; k < qs.size(); ++k) {
-        if (best[k].x >= 0 && best[k].y <= TH_LOW) {                                 // :1316, :1428
-            best_idx_out[q_src[k]] = best[k].x;
-            ++nfused;
-        }
     }
-    if (nfused_out) *nfused_out = nfused;
-    return VSG_OK;
+    const vsg_status st = fuse_search(m, "vsg_fuse_search", 1, &KF, variant == 0 ? &inv_level_sigma2 : nullptr, n, pts, desc, th,
+                                      best_idx_out);
+    if (st == VSG_OK && nfused_out) *nfused_out = (int)std::count_if(best_idx_out, best_idx_out + n, [](int32_t b) { return b >= 0; });
+    return st;
 }
 
 // vsg_fuse_search(..., variant 0, ...) once per target keyframe, all targets in one upload, one launch and one download:
 // the searches of LocalMapping::SearchInNeighbors' loop of Fuse calls (LocalMapping.cc:764-802)
 vsg_status vsg_fuse_search_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *KFs, const float *const *inv_level_sigma2,
                                  int n, const vsg_search_point *pts, const uint8_t *desc, float th, int32_t *best_idx_out) {
-    if (!m || ntargets < 0 || n < 0) {
-        set_error("vsg_fuse_search_multi: %d targets, %d points", ntargets, n);
+    if (ntargets > 0 && !inv_level_sigma2) {
+        set_error("vsg_fuse_search_multi: null level table");
         return VSG_ERR_INVALID;
     }
-    if (ntargets > 0 && (!KFs || !inv_level_sigma2 || (n > 0 && (!pts || !desc || !best_idx_out)))) {
-        set_error("vsg_fuse_search_multi: null target table, level table, points, descriptors or output");
-        return VSG_ERR_INVALID;
-    }
-    for (int t = 0; t < ntargets; ++t) {
-        if (!KFs[t] || !inv_level_sigma2[t]) {
-            set_error("vsg_fuse_search_multi: target %d: null keyframe or level table", t);
-            return VSG_ERR_INVALID;
-        }
-        if (KFs[t]->device != m->device) {
-            set_error("vsg_fuse_search_multi: target %d lives on device %d, the matcher on device %d", t, KFs[t]->device, m->device);
-            return VSG_ERR_INVALID;
-        }
-    }
-    CK(cudaSetDevice(m->device));
-    std::vector<AreaQuery> qs;
-    std::vector<int> q_src, q_tgt;
-    for (int t = 0; t < ntargets; ++t) {
-        const vsg_search_point *tp = pts + (size_t)t * n;
-        const size_t first = qs.size();
-        const vsg_status st = append_queries(KFs[t], n, tp, th, -1, 0, qs, q_src);      // :1246, :1270-1271
-        if (st != VSG_OK) {
-            const std::string why = vsg_last_error();
-            set_error("vsg_fuse_search_multi: target %d: %s", t, why.c_str());
-            return st;
-        }
-        for (size_t k = first; k < qs.size(); ++k) {
-            qs[k].xr = tp[q_src[k]].ur;                                                    // the chi-square gate's right coordinate
-            qs[k].desc_idx = q_src[k];                                                     // desc is shared by all targets
-        }
-        q_tgt.resize(qs.size(), t);
-    }
-    std::vector<int2> best;
-    vsg_status st = area_best_multi(m, ntargets, KFs, inv_level_sigma2, (int)qs.size(), qs.data(), q_tgt.data(), n, desc, best);
-    if (st != VSG_OK) return st;
-    for (size_t i = 0; i < (size_t)ntargets * n; ++i) best_idx_out[i] = -1;
-    for (size_t k = 0; k < qs.size(); ++k)
-        if (best[k].x >= 0 && best[k].y <= TH_LOW) best_idx_out[(size_t)q_tgt[k] * n + q_src[k]] = best[k].x;   // :1316
-    return VSG_OK;
+    return fuse_search(m, "vsg_fuse_search_multi", ntargets, KFs, inv_level_sigma2, n, pts, desc, th, best_idx_out);
 }
 
 // ORBmatcher.cc:1448-1665
@@ -513,11 +487,13 @@ vsg_status vsg_search_by_sim3(vsg_matcher *m, const vsg_frame *KF1, const vsg_fr
         std::vector<int> &out = dir == 0 ? match1 : match2;
         std::vector<AreaQuery> qs;
         std::vector<int> q_src;
-        std::vector<uint8_t> qdesc;
-        vsg_status st = build_queries(target, n, dir == 0 ? pts1 : pts2, dir == 0 ? desc1 : desc2, th, -1, 0, qs, q_src, qdesc);
+        vsg_status st = append_queries(target, n, dir == 0 ? pts1 : pts2, th, -1, 0, qs, q_src);
         if (st != VSG_OK) return st;
+        const std::vector<int> q_tgt(qs.size(), 0);
         std::vector<int2> best;                                                      // independent queries: best on the device
-        if ((st = area_best(m, target, (int)qs.size(), qs.data(), qdesc.data(), nullptr, best)) != VSG_OK) return st;
+        if ((st = area_best_multi(m, 1, &target, nullptr, (int)qs.size(), qs.data(), q_tgt.data(), n, dir == 0 ? desc1 : desc2,
+                                  best)) != VSG_OK)
+            return st;
         for (size_t k = 0; k < qs.size(); ++k)
             if (best[k].x >= 0 && best[k].y <= TH_HIGH) out[q_src[k]] = best[k].x;   // :1556, :1631
     }
@@ -531,25 +507,20 @@ vsg_status vsg_search_by_sim3(vsg_matcher *m, const vsg_frame *KF1, const vsg_fr
     return VSG_OK;
 }
 
-// ORBmatcher.cc:758-900
+// ORBmatcher.cc:758-900: vsg_search_by_bow_kf_multi with one target
 vsg_status vsg_search_by_bow_kf(vsg_matcher *m, const vsg_frame_view *KF1, const uint8_t *mp_valid1,
                                 const vsg_frame_view *KF2, const uint8_t *mp_valid2, int nnodes1,
                                 const int32_t *nodes1, const int32_t *ptr1, const int32_t *idx1, int nnodes2,
                                 const int32_t *nodes2, const int32_t *ptr2, const int32_t *idx2, float nnratio,
                                 int check_ori, int32_t *matches12_out, int *nmatches_out) {
-    if (!m || !KF1 || !KF2 || !featvec_ok(nnodes1, nodes1, ptr1, idx1) || !featvec_ok(nnodes2, nodes2, ptr2, idx2) ||
-        (KF1->n > 0 && (!mp_valid1 || !matches12_out)) || (KF2->n > 0 && !mp_valid2))
+    if (!KF1 || !KF2) {
+        set_error("vsg_search_by_bow_kf: null keyframe");
         return VSG_ERR_INVALID;
-    CK(cudaSetDevice(m->device));
-    const BowWalk w{KF1, mp_valid1, FeatVec{nnodes1, nodes1, ptr1, idx1}, KF2, FeatVec{nnodes2, nodes2, ptr2, idx2}};
-    std::vector<BowSeg> segs;
-    int64_t npairs = 0;
-    const uint16_t *dist;
-    const vsg_status st = bow_walk_dists(m, w, segs, &npairs, &dist);
-    if (st != VSG_OK) return st;
-    const int nmatches = bow_replay_kf(KF1, KF2, mp_valid2, w.b, segs.data(), (int)segs.size(), dist, nnratio, check_ori, matches12_out);
-    if (nmatches_out) *nmatches_out = nmatches;
-    return VSG_OK;
+    }
+    const vsg_bow_side k1{*KF1, mp_valid1, nnodes1, nodes1, ptr1, idx1}, k2{*KF2, mp_valid2, nnodes2, nodes2, ptr2, idx2};
+    const vsg_bow_side *k2s = &k2;
+    int nmatches;
+    return vsg_search_by_bow_kf_multi(m, &k1, 1, &k2s, nnratio, check_ori, matches12_out, nmatches_out ? nmatches_out : &nmatches);
 }
 
 // vsg_search_by_bow_kf(KF1 against KF2s[t]) for every target in one upload, one launch and one download
@@ -608,8 +579,10 @@ vsg_status vsg_bow_pair_distances(vsg_matcher *m, const vsg_frame_view *KF1, con
     std::vector<BowSeg> segs;
     int64_t npairs = 0;
     const uint16_t *dist;
-    const vsg_status st = bow_walk_dists(m, w, segs, &npairs, &dist);
+    vsg_status st = bow_walk(w, segs, &npairs);
     if (st != VSG_OK) return st;
+    const int seg_ptr[2] = {0, (int)segs.size()};
+    if ((st = bow_dists(m, 1, &w, segs, seg_ptr, npairs, &dist)) != VSG_OK) return st;
     *nq_out = (int)segs.size();
     *total_out = (int)npairs;
     if ((int)segs.size() > q_capacity || npairs > capacity) return VSG_ERR_CAPACITY;

@@ -95,9 +95,9 @@ enum DevSlot : int {
     kSlotArg5,             // vsg_match_window: train levels and skip flags
     kSlotOut,              // one-shot results (vsg_match_window, stereo.cu, mappoint.cu, bow.cu), undistort input (frame_ops.cu);
                            // area_search_ordered: the entries in query order
-    kSlotAreaQueries,      // area_search_raw / _ordered, area_best: the queries; second one-shot result (frame_ops.cu, stereo.cu)
-    kSlotAreaQdesc,        // area_search_raw / _ordered, area_best: the query descriptors
-    kSlotAreaCounts,       // area_search_raw / _ordered: per-query offset and count, the total; area_best: the results
+    kSlotAreaQueries,      // area_search_raw / _ordered: the queries; second one-shot result (frame_ops.cu, stereo.cu)
+    kSlotAreaQdesc,        // area_search_raw / _ordered: the query descriptors
+    kSlotAreaCounts,       // area_search_raw / _ordered: per-query offset and count, the total
     kSlotAreaRaw,          // area_search_raw / _ordered: the entries as the kernel writes them (its size carries over as the
                            // next search's first capacity)
     kSlotAreaOrder,        // area_search_ordered: list pointers and the query of every entry
@@ -115,7 +115,7 @@ enum DevSlot : int {
 // Pinned host staging slots of a matcher (vsg_matcher::hbuf): results come back without page faults.  Same rule as DevSlot.
 enum HostSlot : int {
     kHostAreaCounts = 0,   // area_search_raw: offsets, counts and total (AreaLists::off / cnt); area_search_ordered: list
-                           // pointers (OrderedLists::ptr) — both valid until the next area search; area_best: its results
+                           // pointers (OrderedLists::ptr) — both valid until the next area search
     kHostAreaEnt,          // area_search_raw / _ordered: the entries (AreaLists::raw, OrderedLists::ent), valid until the next
                            // area search
     kHostFrameStaging,     // vsg_frame_create: the frame's arrays on their way to the device

@@ -205,25 +205,10 @@ protected:
         std::vector<float> scale;
         vsg_frame_view view;
     };
+    // mvKeysUn, its descriptor rows and mvuRight (if any)
     template <class FrameT>
     static void Flatten(const FrameT &F, Flat &out) {
-        static_assert(sizeof(cv::KeyPoint) == sizeof(vsg_keypoint), "cv::KeyPoint layout");
-        const int n = (int)F.mvKeysUn.size();
-        out.keys.resize(n);
-        if (n) std::memcpy(out.keys.data(), F.mvKeysUn.data(), (size_t)n * sizeof(vsg_keypoint));
-        out.desc.resize((size_t)n * 32);
-        for (int i = 0; i < n; ++i) std::memcpy(&out.desc[(size_t)i * 32], F.mDescriptors.ptr(i), 32);
-        out.scale.assign(F.mvScaleFactors.begin(), F.mvScaleFactors.end());
-        vsg_frame_view &v = out.view;
-        v.n = n;
-        v.keys = out.keys.data();
-        v.descriptors = out.desc.data();
-        v.u_right = F.mvuRight.empty() ? nullptr : F.mvuRight.data();
-        v.min_x = F.mnMinX; v.min_y = F.mnMinY; v.max_x = F.mnMaxX; v.max_y = F.mnMaxY;
-        v.grid_inv_w = F.mfGridElementWidthInv; v.grid_inv_h = F.mfGridElementHeightInv;
-        v.grid_cols = FRAME_GRID_COLS; v.grid_rows = FRAME_GRID_ROWS;
-        v.scale_factors = out.scale.data();
-        v.n_levels = (int)out.scale.size();
+        FlattenKeys(F, F.mvKeysUn, nullptr, 0, F.mvuRight.empty() ? nullptr : F.mvuRight.data(), out);
     }
     struct CacheEntry;
     struct FrameGuard {   // RAII for an uploaded frame; a frame that lives in the thread's cache is only borrowed (and pinned)
@@ -426,6 +411,11 @@ protected:
     template <class KeyFrameT, class MapPointT, class OnReplace>
     static int FuseReplay(KeyFrameT *pKF, bool bRight, const std::vector<MapPointT *> &vpMapPoints, const int32_t *best,
                           OnReplace onReplace);
+    // Fuse(pKF, vpMapPoints, th, bRight) for each (pKF, bRight) of targets in order, the searches in one device call; returns
+    // the sum of their counts
+    template <class KeyFrameT, class MapPointT>
+    static int FuseTargets(const std::vector<std::pair<KeyFrameT *, bool>> &targets, const std::vector<MapPointT *> &vpMapPoints,
+                           const float th);
     // ---- SearchForTriangulation (ORBmatcher.cc:902-1146) in the parts the one-target and the multi-target forms share ----
     // epipole of KF1 in KF2 and the fundamental matrix of Pinhole::epipolarConstrain (Pinhole.cpp:120-124), built with the
     // reference's own Eigen expressions (f12 is left zero when bCoarse: nothing reads it)
@@ -602,20 +592,9 @@ int ORBmatcher::SearchByProjection(FrameT &CurrentFrame, const FrameT &LastFrame
 
 template <class KeyFrameT, class FrameT, class MapPointT>
 int ORBmatcher::SearchByBoW(KeyFrameT *pKF, FrameT &F, std::vector<MapPointT *> &vpMapPointMatches) {
-    const std::vector<MapPointT *> vpMapPointsKF = pKF->GetMapPointMatches();
-    vpMapPointMatches = std::vector<MapPointT *>(F.N, static_cast<MapPointT *>(nullptr));
-    BowSide kf, fr;
-    // two-camera frames / keyframes: the left camera's keypoints followed by the right camera's, the order of
-    // mDescriptors and of the indices in mFeatVec (:298-322, :341-343, :348-350)
-    FlattenBowSide(*pKF, pKF->mpCamera2 != nullptr, (size_t)-1, &vpMapPointsKF, kf);
-    FlattenBowSide(F, F.Nleft != -1, (size_t)-1, static_cast<const std::vector<MapPointT *> *>(nullptr), fr);
-    std::vector<int32_t> matches(fr.flat.view.n, -1);
-    int nmatches = 0;
-    Check(vsg_search_by_bow_2cam(Workspace(), &kf.flat.view, kf.valid.data(), &fr.flat.view, F.Nleft, kf.side.nnodes, kf.side.nodes,
-                                 kf.side.ptr, kf.side.idx, fr.side.nnodes, fr.side.nodes, fr.side.ptr, fr.side.idx, mfNNratio,
-                                 mbCheckOrientation ? 1 : 0, matches.data(), &nmatches), "vsg_search_by_bow");
-    for (int j = 0; j < fr.flat.view.n; ++j)
-        if (matches[j] >= 0) vpMapPointMatches[j] = vpMapPointsKF[matches[j]];               // :339
+    std::vector<std::vector<MapPointT *>> vvpMatches;
+    const int nmatches = SearchByBoW(std::vector<KeyFrameT *>{pKF}, F, vvpMatches)[0];
+    vpMapPointMatches = std::move(vvpMatches[0]);
     return nmatches;
 }
 
@@ -626,7 +605,9 @@ std::vector<int> ORBmatcher::SearchByBoW(const std::vector<KeyFrameT *> &vpKFs, 
     std::vector<std::vector<MapPointT *>> vpMapPointsKF(T);
     std::vector<BowSide> kfs(T);
     std::vector<const vsg_bow_side *> table(T);
-    for (size_t t = 0; t < T; ++t) {                                                  // each target as the one-target call has it
+    // two-camera frames / keyframes: the left camera's keypoints followed by the right camera's, the order of
+    // mDescriptors and of the indices in mFeatVec (:298-322, :341-343, :348-350)
+    for (size_t t = 0; t < T; ++t) {
         vpMapPointsKF[t] = vpKFs[t]->GetMapPointMatches();
         FlattenBowSide(*vpKFs[t], vpKFs[t]->mpCamera2 != nullptr, (size_t)-1, &vpMapPointsKF[t], kfs[t]);
         table[t] = &kfs[t].side;
@@ -712,37 +693,27 @@ int ORBmatcher::SearchByProjection(FrameT &CurrentFrame, KeyFrameT *pKF, const s
 // ---- SearchByBoW(KF, KF) (ORBmatcher.cc:758-900) ----
 template <class KeyFrameT, class MapPointT>
 int ORBmatcher::SearchByBoW(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<MapPointT *> &vpMatches12) {
-    // two-camera keyframes: only the features with an entry in mvKeysUn take part (`idx >= mvKeysUn.size()` -> continue,
-    // :793-796, :814-817); they are dropped from the flattened FeatureVectors
-    const std::vector<MapPointT *> vpMapPoints1 = pKF1->GetMapPointMatches();
-    const std::vector<MapPointT *> vpMapPoints2 = pKF2->GetMapPointMatches();
-    vpMatches12 = std::vector<MapPointT *>(vpMapPoints1.size(), static_cast<MapPointT *>(nullptr));
-    BowSide k1, k2;
-    FlattenBowSide(*pKF1, false, BowKFLimit(pKF1), &vpMapPoints1, k1);                 // :800-804
-    FlattenBowSide(*pKF2, false, BowKFLimit(pKF2), &vpMapPoints2, k2);                 // :820-826
-    std::vector<int32_t> m12(k1.flat.view.n, -1);
-    int nmatches = 0;
-    Check(vsg_search_by_bow_kf(Workspace(), &k1.flat.view, k1.valid.data(), &k2.flat.view, k2.valid.data(), k1.side.nnodes,
-                               k1.side.nodes, k1.side.ptr, k1.side.idx, k2.side.nnodes, k2.side.nodes, k2.side.ptr, k2.side.idx,
-                               mfNNratio, mbCheckOrientation ? 1 : 0, m12.data(), &nmatches), "vsg_search_by_bow_kf");
-    for (int i = 0; i < k1.flat.view.n; ++i)
-        if (m12[i] >= 0) vpMatches12[i] = vpMapPoints2[m12[i]];                           // :847
+    std::vector<std::vector<MapPointT *>> vvpMatches;
+    const int nmatches = SearchByBoW(pKF1, std::vector<KeyFrameT *>{pKF2}, vvpMatches)[0];
+    vpMatches12 = std::move(vvpMatches[0]);
     return nmatches;
 }
 
 template <class KeyFrameT, class MapPointT>
 std::vector<int> ORBmatcher::SearchByBoW(KeyFrameT *pKF1, const std::vector<KeyFrameT *> &vpKF2s,
                                          std::vector<std::vector<MapPointT *>> &vvpMatches12) {
+    // two-camera keyframes: only the features with an entry in mvKeysUn take part (`idx >= mvKeysUn.size()` -> continue,
+    // :793-796, :814-817); they are dropped from the flattened FeatureVectors
     const size_t T = vpKF2s.size();
     const std::vector<MapPointT *> vpMapPoints1 = pKF1->GetMapPointMatches();
     BowSide k1;
-    FlattenBowSide(*pKF1, false, BowKFLimit(pKF1), &vpMapPoints1, k1);
+    FlattenBowSide(*pKF1, false, BowKFLimit(pKF1), &vpMapPoints1, k1);                 // :800-804
     std::vector<std::vector<MapPointT *>> vpMapPoints2(T);
     std::vector<BowSide> k2s(T);
     std::vector<const vsg_bow_side *> table(T);
-    for (size_t t = 0; t < T; ++t) {                                                  // each target as the one-target call has it
+    for (size_t t = 0; t < T; ++t) {
         vpMapPoints2[t] = vpKF2s[t]->GetMapPointMatches();
-        FlattenBowSide(*vpKF2s[t], false, BowKFLimit(vpKF2s[t]), &vpMapPoints2[t], k2s[t]);
+        FlattenBowSide(*vpKF2s[t], false, BowKFLimit(vpKF2s[t]), &vpMapPoints2[t], k2s[t]);   // :820-826
         table[t] = &k2s[t].side;
     }
     const size_t n = (size_t)k1.flat.view.n;
@@ -830,19 +801,7 @@ int ORBmatcher::FuseReplay(KeyFrameT *pKF, bool bRight, const std::vector<MapPoi
 template <class KeyFrameT, class MapPointT>
 int ORBmatcher::Fuse(KeyFrameT *pKF, const std::vector<MapPointT *> &vpMapPoints, const float th, const bool bRight) {
     if (bRight && pKF->NLeft == -1) throw std::runtime_error("vsg ORBmatcher::Fuse: bRight needs a two-camera keyframe");
-    Flat flatLocal;
-    FrameGuard fr;
-    UploadFuseTarget(pKF, bRight, flatLocal, fr);
-    const int nMPs = (int)vpMapPoints.size();
-    std::vector<vsg_search_point> pts(nMPs);
-    ProjectForFuse(pKF, bRight, vpMapPoints, pts.data());
-    std::vector<uint8_t> desc((size_t)nMPs * 32, 0);
-    for (int i = 0; i < nMPs; ++i)
-        if (pts[i].valid) CopyDescriptor(vpMapPoints[i], desc, (size_t)i);
-    std::vector<int32_t> best(nMPs, -1);
-    Check(vsg_fuse_search(Workspace(), fr.h, nMPs, pts.data(), desc.data(), th, pKF->mvInvLevelSigma2.data(), 0, best.data(),
-                          nullptr), "vsg_fuse_search");
-    return FuseReplay(pKF, bRight, vpMapPoints, best.data(), [](MapPointT *) {});
+    return FuseTargets(std::vector<std::pair<KeyFrameT *, bool>>{{pKF, bRight}}, vpMapPoints, th);
 }
 
 template <class KeyFrameT, class MapPointT>
@@ -852,6 +811,12 @@ int ORBmatcher::Fuse(const std::vector<KeyFrameT *> &vpTargetKFs, const std::vec
         targets.emplace_back(pKF, false);
         if (pKF->NLeft != -1) targets.emplace_back(pKF, true);
     }
+    return FuseTargets(targets, vpMapPoints, th);
+}
+
+template <class KeyFrameT, class MapPointT>
+int ORBmatcher::FuseTargets(const std::vector<std::pair<KeyFrameT *, bool>> &targets, const std::vector<MapPointT *> &vpMapPoints,
+                            const float th) {
     const int T = (int)targets.size(), n = (int)vpMapPoints.size();
     if (T == 0) return 0;
     std::vector<Flat> local(T);
@@ -1124,21 +1089,16 @@ int ORBmatcher::SearchForTriangulation(KeyFrameT *pKF1, KeyFrameT *pKF2, std::ve
     if (TwoCameraKF(pKF1) || TwoCameraKF(pKF2)) return SearchForTriangulationTwoCameras(pKF1, pKF2, vMatchedPairs, bOnlyStereo, bCoarse);
     float f12[9], epf[2];
     TriangulationGeometry(pKF1, pKF2, bCoarse, f12, epf);
-    Flat k1, k2;
-    Flatten(*pKF1, k1);
-    Flatten(*pKF2, k2);
-    std::vector<uint8_t> h1(k1.view.n, 0), h2(k2.view.n, 0);
-    for (int i = 0; i < k1.view.n; ++i) h1[i] = pKF1->GetMapPoint(i) ? 1 : 0;               // :968
-    for (int i = 0; i < k2.view.n; ++i) h2[i] = pKF2->GetMapPoint(i) ? 1 : 0;               // :998
-    std::vector<int32_t> n1, p1, i1, n2, p2, i2;
-    FlattenFeatVec(pKF1->mFeatVec, n1, p1, i1);
-    FlattenFeatVec(pKF2->mFeatVec, n2, p2, i2);
-    std::vector<int32_t> m12(k1.view.n, -1);
+    BowSide k1, k2;
+    FlattenTriangulationSide(*pKF1, k1);
+    FlattenTriangulationSide(*pKF2, k2);
+    const vsg_bow_side &s1 = k1.side, &s2 = k2.side;
+    std::vector<int32_t> m12(s1.view.n, -1);
     int nmatches = 0;
-    Check(vsg_search_for_triangulation(Workspace(), &k1.view, h1.data(), &k2.view, h2.data(), (int)n1.size(), n1.data(),
-                                       p1.data(), i1.data(), (int)n2.size(), n2.data(), p2.data(), i2.data(),
-                                       bOnlyStereo ? 1 : 0, bCoarse ? 1 : 0, f12, epf, pKF2->mvLevelSigma2.data(),
-                                       mbCheckOrientation ? 1 : 0, m12.data(), &nmatches), "vsg_search_for_triangulation");
+    Check(vsg_search_for_triangulation(Workspace(), &s1.view, s1.mp_valid, &s2.view, s2.mp_valid, s1.nnodes, s1.nodes, s1.ptr, s1.idx,
+                                       s2.nnodes, s2.nodes, s2.ptr, s2.idx, bOnlyStereo ? 1 : 0, bCoarse ? 1 : 0, f12, epf,
+                                       pKF2->mvLevelSigma2.data(), mbCheckOrientation ? 1 : 0, m12.data(), &nmatches),
+          "vsg_search_for_triangulation");
     vMatchedPairs.clear();
     vMatchedPairs.reserve(nmatches);
     for (size_t i = 0, iend = m12.size(); i < iend; i++) {                                  // :1136-1143
