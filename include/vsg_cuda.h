@@ -447,6 +447,18 @@ vsg_status vsg_fuse_search_multi(vsg_matcher *m, int ntargets, const vsg_frame *
                                  const float *const *inv_level_sigma2, int n, const vsg_search_point *pts,
                                  const uint8_t *desc, float th, int32_t *best_idx_out);
 
+/* The searches of LoopClosing::SearchAndFuse's loop `for (pKFi, Scw : CorrectedPosesMap) matcher.Fuse(pKFi, Scw, vpMapPoints,
+ * 4, vpReplacePoints)` (LoopClosing.cc:1994-2054; loop correction and map merging) in one call: vsg_fuse_search(m, KFs[t], n,
+ * pts + t * n, desc, th, NULL, 1, best_idx_out + t * n, NULL) for every t < ntargets, with one upload, one kernel launch and
+ * one download whatever ntargets is (none if ntargets or n is 0).  pts and best_idx_out are [ntargets][n] (point i projected
+ * into target t with that target's Scw and camera); desc (n x 32) is shared by all targets.  The same keyframe may appear
+ * more than once.  Argument rules as vsg_fuse_search_multi without the level tables: negative counts, a null target and a
+ * target on another device than the matcher's are rejected with VSG_ERR_INVALID before anything is launched, and
+ * vsg_last_error names the target.  The caller replays the bookkeeping target by target; a map point whose descriptor
+ * changes during that replay (MapPoint::Replace recomputes the survivor's) must be searched again in the later targets. */
+vsg_status vsg_fuse_search_sim3_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *KFs, int n,
+                                      const vsg_search_point *pts, const uint8_t *desc, float th, int32_t *best_idx_out);
+
 /* SearchBySim3(pKF1, pKF2, vpMatches12, S12, th) (ORBmatcher.cc:1448-1665).  pts1[i1] (KF1.n entries): map point
  * i1 of KF1 projected into KF2 (valid = present, not already matched, not bad, depth/image/distance gates);
  * pts2[i2] likewise into KF1.  matches12_out[i1] = i2 where both directions agree, else -1. */

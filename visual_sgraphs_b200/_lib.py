@@ -149,6 +149,8 @@ _SIGNATURES = {
                                   C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
     "vsg_fuse_search_multi": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                         C.c_float, C.c_void_p]),
+    "vsg_fuse_search_sim3_multi": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_float,
+                                             C.c_void_p]),
     "vsg_search_by_sim3": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                      C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.POINTER(C.c_int)]),
     "vsg_search_by_bow_kf": (C.c_int, [C.c_void_p, C.POINTER(FrameView), C.c_void_p, C.POINTER(FrameView), C.c_void_p,

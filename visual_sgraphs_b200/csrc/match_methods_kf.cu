@@ -358,6 +358,9 @@ static vsg_status fuse_search(vsg_matcher *m, const char *who, int ntargets, con
     CK(cudaSetDevice(m->device));
     std::vector<AreaQuery> qs;
     std::vector<int> q_src, q_tgt;
+    qs.reserve((size_t)ntargets * n);      // a loop-closure-sized call stages ~10^6 queries: no regrowth copies
+    q_src.reserve((size_t)ntargets * n);
+    q_tgt.reserve((size_t)ntargets * n);
     for (int t = 0; t < ntargets; ++t) {
         const vsg_search_point *tp = pts + (size_t)t * n;
         const size_t first = qs.size();
@@ -465,6 +468,13 @@ vsg_status vsg_fuse_search_multi(vsg_matcher *m, int ntargets, const vsg_frame *
         return VSG_ERR_INVALID;
     }
     return fuse_search(m, "vsg_fuse_search_multi", ntargets, KFs, inv_level_sigma2, n, pts, desc, th, best_idx_out);
+}
+
+// vsg_fuse_search(..., variant 1, ...) once per target keyframe, all targets in one upload, one launch and one download:
+// the searches of LoopClosing::SearchAndFuse's loop of Fuse(KF, Scw, ...) calls (LoopClosing.cc:1994-2054)
+vsg_status vsg_fuse_search_sim3_multi(vsg_matcher *m, int ntargets, const vsg_frame *const *KFs, int n, const vsg_search_point *pts,
+                                      const uint8_t *desc, float th, int32_t *best_idx_out) {
+    return fuse_search(m, "vsg_fuse_search_sim3_multi", ntargets, KFs, nullptr, n, pts, desc, th, best_idx_out);
 }
 
 // ORBmatcher.cc:1448-1665

@@ -362,6 +362,19 @@ class ORBmatcher:
         check(self._L.vsg_fuse_search_multi(self._h, T, frames, sig_ptrs, n, ptr(pts), ptr(desc), float(th), ptr(best)))
         return best
 
+    def fuse_search_sim3_multi(self, kf_frames, search_points, desc, th=4.0):
+        """FuseSearch with sim3_variant (the search of Fuse(KeyFrame*, Sim3f&, ...)) into every keyframe of kf_frames with
+        one upload, one launch and one download: the searches of LoopClosing::SearchAndFuse. search_points is [ntargets][n]
+        (the points projected into each target with its Scw), desc (n x 32) is shared. Returns best_idx[ntargets][n]."""
+        T = len(kf_frames)
+        desc = np.ascontiguousarray(desc, np.uint8).reshape(-1, 32)
+        n = len(desc)
+        pts = np.ascontiguousarray(search_points, SEARCH_POINT_DTYPE).reshape(T, n)
+        frames = (C.c_void_p * max(T, 1))(*[f._h.value for f in kf_frames])
+        best = np.zeros((T, n), np.int32)
+        check(self._L.vsg_fuse_search_sim3_multi(self._h, T, frames, n, ptr(pts), ptr(desc), float(th), ptr(best)))
+        return best
+
     def SearchBySim3(self, kf1_frame, kf2_frame, pts1, desc1, pts2, desc2, th):
         """ORBmatcher.cc:1448-1665 with both projections done by the caller. Returns (nFound, matches12[N1])."""
         pts1 = np.ascontiguousarray(pts1, SEARCH_POINT_DTYPE)

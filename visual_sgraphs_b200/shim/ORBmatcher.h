@@ -34,6 +34,7 @@
 #include <utility>
 #include <stdexcept>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/vsg_cuda.h"
@@ -128,6 +129,22 @@ public:
     template <class KeyFrameT, class MapPointT>
     int Fuse(KeyFrameT *pKF, Sophus::Sim3f &Scw, const std::vector<MapPointT *> &vpPoints, float th,
              std::vector<MapPointT *> &vpReplacePoint);
+    // LoopClosing::SearchAndFuse's loop `for (k) { Fuse(vpKFs[k], vScw[k], vpPoints, th, vpReplacePoint); <Replace loop> }`
+    // (LoopClosing.cc:1994-2054) in two halves: one device call for every target up front, then, inside the loop,
+    // Fuse(search, k, vpReplacePoint), which returns what Fuse(vpKFs[k], vScw[k], vpPoints, th, vpReplacePoint) returns at
+    // that moment, with the same side effects.  The batch projects and searches every point that is not bad in every target;
+    // a resolve takes GetMapPoints() and replays the bookkeeping in point order.  Between two resolves only the Replace calls
+    // of the loop body may change the searched points: a point that an earlier resolve named as a survivor (vpReplacePoint[i]
+    // set) and whose descriptor has changed since is searched again, in the targets not yet resolved.  Each target is resolved
+    // at most once, on the thread that made the batch call (its frames are pinned in that thread's upload cache); misuse
+    // throws std::runtime_error.
+    template <class KeyFrameT, class MapPointT>
+    struct FuseSim3Search;
+    template <class KeyFrameT, class MapPointT>
+    FuseSim3Search<KeyFrameT, MapPointT> Fuse(const std::vector<KeyFrameT *> &vpKFs, const std::vector<Sophus::Sim3f> &vScw,
+                                              const std::vector<MapPointT *> &vpPoints, float th);
+    template <class KeyFrameT, class MapPointT>
+    int Fuse(FuseSim3Search<KeyFrameT, MapPointT> &search, size_t k, std::vector<MapPointT *> &vpReplacePoint);
 #endif
 
     // Matching to triangulate new MapPoints, epipolar constraint (ORBmatcher.cc:902-1146; pinhole, mpCamera2 == NULL).
@@ -345,20 +362,71 @@ protected:
     // The gates the Sim3 / Fuse projections share between the depth test and GetFeaturesInArea
     // (e.g. ORBmatcher.cc:468-486): scale-invariance range, viewing angle, predicted level.
     template <class MapPointT, class KeyFrameT, class Vec3T>
-    static bool DistanceAndNormalGates(MapPointT *pMP, KeyFrameT *pKF, const Vec3T &p3Dw, const Vec3T &Ow, bool bCheckNormal,
-                                       vsg_search_point &p) {
+    static bool DistanceAndNormalGates(MapPointT *pMP, KeyFrameT *pKF, const Vec3T &p3Dw, const Vec3T &Ow, vsg_search_point &p) {
         const float maxDistance = pMP->GetMaxDistanceInvariance();
         const float minDistance = pMP->GetMinDistanceInvariance();
+        return DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, minDistance, maxDistance, [&] { return pMP->GetNormal(); }, p);
+    }
+    // ... with the distance bounds already read; normal() is called only when the distance gate passes
+    template <class MapPointT, class KeyFrameT, class Vec3T, class NormalF>
+    static bool DistanceAndNormalGates(MapPointT *pMP, KeyFrameT *pKF, const Vec3T &p3Dw, const Vec3T &Ow, float minDistance,
+                                       float maxDistance, NormalF normal, vsg_search_point &p) {
         Vec3T PO = p3Dw - Ow;
         const float dist = PO.norm();
         if (dist < minDistance || dist > maxDistance) return false;
-        if (bCheckNormal) {
-            Vec3T Pn = pMP->GetNormal();
-            if (PO.dot(Pn) < 0.5 * dist) return false;
-        }
+        Vec3T Pn = normal();
+        if (PO.dot(Pn) < 0.5 * dist) return false;
         p.level = pMP->PredictScale(dist, pKF);
         return true;
     }
+    // Stale descriptors in the multi-target Fuse forms.  Each target is searched with the descriptors the map points have
+    // when its Fuse starts, and MapPoint::Replace ends with the survivor's ComputeDistinctiveDescriptors(): a survivor that is
+    // one of the searched points may enter a later target with a new descriptor and pick another keypoint there.  Survived()
+    // notes such a survivor.  Refresh() compares the noted points' descriptors with the rows in desc, copies the changed ones
+    // into desc, and searches them again in the given targets with one call search(targets, ns, pts, desc, best) over
+    // [targets][ns] points, writing the answers into best ([T][n], as pts).
+    template <class MapPointT>
+    struct StaleRows {
+        std::vector<std::pair<MapPointT *, int>> queryOf;                                  // searched map point -> its indices
+        std::vector<int> survivors;
+        StaleRows() = default;
+        StaleRows(const std::vector<MapPointT *> &vp, const std::vector<uint8_t> &searched) {
+            for (size_t i = 0; i < vp.size(); ++i)
+                if (searched[i]) queryOf.emplace_back(vp[i], (int)i);
+            std::sort(queryOf.begin(), queryOf.end());
+        }
+        void Survived(MapPointT *pSurvivor) {
+            auto it = std::lower_bound(queryOf.begin(), queryOf.end(), std::make_pair(pSurvivor, 0));
+            for (; it != queryOf.end() && it->first == pSurvivor; ++it) survivors.push_back(it->second);
+        }
+        template <class Search>
+        void Refresh(const std::vector<MapPointT *> &vp, std::vector<uint8_t> &desc, const std::vector<vsg_search_point> &pts,
+                     std::vector<int32_t> &best, const std::vector<int> &targets, Search search) {
+            if (survivors.empty()) return;
+            std::sort(survivors.begin(), survivors.end());
+            survivors.erase(std::unique(survivors.begin(), survivors.end()), survivors.end());
+            std::vector<int> stale;
+            for (int i : survivors) {
+                const cv::Mat d = vp[i]->GetDescriptor();
+                if (std::memcmp(d.ptr(0), &desc[(size_t)i * 32], 32) == 0) continue;
+                std::memcpy(&desc[(size_t)i * 32], d.ptr(0), 32);
+                stale.push_back(i);
+            }
+            survivors.clear();
+            if (stale.empty() || targets.empty()) return;
+            const size_t n = vp.size(), R = targets.size(), ns = stale.size();
+            std::vector<vsg_search_point> rpts(R * ns);
+            std::vector<uint8_t> rdesc(ns * 32);
+            for (size_t j = 0; j < ns; ++j) {
+                std::memcpy(&rdesc[j * 32], &desc[(size_t)stale[j] * 32], 32);
+                for (size_t r = 0; r < R; ++r) rpts[r * ns + j] = pts[(size_t)targets[r] * n + stale[j]];
+            }
+            std::vector<int32_t> rbest(R * ns);
+            search(targets, (int)ns, rpts.data(), rdesc.data(), rbest.data());
+            for (size_t r = 0; r < R; ++r)
+                for (size_t j = 0; j < ns; ++j) best[(size_t)targets[r] * n + stale[j]] = rbest[r * ns + j];
+        }
+    };
     // Keys (one or two lists back to back) + descriptor rows [row0, row0 + n) of a frame / keyframe as a view.
     template <class FrameT>
     static void FlattenKeys(const FrameT &F, const std::vector<cv::KeyPoint> &keysA, const std::vector<cv::KeyPoint> *keysB,
@@ -416,6 +484,22 @@ protected:
     template <class KeyFrameT, class MapPointT>
     static int FuseTargets(const std::vector<std::pair<KeyFrameT *, bool>> &targets, const std::vector<MapPointT *> &vpMapPoints,
                            const float th);
+#ifdef SOPHUS_SIM3_HPP
+    // ---- Fuse(KF, Scw, ...) in one or several targets.  The device search has the signature of vsg_fuse_search_sim3_multi;
+    // the single-target Fuse passes FuseSim3One, which is vsg_fuse_search(..., variant 1), the entry point that call has
+    // always made, so a program that uses only the single-target form links against any implementation of the C ABI that
+    // predates vsg_fuse_search_sim3_multi.  Defined below the class. ----
+    using FuseSim3Fn = vsg_status (*)(vsg_matcher *, int, const vsg_frame *const *, int, const vsg_search_point *, const uint8_t *,
+                                      float, int32_t *);
+    static vsg_status FuseSim3One(vsg_matcher *m, int ntargets, const vsg_frame *const *KFs, int n, const vsg_search_point *pts,
+                                  const uint8_t *desc, float th, int32_t *best_idx_out) {
+        if (ntargets != 1) throw std::logic_error("vsg ORBmatcher: FuseSim3One searches exactly one target");
+        return vsg_fuse_search(m, KFs[0], n, pts, desc, th, nullptr, 1, best_idx_out, nullptr);
+    }
+    template <class KeyFrameT, class MapPointT>
+    FuseSim3Search<KeyFrameT, MapPointT> FuseSim3Batch(const std::vector<KeyFrameT *> &vpKFs, const std::vector<Sophus::Sim3f> &vScw,
+                                                       const std::vector<MapPointT *> &vpPoints, float th, FuseSim3Fn search);
+#endif
     // ---- SearchForTriangulation (ORBmatcher.cc:902-1146) in the parts the one-target and the multi-target forms share ----
     // epipole of KF1 in KF2 and the fundamental matrix of Pinhole::epipolarConstrain (Pinhole.cpp:120-124), built with the
     // reference's own Eigen expressions (f12 is left zero when bCoarse: nothing reads it)
@@ -765,7 +849,7 @@ void ORBmatcher::ProjectForFuse(KeyFrameT *pKF, bool bRight, const std::vector<M
         const auto uv = pCamera->project(p3Dc);
         if (!pKF->IsInImage(uv(0), uv(1))) continue;
         p.ur = uv(0) - bf * invz;
-        if (!DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, true, p)) continue;
+        if (!DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, p)) continue;
         p.u = uv(0); p.v = uv(1);
         p.valid = 1;
     }
@@ -838,47 +922,23 @@ int ORBmatcher::FuseTargets(const std::vector<std::pair<KeyFrameT *, bool>> &tar
     std::vector<int32_t> best((size_t)T * n, -1);
     Check(vsg_fuse_search_multi(Workspace(), T, frames.data(), sigma.data(), n, pts.data(), desc.data(), th, best.data()),
           "vsg_fuse_search_multi");
-    // Stale descriptors.  The loop searches target t with the descriptors the map points have when Fuse(target t) starts, and
-    // MapPoint::Replace ends with the survivor's ComputeDistinctiveDescriptors(): a survivor that is one of vpMapPoints may
-    // enter the later targets with a new descriptor and pick another keypoint there.  So after each target's replay, every
-    // query that survived a Replace is compared with its uploaded row; the ones that changed are searched again, with the
-    // new rows, in all later targets (one more call), before the next target is replayed.
-    std::vector<std::pair<MapPointT *, int>> queryOf;                                         // map point -> its query indices
-    for (int i = 0; i < n; ++i)
-        if (searched[i]) queryOf.emplace_back(vpMapPoints[i], i);
-    std::sort(queryOf.begin(), queryOf.end());
-    std::vector<int> survivors, stale;
-    auto onReplace = [&](MapPointT *pSurvivor) {
-        auto it = std::lower_bound(queryOf.begin(), queryOf.end(), std::make_pair(pSurvivor, 0));
-        for (; it != queryOf.end() && it->first == pSurvivor; ++it) survivors.push_back(it->second);
+    // after each target's replay, the survivors whose descriptor changed are searched again in all later targets, before the
+    // next target is replayed
+    StaleRows<MapPointT> stale(vpMapPoints, searched);
+    auto research = [&](const std::vector<int> &tg, int ns, const vsg_search_point *rpts, const uint8_t *rdesc, int32_t *rbest) {
+        // tg is t + 1 ... T - 1
+        Check(vsg_fuse_search_multi(Workspace(), (int)tg.size(), frames.data() + tg[0], sigma.data() + tg[0], ns, rpts, rdesc, th,
+                                    rbest), "vsg_fuse_search_multi");
     };
+    std::vector<int> later;
     int nFused = 0;
     for (int t = 0; t < T; ++t) {
-        nFused += FuseReplay(targets[t].first, targets[t].second, vpMapPoints, &best[(size_t)t * n], onReplace);
-        if (t + 1 == T || survivors.empty()) continue;
-        std::sort(survivors.begin(), survivors.end());
-        survivors.erase(std::unique(survivors.begin(), survivors.end()), survivors.end());
-        stale.clear();
-        for (int i : survivors) {
-            const cv::Mat d = vpMapPoints[i]->GetDescriptor();
-            if (std::memcmp(d.ptr(0), &desc[(size_t)i * 32], 32) == 0) continue;
-            std::memcpy(&desc[(size_t)i * 32], d.ptr(0), 32);
-            stale.push_back(i);
-        }
-        survivors.clear();
-        if (stale.empty()) continue;
-        const int R = T - t - 1, ns = (int)stale.size();
-        std::vector<vsg_search_point> rpts((size_t)R * ns);
-        std::vector<uint8_t> rdesc((size_t)ns * 32);
-        for (int j = 0; j < ns; ++j) {
-            std::memcpy(&rdesc[(size_t)j * 32], &desc[(size_t)stale[j] * 32], 32);
-            for (int r = 0; r < R; ++r) rpts[(size_t)r * ns + j] = pts[(size_t)(t + 1 + r) * n + stale[j]];
-        }
-        std::vector<int32_t> rbest((size_t)R * ns);
-        Check(vsg_fuse_search_multi(Workspace(), R, frames.data() + t + 1, sigma.data() + t + 1, ns, rpts.data(), rdesc.data(), th,
-                                    rbest.data()), "vsg_fuse_search_multi");
-        for (int r = 0; r < R; ++r)
-            for (int j = 0; j < ns; ++j) best[(size_t)(t + 1 + r) * n + stale[j]] = rbest[(size_t)r * ns + j];
+        nFused += FuseReplay(targets[t].first, targets[t].second, vpMapPoints, &best[(size_t)t * n],
+                             [&](MapPointT *pSurvivor) { stale.Survived(pSurvivor); });
+        if (t + 1 == T) continue;
+        later.clear();
+        for (int r = t + 1; r < T; ++r) later.push_back(r);
+        stale.Refresh(vpMapPoints, desc, pts, best, later, research);
     }
     return nFused;
 }
@@ -927,7 +987,7 @@ int ORBmatcher::SearchByProjection(KeyFrameT *pKF, Sophus::Sim3<float> &Scw, con
             u = uv(0); v = uv(1);
         }
         if (!pKF->IsInImage(u, v)) continue;
-        if (!DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, true, p)) continue;
+        if (!DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, p)) continue;
         p.u = u; p.v = v;
         p.valid = 1;
         CopyDescriptor(pMP, desc, (size_t)iMP);
@@ -1009,44 +1069,139 @@ int ORBmatcher::SearchBySim3(KeyFrameT *pKF1, KeyFrameT *pKF2, std::vector<MapPo
     return nFound;
 }
 
-// ---- Fuse(KF, Scw, vpPoints, th, vpReplacePoint) (ORBmatcher.cc:1337-1446) ----
+// ---- Fuse(KF, Scw, vpPoints, th, vpReplacePoint) (ORBmatcher.cc:1337-1446): the batch with one target, resolved at once ----
 template <class KeyFrameT, class MapPointT>
 int ORBmatcher::Fuse(KeyFrameT *pKF, Sophus::Sim3f &Scw, const std::vector<MapPointT *> &vpPoints, float th,
                      std::vector<MapPointT *> &vpReplacePoint) {
-    Flat flatLocal;
-    FrameGuard fr;
-    const Flat &flat = Upload(*pKF, pKF->NLeft != -1 ? 1 : 0, [&](Flat &o) { FlattenSearched(*pKF, pKF->NLeft, o); }, flatLocal, fr);
-    Sophus::SE3f Tcw = Sophus::SE3f(Scw.rotationMatrix(), Scw.translation() / Scw.scale());
-    const auto Ow = Tcw.inverse().translation();
-    const std::set<MapPointT *> spAlreadyFound = pKF->GetMapPoints();
-    const int nPoints = (int)vpPoints.size();
-    std::vector<vsg_search_point> pts(nPoints);
-    std::vector<uint8_t> desc((size_t)nPoints * 32, 0);
-    for (int iMP = 0; iMP < nPoints; ++iMP) {
-        vsg_search_point &p = pts[iMP];
-        std::memset(&p, 0, sizeof(p));
-        MapPointT *pMP = vpPoints[iMP];
-        if (spAlreadyFound.count(pMP)) continue;            // isBad() is re-checked in order below
-        const auto p3Dw = pMP->GetWorldPos();
-        const auto p3Dc = Tcw * p3Dw;
-        if (p3Dc(2) < 0.0f) continue;
-        const auto uv = pKF->mpCamera->project(p3Dc);
-        if (!pKF->IsInImage(uv(0), uv(1))) continue;
-        if (!DistanceAndNormalGates(pMP, pKF, p3Dw, Ow, true, p)) continue;
-        p.u = uv(0); p.v = uv(1);
-        p.valid = 1;
-        CopyDescriptor(pMP, desc, (size_t)iMP);
+    FuseSim3Search<KeyFrameT, MapPointT> search =
+        FuseSim3Batch(std::vector<KeyFrameT *>{pKF}, std::vector<Sophus::Sim3f>{Scw}, vpPoints, th, &FuseSim3One);
+    return Fuse(search, 0, vpReplacePoint);
+}
+
+template <class KeyFrameT, class MapPointT>
+struct ORBmatcher::FuseSim3Search {
+    std::vector<KeyFrameT *> vpKFs;
+    std::vector<MapPointT *> vpPoints;
+    float th = 0;
+    FuseSim3Fn search = nullptr;                                                              // the device search
+    std::thread::id thread;
+    // the uploaded targets (held for the re-searches), the points projected into them ([T][n]), the descriptor rows the
+    // current answers were searched with, the answers ([T][n], -1: none) and which targets are resolved
+    std::vector<FrameGuard> fr;
+    std::vector<const vsg_frame *> frames;
+    std::vector<vsg_search_point> pts;
+    std::vector<uint8_t> desc;
+    std::vector<int32_t> best;
+    std::vector<uint8_t> resolved;
+    StaleRows<MapPointT> stale;
+    FuseSim3Search() = default;
+    FuseSim3Search(FuseSim3Search &&) = default;
+    FuseSim3Search(const FuseSim3Search &) = delete;
+    FuseSim3Search &operator=(const FuseSim3Search &) = delete;
+};
+
+template <class KeyFrameT, class MapPointT>
+ORBmatcher::FuseSim3Search<KeyFrameT, MapPointT> ORBmatcher::Fuse(const std::vector<KeyFrameT *> &vpKFs,
+                                                                  const std::vector<Sophus::Sim3f> &vScw,
+                                                                  const std::vector<MapPointT *> &vpPoints, float th) {
+    return FuseSim3Batch(vpKFs, vScw, vpPoints, th, &vsg_fuse_search_sim3_multi);
+}
+
+template <class KeyFrameT, class MapPointT>
+ORBmatcher::FuseSim3Search<KeyFrameT, MapPointT> ORBmatcher::FuseSim3Batch(const std::vector<KeyFrameT *> &vpKFs,
+                                                                           const std::vector<Sophus::Sim3f> &vScw,
+                                                                           const std::vector<MapPointT *> &vpPoints, float th,
+                                                                           FuseSim3Fn search) {
+    if (vScw.size() != vpKFs.size())
+        throw std::runtime_error("vsg ORBmatcher::Fuse: " + std::to_string(vpKFs.size()) + " keyframes but " +
+                                 std::to_string(vScw.size()) + " Sim3 poses");
+    const int T = (int)vpKFs.size(), n = (int)vpPoints.size();
+    FuseSim3Search<KeyFrameT, MapPointT> s;
+    s.vpKFs = vpKFs;
+    s.vpPoints = vpPoints;
+    s.th = th;
+    s.search = search;
+    s.thread = std::this_thread::get_id();
+    s.fr = std::vector<FrameGuard>(T);
+    s.frames.resize(T);
+    s.pts.assign((size_t)T * n, vsg_search_point());
+    s.desc.assign((size_t)n * 32, 0);
+    s.best.assign((size_t)T * n, -1);
+    s.resolved.assign(T, 0);
+    // What the projection reads of a point, once for all targets: Replace does not change it (no UpdateNormalAndDepth).  A
+    // point bad now stays bad; isBad() and spAlreadyFound are evaluated by the resolve, at the top of the iteration.
+    using Vec3T = typename std::decay<decltype(vpPoints[0]->GetWorldPos())>::type;
+    struct Geometry { Vec3T p3Dw, Pn; float maxDistance, minDistance; };
+    std::vector<Geometry> geo(n);
+    std::vector<uint8_t> good(n, 0), searched(n, 0);
+    for (int i = 0; i < n; ++i) {
+        MapPointT *pMP = vpPoints[i];
+        if (!pMP || pMP->isBad()) continue;
+        good[i] = 1;
+        geo[i] = Geometry{pMP->GetWorldPos(), pMP->GetNormal(), pMP->GetMaxDistanceInvariance(), pMP->GetMinDistanceInvariance()};
     }
-    std::vector<int32_t> best(nPoints, -1);
-    Check(vsg_fuse_search(Workspace(), fr.h, nPoints, pts.data(), desc.data(), th, nullptr, 1, best.data(), nullptr),
-          "vsg_fuse_search");
+    Flat flatLocal;
+    for (int t = 0; t < T; ++t) {
+        KeyFrameT *pKF = vpKFs[t];
+        Upload(*pKF, pKF->NLeft != -1 ? 1 : 0, [&](Flat &o) { FlattenSearched(*pKF, pKF->NLeft, o); }, flatLocal, s.fr[t]);
+        s.frames[t] = s.fr[t].h;
+        const Sophus::Sim3f &Scw = vScw[t];
+        Sophus::SE3f Tcw = Sophus::SE3f(Scw.rotationMatrix(), Scw.translation() / Scw.scale());
+        const auto Ow = Tcw.inverse().translation();
+        vsg_search_point *pts = &s.pts[(size_t)t * n];
+        for (int i = 0; i < n; ++i) {
+            if (!good[i]) continue;
+            const Geometry &g = geo[i];
+            vsg_search_point &p = pts[i];
+            const auto p3Dc = Tcw * g.p3Dw;
+            if (p3Dc(2) < 0.0f) continue;
+            const auto uv = pKF->mpCamera->project(p3Dc);
+            if (!pKF->IsInImage(uv(0), uv(1))) continue;
+            if (!DistanceAndNormalGates(vpPoints[i], pKF, g.p3Dw, Ow, g.minDistance, g.maxDistance, [&] { return g.Pn; }, p)) continue;
+            p.u = uv(0); p.v = uv(1);
+            p.valid = 1;
+            searched[i] = 1;
+        }
+    }
+    for (int i = 0; i < n; ++i)
+        if (searched[i]) CopyDescriptor(vpPoints[i], s.desc, (size_t)i);
+    s.stale = StaleRows<MapPointT>(vpPoints, searched);
+    Check(search(Workspace(), T, s.frames.data(), n, s.pts.data(), s.desc.data(), th, s.best.data()), "vsg_fuse_search_sim3_multi");
+    return s;
+}
+
+template <class KeyFrameT, class MapPointT>
+int ORBmatcher::Fuse(FuseSim3Search<KeyFrameT, MapPointT> &s, size_t k, std::vector<MapPointT *> &vpReplacePoint) {
+    const size_t T = s.vpKFs.size();
+    if (k >= T) throw std::runtime_error("vsg ORBmatcher::Fuse: target " + std::to_string(k) + " of a search over " + std::to_string(T));
+    if (s.resolved[k]) throw std::runtime_error("vsg ORBmatcher::Fuse: target " + std::to_string(k) + " resolved twice");
+    if (std::this_thread::get_id() != s.thread)
+        throw std::runtime_error("vsg ORBmatcher::Fuse: a resolve on another thread than the batch call's");
+    // the survivors of the Replace calls since the last resolve: changed descriptors are searched again where still needed
+    std::vector<int> open;
+    for (size_t t = 0; t < T; ++t)
+        if (!s.resolved[t]) open.push_back((int)t);
+    s.stale.Refresh(s.vpPoints, s.desc, s.pts, s.best, open,
+                    [&](const std::vector<int> &tg, int ns, const vsg_search_point *rpts, const uint8_t *rdesc, int32_t *rbest) {
+        std::vector<const vsg_frame *> frames;
+        for (int t : tg) frames.push_back(s.frames[t]);
+        Check(s.search(Workspace(), (int)tg.size(), frames.data(), ns, rpts, rdesc, s.th, rbest), "vsg_fuse_search_sim3_multi");
+    });
+    s.resolved[k] = 1;
+    KeyFrameT *pKF = s.vpKFs[k];
+    const std::set<MapPointT *> spAlreadyFound = pKF->GetMapPoints();
+    const size_t n = s.vpPoints.size();
+    const int32_t *best = &s.best[k * n];
     int nFused = 0;
-    for (int iMP = 0; iMP < nPoints; ++iMP) {                                               // :1353-1442 in order
-        MapPointT *pMP = vpPoints[iMP];
-        if (pMP->isBad() || best[iMP] < 0) continue;
+    for (size_t iMP = 0; iMP < n; ++iMP) {                                                    // :1353-1442 in order
+        MapPointT *pMP = s.vpPoints[iMP];
+        if (!pMP || pMP->isBad() || spAlreadyFound.count(pMP) || best[iMP] < 0) continue;
         MapPointT *pMPinKF = pKF->GetMapPoint(best[iMP]);
         if (pMPinKF) {
-            if (!pMPinKF->isBad()) vpReplacePoint[iMP] = pMPinKF;
+            if (!pMPinKF->isBad()) {
+                vpReplacePoint[iMP] = pMPinKF;
+                s.stale.Survived(pMP);                                                        // the caller's pMPinKF->Replace(pMP)
+            }
         } else {
             pMP->AddObservation(pKF, best[iMP]);
             pKF->AddMapPoint(pMP, best[iMP]);
