@@ -88,9 +88,9 @@ namespace vsg {
 enum DevSlot : int {
     kSlotKnnParts = 0,     // knn2_device (match.cu): per-chunk top-2 partials
     kSlotArg1,             // one-shot inputs: query descriptors (vsg_descriptor_distance, vsg_knn2, vsg_match_window), left
-                           // keypoints (stereo.cu), descriptors (mappoint.cu, bow.cu)
+                           // keypoints (stereo.cu), descriptors (bow.cu), descriptors, list offsets and long points (mappoint.cu)
     kSlotArg2,             // train descriptors (match.cu), left descriptors (stereo.cu)
-    kSlotArg3,             // distances / indices (match.cu), right keypoints (stereo.cu), list offsets (mappoint.cu)
+    kSlotArg3,             // distances / indices (match.cu), right keypoints (stereo.cu)
     kSlotArg4,             // distances / candidates (match.cu), right descriptors (stereo.cu)
     kSlotArg5,             // vsg_match_window: train levels and skip flags
     kSlotOut,              // one-shot results (vsg_match_window, stereo.cu, mappoint.cu, bow.cu), undistort input (frame_ops.cu);
@@ -125,6 +125,7 @@ enum HostSlot : int {
     kHostMapShardToken,    // vsg_search_by_projection_map_sharded: claim token and per-rank records
     kHostBestMultiIn,      // area_best_multi: targets, queries and descriptors
     kHostBow,              // bow_dists: inputs, then the distances (valid until the next BoW call); triangulation_candidates
+    kHostDistinctive,      // vsg_distinctive_descriptors (mappoint.cu): inputs, then the results
     kNumHostSlots
 };
 

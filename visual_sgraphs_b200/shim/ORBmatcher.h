@@ -167,6 +167,15 @@ public:
     template <class KeyFrameT>
     int SearchForTriangulation(TriangulationSearch<KeyFrameT> &search, size_t i, std::vector<std::pair<size_t, size_t>> &vMatchedPairs);
 
+    // LocalMapping's loops of MapPoint::ComputeDistinctiveDescriptors() (MapPoint.cc:340-417) over a keyframe's map points
+    // (ProcessNewKeyFrame, the update loop of SearchInNeighbors) in one device call.  Each non-NULL point that is not bad
+    // gets what its own ComputeDistinctiveDescriptors() would give: the rows of its observations in map order (left index,
+    // then right index, of each keyframe that is not bad), the row with the smallest median distance to the others, first
+    // one on ties, written back through MapPoint::SetDistinctiveDescriptor (INTEGRATION.md).  A point without rows is left
+    // alone.  The result depends only on the points' observations and the keyframes' descriptors.
+    template <class MapPointT>
+    static void ComputeDistinctiveDescriptors(const std::vector<MapPointT *> &vpMPs);
+
 public:
     static const int TH_LOW = 50;
     static const int TH_HIGH = 100;
@@ -1481,6 +1490,36 @@ int ORBmatcher::SearchForTriangulationTwoCameras(KeyFrameT *pKF1, KeyFrameT *pKF
     }
     (void)n2;
     return nmatches;
+}
+
+template <class MapPointT>
+void ORBmatcher::ComputeDistinctiveDescriptors(const std::vector<MapPointT *> &vpMPs) {
+    std::vector<MapPointT *> points;                // the points with rows, in vpMPs' order
+    std::vector<int32_t> ptr(1, 0);
+    std::vector<uint8_t> desc;
+    for (MapPointT *pMP : vpMPs) {
+        if (!pMP || pMP->isBad()) continue;
+        const auto observations = pMP->GetObservations();
+        const size_t before = desc.size();
+        for (auto mit = observations.begin(), mend = observations.end(); mit != mend; ++mit) {
+            auto *pKF = mit->first;
+            if (pKF->isBad()) continue;
+            for (const int idx : {std::get<0>(mit->second), std::get<1>(mit->second)}) {
+                if (idx == -1) continue;
+                const uint8_t *row = pKF->mDescriptors.ptr(idx);
+                desc.insert(desc.end(), row, row + 32);
+            }
+        }
+        if (desc.size() == before) continue;        // the reference returns without touching mDescriptor (:379)
+        points.push_back(pMP);
+        ptr.push_back((int32_t)(desc.size() / 32));
+    }
+    if (points.empty()) return;
+    std::vector<int32_t> best(points.size());
+    Check(vsg_distinctive_descriptors(Workspace(), desc.data(), ptr.data(), (int)points.size(), best.data()),
+          "vsg_distinctive_descriptors");
+    for (size_t k = 0; k < points.size(); ++k)     // mDescriptor = vDescriptors[BestIdx].clone() under mMutexFeatures
+        points[k]->SetDistinctiveDescriptor(cv::Mat(1, 32, CV_8U, desc.data() + 32 * ((size_t)ptr[k] + best[k]), 32));
 }
 
 }  // namespace VS_GRAPHS
